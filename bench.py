@@ -14,6 +14,8 @@ device, advance every env one frame (tbx_step), render every env (tbx_render).  
                                             NCCL all-reduce of the episode statistics every 256 steps (inside the timed region)
     python bench.py --wrapped [--game G]    supplementary: the fused DeepMind wrapper stack (agent steps/s; 1 agent step = 4 frames)
     python bench.py --policy track --presteps 3000    supplementary: mid-game Breakout states (scripted ball-tracking policy)
+    python bench.py --dump-outputs DIR      also write what the last timed step returned (a seeded sample) as DIR/*.npy, so that
+                                            two builds can be compared output for output on the same seeded inputs
 
 The pool is in steady state when the clock starts (--presteps 2000 untimed step-only frames, default); the line also carries the survey's
 protocol (warm-up 100, 5 x 1,000 steps: best, mean, SEM), fresh-game / mid-game sub-records, the e2e leg with its own PCIe roofline
@@ -29,6 +31,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as build() left it (it may be read-only)
 
 GAME_DTYPE = {"breakout": "f64+u8", "amidar": "i32+u8", "space_invaders": "i32+u8"}
 ACTION_SEED = 0xB200
@@ -59,7 +62,13 @@ def parse():
                          "gray84, NCCL all-reduce of the episode statistics every 256 steps")
     ap.add_argument("--wrapped", action="store_true",
                     help="supplementary line: the fused DeepMind wrapper stack (frame skip 4, max of 2 frames, 84x84, FrameStack 4)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last of the --steps timed steps returned (observations, reward, done, score, lives of a fixed "
+                         "seeded sample of rank 0's envs, and the episode statistics) as DIR/<name>.npy, float32 / float64, <= 64 MB")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.mixed or args.wrapped or args.interventions):
+        ap.error("--dump-outputs applies to the headline measurement only")
+    return args
 
 
 def obs_bytes(game, obs):
@@ -69,6 +78,33 @@ def obs_bytes(game, obs):
 
 def workload_name(game, envs, obs):
     return "%s batched %d envs/GPU, %s obs, uniform random legal actions, auto-reset" % (game, envs, obs)
+
+
+DUMP_BYTES = 48 << 20       # the dumped sample stays under 64 MB whatever --envs / --obs ask for
+
+
+def sample_outputs(ro, stats_dev, env0):
+    """Host copies of what the pool's last step returned, for a fixed seeded sample of its envs: the observations as float32,
+    the per-env scalars and the episode statistics as float64 (every value is an integer, so both are exact)."""
+    import numpy as np
+    import torch
+    n, fb = ro.n, ro.obs[0].numel()
+    k = min(n, DUMP_BYTES // (4 * fb + 8 * 4))
+    ids = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    idx = torch.from_numpy(ids).to(ro.obs.device)
+    out = {"env_ids": (env0 + ids).astype(np.float64),
+           "obs": ro.obs.index_select(0, idx).float().cpu().numpy(),
+           "episode_stats": stats_dev.double().cpu().numpy()}
+    for name in ("reward", "done", "score", "lives"):
+        out[name] = getattr(ro.pool, name).index_select(0, idx).double().cpu().numpy()
+    return out
+
+
+def dump_outputs(outputs, path):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # --------------------------------------------------------------------------------------------- CPU arm
@@ -585,6 +621,8 @@ def main():
     pool.check()
     value = world * n * K / (ms * 1e-3)
     stats = [int(v) for v in stats_dev.cpu()]
+    # copied now: the protocol repeats and the e2e leg below advance the same pool
+    outputs = sample_outputs(ro, stats_dev, ro.env0) if args.dump_outputs and rank == 0 else None
 
     # ---- the survey's protocol (SURVEY 8d, after test/benchmark.py:119-166): warm-up 100, T = 1,000 timed steps, best of 5 and
     # mean +- SEM over the 5 repeats -- measured in the same run, after the driver's K-step region above
@@ -811,6 +849,8 @@ def main():
         "clocks": clocks, "episode_stats": {"episodes": stats[0], "sum_return": stats[1], "sum_length": stats[2], "max_return": stats[3],
                                             "scope": "all ranks (NCCL-reduced), since pool creation"},
     }
+    if outputs is not None:
+        dump_outputs(outputs, args.dump_outputs)
     print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()

@@ -69,6 +69,22 @@ def main():
         out[name + "_dst_blocky"] = cv2.resize(blocky, (84, 84), interpolation=cv2.INTER_AREA)
         out[name + "_dst_noise_100x60"] = cv2.resize(img, (100, 60), interpolation=cv2.INTER_AREA)
     np.savez_compressed(os.path.join(HERE, "area_golden.npz"), **out)
+    area_cv2_seed5()
+
+
+def area_cv2_seed5():
+    """area_cv2_seed5.json: SHA-256 of the noise frames of tests/test_oracle_golden.py::test_area_resize_equals_live_cv2
+    (default_rng(5), 5 per game) and of their cv2 INTER_AREA 84x84 outputs."""
+    import hashlib
+    import cv2
+    rng = np.random.default_rng(5)
+    out = {"cv2_version": cv2.__version__, "src_sha256": [], "dst_sha256": []}
+    for (w, h) in ((240, 160), (160, 250), (320, 210)):
+        for _ in range(5):
+            src = rng.integers(0, 256, size=(h, w), dtype=np.uint8)
+            out["src_sha256"].append(hashlib.sha256(src.tobytes()).hexdigest())
+            out["dst_sha256"].append(hashlib.sha256(cv2.resize(src, (84, 84), interpolation=cv2.INTER_AREA).tobytes()).hexdigest())
+    json.dump(out, open(os.path.join(HERE, "area_cv2_seed5.json"), "w"), indent=1)
 
 
 if __name__ == "__main__":

@@ -3,8 +3,8 @@ module backed by
   (a) the host build of the product's engines + JSON codec (tests/emu)            -- CPU tier
   (b) the oracle                                                                    -- CPU tier
   (c) the CUDA library itself, through toybox_b200.ctoybox.Toybox (batch of 1)      -- GPU tier
-The reference's Python comes from /root/reference where that exists (this container) and otherwise from the byte-identical
-snapshot tests/golden/reference_py/ (made by tests/golden/make_golden.py), so that (c) runs on the GPU box."""
+The reference's Python is the byte-identical snapshot tests/golden/reference_py/ (made by tests/golden/make_golden.py), so
+that every tier runs the same files on any machine."""
 import os
 import sys
 import types
@@ -13,7 +13,7 @@ import unittest
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference" if os.path.isdir("/root/reference/test/interventions") else os.path.join(HERE, "golden", "reference_py")
+REF = os.path.join(HERE, "golden", "reference_py")
 
 
 def install_ctoybox(toybox_cls, input_cls):
