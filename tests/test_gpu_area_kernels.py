@@ -1,6 +1,7 @@
-"""GPU tier: every code path of the INTER_AREA (WarpFrame) render -- the warp-per-env tile kernel with its list,
-sweep and per-tile rebuild paths, and the CTA-canvas kernel -- against the oracle's cv2-exact resize, on mid-game
-states of all three games and on several output sizes."""
+"""GPU tier: every code path of the INTER_AREA (WarpFrame) render -- the direct kernels and the warp-per-env tile
+kernel with its list, sweep and per-tile rebuild paths, at up to 5 x 4 and at 8 x 8 taps -- against the oracle's
+cv2-exact resize, on mid-game states of all three games and on several output sizes; and the native layouts'
+broadcast + patch render with its dense-env hand-over to the canvas kernel."""
 import os
 
 import numpy as np
@@ -9,10 +10,11 @@ import pytest
 pytestmark = pytest.mark.gpu
 GAMES = ["breakout", "amidar", "space_invaders"]
 TILE = {"TBX_AREA_KERNEL": "tile"}        # Breakout: without the direct kernel (tbx_render_direct.cuh) in front of the tile kernel
-VARIANTS = [{}, TILE, dict(TILE, TBX_AREA_DIGIT_CACHE="0"), dict(TILE, TBX_AREA_LCAP="24"), dict(TILE, TBX_AREA_LCAP="3"), {"TBX_AREA_KERNEL": "cta"},
-            dict(TILE, TBX_AREA_THREADS="128"), dict(TILE, TBX_AREA_TILE_H="4", TBX_AREA_MAX_RUN="8"), dict(TILE, TBX_AREA_TILE_H="16"),
-            dict(TILE, TBX_AREA_MAX_RUN="1", TBX_AREA_LCAP="40"), {"TBX_AREA_LCAP": "3"}]
+VARIANTS = [{}, TILE, dict(TILE, TBX_AREA_DIGIT_CACHE="0"), dict(TILE, TBX_AREA_LCAP="24"), dict(TILE, TBX_AREA_LCAP="3"),
+            dict(TILE, TBX_AREA_LCAP="40"), {"TBX_AREA_LCAP": "3"}]
 SIZES = [(84, 84), (96, 80), (64, 64), (48, 60), (100, 37)]
+# per game: the accepted size with the largest tile-kernel scratch window (8 x 8 taps); each is refused for another game
+WORST_SIZE = {"breakout": (32, 20), "space_invaders": (40, 28), "amidar": (23, 35)}
 
 
 def _advance(tbx, oracle_mod, game, n, steps, seed):
@@ -36,7 +38,7 @@ def _advance(tbx, oracle_mod, game, n, steps, seed):
 
 
 def _set_env(v):
-    for k in ("TBX_AREA_LCAP", "TBX_AREA_KERNEL", "TBX_AREA_THREADS", "TBX_AREA_TILE_H", "TBX_AREA_MAX_RUN", "TBX_AREA_DIGIT_CACHE"):
+    for k in ("TBX_AREA_LCAP", "TBX_AREA_KERNEL", "TBX_AREA_DIGIT_CACHE"):
         os.environ.pop(k, None)
     os.environ.update(v)
 
@@ -46,7 +48,7 @@ def test_area_render_paths_bit_exact(tbx, oracle_mod, game):
     n = 45                                   # ragged: the last chunk holds 5 envs
     pool, ref = _advance(tbx, oracle_mod, game, n, 1200 if game == "breakout" else 400, 77)
     try:
-        for ow, oh in SIZES:
+        for ow, oh in SIZES + [WORST_SIZE[game]]:
             want = ref.render("gray84", ow, oh).reshape(n, -1)
             for v in VARIANTS:
                 _set_env(v)
@@ -60,24 +62,21 @@ def test_area_render_paths_bit_exact(tbx, oracle_mod, game):
 
 @pytest.mark.parametrize("game", GAMES)
 def test_native_render_paths_bit_exact(tbx, oracle_mod, game):
-    """native layouts: broadcast + patch with its dense-env hand-over to the canvas kernel (never / always / mixed), and the
-    canvas kernel alone"""
+    """native layouts: broadcast + patch with its dense-env hand-over to the canvas kernel (never / always / mixed; Breakout and
+    Amidar -- Space Invaders is always patched)"""
     n = 45
     pool, ref = _advance(tbx, oracle_mod, game, n, 1200 if game == "breakout" else 400, 78)
-    keys = ("TBX_NATIVE_KERNEL", "TBX_NATIVE_DENSE")
     try:
         for mode in ("rgb", "rgba", "gray"):
             want = ref.render(mode).reshape(n, -1)
-            for v in ({}, {"TBX_NATIVE_DENSE": "-1"}, {"TBX_NATIVE_DENSE": "0"}, {"TBX_NATIVE_DENSE": "3"}, {"TBX_NATIVE_KERNEL": "canvas"}):
-                for k in keys:
-                    os.environ.pop(k, None)
+            for v in ({}, {"TBX_NATIVE_DENSE": "-1"}, {"TBX_NATIVE_DENSE": "0"}, {"TBX_NATIVE_DENSE": "3"}):
+                os.environ.pop("TBX_NATIVE_DENSE", None)
                 os.environ.update(v)
                 got = pool.render(obs=mode).cpu().numpy().reshape(n, -1)
                 bad = np.argwhere(got != want)
                 assert bad.size == 0, (game, mode, v, bad[:5], got[tuple(bad[0])], want[tuple(bad[0])])
     finally:
-        for k in keys:
-            os.environ.pop(k, None)
+        os.environ.pop("TBX_NATIVE_DENSE", None)
         pool.close()
 
 
@@ -230,21 +229,16 @@ def test_si_direct_kernel_adversarial_states(tbx, oracle_mod):
                     got = pool.render(obs=("gray_area", ow, oh)).cpu().numpy().reshape(n, -1)
                     bad = np.argwhere(got != want)
                     assert bad.size == 0, (rnd, ow, oh, v, bad[:5], got[tuple(bad[0])], want[tuple(bad[0])])
-            for mode in ("rgb", "gray", "rgba"):              # native layouts: broadcast + patch / canvas kernel
+            for mode in ("rgb", "gray", "rgba"):              # native layouts: broadcast + patch
                 want = ref.render(mode).reshape(n, -1)
-                for v in ({}, {"TBX_NATIVE_KERNEL": "canvas"}):
-                    for k in ("TBX_NATIVE_KERNEL",):
-                        os.environ.pop(k, None)
-                    os.environ.update(v)
-                    got = pool.render(obs=mode).cpu().numpy().reshape(n, -1)
-                    bad = np.argwhere(got != want)
-                    assert bad.size == 0, (rnd, mode, v, bad[:5], got[tuple(bad[0])], want[tuple(bad[0])])
+                got = pool.render(obs=mode).cpu().numpy().reshape(n, -1)
+                bad = np.argwhere(got != want)
+                assert bad.size == 0, (rnd, mode, bad[:5], got[tuple(bad[0])], want[tuple(bad[0])])
             for t in range(30):
                 acts = legal[[oracle_mod.action_index(0xB200, i, 500 + t, len(legal)) for i in range(n)]]
                 pool.apply_ale_action(acts, auto_reset=True)
                 ref.step(acts, auto_reset=True)
     finally:
-        os.environ.pop("TBX_NATIVE_KERNEL", None)
         _set_env({})
         pool.close()
 
@@ -282,12 +276,11 @@ def test_amidar_painted_corridors_every_layout(tbx, oracle_mod):
         ref.write_state_json(i, js)
         states.append(js)
     pool.write_state_json(states)
-    keys = ("TBX_NATIVE_KERNEL", "TBX_NATIVE_DENSE", "TBX_AREA_LCAP", "TBX_AREA_KERNEL")
+    keys = ("TBX_NATIVE_DENSE", "TBX_AREA_LCAP", "TBX_AREA_KERNEL")
     try:
         for mode, omode in (("gray84", "gray84"), ("rgb", "rgb"), ("gray", "gray"), ("rgba", "rgba")):
             want = ref.render(omode).reshape(n, -1)
-            for v in ({}, TILE, {"TBX_NATIVE_KERNEL": "canvas"}, {"TBX_NATIVE_DENSE": "-1"}, {"TBX_NATIVE_DENSE": "4"}, dict(TILE, TBX_AREA_LCAP="16"),
-                      {"TBX_AREA_KERNEL": "cta"}):
+            for v in ({}, TILE, {"TBX_NATIVE_DENSE": "0"}, {"TBX_NATIVE_DENSE": "-1"}, {"TBX_NATIVE_DENSE": "4"}, dict(TILE, TBX_AREA_LCAP="16")):
                 for k in keys:
                     os.environ.pop(k, None)
                 os.environ.update(v)

@@ -38,7 +38,7 @@ def build(force=False, verbose=False):
     """Compile toybox_b200/libtoybox_b200.so for sm_100a (cross-compiles without a GPU): one object per translation unit
     under toybox_b200/build/, rebuilt only when the unit or a header it includes changed, compiled in parallel."""
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    extra = os.environ.get("TBX_NVCC_EXTRA", "").split()          # tuning experiments, e.g. -DTBX_RENDER_THREADS=128
+    extra = os.environ.get("TBX_NVCC_EXTRA", "").split()          # tuning experiments, e.g. -DTBX_AREA_MIN_CTAS=2
     os.makedirs(_OBJ, exist_ok=True)
     jobs, objs = [], []
     for src in SOURCES:

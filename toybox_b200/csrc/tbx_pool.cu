@@ -359,17 +359,15 @@ static int ensure_area(tbx_pool *p, int out_w, int out_h, AreaRes **out) {
 
 static int align16(int v) { return (v + 15) & ~15; }
 
-template <int GAME, int MODE, int TX, int TY> static int launch_render(const RenderArgs &a, const void *cfg_host, const TbxAreaPlan *plan_host, int smem, cudaStream_t s) {
+/* the canvas kernel (tbx_render.cuh): the dense Breakout / Amidar envs the patch kernel lists */
+template <int GAME, int MODE> static int launch_render(const RenderArgs &a, const void *cfg_host, int smem, cudaStream_t s) {
   /* the opt-in is per device (a process may hold pools on several GPUs): set it on every launch, a cheap host-side call */
-  CK((cudaFuncSetAttribute(render_kernel<GAME, MODE, TX, TY>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem > 160 * 1024 ? smem : 160 * 1024)));
+  CK((cudaFuncSetAttribute(render_kernel<GAME, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem > 160 * 1024 ? smem : 160 * 1024)));
   const int H = Traits<GAME>::H;
-  dim3 grid(blocks(a.n, TBX_EPC), ((MODE == TBX_OBS_GRAY_AREA ? a.out_h : H) + a.band_rows - 1) / a.band_rows);
+  dim3 grid(blocks(a.n, TBX_EPC), (H + a.band_rows - 1) / a.band_rows);
   /* measured: Breakout's few primitives keep 4 warps busy, the sprite-heavy games use 8 (profiles/r1_native_layouts.md) */
-  int threads = (MODE == TBX_OBS_GRAY_AREA || GAME == TBX_BREAKOUT) ? 128 : 256;
-  if (const char *env = getenv("TBX_RENDER_THREADS")) threads = atoi(env); /* tuning: 32, 64, 128 or 256 */
-  if (threads != 32 && threads != 64 && threads != 128 && threads != 256) threads = 128;
-  static const TbxAreaPlan no_plan = TbxAreaPlan();
-  render_kernel<GAME, MODE, TX, TY><<<grid, threads, smem, s>>>(a, *(const typename Traits<GAME>::Cfg *)cfg_host, plan_host ? *plan_host : no_plan);
+  const int threads = GAME == TBX_BREAKOUT ? 128 : 256;
+  render_kernel<GAME, MODE><<<grid, threads, smem, s>>>(a, *(const typename Traits<GAME>::Cfg *)cfg_host);
   CK(cudaGetLastError());
   return TBX_OK;
 }
@@ -402,44 +400,34 @@ static int launch_native(const tbx_pool *p, int mode, const RenderArgs &a, int b
 }
 
 /* INTER_AREA, one warp per env (tbx_render_area.cuh) */
-template <int GAME, int TX, int TY, bool DUAL> static int launch_area_tile_dual(const RenderArgs &a, const void *cfg_host, const TbxAreaPlan *plan_host, int smem, int threads, cudaStream_t s) {
+template <int GAME, int TX, int TY, bool DUAL> static int launch_area_tile_dual(const RenderArgs &a, const void *cfg_host, const TbxAreaPlan *plan_host, int smem, cudaStream_t s) {
   CK((cudaFuncSetAttribute(area_tile_kernel<GAME, TX, TY, DUAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
   /* env-list mode (the envs the direct kernel handed over, normally none): a small grid walks the list */
   const int grid = a.env_list ? (blocks(a.n, TBX_EPC) < 296 ? blocks(a.n, TBX_EPC) : 296) : blocks(a.n, TBX_EPC);
-  area_tile_kernel<GAME, TX, TY, DUAL><<<grid, threads, smem, s>>>(a, *(const typename Traits<GAME>::Cfg *)cfg_host, *plan_host);
+  area_tile_kernel<GAME, TX, TY, DUAL><<<grid, TBX_TILE_THREADS, smem, s>>>(a, *(const typename Traits<GAME>::Cfg *)cfg_host, *plan_host);
   CK(cudaGetLastError());
   return TBX_OK;
 }
-template <int GAME, int TX, int TY> static int launch_area_tile(const RenderArgs &a, const void *cfg_host, const TbxAreaPlan *plan_host, int smem, int threads, cudaStream_t s) {
-  if (a.planes2) return launch_area_tile_dual<GAME, TX, TY, true>(a, cfg_host, plan_host, smem, threads, s);
-  return launch_area_tile_dual<GAME, TX, TY, false>(a, cfg_host, plan_host, smem, threads, s);
+template <int GAME, int TX, int TY> static int launch_area_tile(const RenderArgs &a, const void *cfg_host, const TbxAreaPlan *plan_host, int smem, cudaStream_t s) {
+  if (a.planes2) return launch_area_tile_dual<GAME, TX, TY, true>(a, cfg_host, plan_host, smem, s);
+  return launch_area_tile_dual<GAME, TX, TY, false>(a, cfg_host, plan_host, smem, s);
 }
-template <int GAME> static int launch_area_tile_taps(int tx, int ty, const RenderArgs &a, const void *c, const TbxAreaPlan *pl, int smem, int threads, cudaStream_t s) {
+/* the smallest instantiated tap counts that cover the plan; plans over 5 x 4 taps render single frames only */
+template <int GAME> static int launch_area_tile_taps(int tx, int ty, const RenderArgs &a, const void *c, const TbxAreaPlan *pl, int smem, cudaStream_t s) {
+  if (tx > 5 || ty > 4) return launch_area_tile_dual<GAME, 8, 8, false>(a, c, pl, smem, s);
   if (ty <= 3) {
-    if (tx <= 3) return launch_area_tile<GAME, 3, 3>(a, c, pl, smem, threads, s);
-    if (tx <= 4) return launch_area_tile<GAME, 4, 3>(a, c, pl, smem, threads, s);
-    return launch_area_tile<GAME, 5, 3>(a, c, pl, smem, threads, s);
+    if (tx <= 3) return launch_area_tile<GAME, 3, 3>(a, c, pl, smem, s);
+    if (tx <= 4) return launch_area_tile<GAME, 4, 3>(a, c, pl, smem, s);
+    return launch_area_tile<GAME, 5, 3>(a, c, pl, smem, s);
   }
-  if (tx <= 3) return launch_area_tile<GAME, 3, 4>(a, c, pl, smem, threads, s);
-  if (tx <= 4) return launch_area_tile<GAME, 4, 4>(a, c, pl, smem, threads, s);
-  return launch_area_tile<GAME, 5, 4>(a, c, pl, smem, threads, s);
+  if (tx <= 3) return launch_area_tile<GAME, 3, 4>(a, c, pl, smem, s);
+  if (tx <= 4) return launch_area_tile<GAME, 4, 4>(a, c, pl, smem, s);
+  return launch_area_tile<GAME, 5, 4>(a, c, pl, smem, s);
 }
-/* INTER_AREA: the smallest instantiated tap counts that cover the plan */
-template <int GAME, int TY> static int launch_area_tx(int tx, const RenderArgs &a, const void *c, const TbxAreaPlan *pl, int smem, cudaStream_t s) {
-  if (tx <= 3) return launch_render<GAME, TBX_OBS_GRAY_AREA, 3, TY>(a, c, pl, smem, s);
-  if (tx <= 4) return launch_render<GAME, TBX_OBS_GRAY_AREA, 4, TY>(a, c, pl, smem, s);
-  return launch_render<GAME, TBX_OBS_GRAY_AREA, 5, TY>(a, c, pl, smem, s);
-}
-template <int GAME> static int launch_render_mode(int mode, int tx, int ty, const RenderArgs &a, const void *c, const TbxAreaPlan *pl, int smem, cudaStream_t s) {
-  switch (mode) {
-    case TBX_OBS_RGBA: return launch_render<GAME, TBX_OBS_RGBA, 1, 1>(a, c, pl, smem, s);
-    case TBX_OBS_RGB: return launch_render<GAME, TBX_OBS_RGB, 1, 1>(a, c, pl, smem, s);
-    case TBX_OBS_GRAY: return launch_render<GAME, TBX_OBS_GRAY, 1, 1>(a, c, pl, smem, s);
-    default:
-      if (tx > 5 || ty > 4) return launch_render<GAME, TBX_OBS_GRAY_AREA, 8, 8>(a, c, pl, smem, s);
-      if (ty <= 3) return launch_area_tx<GAME, 3>(tx, a, c, pl, smem, s);
-      return launch_area_tx<GAME, 4>(tx, a, c, pl, smem, s);
-  }
+template <int GAME> static int launch_render_mode(int mode, const RenderArgs &a, const void *c, int smem, cudaStream_t s) {
+  if (mode == TBX_OBS_RGBA) return launch_render<GAME, TBX_OBS_RGBA>(a, c, smem, s);
+  if (mode == TBX_OBS_RGB) return launch_render<GAME, TBX_OBS_RGB>(a, c, smem, s);
+  return launch_render<GAME, TBX_OBS_GRAY>(a, c, smem, s);
 }
 
 extern "C" {
@@ -466,15 +454,13 @@ static int render_impl(tbx_pool *p, uint8_t *dst, int mode, int out_w, int out_h
   a.planes2 = dual ? dual->planes2 : 0; a.reset_flags = dual ? dual->reset_flags : 0;
   a.stack_k = dual ? dual->stack_k : 1; a.stack_slot = dual ? dual->stack_slot : 0; a.stack_mode = dual ? dual->stack_mode : 0; a.env_stride = fb * (size_t)a.stack_k; a.tile_bytes = 0;
   a.patches[0] = a.patches[1] = 0; a.dense_list = 0; a.dense_count = 0; a.dense_flag = 0; a.dense_threshold = 0; a.env_list = 0; a.env_count = 0;
-  a.dst = dst; a.frame_bytes = fb; a.plan = 0; a.out_h = out_h; a.tile_stride = 0; a.warp_bytes = 0; a.list_cap = 0; a.tile_hshift = 0; a.max_run = 0; a.band_rows = 0; a.smem_rects = 0;
+  a.dst = dst; a.frame_bytes = fb; a.plan = 0; a.tile_stride = 0; a.warp_bytes = 0; a.list_cap = 0; a.band_rows = 0; a.smem_rects = 0;
   for (int b = 0; b < 2; b++) {
     a.base[b] = pix == 4 ? p->d_base_rgba[b] : pix == 3 ? p->d_base_rgb[b] : p->d_base_gray[b];
     a.base_out[b] = 0; /* INTER_AREA: set below */
   }
   a.smem_canvas = align16(p->info->rec_words * TBX_EPC * 4) * (dual ? 2 : 1);
-  int smem_total, tx = 1, ty = 1;
-  bool patch_first = false;
-  const TbxAreaPlan *host_plan = 0;
+  cudaStream_t s = (cudaStream_t)stream;
   if (mode == TBX_OBS_GRAY_AREA) {
     AreaRes *ar = 0;
     r = ensure_area(p, out_w, out_h, &ar);
@@ -485,120 +471,90 @@ static int render_impl(tbx_pool *p, uint8_t *dst, int mode, int out_w, int out_h
       const bool on = !(env && atoi(env) == 0);
       a.patches[0] = on ? ar->d_patches[0] : 0; a.patches[1] = on ? ar->d_patches[1] : 0;
     }
-    tx = ar->tx; ty = ar->ty;
-    host_plan = &ar->plan;
-    /* Bands of output rows: each (chunk, band) CTA keeps only the canvas rows that feed its output rows, which
-     * multiplies the number of independent CTAs per SM.  Surplus (zero-weight) taps may read up to TY-1 rows past
-     * the band's last real row: the canvas allocation covers them. */
-    const int ty_inst = (tx > 5 || ty > 4) ? 8 : (ty <= 3 ? 3 : 4);
-    /* default: one warp per env over 16x4 output tiles; plans with many taps (or TBX_AREA_KERNEL=cta) use the
-     * CTA-wide canvas kernel below */
+    const int tx = ar->tx, ty = ar->ty;
+    const bool many_taps = tx > 5 || ty > 4;
+    if (dual && many_taps) return set_err(TBX_EINVAL, "wrapped observations need an output size the tile kernel supports (at most 5 x 4 taps)");
+    /* one warp per env over tiles of 16 x 8 output pixels, runs of at most TBX_TILE_MAX_RUN tiles: the scratch holds the
+     * widest / tallest run window of the instantiated tap counts */
+    const int tx_inst = many_taps ? 8 : tx <= 3 ? 3 : tx <= 4 ? 4 : 5, ty_inst = many_taps ? 8 : ty <= 3 ? 3 : 4;
+    const int tile_h = 1 << TBX_TILE_HSHIFT;
+    int stride = 0, rows = 0;
+    for (int dxA = 0; dxA < out_w; dxA += 16) {
+      const int dxL = dxA + 16 * TBX_TILE_MAX_RUN - 1 < out_w ? dxA + 16 * TBX_TILE_MAX_RUN - 1 : out_w - 1;
+      const int wdt = ((ar->plan.xs0[dxL] + tx_inst + 3) & ~3) - (ar->plan.xs0[dxA] & ~3);
+      if (wdt > stride) stride = wdt;
+    }
+    for (int dyA = 0; dyA < out_h; dyA += tile_h) {
+      const int dyL = dyA + tile_h - 1 < out_h ? dyA + tile_h - 1 : out_h - 1;
+      const int rws = ar->plan.ys0[dyL] + ty_inst - ar->plan.ys0[dyA];
+      if (rws > rows) rows = rws;
+    }
+    /* every plan build_area_plan accepts fits, for all three games (at most 256 B x 64 rows) */
+    if (stride > 512 || rows > 96 || W % 4 != 0)
+      return set_err(TBX_EINVAL, "INTER_AREA " + std::to_string(out_w) + "x" + std::to_string(out_h) + ": the tile kernel's scratch window (" +
+                                     std::to_string(stride) + " B x " + std::to_string(rows) + " rows) exceeds its limit of 512 B x 96 rows");
+    a.tile_stride = stride;
+    a.list_cap = TBX_TILE_LCAP;
+    if (const char *env = getenv("TBX_AREA_LCAP")) a.list_cap = atoi(env); /* tests: small lists force the sweep / per-tile paths */
+    if (a.list_cap < 1 || a.list_cap > TBX_TILE_LCAP) a.list_cap = TBX_TILE_LCAP;
+    a.tile_bytes = align16(stride * rows);
+    a.warp_bytes = TBX_TILE_LCAP * 20 + 32 + a.tile_bytes * (dual ? 2 : 1);
+    const int smem = a.smem_canvas + (TBX_TILE_THREADS / 32) * a.warp_bytes;
+    int smem_optin = 0;
+    CK(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, p->device));
+    if (smem > smem_optin)
+      return set_err(TBX_EINVAL, "INTER_AREA " + std::to_string(out_w) + "x" + std::to_string(out_h) + ": the tile kernel needs " + std::to_string(smem) +
+                                     " B of shared memory per CTA, the device allows " + std::to_string(smem_optin));
+    /* Direct kernel first (tbx_render_direct.cuh; TBX_AREA_KERNEL=tile turns it off): closed forms for the envs they
+     * cover, the rest are listed and rendered by the tile kernel in env-list mode right after (usually an empty list) */
     const char *ksel = getenv("TBX_AREA_KERNEL");
-    if (tx <= 5 && ty <= 4 && !(ksel && !strcmp(ksel, "cta"))) {
-      const int tx_inst = tx <= 3 ? 3 : tx <= 4 ? 4 : 5;
-      /* tiles of 16 x 8 output pixels, runs of at most 2 tiles: the scratch holds the widest / tallest run window */
-      int ths = 3, max_run = 2;
-      if (const char *env = getenv("TBX_AREA_TILE_H")) ths = atoi(env) == 4 ? 2 : atoi(env) == 16 ? 4 : 3;
-      if (const char *env = getenv("TBX_AREA_MAX_RUN")) max_run = atoi(env);
-      if (max_run < 1) max_run = 1;
-      if (max_run > 8) max_run = 8;
-      int stride = 0, rows = 0;
-      for (int dxA = 0; dxA < out_w; dxA += 16) {
-        const int dxL = dxA + 16 * max_run - 1 < out_w ? dxA + 16 * max_run - 1 : out_w - 1;
-        const int wdt = ((ar->plan.xs0[dxL] + tx_inst + 3) & ~3) - (ar->plan.xs0[dxA] & ~3);
-        if (wdt > stride) stride = wdt;
-      }
-      for (int dyA = 0; dyA < out_h; dyA += 1 << ths) {
-        const int dyL = dyA + (1 << ths) - 1 < out_h ? dyA + (1 << ths) - 1 : out_h - 1;
-        const int rws = ar->plan.ys0[dyL] + ty_inst - ar->plan.ys0[dyA];
-        if (rws > rows) rows = rws;
-      }
-      if (stride <= 512 && rows <= 96 && W % 4 == 0) {
-        int threads = 256;
-        if (const char *env = getenv("TBX_AREA_THREADS")) threads = atoi(env);
-        if (threads != 32 && threads != 64 && threads != 128 && threads != 256) threads = 256;
-        a.tile_stride = stride;
-        a.tile_hshift = ths;
-        a.max_run = max_run;
-        a.list_cap = TBX_TILE_LCAP;
-        if (const char *env = getenv("TBX_AREA_LCAP")) a.list_cap = atoi(env); /* tests: small lists force the sweep / per-tile paths */
-        if (a.list_cap < 1 || a.list_cap > TBX_TILE_LCAP) a.list_cap = TBX_TILE_LCAP;
-        a.tile_bytes = align16(stride * rows);
-        a.warp_bytes = TBX_TILE_LCAP * 20 + 32 + a.tile_bytes * (dual ? 2 : 1);
-        const int smem = a.smem_canvas + (threads / 32) * a.warp_bytes;
-        cudaStream_t s = (cudaStream_t)stream;
-        /* Direct kernel first (tbx_render_direct.cuh; TBX_AREA_KERNEL=tile turns it off): closed forms for the envs they
-         * cover, the rest are listed and rendered by the tile kernel in env-list mode right after (usually an empty list) */
-        if (ar->direct_ok && !dual && !(ksel && !strcmp(ksel, "tile"))) {
-          if (!p->d_fb) { CK(cudaMalloc(&p->d_fb, ((size_t)p->n_pad + 8) * sizeof(int32_t))); CK(cudaMemsetAsync(p->d_fb, 0, 8 * sizeof(int32_t), s)); }
-          DirectArgs da;
-          da.aux = ar->d_direct; da.aux2 = ar->d_direct2; da.fb_list = p->d_fb + 8; da.fb_count = p->d_fb; da.sched = p->d_fb + 2;
-          tbx_direct_geometry(p->game, out_w, out_h, p->game == TBX_BREAKOUT ? p->cfg.brk.n_rows : 0, da);
-          CK(tbx_launch_direct(p->game, tx, ty, a, cfg_ptr(p), ar->plan, da, s));
-          if (p->game == TBX_SPACE_INVADERS) return TBX_OK; /* covers every env: nothing is handed over */
-          a.env_list = p->d_fb + 8;
-          a.env_count = p->d_fb;
-        }
-        if (p->game == TBX_BREAKOUT) return launch_area_tile_taps<TBX_BREAKOUT>(tx, ty, a, cfg_ptr(p), host_plan, smem, threads, s);
-        if (p->game == TBX_AMIDAR) return launch_area_tile_taps<TBX_AMIDAR>(tx, ty, a, cfg_ptr(p), host_plan, smem, threads, s);
-        return launch_area_tile_taps<TBX_SPACE_INVADERS>(tx, ty, a, cfg_ptr(p), host_plan, smem, threads, s);
-      }
+    if (ar->direct_ok && !dual && !(ksel && !strcmp(ksel, "tile"))) {
+      if (!p->d_fb) { CK(cudaMalloc(&p->d_fb, ((size_t)p->n_pad + 8) * sizeof(int32_t))); CK(cudaMemsetAsync(p->d_fb, 0, 8 * sizeof(int32_t), s)); }
+      DirectArgs da;
+      da.aux = ar->d_direct; da.aux2 = ar->d_direct2; da.fb_list = p->d_fb + 8; da.fb_count = p->d_fb; da.sched = p->d_fb + 2;
+      tbx_direct_geometry(p->game, out_w, out_h, p->game == TBX_BREAKOUT ? p->cfg.brk.n_rows : 0, da);
+      CK(tbx_launch_direct(p->game, tx, ty, a, cfg_ptr(p), ar->plan, da, s));
+      if (p->game == TBX_SPACE_INVADERS) return TBX_OK; /* covers every env: nothing is handed over */
+      a.env_list = p->d_fb + 8;
+      a.env_count = p->d_fb;
     }
-    if (dual) return set_err(TBX_EINVAL, "wrapped observations need an output size the tile kernel supports (at most 5 x 4 taps)");
-    int nb = p->game == TBX_AMIDAR ? 1 : 2;
-    if (const char *env = getenv("TBX_AREA_BANDS")) nb = atoi(env);
-    if (nb < 1) nb = 1;
-    if (nb > out_h) nb = out_h;
-    a.band_rows = (out_h + nb - 1) / nb;
-    int canvas_rows = 0;
-    for (int d0 = 0; d0 < out_h; d0 += a.band_rows) {
-      int d1 = d0 + a.band_rows < out_h ? d0 + a.band_rows : out_h;
-      int rows = ar->plan.ys0[d1 - 1] + ty_inst - ar->plan.ys0[d0];
-      if (rows > canvas_rows) canvas_rows = rows;
-    }
-    a.smem_rects = a.smem_canvas + align16(canvas_rows * W + 16);
-  } else {
-    /* Default: broadcast + patch (tbx_render_native.cuh) -- the base frame leaves through the TMA engine at HBM speed, what
-     * differs from it is painted straight into the frame.  Envs that differ in many places (a Breakout wall with more
-     * than 20 holes, an Amidar maze with more than 48 painted tiles / boxes; TBX_NATIVE_DENSE overrides) are cheaper
-     * to repaint in shared memory: the patch kernel lists them and the canvas kernel below renders exactly those.
-     * TBX_NATIVE_KERNEL=canvas renders everything with the canvas kernel. */
-    const char *ksel = getenv("TBX_NATIVE_KERNEL");
-    patch_first = !(ksel && !strcmp(ksel, "canvas")) && !dual;
-    /* canvas bands of at most ~40 KB so that five CTAs stay resident per SM */
-    int max_rows = (40 * 1024) / (W * pix);
-    if (max_rows < 1) max_rows = 1;
-    int nb = (H + max_rows - 1) / max_rows;
-    a.band_rows = (H + nb - 1) / nb;
-    a.smem_rects = a.smem_canvas + align16(a.band_rows * W * pix);
+    if (p->game == TBX_BREAKOUT) return launch_area_tile_taps<TBX_BREAKOUT>(tx, ty, a, cfg_ptr(p), &ar->plan, smem, s);
+    if (p->game == TBX_AMIDAR) return launch_area_tile_taps<TBX_AMIDAR>(tx, ty, a, cfg_ptr(p), &ar->plan, smem, s);
+    return launch_area_tile_taps<TBX_SPACE_INVADERS>(tx, ty, a, cfg_ptr(p), &ar->plan, smem, s);
   }
-  smem_total = a.smem_rects + 2 * TBX_MAX_RECTS * (int)sizeof(int4) + 128 + TBX_MAX_BIG * (int)sizeof(uint4); /* + list counts, per-env base / env ids, the big-primitive queue */
+  /* Native layouts: broadcast + patch (tbx_render_native.cuh) -- the base frame leaves through the TMA engine at HBM speed,
+   * what differs from it is painted straight into the frame.  Breakout and Amidar envs that differ in many places (a wall
+   * with more than 20 holes, a maze with more than 48 painted tiles / boxes; TBX_NATIVE_DENSE overrides) are cheaper to
+   * repaint in shared memory: the patch kernel lists them and the canvas kernel below renders exactly those.  Space
+   * Invaders' ~50 sprites are always patched. */
+  /* canvas bands of at most ~40 KB so that five CTAs stay resident per SM */
+  int max_rows = (40 * 1024) / (W * pix);
+  if (max_rows < 1) max_rows = 1;
+  const int nb = (H + max_rows - 1) / max_rows;
+  a.band_rows = (H + nb - 1) / nb;
+  a.smem_rects = a.smem_canvas + align16(a.band_rows * W * pix);
+  const int smem_total = a.smem_rects + 2 * TBX_MAX_RECTS * (int)sizeof(int4) + 128 + TBX_MAX_BIG * (int)sizeof(uint4); /* + list counts, per-env base / env ids, the big-primitive queue */
   if (smem_total > 220 * 1024) return set_err(TBX_EINVAL, "observation size needs more shared memory than one SM has");
-  cudaStream_t s = (cudaStream_t)stream;
-  if (patch_first) {
-    int thr = p->game == TBX_BREAKOUT ? 20 : p->game == TBX_AMIDAR ? 48 : INT32_MAX;
-    if (const char *env = getenv("TBX_NATIVE_DENSE")) thr = atoi(env) < 0 ? INT32_MAX : atoi(env);
-    RenderArgs f = a; /* same bands for the broadcast */
-    if (thr != INT32_MAX) {
-      if (!p->d_dense) CK(cudaMalloc(&p->d_dense, ((size_t)p->n_pad + 8) * sizeof(int32_t) + (size_t)p->n_pad));
-      f.dense_list = p->d_dense + 8;
-      f.dense_count = p->d_dense;
-      f.dense_flag = reinterpret_cast<uint8_t *>(p->d_dense + 8 + p->n_pad);
-      f.dense_threshold = thr;
-      CK(cudaMemsetAsync(p->d_dense, 0, sizeof(int32_t), s));
-      if (p->game == TBX_BREAKOUT) dense_classify_kernel<TBX_BREAKOUT><<<blocks(p->n, 8), 256, 0, s>>>(f, p->cfg.brk);
-      else if (p->game == TBX_AMIDAR) dense_classify_kernel<TBX_AMIDAR><<<blocks(p->n, 8), 256, 0, s>>>(f, p->cfg.ami);
-      else dense_classify_kernel<TBX_SPACE_INVADERS><<<blocks(p->n, 8), 256, 0, s>>>(f, p->cfg.si);
-      CK(cudaGetLastError());
-    }
-    r = launch_native(p, mode, f, align16(a.band_rows * W * pix), s);
-    if (r || thr == INT32_MAX) return r;
-    a.env_list = p->d_dense + 8;
-    a.env_count = p->d_dense;
+  int thr = p->game == TBX_BREAKOUT ? 20 : p->game == TBX_AMIDAR ? 48 : INT32_MAX;
+  const char *dense_env = getenv("TBX_NATIVE_DENSE");
+  if (dense_env && thr != INT32_MAX) thr = atoi(dense_env) < 0 ? INT32_MAX : atoi(dense_env);
+  if (thr != INT32_MAX) {
+    if (!p->d_dense) CK(cudaMalloc(&p->d_dense, ((size_t)p->n_pad + 8) * sizeof(int32_t) + (size_t)p->n_pad));
+    a.dense_list = p->d_dense + 8;
+    a.dense_count = p->d_dense;
+    a.dense_flag = reinterpret_cast<uint8_t *>(p->d_dense + 8 + p->n_pad);
+    a.dense_threshold = thr;
+    CK(cudaMemsetAsync(p->d_dense, 0, sizeof(int32_t), s));
+    if (p->game == TBX_BREAKOUT) dense_classify_kernel<TBX_BREAKOUT><<<blocks(p->n, 8), 256, 0, s>>>(a, p->cfg.brk);
+    else dense_classify_kernel<TBX_AMIDAR><<<blocks(p->n, 8), 256, 0, s>>>(a, p->cfg.ami);
+    CK(cudaGetLastError());
   }
-  if (p->game == TBX_BREAKOUT) return launch_render_mode<TBX_BREAKOUT>(mode, tx, ty, a, cfg_ptr(p), host_plan, smem_total, s);
-  if (p->game == TBX_AMIDAR) return launch_render_mode<TBX_AMIDAR>(mode, tx, ty, a, cfg_ptr(p), host_plan, smem_total, s);
-  return launch_render_mode<TBX_SPACE_INVADERS>(mode, tx, ty, a, cfg_ptr(p), host_plan, smem_total, s);
+  r = launch_native(p, mode, a, align16(a.band_rows * W * pix), s);
+  if (r || thr == INT32_MAX) return r;
+  a.env_list = p->d_dense + 8;
+  a.env_count = p->d_dense;
+  if (p->game == TBX_BREAKOUT) return launch_render_mode<TBX_BREAKOUT>(mode, a, cfg_ptr(p), smem_total, s);
+  return launch_render_mode<TBX_AMIDAR>(mode, a, cfg_ptr(p), smem_total, s);
 }
 
 /* ---- the fused wrapper stack (tbx_wrap.cuh) */

@@ -1,4 +1,8 @@
-/* tbx_render.cuh -- the render kernel (Toybox.get_state / get_rgb_frame for a whole pool; fused WarpFrame).
+/* tbx_render.cuh -- the canvas render kernel (Toybox.get_state / get_rgb_frame), and the draw-list helpers the other
+ * renderers share.
+ *
+ * The native layouts (RGBA / RGB / gray) are rendered as broadcast + patch (tbx_render_native.cuh).  Breakout and
+ * Amidar envs that differ from their base frame in many places are handed to this kernel instead.
  *
  * DELTA RENDERING over a persistent shared-memory canvas.  One CTA owns a band of canvas rows and renders it for a
  * chunk of TBX_EPC = 8 consecutive envs (8 envs x 4 B = one 32-byte sector per state word, so the word-major
@@ -12,9 +16,7 @@
  *     primitives are painted warp-cooperatively; groups that may conflict are painted by one warp strictly in
  *     order.  The result equals the painter's algorithm over the full draw list.  Painted areas are recorded as
  *     dirty rectangles.
- *   - Native layouts (RGBA / RGB / gray) stream the canvas band to HBM with 16-byte coalesced streaming stores.
- *     The INTER_AREA layout copies the pre-computed down-sample of the base frame to the destination and then
- *     recomputes only the output pixels whose taps touch a dirty rectangle, with cv2's exact f32 tap order.
+ *   - The painted band leaves for the destination frame through the TMA engine.
  *   - Afterwards the dirty rectangles are restored from the base frame, so per-env work is proportional to what
  *     differs from the base, not to the frame size.
  */
@@ -28,8 +30,7 @@
 namespace tbxk {
 
 /* The kernel is compiled for up to 256 threads and 64 registers per thread (4 x 256 or 8 x 128 threads per SM);
- * the launch picks the CTA size per layout: the INTER_AREA layout does little work per env and runs best as many
- * small CTAs, the native layouts stream whole bands and like wide ones.  The CTA size is a power of two. */
+ * the launch picks the CTA size per game.  The CTA size is a power of two. */
 #define TBX_RENDER_MAX_THREADS 256
 #define TBX_RENDER_MIN_CTAS 4
 #define TBX_NT ((int)blockDim.x)
@@ -125,8 +126,7 @@ struct RenderArgs {
   const uint8_t *base[2];     /* base frames 0/1 in the canvas format: gray bytes, packed RGB or RGBA */
   const uint8_t *base_out[2]; /* INTER_AREA: their down-samples */
   const TbxAreaPlan *plan;    /* INTER_AREA */
-  int band_rows;              /* per CTA (blockIdx.y selects the band): canvas rows (native layouts) / output rows (INTER_AREA) */
-  int out_h;                  /* INTER_AREA: output rows (host-side launch geometry) */
+  int band_rows;              /* native layouts: frame rows per CTA (blockIdx.y selects the band) */
   int smem_canvas, smem_rects; /* byte offsets into dynamic shared memory */
   /* dual mode (tbx_wrap.cuh): observation = INTER_AREA(max(frame(planes), frame(planes2))), written into slot
    * `stack_slot` of a ring of `stack_k` frames per env; envs flagged in reset_flags get the frame in every slot */
@@ -145,7 +145,7 @@ struct RenderArgs {
   const int32_t *env_list;
   const int *env_count;
   const TbxDigitPatch *patches[2]; /* INTER_AREA: pre-resolved HUD digit patches per base frame, [slot * 10 + digit]; NULL = off */
-  int tile_stride, warp_bytes, list_cap, tile_hshift, max_run; /* INTER_AREA tile kernel (tbx_render_area.cuh): scratch row pitch, shared memory per warp */
+  int tile_stride, warp_bytes, list_cap; /* INTER_AREA tile kernel (tbx_render_area.cuh): scratch row pitch, shared memory per warp */
 };
 
 /* The canvas is a byte array with PIX bytes per pixel: 1 = gray, 3 = packed RGB, 4 = RGBA.  `val` is the colour
@@ -379,14 +379,11 @@ __device__ __forceinline__ void restore_canvas(uint8_t *canvas, const uint8_t *b
   }
 }
 
-/* MODE: TBX_OBS_RGBA (0), TBX_OBS_RGB (1), TBX_OBS_GRAY (2), TBX_OBS_GRAY_AREA (3).
- * TX, TY: taps per output column / row of the INTER_AREA plan (>= plan.tx, plan.ty; surplus taps have zero weight). */
-template <int GAME, int MODE, int TX, int TY>
-__global__ void __launch_bounds__(TBX_RENDER_MAX_THREADS, TBX_RENDER_MIN_CTAS) render_kernel(const __grid_constant__ RenderArgs a, const __grid_constant__ typename Traits<GAME>::Cfg cfg_c,
-                                                                                          const __grid_constant__ TbxAreaPlan plan_c) {
-  /* The pool's config and the INTER_AREA plan travel as kernel parameters: warp-uniform reads of them (colours,
-   * row taps, inverse maps) come from the constant bank instead of global memory.  Reads indexed per lane (column
-   * taps) still go through `a.plan` in global memory / L1, where they coalesce. */
+/* MODE: TBX_OBS_RGBA (0), TBX_OBS_RGB (1), TBX_OBS_GRAY (2) */
+template <int GAME, int MODE>
+__global__ void __launch_bounds__(TBX_RENDER_MAX_THREADS, TBX_RENDER_MIN_CTAS) render_kernel(const __grid_constant__ RenderArgs a, const __grid_constant__ typename Traits<GAME>::Cfg cfg_c) {
+  /* The pool's config travels as a kernel parameter: warp-uniform reads of it (colours) come from the constant bank
+   * instead of global memory. */
   typedef Traits<GAME> T;
   constexpr int W = T::W, H = T::H, RW = T::RW;
   constexpr int PIX = MODE == 0 ? 4 : MODE == 1 ? 3 : 1; /* canvas bytes per pixel = output bytes per pixel */
@@ -401,7 +398,7 @@ __global__ void __launch_bounds__(TBX_RENDER_MAX_THREADS, TBX_RENDER_MIN_CTAS) r
   uint4 *big_buf = reinterpret_cast<uint4 *>(rect_n + 32);
   const typename T::Cfg &cfg = cfg_c;
   const typename T::Table *tables = (const typename T::Table *)a.tables;
-  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  const int tid = threadIdx.x;
   const int e0 = blockIdx.x * TBX_EPC;
   const int ne = min(TBX_EPC, (a.env_count ? *a.env_count : a.n) - e0);
   if (ne <= 0) return; /* env-list mode: nothing (left) to repaint */
@@ -421,95 +418,8 @@ __global__ void __launch_bounds__(TBX_RENDER_MAX_THREADS, TBX_RENDER_MIN_CTAS) r
   if (tid < ne) env_base[tid] = T::base_id(recs + tid * RW, cfg, tables);
   __syncthreads();
 
-  if constexpr (MODE == 3) {
-    const TbxAreaPlan *__restrict__ plan = a.plan;
-    const TbxAreaPlan &cplan = plan_c;
-    const int dw = cplan.dw, dh = cplan.dh;
-    /* this CTA's band: output rows [d0,d1) and the canvas rows [r0,r1) that feed them (TY taps per output row) */
-    const int d0 = blockIdx.y * a.band_rows, d1 = min(dh, d0 + a.band_rows);
-    const int r0 = cplan.ys0[d0], r1 = min(H, (int)cplan.ys0[d1 - 1] + TY);
-    /* the static part of the band in every output frame of the chunk: the base frame's down-sample, global ->
-     * global (16-, 4- or 1-byte units, whatever the band's byte range allows) */
-    {
-      const int b0 = d0 * dw, b1 = d1 * dw;
-      const int align = (int)(a.frame_bytes | (size_t)b0 | (size_t)b1);
-      for (int j = 0; j < ne; j++) {
-        const uint8_t *src = env_base[j] ? a.base_out[1] : a.base_out[0];
-        uint8_t *dst = a.dst + (size_t)env_id[j] * a.frame_bytes;
-        if ((align & 15) == 0) {
-          for (int i = (b0 >> 4) + tid; i < (b1 >> 4); i += TBX_NT) reinterpret_cast<uint4 *>(dst)[i] = __ldg(reinterpret_cast<const uint4 *>(src) + i);
-        } else if ((align & 3) == 0) {
-          for (int i = (b0 >> 2) + tid; i < (b1 >> 2); i += TBX_NT) reinterpret_cast<uint32_t *>(dst)[i] = __ldg(reinterpret_cast<const uint32_t *>(src) + i);
-        } else {
-          for (int i = b0 + tid; i < b1; i += TBX_NT) dst[i] = __ldg(src + i);
-        }
-      }
-    }
-    int canvas_base = -1;
-    for (int j = 0; j < ne; j++) {
-      const uint32_t *R = recs + j * RW;
-      const int base = env_base[j];
-      int4 *rects = rect_buf + (j & 1) * TBX_MAX_RECTS;
-      int *n_rects = rect_n + (j & 1);
-      /* bring the canvas back to the base frame (the barrier after the previous env's recompute precedes this) */
-      if (canvas_base != base) load_canvas<1, W>(canvas, (base ? a.base[1] : a.base[0]), r0, r1);
-      else restore_canvas<1, W>(canvas, (base ? a.base[1] : a.base[0]), r0, r1, rect_buf + ((j - 1) & 1) * TBX_MAX_RECTS, rect_n[(j - 1) & 1]);
-      canvas_base = base;
-      __syncthreads();
-      if (tid == 0) rect_n[(j - 1) & 1] = 0; /* that list is reused by env j+1 */
-      paint_env<GAME, 1>(R, cfg, tables, base, canvas, r0, r1, rects, n_rects, big_buf, n_big);
-      /* Recompute the band's output pixels fed by a dirty rectangle and patch them into the destination frame
-       * (the barriers above order these byte stores after the band's base copy).  Lanes own output columns (their
-       * taps stay in registers), warps own output rows; narrow rectangles pack several rows into one warp.
-       * Straight-line TX x TY taps, surplus taps carry zero weights (x + 0*b == x for these sums). */
-      uint8_t *out = a.dst + (size_t)env_id[j] * a.frame_bytes;
-      int nr = *n_rects;
-      const bool overflow = nr > TBX_MAX_RECTS;
-      if (overflow) nr = 1;
-      for (int r = 0; r < nr; r++) {
-        const int4 rc = overflow ? make_int4(0, r0, W, r1) : rects[r];
-        if (rc.z <= rc.x) continue;
-        /* a small rectangle is recomputed by one warp (round robin), a large one by all warps row-interleaved */
-        const bool shared = (rc.z - rc.x) * (rc.w - rc.y) > 400;
-        if (!shared && (r & (TBX_NW - 1)) != wid) continue;
-        const int wsel = shared ? wid : 0, wcnt = shared ? TBX_NW : 1;
-        const int dx0 = cplan.xdlo[rc.x], dx1 = cplan.xdhi[rc.z - 1];
-        const int dy0 = max((int)cplan.ydlo[rc.y], d0), dy1 = min((int)cplan.ydhi[rc.w - 1], d1 - 1);
-        if (dy0 > dy1) continue;
-        const int ncols = dx1 - dx0 + 1;
-        const int lg = ncols > 16 ? 5 : ncols > 8 ? 4 : ncols > 4 ? 3 : 2; /* columns per warp pass = 1 << lg */
-        const int cpl = 1 << lg, rpi = 32 >> lg, sub = lane >> lg, c = lane & (cpl - 1);
-        for (int dxb = dx0; dxb <= dx1; dxb += cpl) {
-          const bool colok = dxb + c <= dx1;
-          const int dx = colok ? dxb + c : dx1;
-          const uint8_t *col = canvas + __ldg(&plan->xs0[dx]);
-          float al[TX];
-#pragma unroll
-          for (int t = 0; t < TX; t++) al[t] = __ldg(&plan->xalpha[t][dx]);
-          for (int dy = dy0 + wsel * rpi + sub; dy <= dy1; dy += wcnt * rpi) {
-            const uint8_t *row = col + (size_t)((int)cplan.ys0[dy] - r0) * W;
-            float v = 0.0f;
-#pragma unroll
-            for (int k = 0; k < TY; k++) {
-              float h = tbx_fmul(tbx_u8f(row[k * W]), al[0]);
-#pragma unroll
-              for (int t = 1; t < TX; t++) h = tbx_fadd(h, tbx_fmul(tbx_u8f(row[k * W + t]), al[t]));
-              const float bh = tbx_fmul(cplan.yalpha[k][dy], h);
-              v = k == 0 ? bh : tbx_fadd(v, bh);
-            }
-            const int iv = tbx_f2i_rn_small(v);
-            if (colok) out[dy * dw + dx] = (uint8_t)(iv < 0 ? 0 : iv > 255 ? 255 : iv);
-          }
-        }
-      }
-      __syncthreads(); /* the canvas is restored next */
-    }
-    return;
-  }
-
-  /* ---- native layouts (gray, packed RGB, RGBA): the canvas holds the output format, so the painted band IS the
-   * output band and leaves through the TMA engine -- one bulk shared -> global copy per env (cp.async.bulk), no
-   * per-thread load/store instructions. */
+  /* The canvas holds the output format, so the painted band IS the output band and leaves through the TMA engine --
+   * one bulk shared -> global copy per env (cp.async.bulk), no per-thread load/store instructions. */
   const int r0 = blockIdx.y * a.band_rows, r1 = min(H, r0 + a.band_rows);
   int canvas_base = -1;
 #pragma unroll 1 /* the body is large: unrolled over the 8 envs it no longer fits the instruction cache (measured: 2x slower) */

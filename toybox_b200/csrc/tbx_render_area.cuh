@@ -2,12 +2,12 @@
  *
  * The reference produces this observation as get_state() (native gray frame, toybox/envs/atari/base.py:109)
  * followed by cv2.resize(..., INTER_AREA) (baselines/baselines/common/atari_wrappers.py:243).  An output frame is
- * only 7 KB, so a CTA-wide shared canvas with barriers between the phases of every env (tbx_render.cuh, still used
- * for the native layouts) leaves most issue slots idle.  Here a warp renders its env alone -- no CTA barrier after
+ * only 7 KB, so a CTA-wide shared canvas with barriers between the phases of every env (tbx_render.cuh, used for
+ * the native layouts) leaves most issue slots idle.  Here a warp renders its env alone -- no CTA barrier after
  * the record load -- and never materialises the native frame:
  *   1. the pre-computed down-sample of the env's base frame is copied to the destination (16-byte units);
  *   2. the draw-list entries that differ from the base frame are built once (32 slots per pass, one per lane) and
- *      appended, in draw order, to a per-warp list in shared memory; every entry marks the OUTPUT TILES (16 x 4
+ *      appended, in draw order, to a per-warp list in shared memory; every entry marks the OUTPUT TILES (16 x 8
  *      output pixels) its pixels feed;
  *   3. for every run of horizontally adjacent marked tiles the warp copies the run's source window of the base
  *      frame (a few source rows) into a small shared-memory scratch canvas, paints the list entries that touch it in draw order (painter's
@@ -18,6 +18,8 @@
  * the primitives per tile (slow, but always correct).
  * Members of a PARALLEL draw-list group cannot conflict, so inside a tile the small solid ones (bricks, maze tiles)
  * are painted lane-parallel; everything else is painted by the whole warp, one entry at a time, in draw order.
+ * The kernel renders every plan the library accepts: it is instantiated for 3..5 x 3..4 taps, and for 8 x 8 taps
+ * (single frames only) for the plans with more; surplus taps carry zero weight.
  */
 #ifndef TBX_RENDER_AREA_CUH
 #define TBX_RENDER_AREA_CUH
@@ -25,11 +27,16 @@
 
 namespace tbxk {
 
-#define TBX_TILE_LCAP 128 /* list entries per warp */
-#define TBX_AREA_MAX_THREADS 256
+#define TBX_TILE_LCAP 128   /* list entries per warp */
+#define TBX_TILE_THREADS 256 /* CTA size: 8 warps */
+#define TBX_TILE_HSHIFT 3    /* tiles are 16 x (1 << TBX_TILE_HSHIFT) output pixels */
+#define TBX_TILE_MAX_RUN 2   /* a run renders at most this many horizontally adjacent tiles through one scratch window */
 #ifndef TBX_AREA_MIN_CTAS
 #define TBX_AREA_MIN_CTAS 4
 #endif
+/* the 8 x 8 instantiation keeps its eight column weights per lane in registers: at 4 CTAs per SM (64 registers) it
+ * spills, at 2 it needs ~112 and does not */
+#define TBX_TILE_MIN_CTAS(TX, TY) ((TX) > 5 || (TY) > 4 ? 2 : TBX_AREA_MIN_CTAS)
 
 /* a warp paints one primitive into the tile scratch canvas: window columns [wx0, wx1) (wx0 a multiple of 4, the
  * scratch's column 0), rows [wy0, wy1); `stride` bytes per scratch row */
@@ -225,7 +232,7 @@ __device__ __noinline__ void tile_row_rebuild(const uint32_t *R, const uint32_t 
 }
 
 template <int GAME, int TX, int TY, bool DUAL>
-__global__ void __launch_bounds__(TBX_AREA_MAX_THREADS, TBX_AREA_MIN_CTAS) area_tile_kernel(const __grid_constant__ RenderArgs a, const __grid_constant__ typename Traits<GAME>::Cfg cfg_c,
+__global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) area_tile_kernel(const __grid_constant__ RenderArgs a, const __grid_constant__ typename Traits<GAME>::Cfg cfg_c,
                                                                          const __grid_constant__ TbxAreaPlan plan_c) {
   typedef Traits<GAME> T;
   constexpr int W = T::W, H = T::H, RW = T::RW;
@@ -263,7 +270,7 @@ __global__ void __launch_bounds__(TBX_AREA_MAX_THREADS, TBX_AREA_MIN_CTAS) area_
   uint8_t *tile = reinterpret_cast<uint8_t *>(tmask + 8);
   uint8_t *tile2 = tile + a.tile_bytes; /* dual mode: the second state's window */
   const int stride = a.tile_stride;
-  const int ths = a.tile_hshift; /* tiles are 16 x (1 << ths) output pixels */
+  constexpr int ths = TBX_TILE_HSHIFT;
   const int dw = cp.dw, dh = cp.dh, nty = (dh + (1 << ths) - 1) >> ths;
   const uint32_t lt_mask = (1u << lane) - 1u;
 
@@ -452,7 +459,7 @@ __global__ void __launch_bounds__(TBX_AREA_MAX_THREADS, TBX_AREA_MIN_CTAS) area_
         uint32_t rowbits = (tmask[ty >> 2] >> ((ty & 3) * 8)) & 0xffu;
         while (rowbits) {
           const int t0 = __ffs(rowbits) - 1;
-          const int len = min(__ffs(~(rowbits >> t0)) - 1, a.max_run); /* consecutive marked tiles */
+          const int len = min(__ffs(~(rowbits >> t0)) - 1, TBX_TILE_MAX_RUN); /* consecutive marked tiles */
           rowbits &= ~(((1u << len) - 1u) << t0);
           const int rx0 = t0 * 16, rx1 = rx0 + len * 16 - 1, ry0 = ty << ths, ry1 = ry0 + (1 << ths) - 1;
           uint32_t hm[TBX_TILE_LCAP / 32];
