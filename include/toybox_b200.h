@@ -83,7 +83,8 @@ int tbx_step_inputs(tbx_pool *pool, const uint8_t *inputs_dev, int auto_reset, i
  * env i takes legal[index(seed, env0 + i, t)].  One launch instead of two; bit-identical to tbx_fill_actions + tbx_step. */
 int tbx_step_random(tbx_pool *pool, uint64_t seed, uint64_t env0, uint64_t t, int auto_reset, int32_t *reward_dev, uint8_t *done_dev,
                     int32_t *score_dev, int32_t *lives_dev, void *stream);
-/* synchronises `stream` and returns TBX_EACTION if any env received an invalid action id since the last check */
+/* synchronises `stream` and returns TBX_EACTION if any env received an invalid action id since the last check, else
+ * TBX_EINVAL if a state snapshot load or save skipped entries (tbx_state_load below) since the last check */
 int tbx_check(tbx_pool *pool, void *stream);
 
 /* render_current_frame: Toybox.get_state() / get_rgb_frame() for every env (envs/atari/base.py:109,164).
@@ -185,6 +186,48 @@ int tbx_wrap_destroy(tbx_wrap *wrap);
  * real_done: game over; score / lives: before any reset.  Output pointers may be NULL. */
 int tbx_wrap_step(tbx_wrap *wrap, const int32_t *actions_dev, uint8_t *obs_ring_dev, int32_t *reward_dev, uint8_t *done_dev,
                   uint8_t *real_done_dev, int32_t *score_dev, int32_t *lives_dev, int *slot_out, void *stream);
+
+/* ---- Device-resident state snapshots: save, restore and fork envs without the JSON codec (DESIGN.md 4.7).
+ * A snapshot of k envs is a caller-owned device buffer uint32[rows][k], word-major like the pool's planes: column j is one
+ * env's whole record (both rngs, prev_score, the episode counters; rows = tbx_state_rows), followed for a wrapped env by its
+ * 5 wrapper words (EpisodicLife lives, was_real_done, reset counter, Monitor return, Monitor length; rows =
+ * tbx_wrap_state_rows).  A loaded env continues exactly as the saved env would have.  The device-wide episode statistics
+ * (tbx_stats_read) are pool state and are neither saved nor restored.
+ * Breakout and Amidar records index the pool's geometry tables, so a snapshot goes with the tables blob of the moment it was
+ * saved (tbx_state_tables): a tbx_state_blob_header followed by table_count tables of table_bytes bytes each (none for Space
+ * Invaders).  Tables are only ever appended, so every index in a snapshot is below the count exported after saving it.
+ * Snapshots are trusted binary data written by tbx_state_save: a load checks the blob's header on the host (a mismatch returns
+ * TBX_EINVAL before any device work and leaves the pool unchanged) and, on the device, each entry's env id, column and table
+ * index; an entry out of range is skipped and counted, and the next tbx_check returns TBX_EINVAL with the count.  No other field
+ * is re-validated -- to_state_json / write_state_json stay the validated import. */
+#define TBX_STATE_MAGIC 0x53584254u /* "TBXS" */
+#define TBX_STATE_FORMAT 1          /* the record layout; a snapshot of another format is refused */
+typedef struct {
+  uint32_t magic, format;
+  uint32_t game;        /* 0 breakout, 1 amidar, 2 space_invaders */
+  uint32_t rows;        /* rows of the snapshot this blob belongs to */
+  uint32_t table_bytes; /* bytes of one geometry table */
+  uint32_t table_count;
+} tbx_state_blob_header;
+int tbx_state_rows(const tbx_pool *pool);
+int tbx_wrap_state_rows(const tbx_wrap *wrap);
+/* *size = bytes of the blob; it is written to out_host when out_host != NULL (TBX_EINVAL if cap < *size).  Host only. */
+int tbx_state_tables(const tbx_pool *pool, void *out_host, size_t cap, size_t *size);
+int tbx_wrap_state_tables(const tbx_wrap *wrap, void *out_host, size_t cap, size_t *size);
+/* Column j of snap_dev (uint32[rows][k]) <- env ids_dev[j] (ids_dev == NULL: env j).  Ids may repeat. */
+int tbx_state_save(tbx_pool *pool, const int32_t *ids_dev, int k, uint32_t *snap_dev, void *stream);
+/* Env ids_dev[j] <- column cols_dev[j] of snap_dev (uint32[rows][k_snap]), j < n; cols_dev == NULL: column j, ids_dev == NULL:
+ * env j.  An env listed more than once receives the last listed column, whole.  When the blob's tables are byte-identical to
+ * the pool's first table_count tables (always for the pool's own snapshots and for pools of the same config) table indices are
+ * copied as they are; otherwise the blob's tables are added to the pool (this synchronises the device) and the indices
+ * remapped, so snapshots move between pools, configs and GPUs of the same game.
+ * Save and load enqueue all device work on `stream`; in the same-table case neither synchronises nor allocates after a pool's
+ * first load, so save + load + step + render can be captured in a CUDA graph. */
+int tbx_state_load(tbx_pool *pool, const uint32_t *snap_dev, int k_snap, const int32_t *cols_dev, const int32_t *ids_dev, int n,
+                   const void *tables_blob, size_t blob_bytes, void *stream);
+int tbx_wrap_state_save(tbx_wrap *wrap, const int32_t *ids_dev, int k, uint32_t *snap_dev, void *stream);
+int tbx_wrap_state_load(tbx_wrap *wrap, const uint32_t *snap_dev, int k_snap, const int32_t *cols_dev, const int32_t *ids_dev, int n,
+                        const void *tables_blob, size_t blob_bytes, void *stream);
 
 #ifdef __cplusplus
 }

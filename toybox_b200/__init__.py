@@ -7,5 +7,6 @@ environment at a time through `ctoybox`.  See DESIGN.md / INTEGRATION.md.
 """
 from ._lib import ToyboxError, build, lib  # noqa: F401
 from .pool import BatchedToybox, GAMES, schema_for_config, schema_for_state  # noqa: F401
+from .snapshot import StateSnapshot  # noqa: F401
 
-__all__ = ["BatchedToybox", "GAMES", "ToyboxError", "build", "lib", "schema_for_state", "schema_for_config"]
+__all__ = ["BatchedToybox", "GAMES", "ToyboxError", "build", "lib", "schema_for_state", "schema_for_config", "StateSnapshot"]

@@ -111,6 +111,14 @@ def lib():
         "tbx_wrap_set_stack_mode": (i32, [vp, i32]),
         "tbx_wrap_set_episode_outputs": (i32, [vp, vp, vp]),
         "tbx_wrap_step": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(i32), vp]),
+        "tbx_state_rows": (i32, [vp]),
+        "tbx_wrap_state_rows": (i32, [vp]),
+        "tbx_state_tables": (i32, [vp, vp, sz, C.POINTER(sz)]),
+        "tbx_wrap_state_tables": (i32, [vp, vp, sz, C.POINTER(sz)]),
+        "tbx_state_save": (i32, [vp, vp, i32, vp, vp]),
+        "tbx_wrap_state_save": (i32, [vp, vp, i32, vp, vp]),
+        "tbx_state_load": (i32, [vp, vp, i32, vp, vp, i32, vp, sz, vp]),
+        "tbx_wrap_state_load": (i32, [vp, vp, i32, vp, vp, i32, vp, sz, vp]),
     }
     for name, (res, args) in sigs.items():
         f = getattr(L, name)          # AttributeError here = the header and the library disagree
@@ -125,7 +133,9 @@ EXPORTS = ["tbx_last_error", "tbx_version", "tbx_pool_create", "tbx_pool_destroy
            "tbx_step_inputs", "tbx_check", "tbx_render", "tbx_read_scalars", "tbx_step_host", "tbx_state_to_json",
            "tbx_state_from_json", "tbx_config_to_json", "tbx_config_from_json", "tbx_schema_for_state", "tbx_schema_for_config",
            "tbx_query_json", "tbx_free_str", "tbx_stats_read", "tbx_fill_actions", "tbx_fill_actions_policy",
-           "tbx_wrap_create", "tbx_wrap_destroy", "tbx_wrap_step", "tbx_field_lookup", "tbx_field_get", "tbx_field_set", "tbx_fill_actions_at", "tbx_stats_read_device", "tbx_wrap_set_stack_mode", "tbx_wrap_set_episode_outputs", "tbx_breakout_columns", "tbx_step_random"]
+           "tbx_wrap_create", "tbx_wrap_destroy", "tbx_wrap_step", "tbx_field_lookup", "tbx_field_get", "tbx_field_set", "tbx_fill_actions_at", "tbx_stats_read_device", "tbx_wrap_set_stack_mode", "tbx_wrap_set_episode_outputs", "tbx_breakout_columns", "tbx_step_random",
+           "tbx_state_rows", "tbx_wrap_state_rows", "tbx_state_tables", "tbx_wrap_state_tables", "tbx_state_save", "tbx_wrap_state_save",
+           "tbx_state_load", "tbx_wrap_state_load"]
 
 
 def check(rc):

@@ -2,6 +2,7 @@
 #include "../../include/toybox_b200.h"
 #include "tbx_kernels.cuh"
 #include "tbx_wrap.cuh"
+#include "tbx_snapshot.cuh"
 #include "tbx_fields.h"
 #include "tbx_direct_launch.h"
 #include <map>
@@ -40,7 +41,7 @@ struct tbx_pool {
   int d_tables_n;
   uint32_t *planes;
   unsigned long long *d_stats;
-  int *d_bad;
+  int *d_bad; /* [0] = invalid action ids, [1] = skipped snapshot entries, since the last tbx_check */
   int32_t *d_legal;
   /* render resources of the current config: static frame (gray, RGBA) and per output size the INTER_AREA plan */
   uint8_t *d_base_gray[2], *d_base_rgba[2], *d_base_rgb[2];
@@ -56,6 +57,9 @@ struct tbx_pool {
   int32_t *h_actions_dev, *h_reward_dev, *h_score_dev, *h_lives_dev;
   uint8_t *h_done_dev, *h_obs_dev;
   size_t h_obs_cap;
+  /* snapshot loads: owner entry per env (duplicate destinations), blob -> pool table indices (foreign tables) */
+  int32_t *d_owner, *d_remap;
+  int remap_cap;
 };
 
 /* The JSON codec is host work per env (build / walk a document tree, print / parse ~20-40 KB of text): spread the envs of a
@@ -148,6 +152,7 @@ int tbx_pool_destroy(tbx_pool *p) {
   cudaSetDevice(p->device);
   cudaDeviceSynchronize();
   cudaFree(p->d_cfg); cudaFree(p->d_tables); cudaFree(p->planes); cudaFree(p->d_stats); cudaFree(p->d_bad); cudaFree(p->d_legal); cudaFree(p->d_dense); cudaFree(p->d_fb); cudaFree(p->j_ids); cudaFree(p->j_recs); cudaFreeHost(p->j_host);
+  cudaFree(p->d_owner); cudaFree(p->d_remap);
   drop_render_cache(p);
   cudaFree(p->h_actions_dev); cudaFree(p->h_reward_dev); cudaFree(p->h_score_dev); cudaFree(p->h_lives_dev); cudaFree(p->h_done_dev); cudaFree(p->h_obs_dev);
   if (p->hs) cudaStreamDestroy(p->hs);
@@ -170,6 +175,7 @@ int tbx_pool_create(const char *game, int n_envs, int device, const char *cfg_js
   p->game = g; p->n = n_envs; p->n_pad = (n_envs + 31) & ~31; p->device = device; p->info = tbx::game_info(g);
   p->d_cfg = p->d_tables = 0; p->d_base_gray[0] = p->d_base_gray[1] = p->d_base_rgba[0] = p->d_base_rgba[1] = p->d_base_rgb[0] = p->d_base_rgb[1] = 0; p->d_tables_n = 0; p->planes = 0; p->d_stats = 0; p->d_bad = 0; p->d_legal = 0;
   p->hs = 0; p->d_dense = 0; p->d_fb = 0; p->j_ids = 0; p->j_recs = p->j_host = 0; p->j_cap_ids = p->j_cap_words = 0; p->h_actions_dev = p->h_reward_dev = p->h_score_dev = p->h_lives_dev = 0; p->h_done_dev = p->h_obs_dev = 0; p->h_obs_cap = 0;
+  p->d_owner = p->d_remap = 0; p->remap_cap = 0;
   int rc = TBX_OK;
   try {
     tbx::default_config(g, p->cfg);
@@ -183,8 +189,8 @@ int tbx_pool_create(const char *game, int n_envs, int device, const char *cfg_js
     CK(cudaMemset(p->planes, 0, (size_t)p->info->rec_words * p->n_pad * sizeof(uint32_t)));
     CK(cudaMalloc(&p->d_stats, 4 * sizeof(unsigned long long)));
     CK(cudaMemset(p->d_stats, 0, 4 * sizeof(unsigned long long)));
-    CK(cudaMalloc(&p->d_bad, sizeof(int)));
-    CK(cudaMemset(p->d_bad, 0, sizeof(int)));
+    CK(cudaMalloc(&p->d_bad, 2 * sizeof(int)));
+    CK(cudaMemset(p->d_bad, 0, 2 * sizeof(int)));
     CK(cudaMalloc(&p->d_legal, 18 * sizeof(int32_t)));
     CK(cudaMemcpy(p->d_legal, p->info->legal, 18 * sizeof(int32_t), cudaMemcpyHostToDevice));
     int r = upload_cfg(p);
@@ -284,12 +290,17 @@ int tbx_step_inputs(tbx_pool *p, const uint8_t *inputs, int auto_reset, int32_t 
 int tbx_check(tbx_pool *p, void *stream) {
   if (!p) return set_err(TBX_EINVAL, "pool is NULL");
   CK(cudaSetDevice(p->device));
-  int bad = 0;
-  CK(cudaMemcpyAsync(&bad, p->d_bad, sizeof bad, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+  int bad[2] = {0, 0};
+  CK(cudaMemcpyAsync(bad, p->d_bad, sizeof bad, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
   CK(cudaStreamSynchronize((cudaStream_t)stream));
-  if (bad) {
+  if (bad[0]) {
     CK(cudaMemsetAsync(p->d_bad, 0, sizeof(int), (cudaStream_t)stream));
-    return set_err(TBX_EACTION, "Expected to apply action, but failed: " + std::to_string(bad) + " invalid ALE action id(s)");
+    return set_err(TBX_EACTION, "Expected to apply action, but failed: " + std::to_string(bad[0]) + " invalid ALE action id(s)");
+  }
+  if (bad[1]) {
+    CK(cudaMemsetAsync(p->d_bad + 1, 0, sizeof(int), (cudaStream_t)stream));
+    return set_err(TBX_EINVAL, "state snapshot: " + std::to_string(bad[1]) + " entr" + (bad[1] == 1 ? "y" : "ies") +
+                                   " skipped (env id, column or table index out of range)");
   }
   return TBX_OK;
 }
@@ -967,6 +978,164 @@ int tbx_query_json(tbx_pool *p, int env, const char *query, const char *args_jso
     *out = dup_str(tbxjson::dump(res));
   } catch (const std::exception &e) { return set_err(TBX_EJSON, e.what()); }
   return *out ? TBX_OK : set_err(TBX_ENOMEM, "out of host memory");
+}
+
+} /* extern "C" */
+
+/* ---- device-resident state snapshots (tbx_snapshot.cuh) */
+static const int TBX_WRAP_WORDS = 5; /* the wrapper words of tbx_wrap.cuh */
+static size_t table_bytes(const tbx_pool *p) { return p->game == TBX_BREAKOUT ? sizeof(BrkTable) : p->game == TBX_AMIDAR ? sizeof(AmiTable) : 0; }
+static int table_count(const tbx_pool *p) {
+  return p->game == TBX_BREAKOUT ? (int)p->brk_tables.size() : p->game == TBX_AMIDAR ? (int)p->ami_tables.size() : 0;
+}
+static const void *table_data(const tbx_pool *p) {
+  return p->game == TBX_BREAKOUT ? (const void *)p->brk_tables.data() : p->game == TBX_AMIDAR ? (const void *)p->ami_tables.data() : 0;
+}
+
+static int state_tables(const tbx_pool *p, int rows, void *out, size_t cap, size_t *size) {
+  const tbx_state_blob_header h = {TBX_STATE_MAGIC, TBX_STATE_FORMAT, (uint32_t)p->game, (uint32_t)rows, (uint32_t)table_bytes(p),
+                                   (uint32_t)table_count(p)};
+  const size_t need = sizeof h + (size_t)h.table_bytes * h.table_count;
+  *size = need;
+  if (!out) return TBX_OK;
+  if (cap < need) return set_err(TBX_EINVAL, "the tables blob needs " + std::to_string(need) + " bytes, the buffer holds " + std::to_string(cap));
+  memcpy(out, &h, sizeof h);
+  if (need > sizeof h) memcpy((char *)out + sizeof h, table_data(p), need - sizeof h);
+  return TBX_OK;
+}
+
+/* the pool side of a copy: planes, then (wrapped env) the wrapper words */
+static SnapSide pool_side(const tbx_pool *p, uint32_t *wstate, const int32_t *ids) {
+  SnapSide s;
+  s.base0 = p->planes; s.split = p->info->rec_words; s.stride = (size_t)p->n_pad;
+  s.base1 = wstate ? wstate : p->planes + (size_t)s.split * p->n_pad;
+  s.idx = ids; s.lim = p->n;
+  return s;
+}
+static SnapSide snap_side(uint32_t *snap, int k, int rows, const int32_t *cols) {
+  SnapSide s;
+  s.base0 = snap; s.split = rows; s.stride = (size_t)k; s.base1 = snap + (size_t)rows * k;
+  s.idx = cols; s.lim = k;
+  return s;
+}
+static int launch_snap_copy(const SnapArgs &a, cudaStream_t s) {
+  if (a.owner) {
+    snap_owner_kernel<<<blocks(a.k, TBX_SNAP_THREADS), TBX_SNAP_THREADS, 0, s>>>(a);
+    CK(cudaGetLastError());
+  }
+  snap_copy_kernel<<<dim3(blocks(a.k, TBX_SNAP_THREADS), blocks(a.rows, TBX_SNAP_ROWS)), TBX_SNAP_THREADS, 0, s>>>(a);
+  CK(cudaGetLastError());
+  return TBX_OK;
+}
+
+static int state_save(tbx_pool *p, uint32_t *wstate, const int32_t *ids, int k, uint32_t *snap, cudaStream_t s) {
+  if (!snap || k < 0) return set_err(TBX_EINVAL, "snap is NULL or k < 0");
+  if (!ids && k > p->n) return set_err(TBX_EINVAL, "without env ids, k must not exceed the pool's env count");
+  if (k == 0) return TBX_OK;
+  CK(cudaSetDevice(p->device));
+  SnapArgs a;
+  a.rows = p->info->rec_words + (wstate ? TBX_WRAP_WORDS : 0);
+  a.src = pool_side(p, wstate, ids); a.dst = snap_side(snap, k, a.rows, 0);
+  a.k = k; a.tbl_row = -1; a.tbl_lim = -1; a.remap = 0; a.owner = 0; a.bad = p->d_bad + 1;
+  return launch_snap_copy(a, s);
+}
+
+/* The tables a snapshot was saved with.  Byte-identical to the pool's first `count` tables (the pool's own snapshots, and
+ * those of pools with the same config): *remap = NULL and tbl is copied as is, a host-only check.  Otherwise every blob table
+ * is interned into this pool (delta_ok recomputed for this pool's config first, as tbx_state_from_json does) and *remap maps
+ * blob indices to pool indices; that path synchronises the device. */
+static int snapshot_remap(tbx_pool *p, const uint8_t *tabs, int count, const int32_t **remap) {
+  *remap = 0;
+  const size_t tb = table_bytes(p);
+  if (count == 0 || (count <= table_count(p) && memcmp(tabs, table_data(p), (size_t)count * tb) == 0)) return TBX_OK;
+  std::vector<int32_t> map(count);
+  bool identity = true;
+  for (int i = 0; i < count; i++) {
+    if (p->game == TBX_BREAKOUT) {
+      BrkTable t;
+      memcpy(&t, tabs + (size_t)i * tb, tb);
+      tbx::brk_mark_delta_ok(p->cfg, t);
+      map[i] = intern(p->brk_tables, t);
+    } else {
+      AmiTable t;
+      memcpy(&t, tabs + (size_t)i * tb, tb);
+      map[i] = intern(p->ami_tables, t);
+    }
+    identity = identity && map[i] == i;
+  }
+  int r = upload_tables(p);
+  if (r) return r;
+  if (identity) return TBX_OK;
+  CK(cudaDeviceSynchronize()); /* an earlier load may still read the remap buffer */
+  if (p->remap_cap < count) {
+    cudaFree(p->d_remap); p->d_remap = 0; p->remap_cap = 0;
+    CK(cudaMalloc(&p->d_remap, (size_t)count * sizeof(int32_t)));
+    p->remap_cap = count;
+  }
+  CK(cudaMemcpy(p->d_remap, map.data(), (size_t)count * sizeof(int32_t), cudaMemcpyHostToDevice));
+  *remap = p->d_remap;
+  return TBX_OK;
+}
+
+static int state_load(tbx_pool *p, uint32_t *wstate, const uint32_t *snap, int k_snap, const int32_t *cols, const int32_t *ids, int n, const void *blob,
+                      size_t blob_bytes, cudaStream_t s) {
+  const int rows = p->info->rec_words + (wstate ? TBX_WRAP_WORDS : 0);
+  if (k_snap < 0 || n < 0 || (n > 0 && !snap)) return set_err(TBX_EINVAL, "snap is NULL, or k_snap / n < 0");
+  tbx_state_blob_header h;
+  if (!blob || blob_bytes < sizeof h) return set_err(TBX_EINVAL, "state snapshot: the tables blob is missing or truncated");
+  memcpy(&h, blob, sizeof h);
+  if (h.magic != TBX_STATE_MAGIC) return set_err(TBX_EINVAL, "state snapshot: not a tables blob (bad magic)");
+  if (h.format != TBX_STATE_FORMAT)
+    return set_err(TBX_EINVAL, "state snapshot: format " + std::to_string(h.format) + ", this library reads format " + std::to_string(TBX_STATE_FORMAT));
+  if (h.game != (uint32_t)p->game) return set_err(TBX_EINVAL, std::string("state snapshot: saved from another game, this pool runs ") + p->info->name);
+  if (h.rows != (uint32_t)rows)
+    return set_err(TBX_EINVAL, "state snapshot: " + std::to_string(h.rows) + " rows per env, this " + (wstate ? "wrapped env" : "pool") + " needs " + std::to_string(rows));
+  if (h.table_bytes != table_bytes(p) || h.table_count > (1u << 20) || blob_bytes != sizeof h + (size_t)h.table_bytes * h.table_count)
+    return set_err(TBX_EINVAL, "state snapshot: the tables blob's size does not match its header");
+  if (n == 0) return TBX_OK;
+  CK(cudaSetDevice(p->device));
+  const int32_t *remap = 0;
+  int r = snapshot_remap(p, (const uint8_t *)blob + sizeof h, (int)h.table_count, &remap);
+  if (r) return r;
+  if (ids && !p->d_owner) CK(cudaMalloc(&p->d_owner, (size_t)p->n_pad * sizeof(int32_t)));
+  SnapArgs a;
+  a.rows = rows;
+  a.src = snap_side(const_cast<uint32_t *>(snap), k_snap, rows, cols); a.dst = pool_side(p, wstate, ids);
+  a.k = n; a.tbl_row = p->game == TBX_SPACE_INVADERS ? -1 : TBX_HW(tbl); a.tbl_lim = (int)h.table_count; a.remap = remap;
+  a.owner = ids ? p->d_owner : 0; a.bad = p->d_bad + 1;
+  if (a.owner) CK(cudaMemsetAsync(p->d_owner, 0xff, (size_t)p->n_pad * sizeof(int32_t), s)); /* -1: no entry yet */
+  return launch_snap_copy(a, s);
+}
+
+extern "C" {
+
+int tbx_state_rows(const tbx_pool *p) { return p ? p->info->rec_words : 0; }
+int tbx_wrap_state_rows(const tbx_wrap *w) { return w ? w->pool->info->rec_words + TBX_WRAP_WORDS : 0; }
+int tbx_state_tables(const tbx_pool *p, void *out_host, size_t cap, size_t *size) {
+  if (!p || !size) return set_err(TBX_EINVAL, "pool/size is NULL");
+  return state_tables(p, p->info->rec_words, out_host, cap, size);
+}
+int tbx_wrap_state_tables(const tbx_wrap *w, void *out_host, size_t cap, size_t *size) {
+  if (!w || !size) return set_err(TBX_EINVAL, "wrap/size is NULL");
+  return state_tables(w->pool, w->pool->info->rec_words + TBX_WRAP_WORDS, out_host, cap, size);
+}
+int tbx_state_save(tbx_pool *p, const int32_t *ids_dev, int k, uint32_t *snap_dev, void *stream) {
+  if (!p) return set_err(TBX_EINVAL, "pool is NULL");
+  return state_save(p, 0, ids_dev, k, snap_dev, (cudaStream_t)stream);
+}
+int tbx_wrap_state_save(tbx_wrap *w, const int32_t *ids_dev, int k, uint32_t *snap_dev, void *stream) {
+  if (!w) return set_err(TBX_EINVAL, "wrap is NULL");
+  return state_save(w->pool, w->wstate, ids_dev, k, snap_dev, (cudaStream_t)stream);
+}
+int tbx_state_load(tbx_pool *p, const uint32_t *snap_dev, int k_snap, const int32_t *cols_dev, const int32_t *ids_dev, int n, const void *tables_blob,
+                   size_t blob_bytes, void *stream) {
+  if (!p) return set_err(TBX_EINVAL, "pool is NULL");
+  return state_load(p, 0, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream);
+}
+int tbx_wrap_state_load(tbx_wrap *w, const uint32_t *snap_dev, int k_snap, const int32_t *cols_dev, const int32_t *ids_dev, int n, const void *tables_blob,
+                        size_t blob_bytes, void *stream) {
+  if (!w) return set_err(TBX_EINVAL, "wrap is NULL");
+  return state_load(w->pool, w->wstate, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream);
 }
 
 } /* extern "C" */

@@ -9,6 +9,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from . import snapshot as _snap
 
 GAMES = ("breakout", "amidar", "space_invaders")
 OBS_MODES = {"rgba": 0, "rgb": 1, "gray": 2, "gray_area": 3}
@@ -288,6 +289,32 @@ class BatchedToybox:
             if m.numel() != self.n_envs:
                 raise ValueError("expected a mask of %d entries" % self.n_envs)
         _lib.check(self.L.tbx_field_set(self._h, path.encode(), _ptr(v), _ptr(m), _stream(self.device)))
+
+    # ------------------------------------------------------------------ state snapshots (no JSON, no host synchronisation)
+    def save_state(self, env_ids=None):
+        """A StateSnapshot of the listed envs (all by default; ids may repeat): column j holds env env_ids[j].  Enqueued on the
+        current stream.  Ids: a host sequence (checked here) or an int32 device tensor (checked on the device, see check())."""
+        ids = _snap.id_tensor(env_ids, self.n_envs, self.device, "env id")
+        k = self.n_envs if ids is None else ids.numel()
+        data = torch.empty((self.L.tbx_state_rows(self._h), k), dtype=torch.int32, device=self.device)
+        _lib.check(self.L.tbx_state_save(self._h, _ptr(ids), k, _ptr(data), _stream(self.device)))
+        return _snap.StateSnapshot(data, _snap.tables_blob(self.L.tbx_state_tables, self._h))
+
+    def load_state(self, snap, env_ids=None, columns=None):
+        """Env env_ids[j] <- column columns[j] of `snap` (defaults: envs 0.., columns 0..); a loaded env continues exactly as the
+        saved one would have.  An env listed twice receives the last listed column.  Snapshots of another pool, config or
+        GPU of the same game load too (a snapshot on another device is copied here first)."""
+        if getattr(snap, "wrapped", False):
+            raise ValueError("this snapshot holds wrapper state: load it into a DeepmindToybox")
+        data, ids, cols, n = _snap.load_args(snap, self.device, self.n_envs, env_ids, columns)
+        _lib.check(self.L.tbx_state_load(self._h, _ptr(data), data.shape[1], _ptr(cols), _ptr(ids), n, snap.tables, len(snap.tables),
+                                         _stream(self.device)))
+
+    def fork(self, src_ids, dst_ids=None):
+        """Copy the state of env src_ids[j] into env dst_ids[j] (every env by default); one source may feed every destination."""
+        snap = self.save_state(src_ids)
+        dst = _snap.id_tensor(dst_ids, self.n_envs, self.device, "env id")
+        self.load_state(snap, dst, _snap.fork_columns(snap.k, self.n_envs if dst is None else dst.numel(), self.device))
 
     # ------------------------------------------------------------------ JSON (interventions)
     def to_state_json_text(self, env_ids=None):

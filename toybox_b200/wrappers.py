@@ -18,6 +18,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from . import snapshot as _snap
 from .pool import BatchedToybox, _ptr, _stream
 
 
@@ -97,6 +98,54 @@ class DeepmindToybox:
 
     def check(self):
         self.pool.check()
+
+    # ------------------------------------------------------------------ state snapshots
+    def save_state(self, env_ids=None):
+        """A StateSnapshot of the listed wrapped envs: records, wrapper state (EpisodicLife, no-op reset counter, Monitor
+        accumulators) and observation rings.  Ids as BatchedToybox.save_state."""
+        ids = _snap.id_tensor(env_ids, self.n_envs, self.device, "env id")
+        k = self.n_envs if ids is None else ids.numel()
+        data = torch.empty((self.L.tbx_wrap_state_rows(self._w), k), dtype=torch.int32, device=self.device)
+        _lib.check(self.L.tbx_wrap_state_save(self._w, _ptr(ids), k, _ptr(data), _stream(self.device)))
+        # device ids are checked by the kernel; clamped here only so that the gather cannot fault (skipped entries are reported)
+        obs = self.obs.clone() if ids is None else self.obs.index_select(0, ids.long().clamp(0, self.n_envs - 1))
+        return _snap.StateSnapshot(data, _snap.tables_blob(self.L.tbx_wrap_state_tables, self._w), wrapped=True, obs=obs, slot=self.slot)
+
+    def load_state(self, snap, env_ids=None, columns=None):
+        """Env env_ids[j] <- column columns[j] of a wrapped snapshot, as BatchedToybox.load_state.  Ring rows are rotated so that
+        the saved newest frame lands on self.slot: stacked() then equals its value at the moment of the save.  Synchronises
+        (the ring copy selects the entries the kernel applied)."""
+        if not getattr(snap, "wrapped", False) or tuple(snap.obs.shape[1:]) != tuple(self.obs.shape[1:]):
+            raise ValueError("expected a snapshot of wrapped envs with %d x %d x %d observation rings" % (self.k, self.out_h, self.out_w))
+        data, ids, cols, n = _snap.load_args(snap, self.device, self.n_envs, env_ids, columns)
+        _lib.check(self.L.tbx_wrap_state_load(self._w, _ptr(data), data.shape[1], _ptr(cols), _ptr(ids), n, snap.tables, len(snap.tables),
+                                              _stream(self.device)))
+        obs = snap.obs if snap.obs.device == self.device else snap.obs.to(self.device)
+        shift = (self.slot - snap.slot) % self.k
+        if shift:
+            obs = torch.roll(obs, shifts=shift, dims=1)
+        if ids is None and cols is None:      # env j <- column j: every entry applies unless check() reports skipped ones
+            self.obs[:n].copy_(obs[:n])
+            return
+        # the entries the kernel applied: in range, table index below the blob's count, and the last one for each env
+        dev, k = self.device, snap.k
+        ids = torch.arange(n, device=dev) if ids is None else ids.long()
+        cols = torch.arange(n, device=dev) if cols is None else cols.long()
+        valid = (ids >= 0) & (ids < self.n_envs) & (cols >= 0) & (cols < k)
+        if snap.game != "space_invaders":
+            tbl = data[_snap.TBL_WORD].long().index_select(0, cols.clamp(0, k - 1))
+            valid &= (tbl >= 0) & (tbl < snap.table_count)
+        order = torch.arange(n, device=dev)
+        tgt = torch.where(valid, ids, self.n_envs)
+        last = torch.full((self.n_envs + 1,), -1, dtype=torch.long, device=dev).scatter_reduce_(0, tgt, order, reduce="amax")
+        sel = (valid & (last.index_select(0, tgt) == order)).nonzero().squeeze(1)
+        self.obs.index_copy_(0, ids.index_select(0, sel), obs.index_select(0, cols.index_select(0, sel)))
+
+    def fork(self, src_ids, dst_ids=None):
+        """BatchedToybox.fork for wrapped envs, observation rings included."""
+        snap = self.save_state(src_ids)
+        dst = _snap.id_tensor(dst_ids, self.n_envs, self.device, "env id")
+        self.load_state(snap, dst, _snap.fork_columns(snap.k, self.n_envs if dst is None else dst.numel(), self.device))
 
     def order(self):
         """ring slots, oldest observation first"""
