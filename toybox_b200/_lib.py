@@ -56,6 +56,62 @@ def build(force=False, verbose=False):
     return _SO
 
 
+# restype and argtypes of every symbol include/toybox_b200.h declares
+vp, i32, u64, sz, cp = C.c_void_p, C.c_int, C.c_uint64, C.c_size_t, C.c_char_p
+SIGNATURES = {
+    "tbx_last_error": (cp, []),
+    "tbx_version": (i32, []),
+    "tbx_pool_create": (i32, [cp, i32, i32, cp, C.POINTER(vp)]),
+    "tbx_pool_destroy": (i32, [vp]),
+    "tbx_frame_width": (i32, [vp]),
+    "tbx_frame_height": (i32, [vp]),
+    "tbx_n_envs": (i32, [vp]),
+    "tbx_device": (i32, [vp]),
+    "tbx_legal_actions": (i32, [vp, vp, i32]),
+    "tbx_obs_bytes": (sz, [vp, i32, i32, i32]),
+    "tbx_seed": (i32, [vp, vp, vp, i32]),
+    "tbx_new_game": (i32, [vp, vp, vp]),
+    "tbx_step": (i32, [vp, vp, i32, vp, vp, vp, vp, vp]),
+    "tbx_step_inputs": (i32, [vp, vp, i32, vp, vp, vp, vp, vp]),
+    "tbx_step_random": (i32, [vp, u64, u64, u64, i32, vp, vp, vp, vp, vp]),
+    "tbx_check": (i32, [vp, vp]),
+    "tbx_render": (i32, [vp, vp, i32, i32, i32, vp]),
+    "tbx_read_scalars": (i32, [vp, vp, vp, vp, vp]),
+    "tbx_step_host": (i32, [vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp]),
+    "tbx_state_to_json": (i32, [vp, vp, i32, C.POINTER(vp)]),
+    "tbx_state_from_json": (i32, [vp, vp, i32, C.POINTER(cp)]),
+    "tbx_config_to_json": (i32, [vp, C.POINTER(vp)]),
+    "tbx_config_from_json": (i32, [vp, cp]),
+    "tbx_schema_for_state": (i32, [cp, C.POINTER(vp)]),
+    "tbx_schema_for_config": (i32, [cp, C.POINTER(vp)]),
+    "tbx_query_json": (i32, [vp, i32, cp, cp, C.POINTER(vp)]),
+    "tbx_free_str": (None, [vp]),
+    "tbx_stats_read": (i32, [vp, vp, i32, vp]),
+    "tbx_stats_read_device": (i32, [vp, vp, vp]),
+    "tbx_breakout_columns": (i32, [vp, i32, i32, vp, vp, vp]),
+    "tbx_fill_actions": (i32, [vp, vp, u64, u64, u64, vp]),
+    "tbx_fill_actions_at": (i32, [vp, vp, u64, u64, vp, vp]),
+    "tbx_fill_actions_policy": (i32, [vp, vp, i32, u64, vp]),
+    "tbx_field_lookup": (i32, [cp, cp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)]),
+    "tbx_field_get": (i32, [vp, cp, vp, vp]),
+    "tbx_field_set": (i32, [vp, cp, vp, vp, vp]),
+    "tbx_wrap_create": (i32, [vp, i32, i32, i32, i32, i32, i32, i32, i32, u64, u64, C.POINTER(vp)]),
+    "tbx_wrap_destroy": (i32, [vp]),
+    "tbx_wrap_set_stack_mode": (i32, [vp, i32]),
+    "tbx_wrap_set_episode_outputs": (i32, [vp, vp, vp]),
+    "tbx_wrap_step": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(i32), vp]),
+    "tbx_state_rows": (i32, [vp]),
+    "tbx_wrap_state_rows": (i32, [vp]),
+    "tbx_state_tables": (i32, [vp, vp, sz, C.POINTER(sz)]),
+    "tbx_wrap_state_tables": (i32, [vp, vp, sz, C.POINTER(sz)]),
+    "tbx_state_save": (i32, [vp, vp, i32, vp, vp]),
+    "tbx_wrap_state_save": (i32, [vp, vp, i32, vp, vp]),
+    "tbx_state_load": (i32, [vp, vp, i32, vp, vp, i32, vp, sz, vp]),
+    "tbx_wrap_state_load": (i32, [vp, vp, i32, vp, vp, i32, vp, sz, vp]),
+}
+EXPORTS = sorted(SIGNATURES)
+
+
 class ToyboxError(RuntimeError):
     pass
 
@@ -68,74 +124,12 @@ def lib():
         raise ToyboxError("toybox_b200: %s is missing -- run `python -c 'import __graft_entry__ as g; g.build()'` "
                           "(there is no CPU fallback)" % _SO)
     L = C.CDLL(_SO)
-    vp, i32, u64, sz, cp = C.c_void_p, C.c_int, C.c_uint64, C.c_size_t, C.c_char_p
-    sigs = {
-        "tbx_last_error": (cp, []),
-        "tbx_version": (i32, []),
-        "tbx_pool_create": (i32, [cp, i32, i32, cp, C.POINTER(vp)]),
-        "tbx_pool_destroy": (i32, [vp]),
-        "tbx_frame_width": (i32, [vp]),
-        "tbx_frame_height": (i32, [vp]),
-        "tbx_n_envs": (i32, [vp]),
-        "tbx_device": (i32, [vp]),
-        "tbx_legal_actions": (i32, [vp, vp, i32]),
-        "tbx_obs_bytes": (sz, [vp, i32, i32, i32]),
-        "tbx_seed": (i32, [vp, vp, vp, i32]),
-        "tbx_new_game": (i32, [vp, vp, vp]),
-        "tbx_step": (i32, [vp, vp, i32, vp, vp, vp, vp, vp]),
-        "tbx_step_inputs": (i32, [vp, vp, i32, vp, vp, vp, vp, vp]),
-        "tbx_step_random": (i32, [vp, u64, u64, u64, i32, vp, vp, vp, vp, vp]),
-        "tbx_check": (i32, [vp, vp]),
-        "tbx_render": (i32, [vp, vp, i32, i32, i32, vp]),
-        "tbx_read_scalars": (i32, [vp, vp, vp, vp, vp]),
-        "tbx_step_host": (i32, [vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp]),
-        "tbx_state_to_json": (i32, [vp, vp, i32, C.POINTER(vp)]),
-        "tbx_state_from_json": (i32, [vp, vp, i32, C.POINTER(cp)]),
-        "tbx_config_to_json": (i32, [vp, C.POINTER(vp)]),
-        "tbx_config_from_json": (i32, [vp, cp]),
-        "tbx_schema_for_state": (i32, [cp, C.POINTER(vp)]),
-        "tbx_schema_for_config": (i32, [cp, C.POINTER(vp)]),
-        "tbx_query_json": (i32, [vp, i32, cp, cp, C.POINTER(vp)]),
-        "tbx_free_str": (None, [vp]),
-        "tbx_stats_read": (i32, [vp, vp, i32, vp]),
-        "tbx_stats_read_device": (i32, [vp, vp, vp]),
-        "tbx_breakout_columns": (i32, [vp, i32, i32, vp, vp, vp]),
-        "tbx_fill_actions": (i32, [vp, vp, u64, u64, u64, vp]),
-        "tbx_fill_actions_at": (i32, [vp, vp, u64, u64, vp, vp]),
-        "tbx_fill_actions_policy": (i32, [vp, vp, i32, u64, vp]),
-        "tbx_field_lookup": (i32, [cp, cp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)]),
-        "tbx_field_get": (i32, [vp, cp, vp, vp]),
-        "tbx_field_set": (i32, [vp, cp, vp, vp, vp]),
-        "tbx_wrap_create": (i32, [vp, i32, i32, i32, i32, i32, i32, i32, i32, u64, u64, C.POINTER(vp)]),
-        "tbx_wrap_destroy": (i32, [vp]),
-        "tbx_wrap_set_stack_mode": (i32, [vp, i32]),
-        "tbx_wrap_set_episode_outputs": (i32, [vp, vp, vp]),
-        "tbx_wrap_step": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(i32), vp]),
-        "tbx_state_rows": (i32, [vp]),
-        "tbx_wrap_state_rows": (i32, [vp]),
-        "tbx_state_tables": (i32, [vp, vp, sz, C.POINTER(sz)]),
-        "tbx_wrap_state_tables": (i32, [vp, vp, sz, C.POINTER(sz)]),
-        "tbx_state_save": (i32, [vp, vp, i32, vp, vp]),
-        "tbx_wrap_state_save": (i32, [vp, vp, i32, vp, vp]),
-        "tbx_state_load": (i32, [vp, vp, i32, vp, vp, i32, vp, sz, vp]),
-        "tbx_wrap_state_load": (i32, [vp, vp, i32, vp, vp, i32, vp, sz, vp]),
-    }
-    for name, (res, args) in sigs.items():
+    for name, (res, args) in SIGNATURES.items():
         f = getattr(L, name)          # AttributeError here = the header and the library disagree
         f.restype = res
         f.argtypes = args
     _LIB = L
     return L
-
-
-EXPORTS = ["tbx_last_error", "tbx_version", "tbx_pool_create", "tbx_pool_destroy", "tbx_frame_width", "tbx_frame_height",
-           "tbx_n_envs", "tbx_device", "tbx_legal_actions", "tbx_obs_bytes", "tbx_seed", "tbx_new_game", "tbx_step",
-           "tbx_step_inputs", "tbx_check", "tbx_render", "tbx_read_scalars", "tbx_step_host", "tbx_state_to_json",
-           "tbx_state_from_json", "tbx_config_to_json", "tbx_config_from_json", "tbx_schema_for_state", "tbx_schema_for_config",
-           "tbx_query_json", "tbx_free_str", "tbx_stats_read", "tbx_fill_actions", "tbx_fill_actions_policy",
-           "tbx_wrap_create", "tbx_wrap_destroy", "tbx_wrap_step", "tbx_field_lookup", "tbx_field_get", "tbx_field_set", "tbx_fill_actions_at", "tbx_stats_read_device", "tbx_wrap_set_stack_mode", "tbx_wrap_set_episode_outputs", "tbx_breakout_columns", "tbx_step_random",
-           "tbx_state_rows", "tbx_wrap_state_rows", "tbx_state_tables", "tbx_wrap_state_tables", "tbx_state_save", "tbx_wrap_state_save",
-           "tbx_state_load", "tbx_wrap_state_load"]
 
 
 def check(rc):

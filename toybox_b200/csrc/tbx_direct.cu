@@ -1,4 +1,4 @@
-/* tbx_direct.cu -- host side of the direct INTER_AREA kernels (tbx_render_direct.cuh): table upload and launchers.  A
+/* tbx_direct.cu -- host side of the direct INTER_AREA kernels (tbx_render_direct.cuh): table upload and launcher.  A
  * translation unit of its own so that it compiles in parallel with, and rebuilds independently of, tbx_pool.cu. */
 #include <mutex>
 #include "tbx_render_direct.cuh"
@@ -9,63 +9,30 @@ using namespace tbxk;
 
 static int align16(int v) { return (v + 15) & ~15; }
 
-cudaError_t tbx_direct_build(const tbx::Config &c, const BrkTable *brk_default, const tbx::ResizeTab &rs, const TbxAreaPlan &plan, const uint8_t *base0_gray,
-                             void **d_aux, void **d_aux2) {
-  *d_aux = 0;
-  *d_aux2 = 0;
-  cudaError_t e = cudaSuccess;
-  if (c.game == TBX_BREAKOUT && brk_default) {
-    std::vector<TbxBrkDirect> aux(1);
-    tbx::build_brk_direct(c, *brk_default, rs, plan, base0_gray, aux[0]);
-    if (!aux[0].ok) return cudaSuccess;
-    e = cudaMalloc(d_aux, sizeof(TbxBrkDirect));
-    if (e != cudaSuccess) return e;
-    return cudaMemcpy(*d_aux, aux.data(), sizeof(TbxBrkDirect), cudaMemcpyHostToDevice);
-  }
-  if (c.game == TBX_AMIDAR) {
-    std::vector<TbxAmiDirect> aux(1);
-    tbx::build_ami_direct(c, rs, plan, aux[0]);
-    if (!aux[0].ok) return cudaSuccess;
-    e = cudaMalloc(d_aux, sizeof(TbxAmiDirect));
-    if (e != cudaSuccess) return e;
-    return cudaMemcpy(*d_aux, aux.data(), sizeof(TbxAmiDirect), cudaMemcpyHostToDevice);
-  }
-  if (c.game == TBX_SPACE_INVADERS) {
-    std::vector<TbxSiDirect> aux(1);
-    std::vector<TbxSpritePatch> patches;
-    tbx::build_si_direct(c, rs, plan, base0_gray, aux[0], patches);
-    if (!aux[0].ok) return cudaSuccess;
-    e = cudaMalloc(d_aux, sizeof(TbxSiDirect));
-    if (e != cudaSuccess) return e;
-    e = cudaMemcpy(*d_aux, aux.data(), sizeof(TbxSiDirect), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess || patches.empty()) return e;
-    e = cudaMalloc(d_aux2, patches.size() * sizeof(TbxSpritePatch));
-    if (e != cudaSuccess) return e;
-    return cudaMemcpy(*d_aux2, patches.data(), patches.size() * sizeof(TbxSpritePatch), cudaMemcpyHostToDevice);
-  }
-  return cudaSuccess;
+/* the tables a builder filled -> aux; nothing when the pair is outside its limits */
+template <class D> static cudaError_t upload_direct(const std::vector<D> &A, Buf<uint8_t> &aux) {
+  return A[0].ok ? aux.upload(reinterpret_cast<const uint8_t *>(A.data()), sizeof(D)) : cudaSuccess;
 }
 
-void tbx_direct_geometry(int game, int out_w, int out_h, int brk_rows, DirectArgs &d) {
-  d.hstride = (out_w + 3) & ~3;
-  d.smem_base = align16(out_w * out_h);
-  if (game == TBX_BREAKOUT) {
-    if (brk_rows < 1 || brk_rows > TBX_BRK_MAX_ROWS) brk_rows = TBX_BRK_MAX_ROWS;
-    /* the kernel's small tables follow the staged frame: digit patches, base-frame row classes, division table, the wall's H look-up */
-    d.smem_base += TBX_BRK_TAB_BYTES + align16(brk_rows * 4 * d.hstride * (int)sizeof(float));
-    /* per warp: its env's record, the wall's H rows, the movers' records; two record stages */
-    d.warp_bytes = align16(TBX_WORDS(BrkRec) * 4) + align16(brk_rows * d.hstride * (int)sizeof(float)) + 256;
-    d.smem_total = d.smem_base + 2 * TBX_WORDS(BrkRec) * TBX_EPC * 4 + (TBX_DIRECT_THREADS / 32) * d.warp_bytes;
-  } else if (game == TBX_AMIDAR) {
-    /* per warp: its env's record, the tile rows as looks, the movers' records; two record stages */
-    d.warp_bytes = align16(TBX_WORDS(AmiRec) * 4) + 256 + 448;
-    d.smem_total = d.smem_base + 2 * TBX_WORDS(AmiRec) * TBX_EPC * 4 + (TBX_DIRECT_THREADS / 32) * d.warp_bytes;
-  } else {
-    /* per warp: its env's record, the entries, two coverage bitmaps, the evaluated-entry list; one record stage */
-    const int ow = (out_w + 31) / 32;
-    d.warp_bytes = align16(TBX_WORDS(SiRec) * 4) + TBX_SD_MAX_ENTRIES * 32 + align16(2 * out_h * ow * 4) + TBX_SD_MAX_ENTRIES * 8;
-    d.smem_total = d.smem_base + TBX_WORDS(SiRec) * TBX_EPC * 4 + (TBX_DIRECT_THREADS / 32) * d.warp_bytes;
+cudaError_t tbx_direct_build(const tbx::Config &c, const BrkTable *brk_default, const tbx::ResizeTab &rs, const TbxAreaPlan &plan, const uint8_t *base0_gray,
+                             Buf<uint8_t> &aux, Buf<uint8_t> &aux2) {
+  if (c.game == TBX_BREAKOUT) {
+    if (!brk_default) return cudaSuccess;
+    std::vector<TbxBrkDirect> A(1);
+    tbx::build_brk_direct(c, *brk_default, rs, plan, base0_gray, A[0]);
+    return upload_direct(A, aux);
   }
+  if (c.game == TBX_AMIDAR) {
+    std::vector<TbxAmiDirect> A(1);
+    tbx::build_ami_direct(c, rs, plan, A[0]);
+    return upload_direct(A, aux);
+  }
+  std::vector<TbxSiDirect> A(1);
+  std::vector<TbxSpritePatch> patches;
+  tbx::build_si_direct(c, rs, plan, base0_gray, A[0], patches);
+  const cudaError_t e = upload_direct(A, aux);
+  if (e != cudaSuccess || !aux || patches.empty()) return e;
+  return aux2.upload(reinterpret_cast<const uint8_t *>(patches.data()), patches.size() * sizeof(TbxSpritePatch));
 }
 
 /* persistent grid: as many CTAs as the device keeps resident, each walks its share of the chunks.  The residency is cached per
@@ -98,64 +65,52 @@ template <class K> static cudaError_t persistent_grid(K kernel, int smem, int n_
   return cudaSuccess;
 }
 
-template <int TX, int TY> static cudaError_t launch_brk(const RenderArgs &a, const BrkCfg &cfg, const TbxAreaPlan &plan, const DirectArgs &d, cudaStream_t s) {
-  /* the attribute is per device: set it on every launch (a cheap host-side call) rather than caching it per process */
-  const int smem = d.smem_total + brk_plan_smem_bytes(TX, TY, plan.dw, plan.dh); /* the plan's per-pixel tables go behind the rest */
-  cudaError_t e = cudaFuncSetAttribute(brk_direct_kernel<TX, TY>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+/* the attribute is per device: set it on every launch (a cheap host-side call) rather than caching it per process */
+template <class... P, class... A> static cudaError_t launch_persistent(void (*kernel)(P...), int smem, int n, cudaStream_t s, const A &...args) {
+  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return e;
   int grid = 1;
-  e = persistent_grid(brk_direct_kernel<TX, TY>, smem, (a.n + TBX_EPC - 1) / TBX_EPC, &grid);
+  e = persistent_grid(kernel, smem, (n + TBX_EPC - 1) / TBX_EPC, &grid);
   if (e != cudaSuccess) return e;
-  brk_direct_kernel<TX, TY><<<grid, TBX_DIRECT_THREADS, smem, s>>>(a, cfg, plan, d);
-  return cudaGetLastError();
-}
-template <int TX, int TY> static cudaError_t launch_si(const RenderArgs &a, const TbxAreaPlan &plan, const DirectArgs &d, cudaStream_t s) {
-  const int smem = d.smem_total + si_tab_smem_bytes(plan.dw, plan.dh); /* the plain-background map and the division table go behind the rest */
-  cudaError_t e = cudaFuncSetAttribute(si_direct_kernel<TX, TY>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e != cudaSuccess) return e;
-  int grid = 1;
-  e = persistent_grid(si_direct_kernel<TX, TY>, smem, (a.n + TBX_EPC - 1) / TBX_EPC, &grid);
-  if (e != cudaSuccess) return e;
-  si_direct_kernel<TX, TY><<<grid, TBX_DIRECT_THREADS, smem, s>>>(a, plan, d);
+  kernel<<<grid, TBX_DIRECT_THREADS, smem, s>>>(args...);
   return cudaGetLastError();
 }
 
-template <int TX, int TY> static cudaError_t launch_ami(const RenderArgs &a, const TbxAreaPlan &plan, const DirectArgs &d, cudaStream_t s) {
-  const int smem = d.smem_total + ami_tab_smem_bytes(plan.dh); /* three small per-pixel tables go behind the rest */
-  cudaError_t e = cudaFuncSetAttribute(ami_direct_kernel<TX, TY>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e != cudaSuccess) return e;
-  int grid = 1;
-  e = persistent_grid(ami_direct_kernel<TX, TY>, smem, (a.n + TBX_EPC - 1) / TBX_EPC, &grid);
-  if (e != cudaSuccess) return e;
-  ami_direct_kernel<TX, TY><<<grid, TBX_DIRECT_THREADS, smem, s>>>(a, plan, d);
-  return cudaGetLastError();
-}
-
-cudaError_t tbx_launch_direct(int game, int tx, int ty, const RenderArgs &a, const void *cfg_host, const TbxAreaPlan &plan, const DirectArgs &d, cudaStream_t s) {
-  if (game == TBX_AMIDAR) { /* the tables are built for tx <= 4 only */
-    if (ty <= 3) return tx <= 3 ? launch_ami<3, 3>(a, plan, d, s) : launch_ami<4, 3>(a, plan, d, s);
-    return tx <= 3 ? launch_ami<3, 4>(a, plan, d, s) : launch_ami<4, 4>(a, plan, d, s);
-  }
-  if (game == TBX_SPACE_INVADERS) {
-    if (ty <= 3) {
-      if (tx <= 3) return launch_si<3, 3>(a, plan, d, s);
-      if (tx <= 4) return launch_si<4, 3>(a, plan, d, s);
-      return launch_si<5, 3>(a, plan, d, s);
+cudaError_t tbx_launch_direct(const tbx::Config &c, const RenderArgs &a, const TbxAreaPlan &plan, DirectArgs d, cudaStream_t s) {
+  const int out_w = plan.dw, out_h = plan.dh;
+  d.hstride = (out_w + 3) & ~3;
+  d.smem_base = align16(out_w * out_h);
+  return with_game(c.game, [&](auto g) {
+    constexpr int G = decltype(g)::value, RW = Traits<G>::RW;
+    if constexpr (G == TBX_BREAKOUT) {
+      const int brk_rows = c.brk.n_rows < 1 || c.brk.n_rows > TBX_BRK_MAX_ROWS ? TBX_BRK_MAX_ROWS : c.brk.n_rows;
+      /* the kernel's small tables follow the staged frame: digit patches, base-frame row classes, division table, the wall's H look-up */
+      d.smem_base += TBX_BRK_TAB_BYTES + align16(brk_rows * 4 * d.hstride * (int)sizeof(float));
+      /* per warp: its env's record, the wall's H rows, the movers' records; two record stages */
+      d.warp_bytes = align16(RW * 4) + align16(brk_rows * d.hstride * (int)sizeof(float)) + 256;
+      d.smem_total = d.smem_base + 2 * RW * TBX_EPC * 4 + (TBX_DIRECT_THREADS / 32) * d.warp_bytes;
+      return with_taps<5>(plan.tx, plan.ty, [&](auto X, auto Y) {
+        constexpr int TX = decltype(X)::value, TY = decltype(Y)::value;
+        /* the plan's per-pixel tables go behind the rest */
+        return launch_persistent(brk_direct_kernel<TX, TY>, d.smem_total + brk_plan_smem_bytes(TX, TY, out_w, out_h), a.n, s, a, c.brk, plan, d);
+      });
+    } else if constexpr (G == TBX_AMIDAR) {
+      /* per warp: its env's record, the tile rows as looks, the movers' records; two record stages */
+      d.warp_bytes = align16(RW * 4) + 256 + 448;
+      d.smem_total = d.smem_base + 2 * RW * TBX_EPC * 4 + (TBX_DIRECT_THREADS / 32) * d.warp_bytes;
+      return with_taps<4>(plan.tx, plan.ty, [&](auto X, auto Y) { /* three small per-pixel tables go behind the rest */
+        return launch_persistent(ami_direct_kernel<decltype(X)::value, decltype(Y)::value>, d.smem_total + ami_tab_smem_bytes(out_h), a.n, s, a, plan, d);
+      });
+    } else {
+      /* per warp: its env's record, the entries, two coverage bitmaps, the evaluated-entry list; one record stage */
+      const int ow = (out_w + 31) / 32;
+      d.warp_bytes = align16(RW * 4) + TBX_SD_MAX_ENTRIES * 32 + align16(2 * out_h * ow * 4) + TBX_SD_MAX_ENTRIES * 8;
+      d.smem_total = d.smem_base + RW * TBX_EPC * 4 + (TBX_DIRECT_THREADS / 32) * d.warp_bytes;
+      return with_taps<5>(plan.tx, plan.ty, [&](auto X, auto Y) { /* the plain-background map and the division table go behind the rest */
+        return launch_persistent(si_direct_kernel<decltype(X)::value, decltype(Y)::value>, d.smem_total + si_tab_smem_bytes(out_w, out_h), a.n, s, a, plan, d);
+      });
     }
-    if (tx <= 3) return launch_si<3, 4>(a, plan, d, s);
-    if (tx <= 4) return launch_si<4, 4>(a, plan, d, s);
-    return launch_si<5, 4>(a, plan, d, s);
-  }
-  if (game != TBX_BREAKOUT) return cudaErrorInvalidValue;
-  const BrkCfg &cfg = *(const BrkCfg *)cfg_host;
-  if (ty <= 3) {
-    if (tx <= 3) return launch_brk<3, 3>(a, cfg, plan, d, s);
-    if (tx <= 4) return launch_brk<4, 3>(a, cfg, plan, d, s);
-    return launch_brk<5, 3>(a, cfg, plan, d, s);
-  }
-  if (tx <= 3) return launch_brk<3, 4>(a, cfg, plan, d, s);
-  if (tx <= 4) return launch_brk<4, 4>(a, cfg, plan, d, s);
-  return launch_brk<5, 4>(a, cfg, plan, d, s);
+  });
 }
 
 #ifdef TBX_SI_STATS

@@ -6,11 +6,13 @@
 #include "tbx_fields.h"
 #include "tbx_direct_launch.h"
 #include <map>
+#include <memory>
 #include <new>
 #include <string>
 #include <string.h>
 #include <algorithm>
 #include <thread>
+#include <tuple>
 #include <vector>
 
 using namespace tbxk;
@@ -24,43 +26,90 @@ static int set_err(int code, const std::string &msg) { g_err = msg; return code;
     if (e_ != cudaSuccess) return set_err(TBX_ECUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); \
   } while (0)
 
+/* f() with every exception turned into an error code: nothing may unwind through the C ABI into the caller */
+template <class F> static int guarded(F &&f) {
+  try {
+    return f();
+  } catch (const std::bad_alloc &) {
+    return set_err(TBX_ENOMEM, "out of host memory");
+  } catch (const std::exception &e) {
+    return set_err(TBX_EJSON, e.what());
+  }
+}
+
+/* render resources of one INTER_AREA output size */
 struct AreaRes {
-  TbxAreaPlan *d_plan; TbxAreaPlan plan; uint8_t *d_base_out[2]; TbxDigitPatch *d_patches[2]; int dw, dh, tx, ty;
-  void *d_direct, *d_direct2; int direct_ok; /* tables of the direct kernel (tbx_direct.h), NULL / 0 when the pair is not covered */
+  TbxAreaPlan plan;
+  Buf<TbxAreaPlan> d_plan;
+  Buf<uint8_t> d_base_out[2];       /* down-samples of base frames 0/1 */
+  Buf<TbxDigitPatch> d_patches[2];
+  Buf<uint8_t> d_direct, d_direct2; /* tables of the direct kernel (tbx_direct.h), empty when the pair is not covered */
 };
-static void drop_render_cache(struct tbx_pool *p);
+/* base frames 0/1 of the current config (see tbx_render.cuh): gray, RGBA and packed RGB on the device, gray on the host */
+struct BaseFrames {
+  Buf<uint8_t> gray[2], rgba[2], rgb[2];
+  std::vector<uint8_t> h_gray[2];
+};
+/* tbx_step_host's stream and staging */
+struct HostStaging {
+  cudaStream_t s = 0;
+  Buf<int32_t> actions, reward, score, lives;
+  Buf<uint8_t> done, obs;
+  ~HostStaging() { if (s) cudaStreamDestroy(s); }
+};
+
+/* a pool's interned geometry tables, per game: std::get<GAME>(tbx_pool::tabs); Space Invaders has none */
+template <int G> using Tables = std::vector<typename Traits<G>::Table>;
+template <int G> static constexpr bool kTables = G != TBX_SPACE_INVADERS;
+static_assert(TBX_BREAKOUT == 0 && TBX_AMIDAR == 1 && TBX_SPACE_INVADERS == 2, "game ids index tbx_pool::tabs");
 
 struct tbx_pool {
   int game, n, n_pad, device;
   const tbx::GameInfo *info;
   tbx::Config cfg;
-  void *d_cfg;
-  std::vector<BrkTable> brk_tables;
-  std::vector<AmiTable> ami_tables;
-  void *d_tables;
+  Buf<uint8_t> d_cfg;
+  std::tuple<Tables<TBX_BREAKOUT>, Tables<TBX_AMIDAR>, Tables<TBX_SPACE_INVADERS>> tabs;
+  Buf<uint8_t> d_tables;
   int d_tables_n;
-  uint32_t *planes;
-  unsigned long long *d_stats;
-  int *d_bad; /* [0] = invalid action ids, [1] = skipped snapshot entries, since the last tbx_check */
-  int32_t *d_legal;
-  /* render resources of the current config: static frame (gray, RGBA) and per output size the INTER_AREA plan */
-  uint8_t *d_base_gray[2], *d_base_rgba[2], *d_base_rgb[2];
-  std::vector<uint32_t> h_base_rgba[2];
-  std::vector<uint8_t> h_base_gray[2];
-  std::map<std::pair<int, int>, struct AreaRes> area;
-  int32_t *d_dense; /* [0] = count, [8..] = env ids the patch kernel left to the canvas kernel */
-  int32_t *d_fb;    /* [0] = count, [1] = finished CTAs, [8..] = env ids the direct INTER_AREA kernel left to the tile kernel */
+  Buf<uint32_t> planes;
+  Buf<unsigned long long> d_stats;
+  Buf<int> d_bad; /* [0] = invalid action ids, [1] = skipped snapshot entries, since the last tbx_check */
+  Buf<int32_t> d_legal;
+  /* render resources of the current config: base frames, and per output size the INTER_AREA plan */
+  std::unique_ptr<BaseFrames> base;
+  std::map<std::pair<int, int>, AreaRes> area;
+  Buf<int32_t> d_dense; /* [0] = count, [8..] = env ids the patch kernel left to the canvas kernel */
+  Buf<int32_t> d_fb;    /* [0] = count, [1] = finished CTAs, [8..] = env ids the direct INTER_AREA kernel left to the tile kernel */
   /* JSON import / export staging (grown on demand, kept): env ids and AoS records on the device, records in pinned host memory */
-  int32_t *j_ids; uint32_t *j_recs, *j_host; size_t j_cap_ids, j_cap_words;
-  /* tbx_step_host staging */
-  cudaStream_t hs;
-  int32_t *h_actions_dev, *h_reward_dev, *h_score_dev, *h_lives_dev;
-  uint8_t *h_done_dev, *h_obs_dev;
-  size_t h_obs_cap;
+  Buf<int32_t> j_ids;
+  Buf<uint32_t> j_recs;
+  PinnedBuf<uint32_t> j_host;
+  std::unique_ptr<HostStaging> hs;
   /* snapshot loads: owner entry per env (duplicate destinations), blob -> pool table indices (foreign tables) */
-  int32_t *d_owner, *d_remap;
-  int remap_cap;
+  Buf<int32_t> d_owner, d_remap;
 };
+
+template <int G, class P> static auto &tables(P *p) { return std::get<G>(p->tabs); }
+/* the game's part of a config */
+template <int G, class C> static auto &game_cfg(C &c) {
+  if constexpr (G == TBX_BREAKOUT) return c.brk;
+  else if constexpr (G == TBX_AMIDAR) return c.ami;
+  else return c.si;
+}
+static uint64_t *cfg_rand(tbx::Config &c) { return with_game(c.game, [&](auto g) { return game_cfg<decltype(g)::value>(c).rand; }); }
+/* Breakout's default brick table (the base frames show its bricks); NULL for the other games */
+static const BrkTable *brk_default(const tbx_pool *p) { return p->game == TBX_BREAKOUT ? &tables<TBX_BREAKOUT>(p)[p->cfg.brk.default_tbl] : 0; }
+
+/* per-game host codecs, overloaded on the game's record and table types */
+static void fit_table(const tbx::Config &c, BrkTable &t) { tbx::brk_mark_delta_ok(c, t); } /* delta_ok depends on the config */
+static void fit_table(const tbx::Config &, AmiTable &) {}
+static void default_table(const tbx::Config &c, BrkTable &t) { tbx::brk_default_table(c.brk, t); fit_table(c, t); }
+static void default_table(const tbx::Config &c, AmiTable &t) { tbx::ami_default_table(c.ami, t); }
+static Value state_to_json(const BrkRec &r, const BrkTable *t) { return tbx::brk_state_to_json(r, *t); }
+static Value state_to_json(const AmiRec &r, const AmiTable *t) { return tbx::ami_state_to_json(r, *t); }
+static Value state_to_json(const SiRec &r, const int *) { return tbx::si_state_to_json(r); }
+static void state_from_json(const Value &v, BrkRec &r, BrkTable &t) { tbx::brk_state_from_json(v, r, t); }
+static void state_from_json(const Value &v, AmiRec &r, AmiTable &t) { tbx::ami_state_from_json(v, r, t); }
 
 /* The JSON codec is host work per env (build / walk a document tree, print / parse ~20-40 KB of text): spread the envs of a
  * batched call over host threads.  f(i) may throw; the first message is re-thrown on the calling thread. */
@@ -79,32 +128,27 @@ template <class F> static void parallel_for(int n, F f) {
   for (auto &e : errs) if (!e.empty()) throw std::runtime_error(e);
 }
 
-static size_t cfg_bytes(int game) { return game == TBX_BREAKOUT ? sizeof(BrkCfg) : game == TBX_AMIDAR ? sizeof(AmiCfg) : sizeof(SiCfg); }
-static const void *cfg_ptr(const tbx_pool *p) {
-  return p->game == TBX_BREAKOUT ? (const void *)&p->cfg.brk : p->game == TBX_AMIDAR ? (const void *)&p->cfg.ami : (const void *)&p->cfg.si;
-}
 static int blocks(int n, int t) { return (n + t - 1) / t; }
 
 static int upload_cfg(tbx_pool *p) {
-  CK(cudaMemcpy(p->d_cfg, cfg_ptr(p), cfg_bytes(p->game), cudaMemcpyHostToDevice));
-  return TBX_OK;
+  return with_game(p->game, [&](auto g) -> int {
+    const auto &c = game_cfg<decltype(g)::value>(p->cfg);
+    CK(p->d_cfg.grow(sizeof c));
+    CK(cudaMemcpy(p->d_cfg, &c, sizeof c, cudaMemcpyHostToDevice));
+    return TBX_OK;
+  });
 }
 static int upload_tables(tbx_pool *p) {
-  size_t bytes = 0;
-  const void *src = 0;
-  int n = 0;
-  if (p->game == TBX_BREAKOUT) { n = (int)p->brk_tables.size(); bytes = n * sizeof(BrkTable); src = p->brk_tables.data(); }
-  else if (p->game == TBX_AMIDAR) { n = (int)p->ami_tables.size(); bytes = n * sizeof(AmiTable); src = p->ami_tables.data(); }
-  if (n == 0) return TBX_OK;
-  if (n == p->d_tables_n) return TBX_OK;
-  CK(cudaDeviceSynchronize());
-  void *d = 0;
-  CK(cudaMalloc(&d, bytes));
-  CK(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice));
-  if (p->d_tables) cudaFree(p->d_tables);
-  p->d_tables = d;
-  p->d_tables_n = n;
-  return TBX_OK;
+  return with_game(p->game, [&](auto g) -> int {
+    const auto &t = tables<decltype(g)::value>(p);
+    if (t.empty() || (int)t.size() == p->d_tables_n) return TBX_OK;
+    CK(cudaDeviceSynchronize());
+    Buf<uint8_t> d;
+    CK(d.upload(reinterpret_cast<const uint8_t *>(t.data()), t.size() * sizeof t[0]));
+    p->d_tables = std::move(d);
+    p->d_tables_n = (int)t.size();
+    return TBX_OK;
+  });
 }
 /* index of an identical table, appending it if new */
 template <class TT> static int intern(std::vector<TT> &v, const TT &t) {
@@ -113,13 +157,16 @@ template <class TT> static int intern(std::vector<TT> &v, const TT &t) {
   return (int)v.size() - 1;
 }
 static void install_default_table(tbx_pool *p) {
-  if (p->game == TBX_BREAKOUT) { BrkTable t; tbx::brk_default_table(p->cfg.brk, t); tbx::brk_mark_delta_ok(p->cfg, t); p->cfg.brk.default_tbl = intern(p->brk_tables, t); }
-  else if (p->game == TBX_AMIDAR) { AmiTable t; tbx::ami_default_table(p->cfg.ami, t); p->cfg.ami.default_tbl = intern(p->ami_tables, t); }
+  with_game(p->game, [&](auto g) {
+    constexpr int G = decltype(g)::value;
+    if constexpr (kTables<G>) {
+      typename Traits<G>::Table t;
+      default_table(p->cfg, t);
+      game_cfg<G>(p->cfg).default_tbl = intern(tables<G>(p), t);
+    }
+  });
 }
 
-template <int GAME> static void launch_new_game(tbx_pool *p, const uint8_t *mask, cudaStream_t s) {
-  new_game_kernel<GAME><<<blocks(p->n, 128), 128, 0, s>>>(p->planes, p->n, p->n_pad, p->d_cfg, p->d_tables, mask);
-}
 template <int GAME> static int launch_step(tbx_pool *p, const StepArgs &a, cudaStream_t s) {
   /* staged (records through shared memory) where it measures faster; TBX_STEP_STAGED=0/1 overrides (tuning, tests) */
   bool staged = GAME == TBX_SPACE_INVADERS; /* measured, 65,536 envs in steady state: Space Invaders 90 vs 178 us; Breakout 39 vs 37; Amidar 69 vs 61 */
@@ -135,10 +182,33 @@ template <int GAME> static int launch_step(tbx_pool *p, const StepArgs &a, cudaS
   return TBX_OK;
 }
 static int do_new_game(tbx_pool *p, const uint8_t *mask, cudaStream_t s) {
-  if (p->game == TBX_BREAKOUT) launch_new_game<TBX_BREAKOUT>(p, mask, s);
-  else if (p->game == TBX_AMIDAR) launch_new_game<TBX_AMIDAR>(p, mask, s);
-  else launch_new_game<TBX_SPACE_INVADERS>(p, mask, s);
+  with_game(p->game, [&](auto g) {
+    new_game_kernel<decltype(g)::value><<<blocks(p->n, 128), 128, 0, s>>>(p->planes, p->n, p->n_pad, p->d_cfg, p->d_tables, mask);
+  });
   CK(cudaGetLastError());
+  return TBX_OK;
+}
+
+/* device side of tbx_pool_create */
+static int init_device(tbx_pool *p) {
+  const size_t plane_words = (size_t)p->info->rec_words * p->n_pad;
+  CK(cudaSetDevice(p->device));
+  CK(p->planes.alloc(plane_words));
+  CK(cudaMemset(p->planes, 0, plane_words * sizeof(uint32_t)));
+  CK(p->d_stats.alloc(4));
+  CK(cudaMemset(p->d_stats, 0, 4 * sizeof(unsigned long long)));
+  CK(p->d_bad.alloc(2));
+  CK(cudaMemset(p->d_bad, 0, 2 * sizeof(int)));
+  CK(p->d_legal.upload(p->info->legal, 18));
+  int r = upload_cfg(p);
+  if (r) return r;
+  r = upload_tables(p);
+  if (r) return r;
+  const uint64_t *rand = cfg_rand(p->cfg);
+  set_sim_rand_kernel<<<blocks(p->n, 256), 256>>>(p->planes, p->n, p->n_pad, rand[0], rand[1]);
+  CK(cudaGetLastError());
+  for (int k = 0; k < p->info->new_games_at_ctor; k++) { r = do_new_game(p, 0, 0); if (r) return r; }
+  CK(cudaDeviceSynchronize());
   return TBX_OK;
 }
 
@@ -151,11 +221,6 @@ int tbx_pool_destroy(tbx_pool *p) {
   if (!p) return TBX_OK;
   cudaSetDevice(p->device);
   cudaDeviceSynchronize();
-  cudaFree(p->d_cfg); cudaFree(p->d_tables); cudaFree(p->planes); cudaFree(p->d_stats); cudaFree(p->d_bad); cudaFree(p->d_legal); cudaFree(p->d_dense); cudaFree(p->d_fb); cudaFree(p->j_ids); cudaFree(p->j_recs); cudaFreeHost(p->j_host);
-  cudaFree(p->d_owner); cudaFree(p->d_remap);
-  drop_render_cache(p);
-  cudaFree(p->h_actions_dev); cudaFree(p->h_reward_dev); cudaFree(p->h_score_dev); cudaFree(p->h_lives_dev); cudaFree(p->h_done_dev); cudaFree(p->h_obs_dev);
-  if (p->hs) cudaStreamDestroy(p->hs);
   delete p;
   return TBX_OK;
 }
@@ -170,44 +235,17 @@ int tbx_pool_create(const char *game, int n_envs, int device, const char *cfg_js
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
     return set_err(TBX_ECUDA, "no CUDA device available: toybox_b200 has no CPU path");
   if (device < 0 || device >= ndev) return set_err(TBX_EINVAL, "device index out of range");
-  tbx_pool *p = new (std::nothrow) tbx_pool();
-  if (!p) return set_err(TBX_ENOMEM, "out of host memory");
-  p->game = g; p->n = n_envs; p->n_pad = (n_envs + 31) & ~31; p->device = device; p->info = tbx::game_info(g);
-  p->d_cfg = p->d_tables = 0; p->d_base_gray[0] = p->d_base_gray[1] = p->d_base_rgba[0] = p->d_base_rgba[1] = p->d_base_rgb[0] = p->d_base_rgb[1] = 0; p->d_tables_n = 0; p->planes = 0; p->d_stats = 0; p->d_bad = 0; p->d_legal = 0;
-  p->hs = 0; p->d_dense = 0; p->d_fb = 0; p->j_ids = 0; p->j_recs = p->j_host = 0; p->j_cap_ids = p->j_cap_words = 0; p->h_actions_dev = p->h_reward_dev = p->h_score_dev = p->h_lives_dev = 0; p->h_done_dev = p->h_obs_dev = 0; p->h_obs_cap = 0;
-  p->d_owner = p->d_remap = 0; p->remap_cap = 0;
-  int rc = TBX_OK;
-  try {
+  return guarded([&]() -> int {
+    std::unique_ptr<tbx_pool> p(new tbx_pool());
+    p->game = g; p->n = n_envs; p->n_pad = (n_envs + 31) & ~31; p->device = device; p->info = tbx::game_info(g);
     tbx::default_config(g, p->cfg);
     if (cfg_json) tbx::config_from_json(p->cfg, tbxjson::parse(cfg_json));
-    install_default_table(p);
-  } catch (const std::exception &e) { delete p; return set_err(TBX_EJSON, e.what()); }
-  auto body = [&]() -> int {
-    CK(cudaSetDevice(device));
-    CK(cudaMalloc(&p->d_cfg, cfg_bytes(g)));
-    CK(cudaMalloc(&p->planes, (size_t)p->info->rec_words * p->n_pad * sizeof(uint32_t)));
-    CK(cudaMemset(p->planes, 0, (size_t)p->info->rec_words * p->n_pad * sizeof(uint32_t)));
-    CK(cudaMalloc(&p->d_stats, 4 * sizeof(unsigned long long)));
-    CK(cudaMemset(p->d_stats, 0, 4 * sizeof(unsigned long long)));
-    CK(cudaMalloc(&p->d_bad, 2 * sizeof(int)));
-    CK(cudaMemset(p->d_bad, 0, 2 * sizeof(int)));
-    CK(cudaMalloc(&p->d_legal, 18 * sizeof(int32_t)));
-    CK(cudaMemcpy(p->d_legal, p->info->legal, 18 * sizeof(int32_t), cudaMemcpyHostToDevice));
-    int r = upload_cfg(p);
-    if (r) return r;
-    r = upload_tables(p);
-    if (r) return r;
-    const uint64_t *rand = g == TBX_BREAKOUT ? p->cfg.brk.rand : g == TBX_AMIDAR ? p->cfg.ami.rand : p->cfg.si.rand;
-    set_sim_rand_kernel<<<blocks(p->n, 256), 256>>>(p->planes, p->n, p->n_pad, rand[0], rand[1]);
-    CK(cudaGetLastError());
-    for (int k = 0; k < p->info->new_games_at_ctor; k++) { r = do_new_game(p, 0, 0); if (r) return r; }
-    CK(cudaDeviceSynchronize());
+    install_default_table(p.get());
+    const int rc = init_device(p.get());
+    if (rc) { std::string keep = g_err; tbx_pool_destroy(p.release()); g_err = keep; return rc; }
+    *out = p.release();
     return TBX_OK;
-  };
-  rc = body();
-  if (rc) { std::string keep = g_err; tbx_pool_destroy(p); g_err = keep; return rc; }
-  *out = p;
-  return TBX_OK;
+  });
 }
 
 int tbx_frame_width(const tbx_pool *p) { return p ? p->info->width : 0; }
@@ -239,15 +277,13 @@ int tbx_seed(tbx_pool *p, const uint32_t *seeds, const int32_t *ids, int n) {
   if (n == 0) return TBX_OK;
   if (ids) for (int i = 0; i < n; i++) if (ids[i] < 0 || ids[i] >= p->n) return set_err(TBX_EINVAL, "env id out of range");
   CK(cudaSetDevice(p->device));
-  uint32_t *d_seeds = 0;
-  int32_t *d_ids = 0;
-  CK(cudaMalloc(&d_seeds, n * sizeof(uint32_t)));
-  CK(cudaMemcpy(d_seeds, seeds, n * sizeof(uint32_t), cudaMemcpyHostToDevice));
-  if (ids) { CK(cudaMalloc(&d_ids, n * sizeof(int32_t))); CK(cudaMemcpy(d_ids, ids, n * sizeof(int32_t), cudaMemcpyHostToDevice)); }
+  Buf<uint32_t> d_seeds;
+  Buf<int32_t> d_ids;
+  CK(d_seeds.upload(seeds, n));
+  if (ids) CK(d_ids.upload(ids, n));
   seed_kernel<<<blocks(n, 256), 256>>>(p->planes, p->n_pad, d_seeds, d_ids, n);
   CK(cudaGetLastError());
   CK(cudaDeviceSynchronize());
-  cudaFree(d_seeds); cudaFree(d_ids);
   return TBX_OK;
 }
 
@@ -266,9 +302,7 @@ static int do_step(tbx_pool *p, const int32_t *actions, const uint8_t *inputs, i
   a.legal = p->d_legal; a.n_legal = p->info->n_legal;
   a.syn_seed = syn ? syn->seed : 0; a.syn_env0 = syn ? syn->env0 : 0; a.syn_t = syn ? syn->t : 0;
   a.reward = reward; a.done = done; a.score = score; a.lives = lives; a.stats = p->d_stats; a.bad_actions = p->d_bad;
-  if (p->game == TBX_BREAKOUT) return launch_step<TBX_BREAKOUT>(p, a, s);
-  if (p->game == TBX_AMIDAR) return launch_step<TBX_AMIDAR>(p, a, s);
-  return launch_step<TBX_SPACE_INVADERS>(p, a, s);
+  return with_game(p->game, [&](auto g) { return launch_step<decltype(g)::value>(p, a, s); });
 }
 int tbx_step(tbx_pool *p, const int32_t *actions, int auto_reset, int32_t *reward, uint8_t *done, int32_t *score, int32_t *lives, void *stream) {
   if (!p || !actions) return set_err(TBX_EINVAL, "pool/actions is NULL");
@@ -309,82 +343,82 @@ int tbx_check(tbx_pool *p, void *stream) {
 
 /* ---- render */
 static void drop_render_cache(tbx_pool *p) {
-  for (int b = 0; b < 2; b++) { cudaFree(p->d_base_gray[b]); cudaFree(p->d_base_rgba[b]); cudaFree(p->d_base_rgb[b]); p->d_base_gray[b] = p->d_base_rgba[b] = p->d_base_rgb[b] = 0; }
-  for (auto &kv : p->area) { cudaFree(kv.second.d_plan); cudaFree(kv.second.d_base_out[0]); cudaFree(kv.second.d_base_out[1]); cudaFree(kv.second.d_patches[0]); cudaFree(kv.second.d_patches[1]); cudaFree(kv.second.d_direct); cudaFree(kv.second.d_direct2); }
+  p->base.reset();
   p->area.clear();
 }
-/* base frames 0/1 of the current config (see tbx_render.cuh), gray and RGBA, on the device */
+/* base frames 0/1 of the current config (see tbx_render.cuh); kept only once every buffer is in place */
 static int ensure_base(tbx_pool *p) {
-  if (p->d_base_gray[0]) return TBX_OK;
+  if (p->base) return TBX_OK;
+  auto base = std::make_unique<BaseFrames>();
   const int npix = p->info->width * p->info->height;
-  const BrkTable *brk_default = p->game == TBX_BREAKOUT ? &p->brk_tables[p->cfg.brk.default_tbl] : 0;
+  std::vector<uint32_t> rgba(npix);
+  std::vector<uint8_t> rgb((size_t)npix * 3);
   for (int b = 0; b < 2; b++) {
-    p->h_base_rgba[b].resize(npix);
-    p->h_base_gray[b].resize(npix);
-    tbx::build_base_frame(p->cfg, brk_default, b, p->h_base_rgba[b].data());
-    tbx::frame_to_gray(p->h_base_rgba[b].data(), npix, p->h_base_gray[b].data());
-    CK(cudaMalloc(&p->d_base_gray[b], npix + 16)); /* slack: the direct kernel reads whole words around a pixel */
-    CK(cudaMemset(p->d_base_gray[b] + npix, 0, 16));
-    CK(cudaMalloc(&p->d_base_rgba[b], (size_t)npix * 4));
-    CK(cudaMemcpy(p->d_base_gray[b], p->h_base_gray[b].data(), npix, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(p->d_base_rgba[b], p->h_base_rgba[b].data(), (size_t)npix * 4, cudaMemcpyHostToDevice));
-    std::vector<uint8_t> rgb((size_t)npix * 3);
-    for (int i = 0; i < npix; i++) { uint32_t c = p->h_base_rgba[b][i]; rgb[3 * i] = c & 255; rgb[3 * i + 1] = (c >> 8) & 255; rgb[3 * i + 2] = (c >> 16) & 255; }
-    CK(cudaMalloc(&p->d_base_rgb[b], rgb.size()));
-    CK(cudaMemcpy(p->d_base_rgb[b], rgb.data(), rgb.size(), cudaMemcpyHostToDevice));
+    std::vector<uint8_t> &gray = base->h_gray[b];
+    gray.resize(npix);
+    tbx::build_base_frame(p->cfg, brk_default(p), b, rgba.data());
+    tbx::frame_to_gray(rgba.data(), npix, gray.data());
+    CK(base->gray[b].alloc(npix + 16)); /* slack: the direct kernel reads whole words around a pixel */
+    CK(cudaMemset(base->gray[b] + npix, 0, 16));
+    CK(cudaMemcpy(base->gray[b], gray.data(), npix, cudaMemcpyHostToDevice));
+    CK(base->rgba[b].upload(reinterpret_cast<const uint8_t *>(rgba.data()), (size_t)npix * 4));
+    for (int i = 0; i < npix; i++) { uint32_t c = rgba[i]; rgb[3 * i] = c & 255; rgb[3 * i + 1] = (c >> 8) & 255; rgb[3 * i + 2] = (c >> 16) & 255; }
+    CK(base->rgb[b].upload(rgb.data(), rgb.size()));
   }
+  p->base = std::move(base);
   return TBX_OK;
 }
-static int ensure_area(tbx_pool *p, int out_w, int out_h, AreaRes **out) {
+/* the INTER_AREA resources of one output size, built on first use; kept only once every buffer is in place */
+static int ensure_area(tbx_pool *p, int out_w, int out_h, const AreaRes **out) {
   auto key = std::make_pair(out_w, out_h);
   auto it = p->area.find(key);
   if (it == p->area.end()) {
     tbx::ResizeTab rs;
-    TbxAreaPlan plan;
+    AreaRes r;
     try { tbx::build_resize(p->info->width, p->info->height, out_w, out_h, rs); }
     catch (const std::exception &e) { return set_err(TBX_EINVAL, e.what()); }
-    if (!tbx::build_area_plan(rs, plan)) return set_err(TBX_EINVAL, "resize: the fused kernel supports destinations up to 128x128 with at most 8 taps per axis");
-    AreaRes r;
-    r.plan = plan;
-    r.dw = out_w; r.dh = out_h; r.tx = plan.tx; r.ty = plan.ty; r.d_plan = 0; r.d_base_out[0] = r.d_base_out[1] = 0; r.d_patches[0] = r.d_patches[1] = 0;
-    r.d_direct = r.d_direct2 = 0; r.direct_ok = 0;
-    CK(cudaMalloc(&r.d_plan, sizeof plan));
-    CK(cudaMemcpy(r.d_plan, &plan, sizeof plan, cudaMemcpyHostToDevice));
+    if (!tbx::build_area_plan(rs, r.plan)) return set_err(TBX_EINVAL, "resize: the fused kernel supports destinations up to 128x128 with at most 8 taps per axis");
+    CK(r.d_plan.upload(&r.plan, 1));
     for (int b = 0; b < 2; b++) {
+      const uint8_t *gray = p->base->h_gray[b].data();
       std::vector<uint8_t> base_out(((size_t)out_w * out_h + 15) & ~(size_t)15, 0);
-      tbx::area_resize(p->h_base_gray[b].data(), rs, base_out.data());
-      CK(cudaMalloc(&r.d_base_out[b], base_out.size()));
-      CK(cudaMemcpy(r.d_base_out[b], base_out.data(), base_out.size(), cudaMemcpyHostToDevice));
+      tbx::area_resize(gray, rs, base_out.data());
+      CK(r.d_base_out[b].upload(base_out.data(), base_out.size()));
       std::vector<TbxDigitPatch> patches((size_t)TBX_DP_SLOTS * 10);
-      tbx::build_digit_patches(p->cfg, p->game == TBX_BREAKOUT ? &p->brk_tables[p->cfg.brk.default_tbl] : 0, rs, plan, p->h_base_gray[b].data(), patches.data());
-      CK(cudaMalloc(&r.d_patches[b], patches.size() * sizeof(TbxDigitPatch)));
-      CK(cudaMemcpy(r.d_patches[b], patches.data(), patches.size() * sizeof(TbxDigitPatch), cudaMemcpyHostToDevice));
+      tbx::build_digit_patches(p->cfg, brk_default(p), rs, r.plan, gray, patches.data());
+      CK(r.d_patches[b].upload(patches.data(), patches.size()));
     }
-    CK(tbx_direct_build(p->cfg, p->game == TBX_BREAKOUT ? &p->brk_tables[p->cfg.brk.default_tbl] : 0, rs, plan, p->h_base_gray[0].data(), &r.d_direct, &r.d_direct2));
-    r.direct_ok = r.d_direct != 0;
-    it = p->area.insert(std::make_pair(key, r)).first;
+    CK(tbx_direct_build(p->cfg, brk_default(p), rs, r.plan, p->base->h_gray[0].data(), r.d_direct, r.d_direct2));
+    it = p->area.emplace(key, std::move(r)).first;
   }
   *out = &it->second;
   return TBX_OK;
 }
 
 static int align16(int v) { return (v + 15) & ~15; }
+/* canvas bytes per pixel of an observation layout */
+static constexpr int obs_pix(int mode) { return mode == TBX_OBS_RGBA ? 4 : mode == TBX_OBS_RGB ? 3 : 1; }
+/* f(Const<MODE>()) for a native layout */
+template <class F> static int with_layout(int mode, F &&f) {
+  if (mode == TBX_OBS_RGBA) return f(Const<TBX_OBS_RGBA>());
+  if (mode == TBX_OBS_RGB) return f(Const<TBX_OBS_RGB>());
+  return f(Const<TBX_OBS_GRAY>());
+}
 
 /* the canvas kernel (tbx_render.cuh): the dense Breakout / Amidar envs the patch kernel lists */
-template <int GAME, int MODE> static int launch_render(const RenderArgs &a, const void *cfg_host, int smem, cudaStream_t s) {
+template <int GAME, int MODE> static int launch_render(const RenderArgs &a, const typename Traits<GAME>::Cfg &cfg, int smem, cudaStream_t s) {
   /* the opt-in is per device (a process may hold pools on several GPUs): set it on every launch, a cheap host-side call */
   CK((cudaFuncSetAttribute(render_kernel<GAME, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem > 160 * 1024 ? smem : 160 * 1024)));
   const int H = Traits<GAME>::H;
   dim3 grid(blocks(a.n, TBX_EPC), (H + a.band_rows - 1) / a.band_rows);
   /* measured: Breakout's few primitives keep 4 warps busy, the sprite-heavy games use 8 (profiles/r1_native_layouts.md) */
   const int threads = GAME == TBX_BREAKOUT ? 128 : 256;
-  render_kernel<GAME, MODE><<<grid, threads, smem, s>>>(a, *(const typename Traits<GAME>::Cfg *)cfg_host);
+  render_kernel<GAME, MODE><<<grid, threads, smem, s>>>(a, cfg);
   CK(cudaGetLastError());
   return TBX_OK;
 }
 /* native layouts as broadcast + patch (tbx_render_native.cuh) */
-template <int GAME, int PIX> static int launch_native_pix(const tbx_pool *p, const RenderArgs &a, const void *cfg_host, int band_smem, cudaStream_t s) {
-  typedef typename Traits<GAME>::Cfg Cfg;
+template <int GAME, int PIX> static int launch_native(const RenderArgs &a, const typename Traits<GAME>::Cfg &cfg, int band_smem, cudaStream_t s) {
   const int threads = 256;
   const int patch_smem = a.smem_canvas; /* the records of the CTA's 8 envs */
   CK((cudaFuncSetAttribute(base_fill_kernel<GAME, PIX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024)));
@@ -392,152 +426,102 @@ template <int GAME, int PIX> static int launch_native_pix(const tbx_pool *p, con
   if (band_smem > 64 * 1024 || patch_smem > 160 * 1024) return set_err(TBX_EINVAL, "frame too wide for the native render path");
   const int H = Traits<GAME>::H;
   dim3 grid(blocks(a.n, TBX_FILL_ENVS), (H + a.band_rows - 1) / a.band_rows);
-  base_fill_kernel<GAME, PIX><<<grid, 128, band_smem, s>>>(a, *(const Cfg *)cfg_host);
+  base_fill_kernel<GAME, PIX><<<grid, 128, band_smem, s>>>(a, cfg);
   CK(cudaGetLastError());
-  native_patch_kernel<GAME, PIX><<<blocks(a.n, TBX_EPC), threads, patch_smem, s>>>(a, *(const Cfg *)cfg_host);
+  native_patch_kernel<GAME, PIX><<<blocks(a.n, TBX_EPC), threads, patch_smem, s>>>(a, cfg);
   CK(cudaGetLastError());
-  (void)p;
   return TBX_OK;
 }
-template <int GAME> static int launch_native_game(const tbx_pool *p, int mode, const RenderArgs &a, const void *c, int band_smem, cudaStream_t s) {
-  if (mode == TBX_OBS_RGBA) return launch_native_pix<GAME, 4>(p, a, c, band_smem, s);
-  if (mode == TBX_OBS_RGB) return launch_native_pix<GAME, 3>(p, a, c, band_smem, s);
-  return launch_native_pix<GAME, 1>(p, a, c, band_smem, s);
-}
-static int launch_native(const tbx_pool *p, int mode, const RenderArgs &a, int band_smem, cudaStream_t s) {
-  if (p->game == TBX_BREAKOUT) return launch_native_game<TBX_BREAKOUT>(p, mode, a, cfg_ptr(p), band_smem, s);
-  if (p->game == TBX_AMIDAR) return launch_native_game<TBX_AMIDAR>(p, mode, a, cfg_ptr(p), band_smem, s);
-  return launch_native_game<TBX_SPACE_INVADERS>(p, mode, a, cfg_ptr(p), band_smem, s);
-}
-
 /* INTER_AREA, one warp per env (tbx_render_area.cuh) */
-template <int GAME, int TX, int TY, bool DUAL> static int launch_area_tile_dual(const RenderArgs &a, const void *cfg_host, const TbxAreaPlan *plan_host, int smem, cudaStream_t s) {
+template <int GAME, int TX, int TY, bool DUAL> static int launch_area_tile(const RenderArgs &a, const typename Traits<GAME>::Cfg &cfg, const TbxAreaPlan &plan, int smem, cudaStream_t s) {
   CK((cudaFuncSetAttribute(area_tile_kernel<GAME, TX, TY, DUAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
   /* env-list mode (the envs the direct kernel handed over, normally none): a small grid walks the list */
   const int grid = a.env_list ? (blocks(a.n, TBX_EPC) < 296 ? blocks(a.n, TBX_EPC) : 296) : blocks(a.n, TBX_EPC);
-  area_tile_kernel<GAME, TX, TY, DUAL><<<grid, TBX_TILE_THREADS, smem, s>>>(a, *(const typename Traits<GAME>::Cfg *)cfg_host, *plan_host);
+  area_tile_kernel<GAME, TX, TY, DUAL><<<grid, TBX_TILE_THREADS, smem, s>>>(a, cfg, plan);
   CK(cudaGetLastError());
   return TBX_OK;
 }
-template <int GAME, int TX, int TY> static int launch_area_tile(const RenderArgs &a, const void *cfg_host, const TbxAreaPlan *plan_host, int smem, cudaStream_t s) {
-  if (a.planes2) return launch_area_tile_dual<GAME, TX, TY, true>(a, cfg_host, plan_host, smem, s);
-  return launch_area_tile_dual<GAME, TX, TY, false>(a, cfg_host, plan_host, smem, s);
-}
-/* the smallest instantiated tap counts that cover the plan; plans over 5 x 4 taps render single frames only */
-template <int GAME> static int launch_area_tile_taps(int tx, int ty, const RenderArgs &a, const void *c, const TbxAreaPlan *pl, int smem, cudaStream_t s) {
-  if (tx > 5 || ty > 4) return launch_area_tile_dual<GAME, 8, 8, false>(a, c, pl, smem, s);
-  if (ty <= 3) {
-    if (tx <= 3) return launch_area_tile<GAME, 3, 3>(a, c, pl, smem, s);
-    if (tx <= 4) return launch_area_tile<GAME, 4, 3>(a, c, pl, smem, s);
-    return launch_area_tile<GAME, 5, 3>(a, c, pl, smem, s);
-  }
-  if (tx <= 3) return launch_area_tile<GAME, 3, 4>(a, c, pl, smem, s);
-  if (tx <= 4) return launch_area_tile<GAME, 4, 4>(a, c, pl, smem, s);
-  return launch_area_tile<GAME, 5, 4>(a, c, pl, smem, s);
-}
-template <int GAME> static int launch_render_mode(int mode, const RenderArgs &a, const void *c, int smem, cudaStream_t s) {
-  if (mode == TBX_OBS_RGBA) return launch_render<GAME, TBX_OBS_RGBA>(a, c, smem, s);
-  if (mode == TBX_OBS_RGB) return launch_render<GAME, TBX_OBS_RGB>(a, c, smem, s);
-  return launch_render<GAME, TBX_OBS_GRAY>(a, c, smem, s);
-}
 
-extern "C" {
-
-struct DualRender { const uint32_t *planes2; const uint8_t *reset_flags; int stack_k, stack_slot, stack_mode; };
-static int render_impl(tbx_pool *p, uint8_t *dst, int mode, int out_w, int out_h, void *stream, const DualRender *dual);
-
-int tbx_render(tbx_pool *p, uint8_t *dst, int mode, int out_w, int out_h, void *stream) { return render_impl(p, dst, mode, out_w, out_h, stream, 0); }
-
-} /* extern "C" */
-
-static int render_impl(tbx_pool *p, uint8_t *dst, int mode, int out_w, int out_h, void *stream, const DualRender *dual) {
-  if (!p || !dst) return set_err(TBX_EINVAL, "pool/dst is NULL");
-  if (((uintptr_t)dst & 15) != 0) return set_err(TBX_EINVAL, "dst must be 16-byte aligned");
-  size_t fb = tbx_obs_bytes(p, mode, out_w, out_h);
-  if (fb == 0) return set_err(TBX_EINVAL, "unsupported observation layout or size");
-  CK(cudaSetDevice(p->device));
-  int r = ensure_base(p);
+/* INTER_AREA: the direct kernel where it covers the pair, then the tile kernel */
+static int render_area(tbx_pool *p, RenderArgs &a, int out_w, int out_h, cudaStream_t s) {
+  const AreaRes *ar = 0;
+  int r = ensure_area(p, out_w, out_h, &ar);
   if (r) return r;
-  const int W = p->info->width, H = p->info->height;
-  const int pix = mode == TBX_OBS_RGBA ? 4 : mode == TBX_OBS_RGB ? 3 : 1; /* canvas bytes per pixel */
-  RenderArgs a;
-  a.planes = p->planes; a.n = p->n; a.n_pad = p->n_pad; a.cfg = p->d_cfg; a.tables = p->d_tables;
-  a.planes2 = dual ? dual->planes2 : 0; a.reset_flags = dual ? dual->reset_flags : 0;
-  a.stack_k = dual ? dual->stack_k : 1; a.stack_slot = dual ? dual->stack_slot : 0; a.stack_mode = dual ? dual->stack_mode : 0; a.env_stride = fb * (size_t)a.stack_k; a.tile_bytes = 0;
-  a.patches[0] = a.patches[1] = 0; a.dense_list = 0; a.dense_count = 0; a.dense_flag = 0; a.dense_threshold = 0; a.env_list = 0; a.env_count = 0;
-  a.dst = dst; a.frame_bytes = fb; a.plan = 0; a.tile_stride = 0; a.warp_bytes = 0; a.list_cap = 0; a.band_rows = 0; a.smem_rects = 0;
-  for (int b = 0; b < 2; b++) {
-    a.base[b] = pix == 4 ? p->d_base_rgba[b] : pix == 3 ? p->d_base_rgb[b] : p->d_base_gray[b];
-    a.base_out[b] = 0; /* INTER_AREA: set below */
+  const TbxAreaPlan &plan = ar->plan;
+  const bool dual = a.planes2 != 0;
+  a.base_out[0] = ar->d_base_out[0]; a.base_out[1] = ar->d_base_out[1]; a.plan = ar->d_plan;
+  {
+    const char *env = getenv("TBX_AREA_DIGIT_CACHE");
+    const bool on = !(env && atoi(env) == 0);
+    a.patches[0] = on ? ar->d_patches[0].get() : 0; a.patches[1] = on ? ar->d_patches[1].get() : 0;
   }
-  a.smem_canvas = align16(p->info->rec_words * TBX_EPC * 4) * (dual ? 2 : 1);
-  cudaStream_t s = (cudaStream_t)stream;
-  if (mode == TBX_OBS_GRAY_AREA) {
-    AreaRes *ar = 0;
-    r = ensure_area(p, out_w, out_h, &ar);
-    if (r) return r;
-    a.base_out[0] = ar->d_base_out[0]; a.base_out[1] = ar->d_base_out[1]; a.plan = ar->d_plan;
-    {
-      const char *env = getenv("TBX_AREA_DIGIT_CACHE");
-      const bool on = !(env && atoi(env) == 0);
-      a.patches[0] = on ? ar->d_patches[0] : 0; a.patches[1] = on ? ar->d_patches[1] : 0;
-    }
-    const int tx = ar->tx, ty = ar->ty;
-    const bool many_taps = tx > 5 || ty > 4;
-    if (dual && many_taps) return set_err(TBX_EINVAL, "wrapped observations need an output size the tile kernel supports (at most 5 x 4 taps)");
-    /* one warp per env over tiles of 16 x 8 output pixels, runs of at most TBX_TILE_MAX_RUN tiles: the scratch holds the
-     * widest / tallest run window of the instantiated tap counts */
-    const int tx_inst = many_taps ? 8 : tx <= 3 ? 3 : tx <= 4 ? 4 : 5, ty_inst = many_taps ? 8 : ty <= 3 ? 3 : 4;
-    const int tile_h = 1 << TBX_TILE_HSHIFT;
-    int stride = 0, rows = 0;
-    for (int dxA = 0; dxA < out_w; dxA += 16) {
-      const int dxL = dxA + 16 * TBX_TILE_MAX_RUN - 1 < out_w ? dxA + 16 * TBX_TILE_MAX_RUN - 1 : out_w - 1;
-      const int wdt = ((ar->plan.xs0[dxL] + tx_inst + 3) & ~3) - (ar->plan.xs0[dxA] & ~3);
-      if (wdt > stride) stride = wdt;
-    }
-    for (int dyA = 0; dyA < out_h; dyA += tile_h) {
-      const int dyL = dyA + tile_h - 1 < out_h ? dyA + tile_h - 1 : out_h - 1;
-      const int rws = ar->plan.ys0[dyL] + ty_inst - ar->plan.ys0[dyA];
-      if (rws > rows) rows = rws;
-    }
-    /* every plan build_area_plan accepts fits, for all three games (at most 256 B x 64 rows) */
-    if (stride > 512 || rows > 96 || W % 4 != 0)
-      return set_err(TBX_EINVAL, "INTER_AREA " + std::to_string(out_w) + "x" + std::to_string(out_h) + ": the tile kernel's scratch window (" +
-                                     std::to_string(stride) + " B x " + std::to_string(rows) + " rows) exceeds its limit of 512 B x 96 rows");
-    a.tile_stride = stride;
-    a.list_cap = TBX_TILE_LCAP;
-    if (const char *env = getenv("TBX_AREA_LCAP")) a.list_cap = atoi(env); /* tests: small lists force the sweep / per-tile paths */
-    if (a.list_cap < 1 || a.list_cap > TBX_TILE_LCAP) a.list_cap = TBX_TILE_LCAP;
-    a.tile_bytes = align16(stride * rows);
-    a.warp_bytes = TBX_TILE_LCAP * 20 + 32 + a.tile_bytes * (dual ? 2 : 1);
-    const int smem = a.smem_canvas + (TBX_TILE_THREADS / 32) * a.warp_bytes;
-    int smem_optin = 0;
-    CK(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, p->device));
-    if (smem > smem_optin)
-      return set_err(TBX_EINVAL, "INTER_AREA " + std::to_string(out_w) + "x" + std::to_string(out_h) + ": the tile kernel needs " + std::to_string(smem) +
-                                     " B of shared memory per CTA, the device allows " + std::to_string(smem_optin));
-    /* Direct kernel first (tbx_render_direct.cuh; TBX_AREA_KERNEL=tile turns it off): closed forms for the envs they
-     * cover, the rest are listed and rendered by the tile kernel in env-list mode right after (usually an empty list) */
-    const char *ksel = getenv("TBX_AREA_KERNEL");
-    if (ar->direct_ok && !dual && !(ksel && !strcmp(ksel, "tile"))) {
-      if (!p->d_fb) { CK(cudaMalloc(&p->d_fb, ((size_t)p->n_pad + 8) * sizeof(int32_t))); CK(cudaMemsetAsync(p->d_fb, 0, 8 * sizeof(int32_t), s)); }
-      DirectArgs da;
-      da.aux = ar->d_direct; da.aux2 = ar->d_direct2; da.fb_list = p->d_fb + 8; da.fb_count = p->d_fb; da.sched = p->d_fb + 2;
-      tbx_direct_geometry(p->game, out_w, out_h, p->game == TBX_BREAKOUT ? p->cfg.brk.n_rows : 0, da);
-      CK(tbx_launch_direct(p->game, tx, ty, a, cfg_ptr(p), ar->plan, da, s));
-      if (p->game == TBX_SPACE_INVADERS) return TBX_OK; /* covers every env: nothing is handed over */
-      a.env_list = p->d_fb + 8;
-      a.env_count = p->d_fb;
-    }
-    if (p->game == TBX_BREAKOUT) return launch_area_tile_taps<TBX_BREAKOUT>(tx, ty, a, cfg_ptr(p), &ar->plan, smem, s);
-    if (p->game == TBX_AMIDAR) return launch_area_tile_taps<TBX_AMIDAR>(tx, ty, a, cfg_ptr(p), &ar->plan, smem, s);
-    return launch_area_tile_taps<TBX_SPACE_INVADERS>(tx, ty, a, cfg_ptr(p), &ar->plan, smem, s);
+  const Taps taps = inst_taps(plan.tx, plan.ty);
+  if (dual && taps.x == 8) return set_err(TBX_EINVAL, "wrapped observations need an output size the tile kernel supports (at most 5 x 4 taps)");
+  /* one warp per env over tiles of 16 x 8 output pixels, runs of at most TBX_TILE_MAX_RUN tiles: the scratch holds the
+   * widest / tallest run window of the instantiated tap counts */
+  const int tile_h = 1 << TBX_TILE_HSHIFT;
+  int stride = 0, rows = 0;
+  for (int dxA = 0; dxA < out_w; dxA += 16) {
+    const int dxL = dxA + 16 * TBX_TILE_MAX_RUN - 1 < out_w ? dxA + 16 * TBX_TILE_MAX_RUN - 1 : out_w - 1;
+    const int wdt = ((plan.xs0[dxL] + taps.x + 3) & ~3) - (plan.xs0[dxA] & ~3);
+    if (wdt > stride) stride = wdt;
   }
-  /* Native layouts: broadcast + patch (tbx_render_native.cuh) -- the base frame leaves through the TMA engine at HBM speed,
-   * what differs from it is painted straight into the frame.  Breakout and Amidar envs that differ in many places (a wall
-   * with more than 20 holes, a maze with more than 48 painted tiles / boxes; TBX_NATIVE_DENSE overrides) are cheaper to
-   * repaint in shared memory: the patch kernel lists them and the canvas kernel below renders exactly those.  Space
-   * Invaders' ~50 sprites are always patched. */
+  for (int dyA = 0; dyA < out_h; dyA += tile_h) {
+    const int dyL = dyA + tile_h - 1 < out_h ? dyA + tile_h - 1 : out_h - 1;
+    const int rws = plan.ys0[dyL] + taps.y - plan.ys0[dyA];
+    if (rws > rows) rows = rws;
+  }
+  /* every plan build_area_plan accepts fits, for all three games (at most 256 B x 64 rows) */
+  if (stride > 512 || rows > 96 || p->info->width % 4 != 0)
+    return set_err(TBX_EINVAL, "INTER_AREA " + std::to_string(out_w) + "x" + std::to_string(out_h) + ": the tile kernel's scratch window (" +
+                                   std::to_string(stride) + " B x " + std::to_string(rows) + " rows) exceeds its limit of 512 B x 96 rows");
+  a.tile_stride = stride;
+  a.list_cap = TBX_TILE_LCAP;
+  if (const char *env = getenv("TBX_AREA_LCAP")) a.list_cap = atoi(env); /* tests: small lists force the sweep / per-tile paths */
+  if (a.list_cap < 1 || a.list_cap > TBX_TILE_LCAP) a.list_cap = TBX_TILE_LCAP;
+  a.tile_bytes = align16(stride * rows);
+  a.warp_bytes = TBX_TILE_LCAP * 20 + 32 + a.tile_bytes * (dual ? 2 : 1);
+  const int smem = a.smem_canvas + (TBX_TILE_THREADS / 32) * a.warp_bytes;
+  int smem_optin = 0;
+  CK(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, p->device));
+  if (smem > smem_optin)
+    return set_err(TBX_EINVAL, "INTER_AREA " + std::to_string(out_w) + "x" + std::to_string(out_h) + ": the tile kernel needs " + std::to_string(smem) +
+                                   " B of shared memory per CTA, the device allows " + std::to_string(smem_optin));
+  /* Direct kernel first (tbx_render_direct.cuh; TBX_AREA_KERNEL=tile turns it off): closed forms for the envs they
+   * cover, the rest are listed and rendered by the tile kernel in env-list mode right after (usually an empty list) */
+  const char *ksel = getenv("TBX_AREA_KERNEL");
+  if (ar->d_direct && !dual && !(ksel && !strcmp(ksel, "tile"))) {
+    if (!p->d_fb) { /* the counters start at zero; the kernels leave them so */
+      Buf<int32_t> fb;
+      CK(fb.alloc((size_t)p->n_pad + 8));
+      CK(cudaMemsetAsync(fb, 0, 8 * sizeof(int32_t), s));
+      p->d_fb = std::move(fb);
+    }
+    DirectArgs da = {};
+    da.aux = ar->d_direct; da.aux2 = ar->d_direct2; da.fb_list = p->d_fb + 8; da.fb_count = p->d_fb; da.sched = p->d_fb + 2;
+    CK(tbx_launch_direct(p->cfg, a, plan, da, s));
+    if (p->game == TBX_SPACE_INVADERS) return TBX_OK; /* covers every env: nothing is handed over */
+    a.env_list = p->d_fb + 8;
+    a.env_count = p->d_fb;
+  }
+  return with_game(p->game, [&](auto g) {
+    constexpr int G = decltype(g)::value;
+    const auto &cfg = game_cfg<G>(p->cfg);
+    return with_taps<8>(plan.tx, plan.ty, [&](auto X, auto Y) {
+      constexpr int TX = decltype(X)::value, TY = decltype(Y)::value;
+      if constexpr (TX == 8) return launch_area_tile<G, 8, 8, false>(a, cfg, plan, smem, s); /* single frames only (checked above) */
+      else return dual ? launch_area_tile<G, TX, TY, true>(a, cfg, plan, smem, s) : launch_area_tile<G, TX, TY, false>(a, cfg, plan, smem, s);
+    });
+  });
+}
+
+/* Native layouts: broadcast + patch (tbx_render_native.cuh) -- the base frame leaves through the TMA engine at HBM speed,
+ * what differs from it is painted straight into the frame.  Breakout and Amidar envs that differ in many places (a wall
+ * with more than 20 holes, a maze with more than 48 painted tiles / boxes; TBX_NATIVE_DENSE overrides) are cheaper to
+ * repaint in shared memory: the patch kernel lists them and the canvas kernel below renders exactly those.  Space
+ * Invaders' ~50 sprites are always patched. */
+static int render_native(tbx_pool *p, RenderArgs &a, int mode, cudaStream_t s) {
+  const int W = p->info->width, H = p->info->height, pix = obs_pix(mode);
   /* canvas bands of at most ~40 KB so that five CTAs stay resident per SM */
   int max_rows = (40 * 1024) / (W * pix);
   if (max_rows < 1) max_rows = 1;
@@ -546,35 +530,70 @@ static int render_impl(tbx_pool *p, uint8_t *dst, int mode, int out_w, int out_h
   a.smem_rects = a.smem_canvas + align16(a.band_rows * W * pix);
   const int smem_total = a.smem_rects + 2 * TBX_MAX_RECTS * (int)sizeof(int4) + 128 + TBX_MAX_BIG * (int)sizeof(uint4); /* + list counts, per-env base / env ids, the big-primitive queue */
   if (smem_total > 220 * 1024) return set_err(TBX_EINVAL, "observation size needs more shared memory than one SM has");
-  int thr = p->game == TBX_BREAKOUT ? 20 : p->game == TBX_AMIDAR ? 48 : INT32_MAX;
-  const char *dense_env = getenv("TBX_NATIVE_DENSE");
-  if (dense_env && thr != INT32_MAX) thr = atoi(dense_env) < 0 ? INT32_MAX : atoi(dense_env);
-  if (thr != INT32_MAX) {
-    if (!p->d_dense) CK(cudaMalloc(&p->d_dense, ((size_t)p->n_pad + 8) * sizeof(int32_t) + (size_t)p->n_pad));
-    a.dense_list = p->d_dense + 8;
-    a.dense_count = p->d_dense;
-    a.dense_flag = reinterpret_cast<uint8_t *>(p->d_dense + 8 + p->n_pad);
-    a.dense_threshold = thr;
-    CK(cudaMemsetAsync(p->d_dense, 0, sizeof(int32_t), s));
-    if (p->game == TBX_BREAKOUT) dense_classify_kernel<TBX_BREAKOUT><<<blocks(p->n, 8), 256, 0, s>>>(a, p->cfg.brk);
-    else dense_classify_kernel<TBX_AMIDAR><<<blocks(p->n, 8), 256, 0, s>>>(a, p->cfg.ami);
-    CK(cudaGetLastError());
-  }
-  r = launch_native(p, mode, a, align16(a.band_rows * W * pix), s);
-  if (r || thr == INT32_MAX) return r;
-  a.env_list = p->d_dense + 8;
-  a.env_count = p->d_dense;
-  if (p->game == TBX_BREAKOUT) return launch_render_mode<TBX_BREAKOUT>(mode, a, cfg_ptr(p), smem_total, s);
-  return launch_render_mode<TBX_AMIDAR>(mode, a, cfg_ptr(p), smem_total, s);
+  return with_game(p->game, [&](auto g) -> int {
+    constexpr int G = decltype(g)::value;
+    const auto &cfg = game_cfg<G>(p->cfg);
+    auto patch = [&]() { return with_layout(mode, [&](auto m) { return launch_native<G, obs_pix(decltype(m)::value)>(a, cfg, align16(a.band_rows * W * pix), s); }); };
+    if constexpr (G == TBX_SPACE_INVADERS) {
+      return patch();
+    } else {
+      int thr = G == TBX_BREAKOUT ? 20 : 48;
+      if (const char *dense_env = getenv("TBX_NATIVE_DENSE")) thr = atoi(dense_env) < 0 ? INT32_MAX : atoi(dense_env);
+      if (thr != INT32_MAX) {
+        CK(p->d_dense.grow((size_t)p->n_pad + 8 + p->n_pad / 4)); /* + a byte per env */
+        a.dense_list = p->d_dense + 8;
+        a.dense_count = p->d_dense;
+        a.dense_flag = reinterpret_cast<uint8_t *>(p->d_dense + 8 + p->n_pad);
+        a.dense_threshold = thr;
+        CK(cudaMemsetAsync(p->d_dense, 0, sizeof(int32_t), s));
+        dense_classify_kernel<G><<<blocks(p->n, 8), 256, 0, s>>>(a, cfg);
+        CK(cudaGetLastError());
+      }
+      const int r = patch();
+      if (r || thr == INT32_MAX) return r;
+      a.env_list = p->d_dense + 8;
+      a.env_count = p->d_dense;
+      return with_layout(mode, [&](auto m) { return launch_render<G, decltype(m)::value>(a, cfg, smem_total, s); });
+    }
+  });
 }
+
+struct DualRender { const uint32_t *planes2; const uint8_t *reset_flags; int stack_k, stack_slot, stack_mode; };
+static int render_impl(tbx_pool *p, uint8_t *dst, int mode, int out_w, int out_h, void *stream, const DualRender *dual) {
+  if (!p || !dst) return set_err(TBX_EINVAL, "pool/dst is NULL");
+  if (((uintptr_t)dst & 15) != 0) return set_err(TBX_EINVAL, "dst must be 16-byte aligned");
+  size_t fb = tbx_obs_bytes(p, mode, out_w, out_h);
+  if (fb == 0) return set_err(TBX_EINVAL, "unsupported observation layout or size");
+  CK(cudaSetDevice(p->device));
+  int r = ensure_base(p);
+  if (r) return r;
+  const int pix = obs_pix(mode);
+  RenderArgs a = {};
+  a.planes = p->planes; a.n = p->n; a.n_pad = p->n_pad; a.cfg = p->d_cfg; a.tables = p->d_tables;
+  a.planes2 = dual ? dual->planes2 : 0; a.reset_flags = dual ? dual->reset_flags : 0;
+  a.stack_k = dual ? dual->stack_k : 1; a.stack_slot = dual ? dual->stack_slot : 0; a.stack_mode = dual ? dual->stack_mode : 0; a.env_stride = fb * (size_t)a.stack_k;
+  a.dst = dst; a.frame_bytes = fb;
+  for (int b = 0; b < 2; b++) a.base[b] = pix == 4 ? p->base->rgba[b] : pix == 3 ? p->base->rgb[b] : p->base->gray[b];
+  a.smem_canvas = align16(p->info->rec_words * TBX_EPC * 4) * (dual ? 2 : 1);
+  cudaStream_t s = (cudaStream_t)stream;
+  return mode == TBX_OBS_GRAY_AREA ? render_area(p, a, out_w, out_h, s) : render_native(p, a, mode, s);
+}
+
+extern "C" {
+
+int tbx_render(tbx_pool *p, uint8_t *dst, int mode, int out_w, int out_h, void *stream) {
+  return guarded([&] { return render_impl(p, dst, mode, out_w, out_h, stream, 0); });
+}
+
+} /* extern "C" */
 
 /* ---- the fused wrapper stack (tbx_wrap.cuh) */
 struct tbx_wrap {
   tbx_pool *pool;
   int skip, noop_max, episodic_life, fire_reset, clip_rewards, stack_k, out_w, out_h;
   uint64_t noop_seed, env0;
-  uint32_t *planes_prev, *wstate;
-  uint8_t *was_reset;
+  Buf<uint32_t> planes_prev, wstate;
+  Buf<uint8_t> was_reset;
   int head; /* ring slot of the newest frame */
   int stack_mode; /* what a reset observation does to the other k-1 ring slots: 0 = fills them (FrameStack.reset), 1 = zeroes them (VecFrameStack) */
   int32_t *ep_return, *ep_length; /* caller-owned device outputs of Monitor's episode record, or NULL */
@@ -589,29 +608,25 @@ int tbx_wrap_create(tbx_pool *p, int skip, int noop_max, int episodic_life, int 
   if (skip < 1 || skip > 64 || noop_max < 0 || noop_max > 1000 || stack_k < 1 || stack_k > 16) return set_err(TBX_EINVAL, "skip / noop_max / stack_k out of range");
   if (tbx_obs_bytes(p, TBX_OBS_GRAY_AREA, out_w, out_h) == 0) return set_err(TBX_EINVAL, "unsupported observation size");
   CK(cudaSetDevice(p->device));
-  tbx_wrap *w = new (std::nothrow) tbx_wrap();
-  if (!w) return set_err(TBX_ENOMEM, "out of memory");
-  w->pool = p; w->skip = skip; w->noop_max = noop_max; w->episodic_life = episodic_life; w->fire_reset = fire_reset; w->clip_rewards = clip_rewards;
-  w->stack_k = stack_k; w->out_w = out_w; w->out_h = out_h; w->noop_seed = noop_seed; w->env0 = env0; w->head = 0; w->stack_mode = 0; w->ep_return = w->ep_length = 0;
-  w->planes_prev = 0; w->wstate = 0; w->was_reset = 0;
-  const size_t plane_bytes = (size_t)p->info->rec_words * p->n_pad * 4;
-  cudaError_t e = cudaMalloc(&w->planes_prev, plane_bytes);
-  if (e == cudaSuccess) e = cudaMalloc(&w->wstate, 5 * (size_t)p->n_pad * 4);
-  if (e == cudaSuccess) e = cudaMalloc(&w->was_reset, (size_t)p->n_pad);
-  if (e == cudaSuccess) e = cudaMemcpy(w->planes_prev, p->planes, plane_bytes, cudaMemcpyDeviceToDevice);
-  if (e == cudaSuccess) e = cudaMemset(w->wstate, 0, 5 * (size_t)p->n_pad * 4);
-  if (e == cudaSuccess) { /* EpisodicLifeEnv.__init__: lives = 0, was_real_done = True (atari_wrappers.py:155-156) */
-    std::vector<uint32_t> ones((size_t)p->n_pad, 1u);
-    e = cudaMemcpy(w->wstate + p->n_pad, ones.data(), ones.size() * 4, cudaMemcpyHostToDevice);
-  }
-  if (e == cudaSuccess) e = cudaMemset(w->was_reset, 0, (size_t)p->n_pad);
-  if (e != cudaSuccess) {
-    cudaFree(w->planes_prev); cudaFree(w->wstate); cudaFree(w->was_reset);
-    delete w;
-    return set_err(TBX_ECUDA, std::string("tbx_wrap_create: ") + cudaGetErrorString(e));
-  }
-  *out = w;
-  return TBX_OK;
+  return guarded([&]() -> int {
+    std::unique_ptr<tbx_wrap> w(new tbx_wrap());
+    w->pool = p; w->skip = skip; w->noop_max = noop_max; w->episodic_life = episodic_life; w->fire_reset = fire_reset; w->clip_rewards = clip_rewards;
+    w->stack_k = stack_k; w->out_w = out_w; w->out_h = out_h; w->noop_seed = noop_seed; w->env0 = env0;
+    const size_t plane_words = (size_t)p->info->rec_words * p->n_pad;
+    cudaError_t e = w->planes_prev.alloc(plane_words);
+    if (e == cudaSuccess) e = w->wstate.alloc(5 * (size_t)p->n_pad);
+    if (e == cudaSuccess) e = w->was_reset.alloc((size_t)p->n_pad);
+    if (e == cudaSuccess) e = cudaMemcpy(w->planes_prev, p->planes, plane_words * 4, cudaMemcpyDeviceToDevice);
+    if (e == cudaSuccess) e = cudaMemset(w->wstate, 0, 5 * (size_t)p->n_pad * 4);
+    if (e == cudaSuccess) { /* EpisodicLifeEnv.__init__: lives = 0, was_real_done = True (atari_wrappers.py:155-156) */
+      std::vector<uint32_t> ones((size_t)p->n_pad, 1u);
+      e = cudaMemcpy(w->wstate + p->n_pad, ones.data(), ones.size() * 4, cudaMemcpyHostToDevice);
+    }
+    if (e == cudaSuccess) e = cudaMemset(w->was_reset, 0, (size_t)p->n_pad);
+    if (e != cudaSuccess) return set_err(TBX_ECUDA, std::string("tbx_wrap_create: ") + cudaGetErrorString(e));
+    *out = w.release();
+    return TBX_OK;
+  });
 }
 
 int tbx_wrap_set_stack_mode(tbx_wrap *w, int mode) {
@@ -629,7 +644,6 @@ int tbx_wrap_destroy(tbx_wrap *w) {
   if (!w) return TBX_OK;
   cudaSetDevice(w->pool->device);
   cudaDeviceSynchronize();
-  cudaFree(w->planes_prev); cudaFree(w->wstate); cudaFree(w->was_reset);
   delete w;
   return TBX_OK;
 }
@@ -648,15 +662,13 @@ int tbx_wrap_step(tbx_wrap *w, const int32_t *actions, uint8_t *obs_ring, int32_
   a.reward = reward; a.score = score; a.lives = lives; a.done = done; a.real_done = real_done; a.was_reset = w->was_reset;
   a.ep_return = w->ep_return; a.ep_length = w->ep_length;
   a.stats = p->d_stats; a.bad_actions = p->d_bad;
-  if (p->game == TBX_BREAKOUT) wrap_step_kernel<TBX_BREAKOUT><<<blocks(p->n, 128), 128, 0, s>>>(a);
-  else if (p->game == TBX_AMIDAR) wrap_step_kernel<TBX_AMIDAR><<<blocks(p->n, 128), 128, 0, s>>>(a);
-  else wrap_step_kernel<TBX_SPACE_INVADERS><<<blocks(p->n, 128), 128, 0, s>>>(a);
+  with_game(p->game, [&](auto g) { wrap_step_kernel<decltype(g)::value><<<blocks(p->n, 128), 128, 0, s>>>(a); });
   CK(cudaGetLastError());
   if (obs_ring) {
     w->head = (w->head + 1) % w->stack_k;
     DualRender d;
     d.planes2 = w->planes_prev; d.reset_flags = w->was_reset; d.stack_k = w->stack_k; d.stack_slot = w->head; d.stack_mode = w->stack_mode;
-    int r = render_impl(p, obs_ring, TBX_OBS_GRAY_AREA, w->out_w, w->out_h, stream, &d);
+    int r = guarded([&] { return render_impl(p, obs_ring, TBX_OBS_GRAY_AREA, w->out_w, w->out_h, stream, &d); });
     if (r) return r;
   }
   if (slot_out) *slot_out = w->head;
@@ -706,7 +718,7 @@ int tbx_breakout_columns(tbx_pool *p, int op, int col, const uint8_t *mask, int3
   if (!p || p->game != TBX_BREAKOUT) return set_err(TBX_EINVAL, "tbx_breakout_columns needs a breakout pool");
   if (op < 0 || op > 2 || (op == 2 && !out)) return set_err(TBX_EINVAL, "op is 0 (remove column), 1 (fill column) or 2 (count channels into out)");
   CK(cudaSetDevice(p->device));
-  brk_column_kernel<<<blocks(p->n, 128), 128, 0, (cudaStream_t)stream>>>(p->planes, p->n, p->n_pad, (const BrkTable *)p->d_tables, op, col, mask, out);
+  brk_column_kernel<<<blocks(p->n, 128), 128, 0, (cudaStream_t)stream>>>(p->planes, p->n, p->n_pad, reinterpret_cast<const BrkTable *>(p->d_tables.get()), op, col, mask, out);
   CK(cudaGetLastError());
   return TBX_OK;
 }
@@ -766,40 +778,39 @@ int tbx_step_host(tbx_pool *p, const int32_t *actions, int auto_reset, int mode,
   if (!p || !actions) return set_err(TBX_EINVAL, "pool/actions is NULL");
   CK(cudaSetDevice(p->device));
   const size_t n = (size_t)p->n;
-  if (!p->hs) {
-    CK(cudaStreamCreateWithFlags(&p->hs, cudaStreamNonBlocking));
-    CK(cudaMalloc(&p->h_actions_dev, n * 4)); CK(cudaMalloc(&p->h_reward_dev, n * 4)); CK(cudaMalloc(&p->h_score_dev, n * 4));
-    CK(cudaMalloc(&p->h_lives_dev, n * 4)); CK(cudaMalloc(&p->h_done_dev, n));
-  }
-  size_t fb = 0;
-  if (obs) {
-    fb = tbx_obs_bytes(p, mode, out_w, out_h);
-    if (fb == 0) return set_err(TBX_EINVAL, "unsupported observation layout or size");
-    if (p->h_obs_cap < fb * n) {
-      CK(cudaStreamSynchronize(p->hs));
-      cudaFree(p->h_obs_dev);
-      p->h_obs_dev = 0; p->h_obs_cap = 0;
-      CK(cudaMalloc(&p->h_obs_dev, fb * n));
-      p->h_obs_cap = fb * n;
+  return guarded([&]() -> int {
+    if (!p->hs) {
+      auto h = std::make_unique<HostStaging>();
+      CK(cudaStreamCreateWithFlags(&h->s, cudaStreamNonBlocking));
+      CK(h->actions.alloc(n)); CK(h->reward.alloc(n)); CK(h->score.alloc(n)); CK(h->lives.alloc(n)); CK(h->done.alloc(n));
+      p->hs = std::move(h);
     }
-  }
-  CK(cudaMemcpyAsync(p->h_actions_dev, actions, n * 4, cudaMemcpyHostToDevice, p->hs));
-  int r = do_step(p, p->h_actions_dev, 0, auto_reset, p->h_reward_dev, p->h_done_dev, p->h_score_dev, p->h_lives_dev, p->hs);
-  if (r) return r;
-  if (reward) CK(cudaMemcpyAsync(reward, p->h_reward_dev, n * 4, cudaMemcpyDeviceToHost, p->hs));
-  if (done) CK(cudaMemcpyAsync(done, p->h_done_dev, n, cudaMemcpyDeviceToHost, p->hs));
-  if (score) CK(cudaMemcpyAsync(score, p->h_score_dev, n * 4, cudaMemcpyDeviceToHost, p->hs));
-  if (lives) CK(cudaMemcpyAsync(lives, p->h_lives_dev, n * 4, cudaMemcpyDeviceToHost, p->hs));
-  if (obs) {
-    r = tbx_render(p, p->h_obs_dev, mode, out_w, out_h, p->hs);
+    HostStaging &h = *p->hs;
+    size_t fb = 0;
+    if (obs) {
+      fb = tbx_obs_bytes(p, mode, out_w, out_h);
+      if (fb == 0) return set_err(TBX_EINVAL, "unsupported observation layout or size");
+      if (h.obs.size() < fb * n) CK(cudaStreamSynchronize(h.s));
+      CK(h.obs.grow(fb * n));
+    }
+    CK(cudaMemcpyAsync(h.actions, actions, n * 4, cudaMemcpyHostToDevice, h.s));
+    int r = do_step(p, h.actions, 0, auto_reset, h.reward, h.done, h.score, h.lives, h.s);
     if (r) return r;
-    CK(cudaMemcpyAsync(obs, p->h_obs_dev, fb * n, cudaMemcpyDeviceToHost, p->hs));
-  }
-  CK(cudaStreamSynchronize(p->hs));
-  int bad = 0;
-  CK(cudaMemcpy(&bad, p->d_bad, sizeof bad, cudaMemcpyDeviceToHost));
-  if (bad) { cudaMemset(p->d_bad, 0, sizeof(int)); return set_err(TBX_EACTION, "Expected to apply action, but failed: invalid ALE action id"); }
-  return TBX_OK;
+    if (reward) CK(cudaMemcpyAsync(reward, h.reward, n * 4, cudaMemcpyDeviceToHost, h.s));
+    if (done) CK(cudaMemcpyAsync(done, h.done, n, cudaMemcpyDeviceToHost, h.s));
+    if (score) CK(cudaMemcpyAsync(score, h.score, n * 4, cudaMemcpyDeviceToHost, h.s));
+    if (lives) CK(cudaMemcpyAsync(lives, h.lives, n * 4, cudaMemcpyDeviceToHost, h.s));
+    if (obs) {
+      r = render_impl(p, h.obs, mode, out_w, out_h, h.s, 0);
+      if (r) return r;
+      CK(cudaMemcpyAsync(obs, h.obs, fb * n, cudaMemcpyDeviceToHost, h.s));
+    }
+    CK(cudaStreamSynchronize(h.s));
+    int bad = 0;
+    CK(cudaMemcpy(&bad, p->d_bad, sizeof bad, cudaMemcpyDeviceToHost));
+    if (bad) { cudaMemset(p->d_bad, 0, sizeof(int)); return set_err(TBX_EACTION, "Expected to apply action, but failed: invalid ALE action id"); }
+    return TBX_OK;
+  });
 }
 
 /* ---- JSON */
@@ -812,19 +823,10 @@ void tbx_free_str(char *s) { free(s); }
 
 static int ensure_json_staging(tbx_pool *p, int n) {
   const size_t words = (size_t)n * p->info->rec_words;
-  if (p->j_cap_ids < (size_t)n) {
-    cudaFree(p->j_ids); p->j_ids = 0; p->j_cap_ids = 0;
-    const size_t cap = std::max<size_t>(1024, (size_t)n * 2);
-    CK(cudaMalloc(&p->j_ids, cap * sizeof(int32_t)));
-    p->j_cap_ids = cap;
-  }
-  if (p->j_cap_words < words) {
-    cudaFree(p->j_recs); cudaFreeHost(p->j_host); p->j_recs = p->j_host = 0; p->j_cap_words = 0;
-    const size_t cap = std::max<size_t>((size_t)1024 * p->info->rec_words, words * 2);
-    CK(cudaMalloc(&p->j_recs, cap * 4));
-    CK(cudaMallocHost(&p->j_host, cap * 4));
-    p->j_cap_words = cap;
-  }
+  CK(p->j_ids.grow(n, std::max<size_t>(1024, (size_t)n * 2)));
+  const size_t cap = std::max<size_t>((size_t)1024 * p->info->rec_words, words * 2);
+  CK(p->j_recs.grow(words, cap));
+  CK(p->j_host.grow(words, cap));
   return TBX_OK;
 }
 /* records of the listed envs -> p->j_host (AoS).  Runs on the legacy default stream, which is ordered after the work of
@@ -835,7 +837,7 @@ static int fetch_records(tbx_pool *p, const int32_t *ids, int n) {
   CK(cudaSetDevice(p->device));
   int r = ensure_json_staging(p, n);
   if (r) return r;
-  if (p->hs) CK(cudaStreamSynchronize(p->hs));
+  if (p->hs) CK(cudaStreamSynchronize(p->hs->s));
   CK(cudaMemcpyAsync(p->j_ids, ids, n * sizeof(int32_t), cudaMemcpyHostToDevice, 0));
   gather_kernel<<<blocks(n * rw, 256), 256>>>(p->planes, p->n_pad, p->j_ids, n, rw, p->j_recs);
   CK(cudaGetLastError());
@@ -857,63 +859,58 @@ int tbx_state_to_json(tbx_pool *p, const int32_t *ids, int n, char **out) {
   if (!p || !ids || !out || n < 0) return set_err(TBX_EINVAL, "bad arguments");
   for (int i = 0; i < n; i++) out[i] = 0;
   if (n == 0) return TBX_OK;
-  int r = fetch_records(p, ids, n);
-  if (r) return r;
-  const int rw = p->info->rec_words;
-  const uint32_t *recs = p->j_host;
-  try {
-    parallel_for(n, [&](int i) {
-      const uint32_t *R = recs + (size_t)i * rw;
-      Value v;
-      if (p->game == TBX_BREAKOUT) {
-        const BrkRec &rec = *reinterpret_cast<const BrkRec *>(R);
-        if (rec.hdr.tbl < 0 || rec.hdr.tbl >= (int)p->brk_tables.size()) throw std::runtime_error("corrupt table index");
-        v = tbx::brk_state_to_json(rec, p->brk_tables[rec.hdr.tbl]);
-      } else if (p->game == TBX_AMIDAR) {
-        const AmiRec &rec = *reinterpret_cast<const AmiRec *>(R);
-        if (rec.hdr.tbl < 0 || rec.hdr.tbl >= (int)p->ami_tables.size()) throw std::runtime_error("corrupt table index");
-        v = tbx::ami_state_to_json(rec, p->ami_tables[rec.hdr.tbl]);
-      } else v = tbx::si_state_to_json(*reinterpret_cast<const SiRec *>(R));
-      out[i] = dup_str(tbxjson::dump(v));
-      if (!out[i]) throw std::runtime_error("out of host memory");
+  const int r = guarded([&]() -> int {
+    int r = fetch_records(p, ids, n);
+    if (r) return r;
+    const int rw = p->info->rec_words;
+    const uint32_t *recs = p->j_host;
+    with_game(p->game, [&](auto g) {
+      constexpr int G = decltype(g)::value;
+      const auto &tabs = tables<G>(p);
+      parallel_for(n, [&](int i) {
+        const auto &rec = *reinterpret_cast<const typename Traits<G>::Rec *>(recs + (size_t)i * rw);
+        const typename Traits<G>::Table *t = 0;
+        if constexpr (kTables<G>) {
+          if (rec.hdr.tbl < 0 || rec.hdr.tbl >= (int)tabs.size()) throw std::runtime_error("corrupt table index");
+          t = &tabs[rec.hdr.tbl];
+        }
+        out[i] = dup_str(tbxjson::dump(state_to_json(rec, t)));
+        if (!out[i]) throw std::runtime_error("out of host memory");
+      });
     });
-  } catch (const std::exception &e) {
-    for (int i = 0; i < n; i++) { free(out[i]); out[i] = 0; }
-    return set_err(TBX_EJSON, e.what());
-  }
-  return TBX_OK;
+    return TBX_OK;
+  });
+  if (r) for (int i = 0; i < n; i++) { free(out[i]); out[i] = 0; }
+  return r;
 }
 
 int tbx_state_from_json(tbx_pool *p, const int32_t *ids, int n, const char *const *json) {
   if (!p || !ids || !json || n < 0) return set_err(TBX_EINVAL, "bad arguments");
   if (n == 0) return TBX_OK;
-  int r = fetch_records(p, ids, n); /* keeps the fields JSON does not carry (simulator rand, episode counters) */
-  if (r) return r;
-  const int rw = p->info->rec_words;
-  uint32_t *recs = p->j_host;
-  /* parse everything (in parallel) before touching the pool so a bad document leaves it unchanged */
-  std::vector<BrkTable> new_brk(p->game == TBX_BREAKOUT ? n : 0);
-  std::vector<AmiTable> new_ami(p->game == TBX_AMIDAR ? n : 0);
-  try {
-    parallel_for(n, [&](int i) {
-      uint32_t *R = recs + (size_t)i * rw;
-      Value v = tbxjson::parse(json[i]);
-      if (p->game == TBX_BREAKOUT) { tbx::brk_state_from_json(v, *reinterpret_cast<BrkRec *>(R), new_brk[i]); tbx::brk_mark_delta_ok(p->cfg, new_brk[i]); }
-      else if (p->game == TBX_AMIDAR) tbx::ami_state_from_json(v, *reinterpret_cast<AmiRec *>(R), new_ami[i]);
-      else tbx::si_state_from_json(v, *reinterpret_cast<SiRec *>(R));
+  return guarded([&]() -> int {
+    int r = fetch_records(p, ids, n); /* keeps the fields JSON does not carry (simulator rand, episode counters) */
+    if (r) return r;
+    const int rw = p->info->rec_words;
+    uint32_t *recs = p->j_host;
+    with_game(p->game, [&](auto g) {
+      constexpr int G = decltype(g)::value;
+      typedef typename Traits<G>::Rec Rec;
+      /* parse everything (in parallel) before touching the pool so a bad document leaves it unchanged */
+      Tables<G> new_tabs(kTables<G> ? n : 0);
+      parallel_for(n, [&](int i) {
+        Rec &rec = *reinterpret_cast<Rec *>(recs + (size_t)i * rw);
+        const Value v = tbxjson::parse(json[i]);
+        if constexpr (kTables<G>) { state_from_json(v, rec, new_tabs[i]); fit_table(p->cfg, new_tabs[i]); }
+        else tbx::si_state_from_json(v, rec);
+      });
+      for (int i = 0; i < (int)new_tabs.size(); i++) reinterpret_cast<Rec *>(recs + (size_t)i * rw)->hdr.tbl = intern(tables<G>(p), new_tabs[i]);
     });
-  } catch (const std::exception &e) { return set_err(TBX_EJSON, e.what()); }
-  for (int i = 0; i < n; i++) {
-    uint32_t *R = recs + (size_t)i * rw;
-    if (p->game == TBX_BREAKOUT) reinterpret_cast<BrkRec *>(R)->hdr.tbl = intern(p->brk_tables, new_brk[i]);
-    else if (p->game == TBX_AMIDAR) reinterpret_cast<AmiRec *>(R)->hdr.tbl = intern(p->ami_tables, new_ami[i]);
-  }
-  r = upload_tables(p);
-  if (r) return r;
-  return store_records(p, n);
+    r = upload_tables(p);
+    if (r) return r;
+    return store_records(p, n);
+  });
 }
 
-static uint64_t *cfg_rand(tbx::Config &c) { return c.game == TBX_BREAKOUT ? c.brk.rand : c.game == TBX_AMIDAR ? c.ami.rand : c.si.rand; }
 int tbx_config_to_json(tbx_pool *p, char **out) {
   if (!p || !out) return set_err(TBX_EINVAL, "bad arguments");
   /* ctoybox's config_to_json shows the simulator as it is NOW: `rand` is the simulator rng that new_game has advanced.
@@ -925,42 +922,50 @@ int tbx_config_to_json(tbx_pool *p, char **out) {
                   cudaMemcpyDeviceToHost));
   cfg_rand(c)[0] = (uint64_t)w[0] | ((uint64_t)w[1] << 32);
   cfg_rand(c)[1] = (uint64_t)w[2] | ((uint64_t)w[3] << 32);
-  try { *out = dup_str(tbxjson::dump(tbx::config_to_json(c))); } catch (const std::exception &e) { return set_err(TBX_EJSON, e.what()); }
-  return *out ? TBX_OK : set_err(TBX_ENOMEM, "out of host memory");
+  return guarded([&] {
+    *out = dup_str(tbxjson::dump(tbx::config_to_json(c)));
+    return *out ? TBX_OK : set_err(TBX_ENOMEM, "out of host memory");
+  });
 }
 int tbx_config_from_json(tbx_pool *p, const char *json) {
   if (!p || !json) return set_err(TBX_EINVAL, "bad arguments");
-  tbx::Config c = p->cfg;
-  try { tbx::config_from_json(c, tbxjson::parse(json)); } catch (const std::exception &e) { return set_err(TBX_EJSON, e.what()); }
-  CK(cudaSetDevice(p->device));
-  CK(cudaDeviceSynchronize());
-  p->cfg = c;
-  drop_render_cache(p);
-  install_default_table(p);
-  int r = upload_tables(p);
-  if (r) return r;
-  /* write_config_json replaces the simulator, its rng included: every env's simulator rng restarts from the document's */
-  set_sim_rand_kernel<<<blocks(p->n, 256), 256>>>(p->planes, p->n, p->n_pad, cfg_rand(p->cfg)[0], cfg_rand(p->cfg)[1]);
-  CK(cudaGetLastError());
-  return upload_cfg(p);
+  return guarded([&]() -> int {
+    tbx::Config c = p->cfg;
+    tbx::config_from_json(c, tbxjson::parse(json));
+    CK(cudaSetDevice(p->device));
+    CK(cudaDeviceSynchronize());
+    p->cfg = c;
+    drop_render_cache(p);
+    install_default_table(p);
+    int r = upload_tables(p);
+    if (r) return r;
+    /* write_config_json replaces the simulator, its rng included: every env's simulator rng restarts from the document's */
+    set_sim_rand_kernel<<<blocks(p->n, 256), 256>>>(p->planes, p->n, p->n_pad, cfg_rand(p->cfg)[0], cfg_rand(p->cfg)[1]);
+    CK(cudaGetLastError());
+    return upload_cfg(p);
+  });
 }
 int tbx_schema_for_state(const char *game, char **out) {
   int g = tbx::game_from_name(game);
   if (g < 0 || !out) return set_err(TBX_EINVAL, "unknown game");
-  *out = dup_str(tbxjson::dump(tbx::schema_for_state(g)));
-  return *out ? TBX_OK : set_err(TBX_ENOMEM, "out of host memory");
+  return guarded([&] {
+    *out = dup_str(tbxjson::dump(tbx::schema_for_state(g)));
+    return *out ? TBX_OK : set_err(TBX_ENOMEM, "out of host memory");
+  });
 }
 int tbx_schema_for_config(const char *game, char **out) {
   int g = tbx::game_from_name(game);
   if (g < 0 || !out) return set_err(TBX_EINVAL, "unknown game");
-  try { *out = dup_str(tbxjson::dump(tbx::schema_for_config(g))); } catch (const std::exception &e) { return set_err(TBX_EJSON, e.what()); }
-  return *out ? TBX_OK : set_err(TBX_ENOMEM, "out of host memory");
+  return guarded([&] {
+    *out = dup_str(tbxjson::dump(tbx::schema_for_config(g)));
+    return *out ? TBX_OK : set_err(TBX_ENOMEM, "out of host memory");
+  });
 }
 int tbx_query_json(tbx_pool *p, int env, const char *query, const char *args_json, char **out) {
   if (!p || !query || !out) return set_err(TBX_EINVAL, "bad arguments");
   *out = 0;
   if (env < 0 || env >= p->n) return set_err(TBX_EINVAL, "env id out of range");
-  try {
+  return guarded([&]() -> int {
     Value args = tbxjson::parse(args_json ? args_json : "null");
     std::string q(query);
     const uint32_t *rec = 0;
@@ -971,39 +976,40 @@ int tbx_query_json(tbx_pool *p, int env, const char *query, const char *args_jso
       if (r) return r;
       rec = p->j_host;
       int tbl = reinterpret_cast<const BrkRec *>(rec)->hdr.tbl;
-      if (tbl < 0 || tbl >= (int)p->brk_tables.size()) return set_err(TBX_EINVAL, "corrupt table index");
-      brk = &p->brk_tables[tbl];
+      if (tbl < 0 || tbl >= (int)tables<TBX_BREAKOUT>(p).size()) return set_err(TBX_EINVAL, "corrupt table index");
+      brk = &tables<TBX_BREAKOUT>(p)[tbl];
     }
     Value res = tbx::query_json(p->game, rec, brk, q, args);
     *out = dup_str(tbxjson::dump(res));
-  } catch (const std::exception &e) { return set_err(TBX_EJSON, e.what()); }
-  return *out ? TBX_OK : set_err(TBX_ENOMEM, "out of host memory");
+    return *out ? TBX_OK : set_err(TBX_ENOMEM, "out of host memory");
+  });
 }
 
 } /* extern "C" */
 
 /* ---- device-resident state snapshots (tbx_snapshot.cuh) */
 static const int TBX_WRAP_WORDS = 5; /* the wrapper words of tbx_wrap.cuh */
-static size_t table_bytes(const tbx_pool *p) { return p->game == TBX_BREAKOUT ? sizeof(BrkTable) : p->game == TBX_AMIDAR ? sizeof(AmiTable) : 0; }
-static int table_count(const tbx_pool *p) {
-  return p->game == TBX_BREAKOUT ? (int)p->brk_tables.size() : p->game == TBX_AMIDAR ? (int)p->ami_tables.size() : 0;
-}
-static const void *table_data(const tbx_pool *p) {
-  return p->game == TBX_BREAKOUT ? (const void *)p->brk_tables.data() : p->game == TBX_AMIDAR ? (const void *)p->ami_tables.data() : 0;
+/* the pool's interned tables as bytes */
+struct TableView { const void *data; size_t bytes; int count; };
+static TableView table_view(const tbx_pool *p) {
+  return with_game(p->game, [&](auto g) {
+    constexpr int G = decltype(g)::value;
+    const auto &t = tables<G>(p);
+    return TableView{t.data(), kTables<G> ? sizeof t[0] : 0, (int)t.size()};
+  });
 }
 
 static int state_tables(const tbx_pool *p, int rows, void *out, size_t cap, size_t *size) {
-  const tbx_state_blob_header h = {TBX_STATE_MAGIC, TBX_STATE_FORMAT, (uint32_t)p->game, (uint32_t)rows, (uint32_t)table_bytes(p),
-                                   (uint32_t)table_count(p)};
+  const TableView t = table_view(p);
+  const tbx_state_blob_header h = {TBX_STATE_MAGIC, TBX_STATE_FORMAT, (uint32_t)p->game, (uint32_t)rows, (uint32_t)t.bytes, (uint32_t)t.count};
   const size_t need = sizeof h + (size_t)h.table_bytes * h.table_count;
   *size = need;
   if (!out) return TBX_OK;
   if (cap < need) return set_err(TBX_EINVAL, "the tables blob needs " + std::to_string(need) + " bytes, the buffer holds " + std::to_string(cap));
   memcpy(out, &h, sizeof h);
-  if (need > sizeof h) memcpy((char *)out + sizeof h, table_data(p), need - sizeof h);
+  if (need > sizeof h) memcpy((char *)out + sizeof h, t.data, need - sizeof h);
   return TBX_OK;
 }
-
 /* the pool side of a copy: planes, then (wrapped env) the wrapper words */
 static SnapSide pool_side(const tbx_pool *p, uint32_t *wstate, const int32_t *ids) {
   SnapSide s;
@@ -1046,37 +1052,32 @@ static int state_save(tbx_pool *p, uint32_t *wstate, const int32_t *ids, int k, 
  * blob indices to pool indices; that path synchronises the device. */
 static int snapshot_remap(tbx_pool *p, const uint8_t *tabs, int count, const int32_t **remap) {
   *remap = 0;
-  const size_t tb = table_bytes(p);
-  if (count == 0 || (count <= table_count(p) && memcmp(tabs, table_data(p), (size_t)count * tb) == 0)) return TBX_OK;
-  std::vector<int32_t> map(count);
+  std::vector<int32_t> map;
   bool identity = true;
-  for (int i = 0; i < count; i++) {
-    if (p->game == TBX_BREAKOUT) {
-      BrkTable t;
-      memcpy(&t, tabs + (size_t)i * tb, tb);
-      tbx::brk_mark_delta_ok(p->cfg, t);
-      map[i] = intern(p->brk_tables, t);
-    } else {
-      AmiTable t;
-      memcpy(&t, tabs + (size_t)i * tb, tb);
-      map[i] = intern(p->ami_tables, t);
+  with_game(p->game, [&](auto g) {
+    constexpr int G = decltype(g)::value;
+    if constexpr (kTables<G>) {
+      auto &v = tables<G>(p);
+      typename Traits<G>::Table t;
+      if (count <= (int)v.size() && memcmp(tabs, v.data(), (size_t)count * sizeof t) == 0) return;
+      for (int i = 0; i < count; i++) {
+        memcpy(&t, tabs + (size_t)i * sizeof t, sizeof t);
+        fit_table(p->cfg, t);
+        map.push_back(intern(v, t));
+        identity = identity && map[i] == i;
+      }
     }
-    identity = identity && map[i] == i;
-  }
+  });
+  if (map.empty()) return TBX_OK;
   int r = upload_tables(p);
   if (r) return r;
   if (identity) return TBX_OK;
   CK(cudaDeviceSynchronize()); /* an earlier load may still read the remap buffer */
-  if (p->remap_cap < count) {
-    cudaFree(p->d_remap); p->d_remap = 0; p->remap_cap = 0;
-    CK(cudaMalloc(&p->d_remap, (size_t)count * sizeof(int32_t)));
-    p->remap_cap = count;
-  }
+  CK(p->d_remap.grow(count));
   CK(cudaMemcpy(p->d_remap, map.data(), (size_t)count * sizeof(int32_t), cudaMemcpyHostToDevice));
   *remap = p->d_remap;
   return TBX_OK;
 }
-
 static int state_load(tbx_pool *p, uint32_t *wstate, const uint32_t *snap, int k_snap, const int32_t *cols, const int32_t *ids, int n, const void *blob,
                       size_t blob_bytes, cudaStream_t s) {
   const int rows = p->info->rec_words + (wstate ? TBX_WRAP_WORDS : 0);
@@ -1090,19 +1091,19 @@ static int state_load(tbx_pool *p, uint32_t *wstate, const uint32_t *snap, int k
   if (h.game != (uint32_t)p->game) return set_err(TBX_EINVAL, std::string("state snapshot: saved from another game, this pool runs ") + p->info->name);
   if (h.rows != (uint32_t)rows)
     return set_err(TBX_EINVAL, "state snapshot: " + std::to_string(h.rows) + " rows per env, this " + (wstate ? "wrapped env" : "pool") + " needs " + std::to_string(rows));
-  if (h.table_bytes != table_bytes(p) || h.table_count > (1u << 20) || blob_bytes != sizeof h + (size_t)h.table_bytes * h.table_count)
+  if (h.table_bytes != table_view(p).bytes || h.table_count > (1u << 20) || blob_bytes != sizeof h + (size_t)h.table_bytes * h.table_count)
     return set_err(TBX_EINVAL, "state snapshot: the tables blob's size does not match its header");
   if (n == 0) return TBX_OK;
   CK(cudaSetDevice(p->device));
   const int32_t *remap = 0;
   int r = snapshot_remap(p, (const uint8_t *)blob + sizeof h, (int)h.table_count, &remap);
   if (r) return r;
-  if (ids && !p->d_owner) CK(cudaMalloc(&p->d_owner, (size_t)p->n_pad * sizeof(int32_t)));
+  if (ids) CK(p->d_owner.grow(p->n_pad));
   SnapArgs a;
   a.rows = rows;
   a.src = snap_side(const_cast<uint32_t *>(snap), k_snap, rows, cols); a.dst = pool_side(p, wstate, ids);
   a.k = n; a.tbl_row = p->game == TBX_SPACE_INVADERS ? -1 : TBX_HW(tbl); a.tbl_lim = (int)h.table_count; a.remap = remap;
-  a.owner = ids ? p->d_owner : 0; a.bad = p->d_bad + 1;
+  a.owner = ids ? p->d_owner.get() : 0; a.bad = p->d_bad + 1;
   if (a.owner) CK(cudaMemsetAsync(p->d_owner, 0xff, (size_t)p->n_pad * sizeof(int32_t), s)); /* -1: no entry yet */
   return launch_snap_copy(a, s);
 }
@@ -1130,12 +1131,12 @@ int tbx_wrap_state_save(tbx_wrap *w, const int32_t *ids_dev, int k, uint32_t *sn
 int tbx_state_load(tbx_pool *p, const uint32_t *snap_dev, int k_snap, const int32_t *cols_dev, const int32_t *ids_dev, int n, const void *tables_blob,
                    size_t blob_bytes, void *stream) {
   if (!p) return set_err(TBX_EINVAL, "pool is NULL");
-  return state_load(p, 0, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream);
+  return guarded([&] { return state_load(p, 0, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream); });
 }
 int tbx_wrap_state_load(tbx_wrap *w, const uint32_t *snap_dev, int k_snap, const int32_t *cols_dev, const int32_t *ids_dev, int n, const void *tables_blob,
                         size_t blob_bytes, void *stream) {
   if (!w) return set_err(TBX_EINVAL, "wrap is NULL");
-  return state_load(w->pool, w->wstate, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream);
+  return guarded([&] { return state_load(w->pool, w->wstate, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream); });
 }
 
 } /* extern "C" */
