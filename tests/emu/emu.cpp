@@ -14,6 +14,7 @@
 #include "../../toybox_b200/csrc/tbx_direct.h"
 #include <string.h>
 #include <stdlib.h>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -320,6 +321,40 @@ int emu_si_score_strip(Emu *e, int out_w, int out_h, uint8_t *out) {
       if (db < 0) db = 10;
       out[dy * out_w + dx] = A.sc_px[tc][da][db][tr];
     }
+  return 0;
+}
+
+/* Which direct INTER_AREA kernel tables the library builds for this config at out_w x out_h (tbx_direct_build runs the same
+ * builders): out[0] = ok (0: every env of the size goes to the tile kernel), then Breakout nrows / n_cls, Space Invaders
+ * n_sets (0: no sprite patch tables) / sc_ok (0: no score strip), unused entries 0; out[3], out[4] = the plan's taps per output
+ * column / row (the tile kernel's dual mode takes at most 5 x 4).  Returns -1 for a size the library refuses. */
+int emu_direct_info(Emu *e, int out_w, int out_h, int32_t *out) {
+  const int W = e->info->width, H = e->info->height;
+  tbx::ResizeTab rs;
+  TbxAreaPlan pl;
+  try { tbx::build_resize(W, H, out_w, out_h, rs); } catch (const std::exception &ex) { g_err = ex.what(); return -1; }
+  if (!tbx::build_area_plan(rs, pl)) { g_err = "size pair outside the fused kernel's limits"; return -1; }
+  const BrkTable *dt = e->game == TBX_BREAKOUT ? &e->brk_tables[e->cfg.brk.default_tbl] : 0;
+  std::vector<uint32_t> rgba((size_t)W * H);
+  std::vector<uint8_t> base0((size_t)W * H);
+  tbx::build_base_frame(e->cfg, dt, 0, rgba.data());
+  tbx::frame_to_gray(rgba.data(), W * H, base0.data());
+  out[0] = out[1] = out[2] = 0;
+  out[3] = pl.tx; out[4] = pl.ty;
+  if (e->game == TBX_BREAKOUT) {
+    std::unique_ptr<TbxBrkDirect> A(new TbxBrkDirect);
+    tbx::build_brk_direct(e->cfg, *dt, rs, pl, base0.data(), *A);
+    out[0] = A->ok; out[1] = A->nrows; out[2] = A->n_cls;
+  } else if (e->game == TBX_AMIDAR) {
+    std::unique_ptr<TbxAmiDirect> A(new TbxAmiDirect);
+    tbx::build_ami_direct(e->cfg, rs, pl, *A);
+    out[0] = A->ok;
+  } else {
+    std::unique_ptr<TbxSiDirect> A(new TbxSiDirect);
+    std::vector<TbxSpritePatch> patches;
+    tbx::build_si_direct(e->cfg, rs, pl, base0.data(), *A, patches);
+    out[0] = A->ok; out[1] = A->n_sets; out[2] = A->sc_ok;
+  }
   return 0;
 }
 

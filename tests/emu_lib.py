@@ -127,6 +127,22 @@ class Emu:
             raise ValueError(self.L.emu_last_error().decode())
         return None if rc else out
 
+    def direct_info(self, out_w=84, out_h=84):
+        """The direct INTER_AREA kernel's tables for this config at out_w x out_h, as the library builds them: {"ok"} for
+        every game, plus {"nrows", "n_cls"} for Breakout and {"n_sets", "sc_ok"} for Space Invaders.  ok == 0: the tile
+        kernel renders every env of that size; n_sets == 0: no sprite patch tables; sc_ok == 0: no score strip.  "taps" is
+        the resize plan's (taps per output column, taps per output row); wrapped observations take at most (5, 4)."""
+        out = (C.c_int32 * 5)()
+        self.L.emu_direct_info.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p]
+        if self.L.emu_direct_info(self.h, out_w, out_h, out) != 0:
+            raise ValueError(self.L.emu_last_error().decode())
+        info = {"ok": out[0], "taps": (out[3], out[4])}
+        if self.game == "breakout":
+            info.update(nrows=out[1], n_cls=out[2])
+        elif self.game == "space_invaders":
+            info.update(n_sets=out[1], sc_ok=out[2])
+        return info
+
     def state_json(self):
         return json.loads(_take(self.L.emu_state_to_json(self.h)))
 

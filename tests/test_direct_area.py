@@ -128,3 +128,39 @@ def test_si_score_strip_table_equals_full_resize(size):
         bad = np.argwhere(got != want)
         assert bad.size == 0, (size, v, bad[:4], got[tuple(bad[0])], want[tuple(bad[0])])
     assert n_table > 0 or size != (84, 84)          # the table exists at the size the benchmark uses
+
+
+def test_direct_coverage_of_gpu_tier_cases():
+    """The direct kernels' tables exist for every (config, output size) that test_gpu_area_coverage.py renders through them,
+    with the brick rows and Space Invaders sprite patch sets it claims, and the wrapped sizes it uses stay within the dual
+    tile kernel's 5 x 4 taps.  Over every output size the library accepts, Space Invaders' direct kernel runs both with and
+    without sprite patch tables but always with the score strip.  A builder change that drops coverage fails here."""
+    import test_gpu_area_coverage as G
+    for game, sizes in G.A_SIZES.items():
+        for size in sizes:
+            assert emu_lib.Emu(game).direct_info(*size)["ok"] == 1, (game, size)
+    for game, names in (("breakout", list(G.BRK_CONFIGS)), ("amidar", G.AMI_CONFIGS), ("space_invaders", G.SI_CONFIGS)):
+        for name in names:
+            e = emu_lib.Emu(game, G._config(game, name))
+            for size in G.C_SIZES[game]:
+                info = e.direct_info(*size)
+                assert info["ok"] == 1, (game, name, size, info)
+                if game == "breakout":
+                    assert info["nrows"] == G.BRK_CONFIGS[name], (name, size, info)
+                if game == "space_invaders":
+                    assert (info["n_sets"], info["sc_ok"]) == (G.SI_PATCHES[size], 1), (name, size, info)
+    for game, sizes in G.D_SIZES.items():
+        for size in sizes:
+            tx, ty = emu_lib.Emu(game).direct_info(*size)["taps"]
+            assert tx <= 5 and ty <= 4, (game, size, tx, ty)
+    e = emu_lib.Emu("space_invaders")
+    seen = set()
+    for w in range(4, 129, 4):                   # the direct kernel needs a width that is a multiple of 4
+        for h in range(1, 129):
+            try:
+                info = e.direct_info(w, h)
+            except ValueError:                   # a size the library refuses
+                continue
+            if info["ok"]:
+                seen.add((info["n_sets"] > 0, info["sc_ok"]))
+    assert seen == {(True, 1), (False, 1)}, seen
