@@ -32,8 +32,10 @@ enum {
   TBX_OBS_RGBA = 0,  /* uint8[N][H][W][4]  Toybox.get_state() with grayscale=False  (envs/atari/base.py:109) */
   TBX_OBS_RGB = 1,   /* uint8[N][H][W][3]  Toybox.get_rgb_frame()                   (envs/atari/base.py:164) */
   TBX_OBS_GRAY = 2,  /* uint8[N][H][W]     Toybox.get_state() with grayscale=True   (envs/atari/base.py:109) */
-  TBX_OBS_GRAY_AREA = 3 /* uint8[N][out_h][out_w]  cv2.resize(gray, (out_w,out_h), INTER_AREA) = baselines WarpFrame
+  TBX_OBS_GRAY_AREA = 3, /* uint8[N][out_h][out_w]  cv2.resize(gray, (out_w,out_h), INTER_AREA) = baselines WarpFrame
                            (baselines/baselines/common/atari_wrappers.py:230-244), fused into the render */
+  TBX_OBS_RGB_AREA = 4  /* uint8[N][out_h][out_w][3]  cv2.resize(get_rgb_frame(), (out_w,out_h), INTER_AREA): WarpFrame(grayscale=False),
+                           64x64 / 84x84 colour observations; the same output sizes as TBX_OBS_GRAY_AREA */
 };
 
 const char *tbx_last_error(void);
@@ -88,7 +90,7 @@ int tbx_step_random(tbx_pool *pool, uint64_t seed, uint64_t env0, uint64_t t, in
 int tbx_check(tbx_pool *pool, void *stream);
 
 /* render_current_frame: Toybox.get_state() / get_rgb_frame() for every env (envs/atari/base.py:109,164).
- * dst_dev: N * tbx_obs_bytes() bytes, 16-byte aligned.  out_w/out_h are used by TBX_OBS_GRAY_AREA only. */
+ * dst_dev: N * tbx_obs_bytes() bytes, 16-byte aligned.  out_w/out_h are used by TBX_OBS_GRAY_AREA and TBX_OBS_RGB_AREA only. */
 int tbx_render(tbx_pool *pool, uint8_t *dst_dev, int obs_mode, int out_w, int out_h, void *stream);
 
 /* state_lives / state_score / state_level / state_game_over (envs/atari/base.py:20-27,136,145).  Device

@@ -37,18 +37,21 @@ template <class F> static int guarded(F &&f) {
   }
 }
 
-/* render resources of one INTER_AREA output size */
+/* render resources of one INTER_AREA output size: the plan, then those of each layout, built on its first render */
 struct AreaRes {
   TbxAreaPlan plan;
   Buf<TbxAreaPlan> d_plan;
-  Buf<uint8_t> d_base_out[2];       /* down-samples of base frames 0/1 */
+  Buf<uint8_t> d_base_out[2];       /* gray: down-samples of base frames 0/1 */
   Buf<TbxDigitPatch> d_patches[2];
   Buf<uint8_t> d_direct, d_direct2; /* tables of the direct kernel (tbx_direct.h), empty when the pair is not covered */
+  Buf<uint8_t> d_rgb_out[2];        /* RGB: interleaved down-samples of base frames 0/1 */
 };
-/* base frames 0/1 of the current config (see tbx_render.cuh): gray, RGBA and packed RGB on the device, gray on the host */
+/* base frames 0/1 of the current config (see tbx_render.cuh): gray, RGBA and packed RGB on the device, gray on the host;
+ * for the RGB INTER_AREA layout also R, G, B planes of W x H each (the tile kernel reads one channel's source window in
+ * 4-byte words), on the device and the host, built on the first such render */
 struct BaseFrames {
-  Buf<uint8_t> gray[2], rgba[2], rgb[2];
-  std::vector<uint8_t> h_gray[2];
+  Buf<uint8_t> gray[2], rgba[2], rgb[2], planar[2];
+  std::vector<uint8_t> h_gray[2], h_planar[2];
 };
 /* tbx_step_host's stream and staging */
 struct HostStaging {
@@ -265,8 +268,9 @@ size_t tbx_obs_bytes(const tbx_pool *p, int mode, int out_w, int out_h) {
     case TBX_OBS_RGB: return px * 3;
     case TBX_OBS_GRAY: return px;
     case TBX_OBS_GRAY_AREA:
+    case TBX_OBS_RGB_AREA:
       if (out_w < 1 || out_h < 1 || out_w > p->info->width || out_h > p->info->height || out_w > TBX_RS_MAX_DST || out_h > TBX_RS_MAX_DST) return 0;
-      return (size_t)out_w * out_h;
+      return (size_t)out_w * out_h * (mode == TBX_OBS_RGB_AREA ? 3 : 1);
   }
   return 0;
 }
@@ -368,30 +372,72 @@ static int ensure_base(tbx_pool *p) {
   p->base = std::move(base);
   return TBX_OK;
 }
-/* the INTER_AREA resources of one output size, built on first use; kept only once every buffer is in place */
-static int ensure_area(tbx_pool *p, int out_w, int out_h, const AreaRes **out) {
+/* base frames 0/1 as planes for the RGB INTER_AREA layout; kept only once both are in place */
+static int ensure_planar(tbx_pool *p) {
+  BaseFrames &bf = *p->base;
+  if (bf.planar[0]) return TBX_OK;
+  const int npix = p->info->width * p->info->height;
+  std::vector<uint32_t> rgba(npix);
+  std::vector<uint8_t> h[2];
+  Buf<uint8_t> d[2];
+  for (int b = 0; b < 2; b++) {
+    tbx::build_base_frame(p->cfg, brk_default(p), b, rgba.data());
+    h[b].resize((size_t)npix * 3);
+    for (int c = 0; c < 3; c++)
+      for (int i = 0; i < npix; i++) h[b][(size_t)c * npix + i] = (uint8_t)(rgba[i] >> (8 * c));
+    CK(d[b].upload(h[b].data(), h[b].size()));
+  }
+  for (int b = 0; b < 2; b++) { bf.planar[b] = std::move(d[b]); bf.h_planar[b] = std::move(h[b]); }
+  return TBX_OK;
+}
+/* the INTER_AREA resources of one output size and layout, built on first use; each part is kept only once every buffer
+ * of it is in place */
+static int ensure_area(tbx_pool *p, int out_w, int out_h, bool rgb, const AreaRes **out) {
   auto key = std::make_pair(out_w, out_h);
   auto it = p->area.find(key);
+  if (it != p->area.end() && (rgb ? it->second.d_rgb_out[0] : it->second.d_base_out[0])) { *out = &it->second; return TBX_OK; }
+  tbx::ResizeTab rs;
+  try { tbx::build_resize(p->info->width, p->info->height, out_w, out_h, rs); }
+  catch (const std::exception &e) { return set_err(TBX_EINVAL, e.what()); }
   if (it == p->area.end()) {
-    tbx::ResizeTab rs;
     AreaRes r;
-    try { tbx::build_resize(p->info->width, p->info->height, out_w, out_h, rs); }
-    catch (const std::exception &e) { return set_err(TBX_EINVAL, e.what()); }
     if (!tbx::build_area_plan(rs, r.plan)) return set_err(TBX_EINVAL, "resize: the fused kernel supports destinations up to 128x128 with at most 8 taps per axis");
     CK(r.d_plan.upload(&r.plan, 1));
-    for (int b = 0; b < 2; b++) {
-      const uint8_t *gray = p->base->h_gray[b].data();
-      std::vector<uint8_t> base_out(((size_t)out_w * out_h + 15) & ~(size_t)15, 0);
-      tbx::area_resize(gray, rs, base_out.data());
-      CK(r.d_base_out[b].upload(base_out.data(), base_out.size()));
-      std::vector<TbxDigitPatch> patches((size_t)TBX_DP_SLOTS * 10);
-      tbx::build_digit_patches(p->cfg, brk_default(p), rs, r.plan, gray, patches.data());
-      CK(r.d_patches[b].upload(patches.data(), patches.size()));
-    }
-    CK(tbx_direct_build(p->cfg, brk_default(p), rs, r.plan, p->base->h_gray[0].data(), r.d_direct, r.d_direct2));
     it = p->area.emplace(key, std::move(r)).first;
   }
-  *out = &it->second;
+  AreaRes &ar = it->second;
+  if (!rgb && !ar.d_base_out[0]) {
+    Buf<uint8_t> base_out[2], direct, direct2;
+    Buf<TbxDigitPatch> patches[2];
+    for (int b = 0; b < 2; b++) {
+      const uint8_t *gray = p->base->h_gray[b].data();
+      std::vector<uint8_t> h(((size_t)out_w * out_h + 15) & ~(size_t)15, 0);
+      tbx::area_resize(gray, rs, h.data());
+      CK(base_out[b].upload(h.data(), h.size()));
+      std::vector<TbxDigitPatch> hp((size_t)TBX_DP_SLOTS * 10);
+      tbx::build_digit_patches(p->cfg, brk_default(p), rs, ar.plan, gray, hp.data());
+      CK(patches[b].upload(hp.data(), hp.size()));
+    }
+    CK(tbx_direct_build(p->cfg, brk_default(p), rs, ar.plan, p->base->h_gray[0].data(), direct, direct2));
+    for (int b = 0; b < 2; b++) { ar.d_base_out[b] = std::move(base_out[b]); ar.d_patches[b] = std::move(patches[b]); }
+    ar.d_direct = std::move(direct); ar.d_direct2 = std::move(direct2);
+  }
+  if (rgb && !ar.d_rgb_out[0]) { /* the per-channel resize of the planar base frames, interleaved */
+    int r = ensure_planar(p);
+    if (r) return r;
+    const size_t npix = (size_t)p->info->width * p->info->height, nout = (size_t)out_w * out_h;
+    Buf<uint8_t> rgb_out[2];
+    std::vector<uint8_t> plane(nout), h((nout * 3 + 15) & ~(size_t)15, 0);
+    for (int b = 0; b < 2; b++) {
+      for (int c = 0; c < 3; c++) {
+        tbx::area_resize(p->base->h_planar[b].data() + c * npix, rs, plane.data());
+        for (size_t i = 0; i < nout; i++) h[3 * i + c] = plane[i];
+      }
+      CK(rgb_out[b].upload(h.data(), h.size()));
+    }
+    for (int b = 0; b < 2; b++) ar.d_rgb_out[b] = std::move(rgb_out[b]);
+  }
+  *out = &ar;
   return TBX_OK;
 }
 
@@ -432,25 +478,30 @@ template <int GAME, int PIX> static int launch_native(const RenderArgs &a, const
   CK(cudaGetLastError());
   return TBX_OK;
 }
-/* INTER_AREA, one warp per env (tbx_render_area.cuh) */
-template <int GAME, int TX, int TY, bool DUAL> static int launch_area_tile(const RenderArgs &a, const typename Traits<GAME>::Cfg &cfg, const TbxAreaPlan &plan, int smem, cudaStream_t s) {
-  CK((cudaFuncSetAttribute(area_tile_kernel<GAME, TX, TY, DUAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
+/* INTER_AREA, one warp per env (tbx_render_area.cuh); RGB: the single-frame RGB mode */
+template <int GAME, int TX, int TY, bool DUAL, bool RGB = false>
+static int launch_area_tile(const RenderArgs &a, const typename Traits<GAME>::Cfg &cfg, const TbxAreaPlan &plan, int smem, cudaStream_t s) {
+  CK((cudaFuncSetAttribute(area_tile_kernel<GAME, TX, TY, DUAL, RGB>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
   /* env-list mode (the envs the direct kernel handed over, normally none): a small grid walks the list */
   const int grid = a.env_list ? (blocks(a.n, TBX_EPC) < 296 ? blocks(a.n, TBX_EPC) : 296) : blocks(a.n, TBX_EPC);
-  area_tile_kernel<GAME, TX, TY, DUAL><<<grid, TBX_TILE_THREADS, smem, s>>>(a, cfg, plan);
+  area_tile_kernel<GAME, TX, TY, DUAL, RGB><<<grid, TBX_TILE_THREADS, smem, s>>>(a, cfg, plan);
   CK(cudaGetLastError());
   return TBX_OK;
 }
 
-/* INTER_AREA: the direct kernel where it covers the pair, then the tile kernel */
-static int render_area(tbx_pool *p, RenderArgs &a, int out_w, int out_h, cudaStream_t s) {
+/* INTER_AREA: the direct kernel where it covers the pair, then the tile kernel; RGB (single frames): the tile kernel's
+ * RGB mode alone */
+static int render_area(tbx_pool *p, RenderArgs &a, int out_w, int out_h, bool rgb, cudaStream_t s) {
   const AreaRes *ar = 0;
-  int r = ensure_area(p, out_w, out_h, &ar);
+  int r = ensure_area(p, out_w, out_h, rgb, &ar);
   if (r) return r;
   const TbxAreaPlan &plan = ar->plan;
   const bool dual = a.planes2 != 0;
-  a.base_out[0] = ar->d_base_out[0]; a.base_out[1] = ar->d_base_out[1]; a.plan = ar->d_plan;
-  {
+  a.plan = ar->d_plan;
+  if (rgb) {
+    for (int b = 0; b < 2; b++) { a.base[b] = p->base->planar[b]; a.base_out[b] = ar->d_rgb_out[b]; a.patches[b] = 0; }
+  } else {
+    a.base_out[0] = ar->d_base_out[0]; a.base_out[1] = ar->d_base_out[1];
     const char *env = getenv("TBX_AREA_DIGIT_CACHE");
     const bool on = !(env && atoi(env) == 0);
     a.patches[0] = on ? ar->d_patches[0].get() : 0; a.patches[1] = on ? ar->d_patches[1].get() : 0;
@@ -480,7 +531,7 @@ static int render_area(tbx_pool *p, RenderArgs &a, int out_w, int out_h, cudaStr
   if (const char *env = getenv("TBX_AREA_LCAP")) a.list_cap = atoi(env); /* tests: small lists force the sweep / per-tile paths */
   if (a.list_cap < 1 || a.list_cap > TBX_TILE_LCAP) a.list_cap = TBX_TILE_LCAP;
   a.tile_bytes = align16(stride * rows);
-  a.warp_bytes = TBX_TILE_LCAP * 20 + 32 + a.tile_bytes * (dual ? 2 : 1);
+  a.warp_bytes = TBX_TILE_LCAP * (rgb ? 24 : 20) + 32 + a.tile_bytes * (dual ? 2 : 1); /* list, extents (, colours), tile mask, scratch */
   const int smem = a.smem_canvas + (TBX_TILE_THREADS / 32) * a.warp_bytes;
   int smem_optin = 0;
   CK(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, p->device));
@@ -490,7 +541,7 @@ static int render_area(tbx_pool *p, RenderArgs &a, int out_w, int out_h, cudaStr
   /* Direct kernel first (tbx_render_direct.cuh; TBX_AREA_KERNEL=tile turns it off): closed forms for the envs they
    * cover, the rest are listed and rendered by the tile kernel in env-list mode right after (usually an empty list) */
   const char *ksel = getenv("TBX_AREA_KERNEL");
-  if (ar->d_direct && !dual && !(ksel && !strcmp(ksel, "tile"))) {
+  if (ar->d_direct && !dual && !rgb && !(ksel && !strcmp(ksel, "tile"))) {
     if (!p->d_fb) { /* the counters start at zero; the kernels leave them so */
       Buf<int32_t> fb;
       CK(fb.alloc((size_t)p->n_pad + 8));
@@ -509,6 +560,7 @@ static int render_area(tbx_pool *p, RenderArgs &a, int out_w, int out_h, cudaStr
     const auto &cfg = game_cfg<G>(p->cfg);
     return with_taps<8>(plan.tx, plan.ty, [&](auto X, auto Y) {
       constexpr int TX = decltype(X)::value, TY = decltype(Y)::value;
+      if (rgb) return launch_area_tile<G, TX, TY, false, true>(a, cfg, plan, smem, s);
       if constexpr (TX == 8) return launch_area_tile<G, 8, 8, false>(a, cfg, plan, smem, s); /* single frames only (checked above) */
       else return dual ? launch_area_tile<G, TX, TY, true>(a, cfg, plan, smem, s) : launch_area_tile<G, TX, TY, false>(a, cfg, plan, smem, s);
     });
@@ -576,7 +628,8 @@ static int render_impl(tbx_pool *p, uint8_t *dst, int mode, int out_w, int out_h
   for (int b = 0; b < 2; b++) a.base[b] = pix == 4 ? p->base->rgba[b] : pix == 3 ? p->base->rgb[b] : p->base->gray[b];
   a.smem_canvas = align16(p->info->rec_words * TBX_EPC * 4) * (dual ? 2 : 1);
   cudaStream_t s = (cudaStream_t)stream;
-  return mode == TBX_OBS_GRAY_AREA ? render_area(p, a, out_w, out_h, s) : render_native(p, a, mode, s);
+  if (mode == TBX_OBS_GRAY_AREA || mode == TBX_OBS_RGB_AREA) return render_area(p, a, out_w, out_h, mode == TBX_OBS_RGB_AREA, s);
+  return render_native(p, a, mode, s);
 }
 
 extern "C" {

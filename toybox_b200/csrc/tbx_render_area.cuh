@@ -20,6 +20,10 @@
  * are painted lane-parallel; everything else is painted by the whole warp, one entry at a time, in draw order.
  * The kernel renders every plan the library accepts: it is instantiated for 3..5 x 3..4 taps, and for 8 x 8 taps
  * (single frames only) for the plans with more; surplus taps carry zero weight.
+ * RGB mode (RGB = true, single frames): the list, hit tests, sweeps and per-tile rebuild are colour-blind and
+ * shared; each entry also keeps its 24-bit colour, and every run is loaded, painted and resolved once per channel from
+ * planar base frames, so the scratch window keeps its gray size.  The output is interleaved RGB, = cv2's 3-channel
+ * INTER_AREA (which is the per-channel resize).
  */
 #ifndef TBX_RENDER_AREA_CUH
 #define TBX_RENDER_AREA_CUH
@@ -130,8 +134,9 @@ __device__ __forceinline__ void tile_load(uint8_t *tile, int stride, const uint8
 }
 
 /* recompute output pixels [dx0,dx1] x [dy0,dy1] from the scratch and patch them into the frame: TX x TY taps in cv2's
- * order; surplus taps carry zero weights and may read scratch bytes outside the copied window (x + 0*b == x here) */
-template <int TX, int TY>
+ * order; surplus taps carry zero weights and may read scratch bytes outside the copied window (x + 0*b == x here).
+ * CH: bytes per output pixel (3: `out` points at the channel's byte of pixel 0) */
+template <int TX, int TY, int CH = 1>
 __device__ __forceinline__ void tile_resolve(const uint8_t *tile, int stride, int wx0, int wy0, int dx0, int dx1, int dy0, int dy1, int dw,
                                              const TbxAreaPlan *__restrict__ plan, uint8_t *out, int lane) {
   const int ncol = dx1 - dx0 + 1;
@@ -157,7 +162,7 @@ __device__ __forceinline__ void tile_resolve(const uint8_t *tile, int stride, in
         v = k == 0 ? bh : tbx_fadd(v, bh);
       }
       const int iv = tbx_f2i_rn_small(v);
-      if (colok) out[dy * dw + dx] = (uint8_t)(iv < 0 ? 0 : iv > 255 ? 255 : iv);
+      if (colok) out[(dy * dw + dx) * CH] = (uint8_t)(iv < 0 ? 0 : iv > 255 ? 255 : iv);
     }
   }
 }
@@ -174,14 +179,16 @@ __device__ __forceinline__ void tile_max(uint8_t *tile, const uint8_t *tile2, in
     }
 }
 
-__device__ __forceinline__ void paint_entry_coop(uint8_t *tile, int stride, int wx0, int wy0, int wx1, int wy1, const uint4 &q, const uint32_t *R, int lane) {
+/* val: the byte painted (the entry's gray, or one component of its colour in RGB mode) */
+__device__ __forceinline__ void paint_entry_coop(uint8_t *tile, int stride, int wx0, int wy0, int wx1, int wy1, const uint4 &q, uint32_t val, const uint32_t *R, int lane) {
   paint_tile(tile, stride, wx0, wy0, wx1, wy1, (int16_t)(q.x & 0xffffu), (int16_t)(q.x >> 16), (int16_t)(q.y & 0xffffu), (int16_t)(q.y >> 16),
-             q.z & 255u, q.w, R, lane);
+             val, q.w, R, lane);
 }
 
 /* One tile row with more entries than the list holds: every tile of the row re-builds the primitives and paints
- * those that touch it, strictly in draw order (slow, but always correct). */
-template <int GAME, int TX, int TY>
+ * those that touch it, strictly in draw order (slow, but always correct).  CH = 3: once per channel, from the planar base
+ * frames (channel c at bfr + c * W * H), into the interleaved frame. */
+template <int GAME, int TX, int TY, int CH = 1>
 __device__ __noinline__ void tile_row_rebuild(const uint32_t *R, const uint32_t *R2, const typename Traits<GAME>::Cfg &cfg, const typename Traits<GAME>::Table *tables,
                                               int base, int base2, const uint8_t *bfr, const uint8_t *bfr2, const TbxAreaPlan *__restrict__ plan, const TbxAreaPlan &cp,
                                               uint8_t *tile, uint8_t *tile2, int stride,
@@ -194,11 +201,13 @@ __device__ __noinline__ void tile_row_rebuild(const uint32_t *R, const uint32_t 
   for (int dxA = 0; dxA < dw; dxA += 16) {
     const int dxL = min(dxA + 15, dw - 1);
     const int wx0 = cp.xs0[dxA] & ~3, wx1 = min(W, ((int)cp.xs0[dxL] + TX + 3) & ~3);
+#pragma unroll 1
+    for (int ch = 0; ch < CH; ch++) {
     for (int st = 0; st < (R2 ? 2 : 1); st++) {
       const uint32_t *Rs = st ? R2 : R;
       const int bs = st ? base2 : base;
       uint8_t *ts = st ? tile2 : tile;
-      tile_load<W>(ts, stride, st ? bfr2 : bfr, wx0, wy0, wx1, wy1, lane);
+      tile_load<W>(ts, stride, (st ? bfr2 : bfr) + ch * (W * H), wx0, wy0, wx1, wy1, lane);
       __syncwarp();
       for (int g = 0; g < T::NG; g++) {
         int gb, ge, gmode;
@@ -219,22 +228,28 @@ __device__ __noinline__ void tile_row_rebuild(const uint32_t *R, const uint32_t 
             uint4 q;
             q.x = __shfl_sync(0xffffffffu, e.x, l); q.y = __shfl_sync(0xffffffffu, e.y, l);
             q.z = __shfl_sync(0xffffffffu, e.z, l); q.w = __shfl_sync(0xffffffffu, e.w, l);
-            paint_entry_coop(ts, stride, wx0, wy0, wx1, wy1, q, Rs, lane);
+            const uint32_t val = CH == 1 ? q.z & 255u : (__shfl_sync(0xffffffffu, p.color, l) >> (8 * ch)) & 255u;
+            paint_entry_coop(ts, stride, wx0, wy0, wx1, wy1, q, val, Rs, lane);
             __syncwarp();
           }
         }
       }
     }
     if (R2) { tile_max(tile, tile2, stride, wx1 - wx0, wy1 - wy0, lane); __syncwarp(); }
-    tile_resolve<TX, TY>(tile, stride, wx0, wy0, dxA, dxL, dy0, dy1, dw, plan, out, lane);
+    tile_resolve<TX, TY, CH>(tile, stride, wx0, wy0, dxA, dxL, dy0, dy1, dw, plan, out + ch, lane);
     __syncwarp();
+    }
   }
 }
 
-template <int GAME, int TX, int TY, bool DUAL>
+/* RGB (TBX_OBS_RGB_AREA, single frames only): a.base[b] = planar base frame b (R, G, B planes of W x H), a.base_out[b] = its
+ * interleaved down-sample, 3 bytes per output pixel; no HUD digit patches (they are gray) */
+template <int GAME, int TX, int TY, bool DUAL, bool RGB = false>
 __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) area_tile_kernel(const __grid_constant__ RenderArgs a, const __grid_constant__ typename Traits<GAME>::Cfg cfg_c,
                                                                          const __grid_constant__ TbxAreaPlan plan_c) {
+  static_assert(!(DUAL && RGB), "the RGB mode renders single frames");
   typedef Traits<GAME> T;
+  constexpr int CH = RGB ? 3 : 1;
   constexpr int W = T::W, H = T::H, RW = T::RW;
   extern __shared__ uint4 smem_raw[];
   uint8_t *smem = reinterpret_cast<uint8_t *>(smem_raw);
@@ -267,7 +282,8 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
   uint4 *list = reinterpret_cast<uint4 *>(wmem);
   uint32_t *exts = reinterpret_cast<uint32_t *>(wmem + TBX_TILE_LCAP * 16);
   uint32_t *tmask = exts + TBX_TILE_LCAP;
-  uint8_t *tile = reinterpret_cast<uint8_t *>(tmask + 8);
+  uint32_t *cols = tmask + 8; /* RGB mode: each entry's colour (r | g << 8 | b << 16) */
+  uint8_t *tile = reinterpret_cast<uint8_t *>(tmask + 8 + (RGB ? TBX_TILE_LCAP : 0));
   uint8_t *tile2 = tile + a.tile_bytes; /* dual mode: the second state's window */
   const int stride = a.tile_stride;
   constexpr int ths = TBX_TILE_HSHIFT;
@@ -286,7 +302,7 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
     uint8_t *out = a.dst + (size_t)env * a.env_stride + (size_t)a.stack_slot * a.frame_bytes;
     { /* 1. the static part of the frame */
       const uint8_t *src = base ? a.base_out[1] : a.base_out[0];
-      const int nb = dw * dh;
+      const int nb = dw * dh * CH;
       if ((a.frame_bytes & 15) == 0) {
         for (int i = lane; i < (nb >> 4); i += 32) reinterpret_cast<uint4 *>(out)[i] = __ldg(reinterpret_cast<const uint4 *>(src) + i);
       } else if ((a.frame_bytes & 3) == 0) {
@@ -311,7 +327,7 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
       int n = 0;
       bool overflow = false;
       /* whole frame in one sweep: a digit's footprint is not clipped; dual mode: both frames on the same base frame */
-      const bool use_patches = a.patches[0] != 0 && nsw == 1 && (!dual || base == base2);
+      const bool use_patches = !RGB && a.patches[0] != 0 && nsw == 1 && (!dual || base == base2); /* the patches are gray */
       if constexpr (!dual) {
         for (int g = 0; g < T::NG && !overflow; g++) {
           int gb, ge, gmode;
@@ -334,6 +350,7 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
               if (cand) e.z |= (TBX_ENTRY_DIGIT << 16) | ((uint32_t)didx << 24);
               list[slot] = e;
               exts[slot] = ext;
+              if constexpr (RGB) cols[slot] = p.color;
               if (!cand) mark_tiles(tmask, ext, ths); /* candidates are marked below unless their patch can be used */
             }
             n += __popc(m);
@@ -396,7 +413,7 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
       __syncwarp();
 
       if (overflow) {
-        tile_row_rebuild<GAME, TX, TY>(R, R2, cfg, tables, base, base2, bfr, bfr2, plan, cp, tile, tile2, stride, tyA, ths, rA, rB, dyA, dyB, out, lane);
+        tile_row_rebuild<GAME, TX, TY, CH>(R, R2, cfg, tables, base, base2, bfr, bfr2, plan, cp, tile, tile2, stride, tyA, ths, rA, rB, dyA, dyB, out, lane);
         continue;
       }
       /* 2b. HUD digits: a digit entry whose output rectangle meets no other entry's is the only thing that differs from
@@ -482,7 +499,10 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
           if (dx0 > dx1 || dy0 > dy1) continue;
           const int wx0 = cp.xs0[dx0] & ~3, wx1 = min(W, ((int)cp.xs0[dx1] + TX + 3) & ~3);
           const int wy0 = cp.ys0[dy0], wy1 = min(H, (int)cp.ys0[dy1] + TY);
-          tile_load<W>(tile, stride, bfr, wx0, wy0, wx1, wy1, lane);
+          /* RGB mode: channel by channel through the same scratch window */
+#pragma unroll 1
+          for (int ch = 0; ch < CH; ch++) {
+          tile_load<W>(tile, stride, bfr + ch * (W * H), wx0, wy0, wx1, wy1, lane);
           if (dual && two_frames) tile_load<W>(tile2, stride, bfr2, wx0, wy0, wx1, wy1, lane);
           __syncwarp();
 #pragma unroll
@@ -500,8 +520,9 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
               const uint32_t *Rs = st2 ? R2 : R;
               if (!((zl >> 16) & TBX_ENTRY_PAR)) { /* in-order group: one entry at a time */
                 const uint4 q = list[c * 32 + l];
-                paint_entry_coop(ts, stride, wx0, wy0, wx1, wy1, q, Rs, lane);
-                if (twice) paint_entry_coop(tile2, stride, wx0, wy0, wx1, wy1, q, R2, lane);
+                const uint32_t qv = RGB ? (cols[c * 32 + l] >> (8 * ch)) & 255u : q.z & 255u;
+                paint_entry_coop(ts, stride, wx0, wy0, wx1, wy1, q, qv, Rs, lane);
+                if (twice) paint_entry_coop(tile2, stride, wx0, wy0, wx1, wy1, q, qv, R2, lane);
                 __syncwarp();
                 m &= m - 1;
                 continue;
@@ -514,27 +535,30 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
               if (__popc(smalls) < 3) { smalls = 0; small = false; } /* too few to pay for one-lane loops: the warp paints each */
               uint32_t big = same & ~smalls;
               if (small) {
+                const uint32_t ev = RGB ? (cols[c * 32 + lane] >> (8 * ch)) & 255u : e.z & 255u; /* the byte this lane's entry paints */
                 paint_tile_lane(ts, stride, wx0, wy0, wx1, wy1, (int16_t)(e.x & 0xffffu), (int16_t)(e.x >> 16), (int16_t)(e.y & 0xffffu),
-                                (int16_t)(e.y >> 16), e.z & 255u);
+                                (int16_t)(e.y >> 16), ev);
                 if (twice)
                   paint_tile_lane(tile2, stride, wx0, wy0, wx1, wy1, (int16_t)(e.x & 0xffffu), (int16_t)(e.x >> 16), (int16_t)(e.y & 0xffffu),
-                                  (int16_t)(e.y >> 16), e.z & 255u);
+                                  (int16_t)(e.y >> 16), ev);
               }
               __syncwarp();
               while (big) {
                 const int lb = __ffs(big) - 1;
                 big &= big - 1;
                 const uint4 q = list[c * 32 + lb];
-                paint_entry_coop(ts, stride, wx0, wy0, wx1, wy1, q, Rs, lane);
-                if (twice) paint_entry_coop(tile2, stride, wx0, wy0, wx1, wy1, q, R2, lane);
+                const uint32_t qv = RGB ? (cols[c * 32 + lb] >> (8 * ch)) & 255u : q.z & 255u;
+                paint_entry_coop(ts, stride, wx0, wy0, wx1, wy1, q, qv, Rs, lane);
+                if (twice) paint_entry_coop(tile2, stride, wx0, wy0, wx1, wy1, q, qv, R2, lane);
                 __syncwarp();
               }
               m &= ~same;
             }
           }
           if (dual && two_frames) { tile_max(tile, tile2, stride, wx1 - wx0, wy1 - wy0, lane); __syncwarp(); }
-          tile_resolve<TX, TY>(tile, stride, wx0, wy0, dx0, dx1, dy0, dy1, dw, plan, out, lane);
-          __syncwarp(); /* the scratch canvas is overwritten by the next run */
+          tile_resolve<TX, TY, CH>(tile, stride, wx0, wy0, dx0, dx1, dy0, dy1, dw, plan, out + ch, lane);
+          __syncwarp(); /* the scratch canvas is overwritten by the next run or channel */
+          }
         }
       }
       if (use_patches) { /* the isolated digits: their patches go in last (a run's bounding box may have swept over them) */
@@ -561,7 +585,7 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
     if (a.reset_flags && a.stack_k > 1 && a.reset_flags[env]) {
       __syncwarp();
       uint8_t *ring = a.dst + (size_t)env * a.env_stride;
-      const int nb = dw * dh;
+      const int nb = dw * dh * CH;
       const bool zero = a.stack_mode == 1;
       for (int k = 0; k < a.stack_k; k++) {
         if (k == a.stack_slot) continue;

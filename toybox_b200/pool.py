@@ -12,7 +12,7 @@ from . import _lib
 from . import snapshot as _snap
 
 GAMES = ("breakout", "amidar", "space_invaders")
-OBS_MODES = {"rgba": 0, "rgb": 1, "gray": 2, "gray_area": 3}
+OBS_MODES = {"rgba": 0, "rgb": 1, "gray": 2, "gray_area": 3, "rgb_area": 4}
 
 
 def _ptr(t):
@@ -27,7 +27,8 @@ class BatchedToybox:
     """`n_envs` independent environments of `game` on one CUDA device.
 
     obs: 'rgba' uint8[N,H,W,4] | 'rgb' uint8[N,H,W,3] | 'gray' uint8[N,H,W,1] | 'gray84' uint8[N,84,84,1]
-         (= cv2.INTER_AREA of the grayscale frame, baselines WarpFrame) | ('gray_area', out_w, out_h).
+         (= cv2.INTER_AREA of the grayscale frame, baselines WarpFrame) | ('gray_area', out_w, out_h) | 'rgb84' uint8[N,84,84,3]
+         (= cv2.INTER_AREA of the RGB frame, WarpFrame(grayscale=False)) | ('rgb_area', out_w, out_h).
     """
 
     def __init__(self, game, n_envs, device=None, obs="gray84", config=None, seeds=None):
@@ -81,8 +82,8 @@ class BatchedToybox:
     def set_obs(self, obs):
         if isinstance(obs, (tuple, list)):
             mode, ow, oh = obs
-        elif obs == "gray84":
-            mode, ow, oh = "gray_area", 84, 84
+        elif obs in ("gray84", "rgb84"):
+            mode, ow, oh = obs[:-2] + "_area", 84, 84
         else:
             mode, ow, oh = obs, 0, 0
         if mode not in OBS_MODES:
@@ -92,7 +93,7 @@ class BatchedToybox:
             raise ValueError("unsupported observation size %r for %s" % (obs, self.game_name))
         self._mode, self._ow, self._oh, self._obs_bytes = OBS_MODES[mode], ow, oh, nbytes
         H, W = self.height, self.width
-        self.obs_shape = {0: (H, W, 4), 1: (H, W, 3), 2: (H, W, 1), 3: (oh, ow, 1)}[self._mode]
+        self.obs_shape = {0: (H, W, 4), 1: (H, W, 3), 2: (H, W, 1), 3: (oh, ow, 1), 4: (oh, ow, 3)}[self._mode]
         self._obs = None
 
     def get_width(self):
