@@ -174,13 +174,19 @@ int tbx_wrap_create(tbx_pool *pool, int skip, int noop_max, int episodic_life, i
  * (baselines/baselines/common/atari_wrappers.py:262-266, the wrap_deepmind(frame_stack=True) path); 1 = they are zeroed,
  * VecFrameStack (baselines/baselines/common/vec_env/vec_frame_stack.py:17-30, the make_vec_env + VecFrameStack path). */
 int tbx_wrap_set_stack_mode(tbx_wrap *w, int mode);
+/* The layout of the observation ring: TBX_OBS_GRAY_AREA (default; the ring is uint8[N][stack_k][out_h][out_w]) or
+ * TBX_OBS_RGB_AREA, WarpFrame(grayscale=False) (atari_wrappers.py:230-244): the ring is uint8[N][stack_k][out_h][out_w][3],
+ * each observation the colour INTER_AREA down-sample of the pixel-wise max of the two RGB frames.  Both accept the same
+ * output sizes.  TBX_EINVAL for any other layout, or once the wrap has stepped (its ring holds frames of the old layout). */
+int tbx_wrap_set_obs_mode(tbx_wrap *w, int obs_mode);
 /* Device buffers (int32[N] each, caller-owned, may be NULL) that every tbx_wrap_step fills with baselines' Monitor record
  * (bench/monitor.py:58-76; Monitor sits between make_atari and wrap_deepmind, common/cmd_util.py:30-36) of the episode that
  * ended in that agent step: r = sum of raw rewards, l = MaxAndSkipEnv steps since the last real reset.  Valid where real_done. */
 int tbx_wrap_set_episode_outputs(tbx_wrap *w, int32_t *ep_return_dev, int32_t *ep_length_dev);
 int tbx_wrap_destroy(tbx_wrap *wrap);
 /* env.step(action) of the wrapped env for every env (actions_dev: int32[N] gym action indices into the legal set), or
- * env.reset() for every env when actions_dev == NULL.  obs_ring_dev: uint8[N][stack_k][out_h][out_w], a ring of the
+ * env.reset() for every env when actions_dev == NULL.  obs_ring_dev: uint8[N][stack_k][out_h][out_w] (with [3] appended
+ * under TBX_OBS_RGB_AREA, tbx_wrap_set_obs_mode), a ring of the
  * last stack_k observations per env; the newest frame goes to slot *slot_out (host int), older frames follow
  * backwards modulo stack_k (FrameStack order = slots slot+1, ..., slot+stack_k, modulo stack_k).  Envs whose
  * observation comes from a reset get it in every slot (FrameStack.reset).  reward: sum over the skipped frames,

@@ -98,6 +98,7 @@ SIGNATURES = {
     "tbx_wrap_create": (i32, [vp, i32, i32, i32, i32, i32, i32, i32, i32, u64, u64, C.POINTER(vp)]),
     "tbx_wrap_destroy": (i32, [vp]),
     "tbx_wrap_set_stack_mode": (i32, [vp, i32]),
+    "tbx_wrap_set_obs_mode": (i32, [vp, i32]),
     "tbx_wrap_set_episode_outputs": (i32, [vp, vp, vp]),
     "tbx_wrap_step": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(i32), vp]),
     "tbx_state_rows": (i32, [vp]),

@@ -478,7 +478,7 @@ template <int GAME, int PIX> static int launch_native(const RenderArgs &a, const
   CK(cudaGetLastError());
   return TBX_OK;
 }
-/* INTER_AREA, one warp per env (tbx_render_area.cuh); RGB: the single-frame RGB mode */
+/* INTER_AREA, one warp per env (tbx_render_area.cuh); RGB: the RGB mode */
 template <int GAME, int TX, int TY, bool DUAL, bool RGB = false>
 static int launch_area_tile(const RenderArgs &a, const typename Traits<GAME>::Cfg &cfg, const TbxAreaPlan &plan, int smem, cudaStream_t s) {
   CK((cudaFuncSetAttribute(area_tile_kernel<GAME, TX, TY, DUAL, RGB>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
@@ -489,8 +489,8 @@ static int launch_area_tile(const RenderArgs &a, const typename Traits<GAME>::Cf
   return TBX_OK;
 }
 
-/* INTER_AREA: the direct kernel where it covers the pair, then the tile kernel; RGB (single frames): the tile kernel's
- * RGB mode alone */
+/* INTER_AREA: the direct kernel where it covers the pair, then the tile kernel; RGB: the tile kernel's RGB mode alone (single
+ * frames, and the wrapped path's max of two frames) */
 static int render_area(tbx_pool *p, RenderArgs &a, int out_w, int out_h, bool rgb, cudaStream_t s) {
   const AreaRes *ar = 0;
   int r = ensure_area(p, out_w, out_h, rgb, &ar);
@@ -560,9 +560,13 @@ static int render_area(tbx_pool *p, RenderArgs &a, int out_w, int out_h, bool rg
     const auto &cfg = game_cfg<G>(p->cfg);
     return with_taps<8>(plan.tx, plan.ty, [&](auto X, auto Y) {
       constexpr int TX = decltype(X)::value, TY = decltype(Y)::value;
-      if (rgb) return launch_area_tile<G, TX, TY, false, true>(a, cfg, plan, smem, s);
-      if constexpr (TX == 8) return launch_area_tile<G, 8, 8, false>(a, cfg, plan, smem, s); /* single frames only (checked above) */
-      else return dual ? launch_area_tile<G, TX, TY, true>(a, cfg, plan, smem, s) : launch_area_tile<G, TX, TY, false>(a, cfg, plan, smem, s);
+      if constexpr (TX == 8) { /* single frames only (checked above) */
+        return rgb ? launch_area_tile<G, 8, 8, false, true>(a, cfg, plan, smem, s) : launch_area_tile<G, 8, 8, false>(a, cfg, plan, smem, s);
+      } else if (rgb) {
+        return dual ? launch_area_tile<G, TX, TY, true, true>(a, cfg, plan, smem, s) : launch_area_tile<G, TX, TY, false, true>(a, cfg, plan, smem, s);
+      } else {
+        return dual ? launch_area_tile<G, TX, TY, true>(a, cfg, plan, smem, s) : launch_area_tile<G, TX, TY, false>(a, cfg, plan, smem, s);
+      }
     });
   });
 }
@@ -649,6 +653,8 @@ struct tbx_wrap {
   Buf<uint8_t> was_reset;
   int head; /* ring slot of the newest frame */
   int stack_mode; /* what a reset observation does to the other k-1 ring slots: 0 = fills them (FrameStack.reset), 1 = zeroes them (VecFrameStack) */
+  int obs_mode;   /* the ring's layout: TBX_OBS_GRAY_AREA or TBX_OBS_RGB_AREA (WarpFrame(grayscale=False)) */
+  bool stepped;   /* tbx_wrap_step has run: the ring holds frames of obs_mode's layout */
   int32_t *ep_return, *ep_length; /* caller-owned device outputs of Monitor's episode record, or NULL */
 };
 
@@ -664,7 +670,7 @@ int tbx_wrap_create(tbx_pool *p, int skip, int noop_max, int episodic_life, int 
   return guarded([&]() -> int {
     std::unique_ptr<tbx_wrap> w(new tbx_wrap());
     w->pool = p; w->skip = skip; w->noop_max = noop_max; w->episodic_life = episodic_life; w->fire_reset = fire_reset; w->clip_rewards = clip_rewards;
-    w->stack_k = stack_k; w->out_w = out_w; w->out_h = out_h; w->noop_seed = noop_seed; w->env0 = env0;
+    w->stack_k = stack_k; w->out_w = out_w; w->out_h = out_h; w->noop_seed = noop_seed; w->env0 = env0; w->obs_mode = TBX_OBS_GRAY_AREA;
     const size_t plane_words = (size_t)p->info->rec_words * p->n_pad;
     cudaError_t e = w->planes_prev.alloc(plane_words);
     if (e == cudaSuccess) e = w->wstate.alloc(5 * (size_t)p->n_pad);
@@ -687,6 +693,13 @@ int tbx_wrap_set_stack_mode(tbx_wrap *w, int mode) {
   w->stack_mode = mode;
   return TBX_OK;
 }
+int tbx_wrap_set_obs_mode(tbx_wrap *w, int obs_mode) {
+  if (!w || (obs_mode != TBX_OBS_GRAY_AREA && obs_mode != TBX_OBS_RGB_AREA))
+    return set_err(TBX_EINVAL, "wrap is NULL or unsupported observation layout (TBX_OBS_GRAY_AREA or TBX_OBS_RGB_AREA)");
+  if (w->stepped) return set_err(TBX_EINVAL, "the observation layout is set before the first tbx_wrap_step");
+  w->obs_mode = obs_mode;
+  return TBX_OK;
+}
 int tbx_wrap_set_episode_outputs(tbx_wrap *w, int32_t *ep_return_dev, int32_t *ep_length_dev) {
   if (!w) return set_err(TBX_EINVAL, "wrap is NULL");
   w->ep_return = ep_return_dev; w->ep_length = ep_length_dev;
@@ -707,6 +720,7 @@ int tbx_wrap_step(tbx_wrap *w, const int32_t *actions, uint8_t *obs_ring, int32_
   tbx_pool *p = w->pool;
   CK(cudaSetDevice(p->device));
   cudaStream_t s = (cudaStream_t)stream;
+  w->stepped = true;
   WrapArgs a;
   a.planes = p->planes; a.planes_prev = w->planes_prev; a.wstate = w->wstate; a.n = p->n; a.n_pad = p->n_pad; a.cfg = p->d_cfg; a.tables = p->d_tables;
   a.legal = p->d_legal; a.n_legal = p->info->n_legal; a.actions = actions;
@@ -721,7 +735,7 @@ int tbx_wrap_step(tbx_wrap *w, const int32_t *actions, uint8_t *obs_ring, int32_
     w->head = (w->head + 1) % w->stack_k;
     DualRender d;
     d.planes2 = w->planes_prev; d.reset_flags = w->was_reset; d.stack_k = w->stack_k; d.stack_slot = w->head; d.stack_mode = w->stack_mode;
-    int r = guarded([&] { return render_impl(p, obs_ring, TBX_OBS_GRAY_AREA, w->out_w, w->out_h, stream, &d); });
+    int r = guarded([&] { return render_impl(p, obs_ring, w->obs_mode, w->out_w, w->out_h, stream, &d); });
     if (r) return r;
   }
   if (slot_out) *slot_out = w->head;

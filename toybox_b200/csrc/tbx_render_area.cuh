@@ -20,10 +20,11 @@
  * are painted lane-parallel; everything else is painted by the whole warp, one entry at a time, in draw order.
  * The kernel renders every plan the library accepts: it is instantiated for 3..5 x 3..4 taps, and for 8 x 8 taps
  * (single frames only) for the plans with more; surplus taps carry zero weight.
- * RGB mode (RGB = true, single frames): the list, hit tests, sweeps and per-tile rebuild are colour-blind and
- * shared; each entry also keeps its 24-bit colour, and every run is loaded, painted and resolved once per channel from
- * planar base frames, so the scratch window keeps its gray size.  The output is interleaved RGB, = cv2's 3-channel
- * INTER_AREA (which is the per-channel resize).
+ * RGB mode (RGB = true; single frames, and the dual mode of the wrapped path for 3..5 x 3..4 taps): the list, hit tests,
+ * sweeps and per-tile rebuild are colour-blind and shared; each entry also keeps its 24-bit colour, and every run is loaded,
+ * painted and resolved once per channel from planar base frames (both windows in dual mode), so the scratch window keeps its
+ * gray size.  The output is interleaved RGB, = cv2's 3-channel INTER_AREA (which is the per-channel resize).  In dual mode
+ * a slot is "in both frames" only if its colour is the same in both, not just its gray.
  */
 #ifndef TBX_RENDER_AREA_CUH
 #define TBX_RENDER_AREA_CUH
@@ -41,6 +42,12 @@ namespace tbxk {
 /* the 8 x 8 instantiation keeps its eight column weights per lane in registers: at 4 CTAs per SM (64 registers) it
  * spills, at 2 it needs ~112 and does not */
 #define TBX_TILE_MIN_CTAS(TX, TY) ((TX) > 5 || (TY) > 4 ? 2 : TBX_AREA_MIN_CTAS)
+/* dual RGB (two scratch windows, the colour array, a channel loop): it spills at 64 and at 80 registers (4 and 3 CTAs per SM)
+ * and needs ~128 (2).  Its shared memory allows 4 CTAs per SM for Breakout 84 x 84 (55.5 KB), 3 for Amidar (75.6 KB) and 2 for
+ * Space Invaders (90.9 KB) */
+#ifndef TBX_TILE_DUAL_RGB_MIN_CTAS
+#define TBX_TILE_DUAL_RGB_MIN_CTAS 2
+#endif
 
 /* a warp paints one primitive into the tile scratch canvas: window columns [wx0, wx1) (wx0 a multiple of 4, the
  * scratch's column 0), rows [wy0, wy1); `stride` bytes per scratch row */
@@ -187,8 +194,9 @@ __device__ __forceinline__ void paint_entry_coop(uint8_t *tile, int stride, int 
 
 /* One tile row with more entries than the list holds: every tile of the row re-builds the primitives and paints
  * those that touch it, strictly in draw order (slow, but always correct).  CH = 3: once per channel, from the planar base
- * frames (channel c at bfr + c * W * H), into the interleaved frame. */
-template <int GAME, int TX, int TY, int CH = 1>
+ * frames (channel c at bfr + c * W * H), into the interleaved frame.  DUAL_RGB: the dual RGB kernel's own copy -- ptxas
+ * compiles a __noinline__ function once for all its callers, and that kernel has twice the registers of the others. */
+template <int GAME, int TX, int TY, int CH = 1, bool DUAL_RGB = false>
 __device__ __noinline__ void tile_row_rebuild(const uint32_t *R, const uint32_t *R2, const typename Traits<GAME>::Cfg &cfg, const typename Traits<GAME>::Table *tables,
                                               int base, int base2, const uint8_t *bfr, const uint8_t *bfr2, const TbxAreaPlan *__restrict__ plan, const TbxAreaPlan &cp,
                                               uint8_t *tile, uint8_t *tile2, int stride,
@@ -242,12 +250,11 @@ __device__ __noinline__ void tile_row_rebuild(const uint32_t *R, const uint32_t 
   }
 }
 
-/* RGB (TBX_OBS_RGB_AREA, single frames only): a.base[b] = planar base frame b (R, G, B planes of W x H), a.base_out[b] = its
- * interleaved down-sample, 3 bytes per output pixel; no HUD digit patches (they are gray) */
+/* RGB (TBX_OBS_RGB_AREA): a.base[b] = planar base frame b (R, G, B planes of W x H), a.base_out[b] = its interleaved
+ * down-sample, 3 bytes per output pixel; no HUD digit patches (they are gray) */
 template <int GAME, int TX, int TY, bool DUAL, bool RGB = false>
-__global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) area_tile_kernel(const __grid_constant__ RenderArgs a, const __grid_constant__ typename Traits<GAME>::Cfg cfg_c,
+__global__ void __launch_bounds__(TBX_TILE_THREADS, DUAL && RGB ? TBX_TILE_DUAL_RGB_MIN_CTAS : TBX_TILE_MIN_CTAS(TX, TY)) area_tile_kernel(const __grid_constant__ RenderArgs a, const __grid_constant__ typename Traits<GAME>::Cfg cfg_c,
                                                                          const __grid_constant__ TbxAreaPlan plan_c) {
-  static_assert(!(DUAL && RGB), "the RGB mode renders single frames");
   typedef Traits<GAME> T;
   constexpr int CH = RGB ? 3 : 1;
   constexpr int W = T::W, H = T::H, RW = T::RW;
@@ -379,7 +386,8 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
             const bool okA = make_entry<W>(pA, g, gmA, rA, rB, dyA, dyB, plan, eA, xA);
             const bool okB = make_entry<W>(pB, g | 0x80, gmB, rA, rB, dyA, dyB, plan, eB, xB);
             const bool both = merge && okA && okB && eA.x == eB.x && eA.y == eB.y && ((eA.z ^ eB.z) & 0xffu) == 0 && eA.w == eB.w &&
-                              !(eA.w & TBX_PRIM_STATE); /* sprites stored in the record may differ bit by bit */
+                              !(eA.w & TBX_PRIM_STATE) /* sprites stored in the record may differ bit by bit */
+                              && (!RGB || pA.color == pB.color); /* RGB: two colours may share a gray */
             const unsigned m1 = __ballot_sync(0xffffffffu, okA), m2 = __ballot_sync(0xffffffffu, okB && !both);
             if ((m1 | m2) == 0) continue;
             if (n + __popc(m1) + __popc(m2) > a.list_cap) { overflow = true; break; }
@@ -394,11 +402,13 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
               }
               list[slot] = eA;
               exts[slot] = xA;
+              if constexpr (RGB) cols[slot] = pA.color;
               if (!cand) mark_tiles(tmask, xA, ths);
             }
             if (okB && !both) {
               list[slot + (okA ? 1 : 0)] = eB;
               exts[slot + (okA ? 1 : 0)] = xB;
+              if constexpr (RGB) cols[slot + (okA ? 1 : 0)] = pB.color;
               mark_tiles(tmask, xB, ths);
             }
             n += __popc(m1) + __popc(m2);
@@ -413,7 +423,7 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
       __syncwarp();
 
       if (overflow) {
-        tile_row_rebuild<GAME, TX, TY, CH>(R, R2, cfg, tables, base, base2, bfr, bfr2, plan, cp, tile, tile2, stride, tyA, ths, rA, rB, dyA, dyB, out, lane);
+        tile_row_rebuild<GAME, TX, TY, CH, DUAL && RGB>(R, R2, cfg, tables, base, base2, bfr, bfr2, plan, cp, tile, tile2, stride, tyA, ths, rA, rB, dyA, dyB, out, lane);
         continue;
       }
       /* 2b. HUD digits: a digit entry whose output rectangle meets no other entry's is the only thing that differs from
@@ -503,7 +513,7 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, TBX_TILE_MIN_CTAS(TX, TY)) a
 #pragma unroll 1
           for (int ch = 0; ch < CH; ch++) {
           tile_load<W>(tile, stride, bfr + ch * (W * H), wx0, wy0, wx1, wy1, lane);
-          if (dual && two_frames) tile_load<W>(tile2, stride, bfr2, wx0, wy0, wx1, wy1, lane);
+          if (dual && two_frames) tile_load<W>(tile2, stride, bfr2 + ch * (W * H), wx0, wy0, wx1, wy1, lane);
           __syncwarp();
 #pragma unroll
           for (int c = 0; c < TBX_TILE_LCAP / 32; c++) {

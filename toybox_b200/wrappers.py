@@ -19,41 +19,49 @@ import torch
 
 from . import _lib
 from . import snapshot as _snap
-from .pool import BatchedToybox, _ptr, _stream
+from .pool import OBS_MODES, BatchedToybox, _ptr, _stream
 
 
 class DeepmindToybox:
     """N wrapped envs.  step(actions) takes gym action INDICES (0..len(legal)-1, envs/atari/base.py:126) as an int32
     tensor on the pool's device and returns (obs, reward, done, info):
-      obs    uint8[N, k, out_h, out_w]: a RING of the last k observations per env -- the newest is obs[:, self.slot],
-             FrameStack order (oldest first) is slots (self.slot + 1 .. self.slot + k) % k; `stacked()` returns that
-             order as the reference's uint8[N, out_h, out_w, k] (a copy);
+      obs    uint8[N, k, out_h, out_w] (uint8[N, k, out_h, out_w, 3] when grayscale=False): a RING of the last k
+             observations per env -- the newest is obs[:, self.slot], FrameStack order (oldest first) is slots
+             (self.slot + 1 .. self.slot + k) % k; `stacked()` returns that order as the reference's
+             uint8[N, out_h, out_w, k] (uint8[N, out_h, out_w, 3k] in colour) (a copy);
       reward int32[N] (sign of the summed reward when clip_rewards), done uint8[N] (game over, or a lost life when
       episode_life), info = {'lives', 'score', 'real_done'} tensors (values before the reset of a finished env).
     A finished env is reset inside the same call and `obs` then holds its reset observation (VecEnv semantics)."""
 
     def __init__(self, game, n_envs, device=None, seeds=None, config=None, frame_skip=4, noop_max=30, episode_life=True,
-                 fire_reset=True, clip_rewards=True, frame_stack=4, size=(84, 84), noop_seed=0, env0=0, stack_reset="fill"):
+                 fire_reset=True, clip_rewards=True, frame_stack=4, size=(84, 84), noop_seed=0, env0=0, stack_reset="fill",
+                 grayscale=True):
         """stack_reset: what a reset observation does to the other k-1 ring slots -- "fill" (FrameStack.reset,
         atari_wrappers.py:262-266: wrap_deepmind(frame_stack=True), the deepq path) or "zero" (VecFrameStack,
-        vec_env/vec_frame_stack.py:17-30: make_vec_env + VecFrameStack, the ppo2 / a2c path of run.py:123-125)."""
+        vec_env/vec_frame_stack.py:17-30: make_vec_env + VecFrameStack, the ppo2 / a2c path of run.py:123-125).
+        grayscale: WarpFrame's argument (atari_wrappers.py:230-244); False gives colour observations, the INTER_AREA
+        down-sample of the pixel-wise max of the last two RGB frames."""
         if stack_reset not in ("fill", "zero"):
             raise ValueError("stack_reset is 'fill' (FrameStack) or 'zero' (VecFrameStack)")
         self.pool = BatchedToybox(game, n_envs, device=device, obs=("gray_area", size[0], size[1]), config=config, seeds=seeds)
         self.L = self.pool.L
         self.n_envs, self.device = self.pool.n_envs, self.pool.device
         self.k, self.out_w, self.out_h = int(frame_stack), int(size[0]), int(size[1])
+        self.grayscale = bool(grayscale)
+        self.frame_shape = (self.out_h, self.out_w) if self.grayscale else (self.out_h, self.out_w, 3)
         h = C.c_void_p()
         _lib.check(self.L.tbx_wrap_create(self.pool._h, int(frame_skip), int(noop_max), int(bool(episode_life)), int(bool(fire_reset)),
                                           int(bool(clip_rewards)), self.k, self.out_w, self.out_h, int(noop_seed), int(env0), C.byref(h)))
         self._w = h
         _lib.check(self.L.tbx_wrap_set_stack_mode(self._w, 1 if stack_reset == "zero" else 0))
+        if not self.grayscale:
+            _lib.check(self.L.tbx_wrap_set_obs_mode(self._w, OBS_MODES["rgb_area"]))
         n, dev = self.n_envs, self.device
         # Monitor's episode record (bench/monitor.py:58-76) of the episode that ended in the last agent step, where real_done
         self.ep_return = torch.zeros(n_envs, dtype=torch.int32, device=self.device)
         self.ep_length = torch.zeros(n_envs, dtype=torch.int32, device=self.device)
         _lib.check(self.L.tbx_wrap_set_episode_outputs(self._w, _ptr(self.ep_return), _ptr(self.ep_length)))
-        self.obs = torch.zeros((n, self.k, self.out_h, self.out_w), dtype=torch.uint8, device=dev)
+        self.obs = torch.zeros((n, self.k) + self.frame_shape, dtype=torch.uint8, device=dev)
         self.reward = torch.zeros(n, dtype=torch.int32, device=dev)
         self.done = torch.zeros(n, dtype=torch.uint8, device=dev)
         self.real_done = torch.zeros(n, dtype=torch.uint8, device=dev)
@@ -116,7 +124,8 @@ class DeepmindToybox:
         the saved newest frame lands on self.slot: stacked() then equals its value at the moment of the save.  Synchronises
         (the ring copy selects the entries the kernel applied)."""
         if not getattr(snap, "wrapped", False) or tuple(snap.obs.shape[1:]) != tuple(self.obs.shape[1:]):
-            raise ValueError("expected a snapshot of wrapped envs with %d x %d x %d observation rings" % (self.k, self.out_h, self.out_w))
+            raise ValueError("expected a snapshot of wrapped envs with %d x %d x %d observation rings of %d channel%s%s"
+                             % (self.k, self.out_h, self.out_w, self.channels, "" if self.channels == 1 else "s", _got_rings(snap)))
         data, ids, cols, n = _snap.load_args(snap, self.device, self.n_envs, env_ids, columns)
         _lib.check(self.L.tbx_wrap_state_load(self._w, _ptr(data), data.shape[1], _ptr(cols), _ptr(ids), n, snap.tables, len(snap.tables),
                                               _stream(self.device)))
@@ -151,10 +160,29 @@ class DeepmindToybox:
         """ring slots, oldest observation first"""
         return [(self.slot + 1 + i) % self.k for i in range(self.k)]
 
+    @property
+    def channels(self):
+        """bytes per observation pixel: 1 (gray) or 3 (RGB)"""
+        return 1 if self.grayscale else 3
+
     def stacked(self):
-        """FrameStack's observation (atari_wrappers.py:246-275) for every env: uint8[N, out_h, out_w, k], oldest first."""
+        """FrameStack's observation (atari_wrappers.py:246-275) for every env, oldest first: uint8[N, out_h, out_w, k], or in
+        colour uint8[N, out_h, out_w, 3k] with frame-major channels (the oldest frame's R, G, B first), the concatenation
+        along the last axis that LazyFrames and VecFrameStack produce."""
         idx = torch.as_tensor(self.order(), device=self.device)
-        return self.obs.index_select(1, idx).permute(0, 2, 3, 1).contiguous()
+        ring = self.obs.index_select(1, idx)
+        if self.grayscale:
+            return ring.permute(0, 2, 3, 1).contiguous()
+        return ring.permute(0, 2, 3, 1, 4).reshape(self.n_envs, self.out_h, self.out_w, 3 * self.k)
+
+
+def _got_rings(snap):
+    """what a refused snapshot holds, for the message"""
+    if not getattr(snap, "wrapped", False):
+        return " (got a snapshot of unwrapped envs)"
+    sh = tuple(snap.obs.shape[1:])
+    ch = sh[3] if len(sh) > 3 else 1
+    return " (got %s rings of %d channel%s)" % (" x ".join(str(v) for v in sh[:3]), ch, "" if ch == 1 else "s")
 
 
 class _Box:
@@ -182,7 +210,7 @@ class ToyboxVecEnv:
         self.env = DeepmindToybox(game, num_envs, **kw)
         self.num_envs = int(num_envs)
         e = self.env
-        self.observation_space = _Box(0, 255, (e.out_h, e.out_w, e.k), np.uint8)
+        self.observation_space = _Box(0, 255, (e.out_h, e.out_w, e.channels * e.k), np.uint8)
         self.action_space = _Discrete(e.n_actions)
         self._actions = None
         self._t0 = time.time()
