@@ -181,8 +181,24 @@ int tbx_wrap_set_stack_mode(tbx_wrap *w, int mode);
 int tbx_wrap_set_obs_mode(tbx_wrap *w, int obs_mode);
 /* Device buffers (int32[N] each, caller-owned, may be NULL) that every tbx_wrap_step fills with baselines' Monitor record
  * (bench/monitor.py:58-76; Monitor sits between make_atari and wrap_deepmind, common/cmd_util.py:30-36) of the episode that
- * ended in that agent step: r = sum of raw rewards, l = MaxAndSkipEnv steps since the last real reset.  Valid where real_done. */
+ * ended in that agent step: r = sum of raw rewards, l = MaxAndSkipEnv steps since the last real reset.  Valid where real_done
+ * or truncated (tbx_wrap_set_time_limit). */
 int tbx_wrap_set_episode_outputs(tbx_wrap *w, int32_t *ep_return_dev, int32_t *ep_length_dev);
+/* Sticky actions (repeat_action_probability p, ALE's `if (rand() >= p) m_player_a_action = action`): on every game frame the
+ * stack runs -- the skipped frames, the no-ops of NoopResetEnv, the FIRE / RIGHT steps of FireResetEnv, the NOOP step of a
+ * life-loss reset -- env i repeats the ALE id of its previous frame where the draw u of (seed, env0 + i, f) is below
+ * llround(p * 2^32), else applies the requested id.  u is the upper 32 bits of the splitmix64 mix of the action stream, keyed
+ * with seed ^ 0x5354494B59414354; f counts env i's frames and is never reset; a new game sets the remembered id to NOOP.
+ * p > 0 adds two wrapper words per env (remembered id, frame counter: tbx_wrap_state_rows grows by 2), p = 0 (default) turns
+ * the rule off.  TBX_EINVAL for p outside [0, 1] or NaN, or once the wrap has stepped. */
+int tbx_wrap_set_sticky_actions(tbx_wrap *w, double repeat_action_probability, uint64_t seed);
+/* Episode time limit (gym's TimeLimit between MaxAndSkipEnv and Monitor): an env whose Monitor length (MaxAndSkipEnv steps since
+ * the last real reset, reset-chain steps included) reaches max_episode_steps at the end of an agent step reports done, takes
+ * the full reset chain and exports its Monitor record; truncated_dev (uint8[N], caller-owned, may be NULL; written on every
+ * step) flags such an env where its game is not over.  real_done keeps meaning game over.  Reset-chain steps that cross the
+ * limit truncate at the next agent step.  0 (default) = no limit.  TBX_EINVAL for a negative limit, or once the wrap has
+ * stepped. */
+int tbx_wrap_set_time_limit(tbx_wrap *w, int max_episode_steps, uint8_t *truncated_dev);
 int tbx_wrap_destroy(tbx_wrap *wrap);
 /* env.step(action) of the wrapped env for every env (actions_dev: int32[N] gym action indices into the legal set), or
  * env.reset() for every env when actions_dev == NULL.  obs_ring_dev: uint8[N][stack_k][out_h][out_w] (with [3] appended
@@ -190,7 +206,7 @@ int tbx_wrap_destroy(tbx_wrap *wrap);
  * last stack_k observations per env; the newest frame goes to slot *slot_out (host int), older frames follow
  * backwards modulo stack_k (FrameStack order = slots slot+1, ..., slot+stack_k, modulo stack_k).  Envs whose
  * observation comes from a reset get it in every slot (FrameStack.reset).  reward: sum over the skipped frames,
- * its sign when clip_rewards; done: as the agent sees it (game over, or a lost life when episodic_life);
+ * its sign when clip_rewards; done: as the agent sees it (game over, a lost life when episodic_life, or the time limit);
  * real_done: game over; score / lives: before any reset.  Output pointers may be NULL. */
 int tbx_wrap_step(tbx_wrap *wrap, const int32_t *actions_dev, uint8_t *obs_ring_dev, int32_t *reward_dev, uint8_t *done_dev,
                   uint8_t *real_done_dev, int32_t *score_dev, int32_t *lives_dev, int *slot_out, void *stream);
@@ -198,8 +214,8 @@ int tbx_wrap_step(tbx_wrap *wrap, const int32_t *actions_dev, uint8_t *obs_ring_
 /* ---- Device-resident state snapshots: save, restore and fork envs without the JSON codec (DESIGN.md 4.7).
  * A snapshot of k envs is a caller-owned device buffer uint32[rows][k], word-major like the pool's planes: column j is one
  * env's whole record (both rngs, prev_score, the episode counters; rows = tbx_state_rows), followed for a wrapped env by its
- * 5 wrapper words (EpisodicLife lives, was_real_done, reset counter, Monitor return, Monitor length; rows =
- * tbx_wrap_state_rows).  A loaded env continues exactly as the saved env would have.  The device-wide episode statistics
+ * 5 wrapper words (EpisodicLife lives, was_real_done, reset counter, Monitor return, Monitor length), 7 with sticky actions
+ * (+ the remembered ALE id and the frame counter); rows = tbx_wrap_state_rows.  A loaded env continues exactly as the saved env would have.  The device-wide episode statistics
  * (tbx_stats_read) are pool state and are neither saved nor restored.
  * Breakout and Amidar records index the pool's geometry tables, so a snapshot goes with the tables blob of the moment it was
  * saved (tbx_state_tables): a tbx_state_blob_header followed by table_count tables of table_bytes bytes each (none for Space

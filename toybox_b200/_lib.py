@@ -100,6 +100,8 @@ SIGNATURES = {
     "tbx_wrap_set_stack_mode": (i32, [vp, i32]),
     "tbx_wrap_set_obs_mode": (i32, [vp, i32]),
     "tbx_wrap_set_episode_outputs": (i32, [vp, vp, vp]),
+    "tbx_wrap_set_sticky_actions": (i32, [vp, C.c_double, u64]),
+    "tbx_wrap_set_time_limit": (i32, [vp, i32, vp]),
     "tbx_wrap_step": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(i32), vp]),
     "tbx_state_rows": (i32, [vp]),
     "tbx_wrap_state_rows": (i32, [vp]),

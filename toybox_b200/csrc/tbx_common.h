@@ -126,14 +126,21 @@ TBX_HD int tbx_ale_action_to_input(int a) {
   return m;
 }
 
-/* ---- synthetic action stream of the bench / parity tests (SURVEY 8d): counter based, uniform over n_legal */
-TBX_HD uint32_t tbx_action_index(uint64_t seed, uint64_t env, uint64_t t, uint32_t n_legal) {
+/* ---- counter-based draws: the splitmix64 finaliser of (seed, env, t) */
+TBX_HD uint64_t tbx_mix(uint64_t seed, uint64_t env, uint64_t t) {
   uint64_t z = seed + env * 0x9E3779B97F4A7C15ULL + t * 0xD1B54A32D192ED03ULL;
   z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ULL;
   z = (z ^ (z >> 27)) * 0x94D049BB133111EBULL;
-  z ^= z >> 31;
-  return (uint32_t)(((z >> 32) * (uint64_t)n_legal) >> 32);
+  return z ^ (z >> 31);
 }
+/* synthetic action stream of the bench / parity tests (SURVEY 8d), and the no-op counts of the wrapper stack: uniform over n_legal */
+TBX_HD uint32_t tbx_action_index(uint64_t seed, uint64_t env, uint64_t t, uint32_t n_legal) {
+  return (uint32_t)(((tbx_mix(seed, env, t) >> 32) * (uint64_t)n_legal) >> 32);
+}
+/* the sticky-action draw of env `env` on its frame `f` (tbx_wrap.cuh): uniform over [0, 2^32).  The salt separates this stream
+ * from the no-op stream when both use one seed. */
+#define TBX_STICKY_SALT 0x5354494B59414354ULL /* "STIKYACT" */
+TBX_HD uint32_t tbx_sticky_draw(uint64_t seed, uint64_t env, uint64_t f) { return (uint32_t)(tbx_mix(seed ^ TBX_STICKY_SALT, env, f) >> 32); }
 
 /* ---- colour: r | g<<8 | b<<16 | a<<24 (the byte order of an RGBA pixel in memory) */
 TBX_HD uint32_t tbx_rgba(uint32_t r, uint32_t g, uint32_t b, uint32_t a) { return r | (g << 8) | (b << 16) | (a << 24); }

@@ -5,6 +5,7 @@
 #include "tbx_snapshot.cuh"
 #include "tbx_fields.h"
 #include "tbx_direct_launch.h"
+#include <cmath>
 #include <map>
 #include <memory>
 #include <new>
@@ -656,7 +657,12 @@ struct tbx_wrap {
   int obs_mode;   /* the ring's layout: TBX_OBS_GRAY_AREA or TBX_OBS_RGB_AREA (WarpFrame(grayscale=False)) */
   bool stepped;   /* tbx_wrap_step has run: the ring holds frames of obs_mode's layout */
   int32_t *ep_return, *ep_length; /* caller-owned device outputs of Monitor's episode record, or NULL */
+  int words;               /* wrapper words per env in wstate: 5, or 7 with sticky actions (tbx_wrap.cuh) */
+  uint64_t sticky_seed, sticky_thr; /* sticky actions: the draw's seed and llround(p * 2^32); thr 0 = off */
+  int max_steps;           /* episode time limit in agent steps, 0 = none */
+  uint8_t *truncated;      /* caller-owned device output, or NULL */
 };
+static const int TBX_WRAP_WORDS_MAX = 7; /* wstate is allocated for the sticky layout */
 
 extern "C" {
 
@@ -673,10 +679,11 @@ int tbx_wrap_create(tbx_pool *p, int skip, int noop_max, int episodic_life, int 
     w->stack_k = stack_k; w->out_w = out_w; w->out_h = out_h; w->noop_seed = noop_seed; w->env0 = env0; w->obs_mode = TBX_OBS_GRAY_AREA;
     const size_t plane_words = (size_t)p->info->rec_words * p->n_pad;
     cudaError_t e = w->planes_prev.alloc(plane_words);
-    if (e == cudaSuccess) e = w->wstate.alloc(5 * (size_t)p->n_pad);
+    w->words = 5;
+    if (e == cudaSuccess) e = w->wstate.alloc(TBX_WRAP_WORDS_MAX * (size_t)p->n_pad);
     if (e == cudaSuccess) e = w->was_reset.alloc((size_t)p->n_pad);
     if (e == cudaSuccess) e = cudaMemcpy(w->planes_prev, p->planes, plane_words * 4, cudaMemcpyDeviceToDevice);
-    if (e == cudaSuccess) e = cudaMemset(w->wstate, 0, 5 * (size_t)p->n_pad * 4);
+    if (e == cudaSuccess) e = cudaMemset(w->wstate, 0, TBX_WRAP_WORDS_MAX * (size_t)p->n_pad * 4);
     if (e == cudaSuccess) { /* EpisodicLifeEnv.__init__: lives = 0, was_real_done = True (atari_wrappers.py:155-156) */
       std::vector<uint32_t> ones((size_t)p->n_pad, 1u);
       e = cudaMemcpy(w->wstate + p->n_pad, ones.data(), ones.size() * 4, cudaMemcpyHostToDevice);
@@ -698,6 +705,27 @@ int tbx_wrap_set_obs_mode(tbx_wrap *w, int obs_mode) {
     return set_err(TBX_EINVAL, "wrap is NULL or unsupported observation layout (TBX_OBS_GRAY_AREA or TBX_OBS_RGB_AREA)");
   if (w->stepped) return set_err(TBX_EINVAL, "the observation layout is set before the first tbx_wrap_step");
   w->obs_mode = obs_mode;
+  return TBX_OK;
+}
+int tbx_wrap_set_sticky_actions(tbx_wrap *w, double repeat_action_probability, uint64_t seed) {
+  const double p = repeat_action_probability;
+  if (!w || !(p >= 0.0 && p <= 1.0)) return set_err(TBX_EINVAL, "wrap is NULL or repeat_action_probability is not in [0, 1]");
+  if (w->stepped) return set_err(TBX_EINVAL, "sticky actions are set before the first tbx_wrap_step");
+  const int words = p > 0.0 ? 7 : 5;
+  if (words == 7) { /* the remembered ALE id (NOOP) and the frame counter of every env start at 0 */
+    CK(cudaSetDevice(w->pool->device));
+    CK(cudaMemset(w->wstate + 5 * (size_t)w->pool->n_pad, 0, 2 * (size_t)w->pool->n_pad * 4));
+  }
+  w->words = words;
+  w->sticky_seed = seed;
+  w->sticky_thr = (uint64_t)llround(p * 4294967296.0);
+  return TBX_OK;
+}
+int tbx_wrap_set_time_limit(tbx_wrap *w, int max_episode_steps, uint8_t *truncated_dev) {
+  if (!w || max_episode_steps < 0) return set_err(TBX_EINVAL, "wrap is NULL or max_episode_steps < 0");
+  if (w->stepped) return set_err(TBX_EINVAL, "the time limit is set before the first tbx_wrap_step");
+  w->max_steps = max_episode_steps;
+  w->truncated = truncated_dev;
   return TBX_OK;
 }
 int tbx_wrap_set_episode_outputs(tbx_wrap *w, int32_t *ep_return_dev, int32_t *ep_length_dev) {
@@ -728,8 +756,13 @@ int tbx_wrap_step(tbx_wrap *w, const int32_t *actions, uint8_t *obs_ring, int32_
   a.noop_seed = w->noop_seed; a.env0 = w->env0;
   a.reward = reward; a.score = score; a.lives = lives; a.done = done; a.real_done = real_done; a.was_reset = w->was_reset;
   a.ep_return = w->ep_return; a.ep_length = w->ep_length;
+  a.sticky_seed = w->sticky_seed; a.sticky_thr = w->sticky_thr; a.max_steps = w->max_steps; a.truncated = w->truncated;
   a.stats = p->d_stats; a.bad_actions = p->d_bad;
-  with_game(p->game, [&](auto g) { wrap_step_kernel<decltype(g)::value><<<blocks(p->n, 128), 128, 0, s>>>(a); });
+  with_game(p->game, [&](auto g) {
+    constexpr int G = decltype(g)::value;
+    if (w->words == 7) wrap_step_kernel<G, true><<<blocks(p->n, 128), 128, 0, s>>>(a);
+    else wrap_step_kernel<G, false><<<blocks(p->n, 128), 128, 0, s>>>(a);
+  });
   CK(cudaGetLastError());
   if (obs_ring) {
     w->head = (w->head + 1) % w->stack_k;
@@ -1055,7 +1088,6 @@ int tbx_query_json(tbx_pool *p, int env, const char *query, const char *args_jso
 } /* extern "C" */
 
 /* ---- device-resident state snapshots (tbx_snapshot.cuh) */
-static const int TBX_WRAP_WORDS = 5; /* the wrapper words of tbx_wrap.cuh */
 /* the pool's interned tables as bytes */
 struct TableView { const void *data; size_t bytes; int count; };
 static TableView table_view(const tbx_pool *p) {
@@ -1077,7 +1109,7 @@ static int state_tables(const tbx_pool *p, int rows, void *out, size_t cap, size
   if (need > sizeof h) memcpy((char *)out + sizeof h, t.data, need - sizeof h);
   return TBX_OK;
 }
-/* the pool side of a copy: planes, then (wrapped env) the wrapper words */
+/* the pool side of a copy: planes, then (wrapped env) its `words` wrapper words */
 static SnapSide pool_side(const tbx_pool *p, uint32_t *wstate, const int32_t *ids) {
   SnapSide s;
   s.base0 = p->planes; s.split = p->info->rec_words; s.stride = (size_t)p->n_pad;
@@ -1101,13 +1133,13 @@ static int launch_snap_copy(const SnapArgs &a, cudaStream_t s) {
   return TBX_OK;
 }
 
-static int state_save(tbx_pool *p, uint32_t *wstate, const int32_t *ids, int k, uint32_t *snap, cudaStream_t s) {
+static int state_save(tbx_pool *p, uint32_t *wstate, int words, const int32_t *ids, int k, uint32_t *snap, cudaStream_t s) {
   if (!snap || k < 0) return set_err(TBX_EINVAL, "snap is NULL or k < 0");
   if (!ids && k > p->n) return set_err(TBX_EINVAL, "without env ids, k must not exceed the pool's env count");
   if (k == 0) return TBX_OK;
   CK(cudaSetDevice(p->device));
   SnapArgs a;
-  a.rows = p->info->rec_words + (wstate ? TBX_WRAP_WORDS : 0);
+  a.rows = p->info->rec_words + (wstate ? words : 0);
   a.src = pool_side(p, wstate, ids); a.dst = snap_side(snap, k, a.rows, 0);
   a.k = k; a.tbl_row = -1; a.tbl_lim = -1; a.remap = 0; a.owner = 0; a.bad = p->d_bad + 1;
   return launch_snap_copy(a, s);
@@ -1145,9 +1177,9 @@ static int snapshot_remap(tbx_pool *p, const uint8_t *tabs, int count, const int
   *remap = p->d_remap;
   return TBX_OK;
 }
-static int state_load(tbx_pool *p, uint32_t *wstate, const uint32_t *snap, int k_snap, const int32_t *cols, const int32_t *ids, int n, const void *blob,
+static int state_load(tbx_pool *p, uint32_t *wstate, int words, const uint32_t *snap, int k_snap, const int32_t *cols, const int32_t *ids, int n, const void *blob,
                       size_t blob_bytes, cudaStream_t s) {
-  const int rows = p->info->rec_words + (wstate ? TBX_WRAP_WORDS : 0);
+  const int rows = p->info->rec_words + (wstate ? words : 0);
   if (k_snap < 0 || n < 0 || (n > 0 && !snap)) return set_err(TBX_EINVAL, "snap is NULL, or k_snap / n < 0");
   tbx_state_blob_header h;
   if (!blob || blob_bytes < sizeof h) return set_err(TBX_EINVAL, "state snapshot: the tables blob is missing or truncated");
@@ -1178,32 +1210,32 @@ static int state_load(tbx_pool *p, uint32_t *wstate, const uint32_t *snap, int k
 extern "C" {
 
 int tbx_state_rows(const tbx_pool *p) { return p ? p->info->rec_words : 0; }
-int tbx_wrap_state_rows(const tbx_wrap *w) { return w ? w->pool->info->rec_words + TBX_WRAP_WORDS : 0; }
+int tbx_wrap_state_rows(const tbx_wrap *w) { return w ? w->pool->info->rec_words + w->words : 0; }
 int tbx_state_tables(const tbx_pool *p, void *out_host, size_t cap, size_t *size) {
   if (!p || !size) return set_err(TBX_EINVAL, "pool/size is NULL");
   return state_tables(p, p->info->rec_words, out_host, cap, size);
 }
 int tbx_wrap_state_tables(const tbx_wrap *w, void *out_host, size_t cap, size_t *size) {
   if (!w || !size) return set_err(TBX_EINVAL, "wrap/size is NULL");
-  return state_tables(w->pool, w->pool->info->rec_words + TBX_WRAP_WORDS, out_host, cap, size);
+  return state_tables(w->pool, w->pool->info->rec_words + w->words, out_host, cap, size);
 }
 int tbx_state_save(tbx_pool *p, const int32_t *ids_dev, int k, uint32_t *snap_dev, void *stream) {
   if (!p) return set_err(TBX_EINVAL, "pool is NULL");
-  return state_save(p, 0, ids_dev, k, snap_dev, (cudaStream_t)stream);
+  return state_save(p, 0, 0, ids_dev, k, snap_dev, (cudaStream_t)stream);
 }
 int tbx_wrap_state_save(tbx_wrap *w, const int32_t *ids_dev, int k, uint32_t *snap_dev, void *stream) {
   if (!w) return set_err(TBX_EINVAL, "wrap is NULL");
-  return state_save(w->pool, w->wstate, ids_dev, k, snap_dev, (cudaStream_t)stream);
+  return state_save(w->pool, w->wstate, w->words, ids_dev, k, snap_dev, (cudaStream_t)stream);
 }
 int tbx_state_load(tbx_pool *p, const uint32_t *snap_dev, int k_snap, const int32_t *cols_dev, const int32_t *ids_dev, int n, const void *tables_blob,
                    size_t blob_bytes, void *stream) {
   if (!p) return set_err(TBX_EINVAL, "pool is NULL");
-  return guarded([&] { return state_load(p, 0, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream); });
+  return guarded([&] { return state_load(p, 0, 0, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream); });
 }
 int tbx_wrap_state_load(tbx_wrap *w, const uint32_t *snap_dev, int k_snap, const int32_t *cols_dev, const int32_t *ids_dev, int n, const void *tables_blob,
                         size_t blob_bytes, void *stream) {
   if (!w) return set_err(TBX_EINVAL, "wrap is NULL");
-  return guarded([&] { return state_load(w->pool, w->wstate, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream); });
+  return guarded([&] { return state_load(w->pool, w->wstate, w->words, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream); });
 }
 
 } /* extern "C" */

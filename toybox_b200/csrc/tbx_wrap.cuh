@@ -14,9 +14,22 @@
  * (bench/monitor.py:58-76), which sits between make_atari and wrap_deepmind (common/cmd_util.py:30-36, run.py:116-119):
  * the sum of raw rewards and the number of MaxAndSkipEnv steps since the last real reset -- the FIRE / RIGHT steps of
  * FireResetEnv.reset and the NOOP step of a life-loss reset count, the no-op frames of NoopResetEnv (below Monitor) do not.
- * Deviations, both stated in DESIGN.md: the no-op count comes from the counter-based generator of this library
- * (tbx_action_index) instead of gym's np_random (a MT19937 seeded through gym's hash_seed: not part of ctoybox);
- * gym's TimeLimit wrapper (make_wrapper, :324) is not applied.
+ *
+ * Sticky actions (repeat_action_probability, Machado et al. 2018; ALE's `if (rand() >= p) m_player_a_action = action`),
+ * the STICKY instantiation: a layer directly above ToyboxBaseEnv, so the rule holds on every game frame the stack runs --
+ * the skipped frames of an agent step, the no-op frames of NoopResetEnv, the FIRE / RIGHT steps of FireResetEnv and the
+ * NOOP step of a life-loss reset.  Each frame repeats the ALE id of the env's previous frame where the draw
+ * tbx_sticky_draw(sticky_seed, env0 + i, f) < sticky_thr (= llround(p * 2^32)), else applies the requested id; f counts
+ * the env's frames and is never reset, and new_game sets the remembered id to NOOP (ALE's reset_game).  Both are two more
+ * wrapper words (7 per env).
+ * Episode time limit (max_steps > 0; gym's TimeLimit inside make_atari, between MaxAndSkipEnv and Monitor): its step
+ * count is Monitor's length, and it is tested at the end of the agent's own step.  An env at the limit reports done (so
+ * EpisodicLifeEnv sees was_real_done and the full reset chain runs) and Monitor's record, and `truncated` where its game
+ * is not over (gym's info['TimeLimit.truncated'] = not done).
+ * Deviations, all stated in DESIGN.md: the no-op count comes from the counter-based generator of this library
+ * (tbx_action_index) instead of gym's np_random (a MT19937 seeded through gym's hash_seed: not part of ctoybox); the
+ * sticky draws come from the same kind of generator instead of ALE's MT19937; reset-chain steps that cross the time limit
+ * truncate at the next agent step.
  */
 #ifndef TBX_WRAP_CUH
 #define TBX_WRAP_CUH
@@ -26,7 +39,8 @@ namespace tbxk {
 
 struct WrapArgs {
   uint32_t *planes, *planes_prev; /* state after the agent step / before its last frame (max of the two = observation) */
-  uint32_t *wstate;               /* [5][n_pad]: el_lives, was_real_done, resets, monitor return, monitor length */
+  uint32_t *wstate;               /* [5][n_pad]: el_lives, was_real_done, resets, monitor return, monitor length;
+                                     [7][n_pad] when STICKY: + the ALE id of the last frame, the frame counter */
   int n, n_pad;
   const void *cfg, *tables;
   const int32_t *legal; /* the game's legal ALE ids: gym action index -> ALE id (envs/atari/base.py:126) */
@@ -34,9 +48,12 @@ struct WrapArgs {
   const int32_t *actions; /* int32[N] gym action indices; NULL = reset every env (VecEnv.reset) */
   int skip, noop_max, episodic_life, fire_reset, clip_rewards;
   uint64_t noop_seed, env0;
+  uint64_t sticky_seed, sticky_thr; /* STICKY: a frame repeats the last id where tbx_sticky_draw(sticky_seed, env0 + i, f) < sticky_thr */
+  int max_steps;                    /* TimeLimit: 0 = none */
   int32_t *reward, *score, *lives; /* reward: summed over the skipped frames, sign() of it when clip_rewards */
   uint8_t *done, *real_done, *was_reset; /* done as the agent sees it; game over; observation comes from a reset */
-  int32_t *ep_return, *ep_length; /* may be NULL: Monitor's {'r', 'l'} of the episode that ended in this agent step (where real_done) */
+  int32_t *ep_return, *ep_length; /* may be NULL: Monitor's {'r', 'l'} of the episode that ended in this agent step (where real_done or truncated) */
+  uint8_t *truncated;             /* may be NULL: the agent step hit the time limit before the game was over */
   unsigned long long *stats;
   int *bad_actions;
 };
@@ -48,7 +65,7 @@ struct WrapArgs {
 enum { TBX_U_SKIP = 0, TBX_U_NOOP = 1 };
 enum { TBX_ST_MAIN = 0, TBX_ST_ELR_A, TBX_ST_FIRE1, TBX_ST_ELR_B, TBX_ST_FIRE2, TBX_ST_ELR_C, TBX_ST_END };
 
-template <int GAME>
+template <int GAME, bool STICKY>
 __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
   typedef Traits<GAME> T;
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
@@ -63,10 +80,16 @@ __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
   int resets = (int)a.wstate[2 * (size_t)a.n_pad + env];      /* NoopResetEnv resets so far */
   int mon_ret = (int)a.wstate[3 * (size_t)a.n_pad + env];     /* Monitor.rewards: sum and count since Monitor.reset */
   int mon_len = (int)a.wstate[4 * (size_t)a.n_pad + env];
+  int sticky_ale = 0;   /* STICKY: the ALE id applied on the env's last frame */
+  uint32_t frame = 0;   /* STICKY: the env's frame counter, the draw's key */
+  if (STICKY) {
+    sticky_ale = (int)a.wstate[5 * (size_t)a.n_pad + env];
+    frame = a.wstate[6 * (size_t)a.n_pad + env];
+  }
   int unit_rew = 0, ep_ret_out = 0, ep_len_out = 0;
 
   int total = 0, sink = 0;
-  bool out_done = false, out_real = false, reset = false;
+  bool out_done = false, out_real = false, out_trunc = false, reset = false;
   int stage = TBX_ST_END, unit = TBX_U_SKIP, frames_left = 0, ale = 0;
   bool snapped = false, unit_done = false, need_new_game = false;
   int score_out = S.ldi(TBX_HW(score)), lives_out = S.ldi(TBX_HW(lives));
@@ -97,12 +120,22 @@ __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
   }
 
   while (stage != TBX_ST_END) {
-    if (need_new_game) { T::new_game(S, cfg, tables); need_new_game = false; } /* ToyboxBaseEnv.reset (envs/atari/base.py:151-156) */
+    if (need_new_game) { /* ToyboxBaseEnv.reset (envs/atari/base.py:151-156) */
+      T::new_game(S, cfg, tables);
+      need_new_game = false;
+      if (STICKY) sticky_ale = 0; /* ALE's reset_game: the remembered action is NOOP */
+    }
     if (frames_left > 0) {
       if (unit == TBX_U_SKIP && frames_left == 1 && a.skip > 1) { TBX_SNAPSHOT(); snapped = true; } /* the state before the last repeat */
       /* ToyboxBaseEnv.step (base.py:115-149): one transition, reward = max(score - prev, 0), done = lives <= 0 */
       const int lives_before = S.ldi(TBX_HW(lives));
-      T::step(S, cfg, tables, tbx_ale_action_to_input(ale));
+      int applied = ale;
+      if (STICKY) { /* sticky actions: repeat the last frame's id with probability p */
+        if ((uint64_t)tbx_sticky_draw(a.sticky_seed, a.env0 + (uint64_t)env, (uint64_t)frame) >= a.sticky_thr) sticky_ale = ale;
+        frame++;
+        applied = sticky_ale;
+      }
+      T::step(S, cfg, tables, tbx_ale_action_to_input(applied));
       const TbxStepOut o = tbx_bookkeep(S, lives_before);
       if (stage == TBX_ST_MAIN) total += o.reward; else sink += o.reward;
       unit_rew += o.reward;
@@ -124,8 +157,12 @@ __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
     if (unit == TBX_U_NOOP) { resets++; TBX_SNAPSHOT(); }   /* the observation of a reset is a single frame */
     else if (!snapped) TBX_SNAPSHOT();                      /* stopped early: the reference's observation is stale and unused */
     bool done = unit_done;
+    if (stage == TBX_ST_MAIN && a.max_steps > 0 && mon_len >= a.max_steps) { /* TimeLimit.step, on the agent's step only */
+      out_trunc = !done; /* info['TimeLimit.truncated'] = not done */
+      done = true;
+    }
     if (stage == TBX_ST_MAIN || stage == TBX_ST_FIRE1 || stage == TBX_ST_FIRE2) {
-      if (stage == TBX_ST_MAIN) { out_real = done; if (done) { ep_ret_out = mon_ret; ep_len_out = mon_len; } } /* info['episode'] reaches the agent */
+      if (stage == TBX_ST_MAIN) { out_real = unit_done; if (done) { ep_ret_out = mon_ret; ep_len_out = mon_len; } } /* info['episode'] reaches the agent */
       if (a.episodic_life) { /* EpisodicLifeEnv.step (:158-170) */
         was_real_done = done;
         const int lives = S.ldi(TBX_HW(lives));
@@ -171,12 +208,17 @@ __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
   a.wstate[2 * (size_t)a.n_pad + env] = (uint32_t)resets;
   a.wstate[3 * (size_t)a.n_pad + env] = (uint32_t)mon_ret;
   a.wstate[4 * (size_t)a.n_pad + env] = (uint32_t)mon_len;
+  if (STICKY) {
+    a.wstate[5 * (size_t)a.n_pad + env] = (uint32_t)sticky_ale;
+    a.wstate[6 * (size_t)a.n_pad + env] = frame;
+  }
   if (a.ep_return) a.ep_return[env] = ep_ret_out;
   if (a.ep_length) a.ep_length[env] = ep_len_out;
   if (a.reward) a.reward[env] = a.clip_rewards ? (total > 0 ? 1 : total < 0 ? -1 : 0) : total;
   if (a.done) a.done[env] = (uint8_t)out_done;
   if (a.real_done) a.real_done[env] = (uint8_t)out_real;
   if (a.was_reset) a.was_reset[env] = (uint8_t)reset;
+  if (a.truncated) a.truncated[env] = (uint8_t)out_trunc;
   if (a.score) a.score[env] = score_out;
   if (a.lives) a.lives[env] = lives_out;
 }

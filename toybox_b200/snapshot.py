@@ -15,8 +15,9 @@ TBL_WORD = 14                                             # TbxHdr.tbl: the reco
 
 
 class StateSnapshot:
-    """The state of k envs: `data` int32[rows, k] (column j = one env's record, plus its 5 wrapper words when `wrapped`),
-    `tables` the blob of geometry tables the records index, and for a wrapped env `obs` uint8[k, stack, out_h, out_w], the
+    """The state of k envs: `data` int32[rows, k] (column j = one env's record, plus its wrapper words when `wrapped`: 5, or 7
+    with sticky actions), `tables` the blob of geometry tables the records index, and for a wrapped env `obs`
+    uint8[k, stack, out_h, out_w], the
     envs' observation rings, whose newest frame is in ring slot `slot`.  `game`, `rows`, `format` and `table_count` come from
     the blob's header.  Picklable (torch.save / torch.load); `.to(device)` moves it to another GPU."""
 

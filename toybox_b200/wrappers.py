@@ -29,18 +29,27 @@ class DeepmindToybox:
              observations per env -- the newest is obs[:, self.slot], FrameStack order (oldest first) is slots
              (self.slot + 1 .. self.slot + k) % k; `stacked()` returns that order as the reference's
              uint8[N, out_h, out_w, k] (uint8[N, out_h, out_w, 3k] in colour) (a copy);
-      reward int32[N] (sign of the summed reward when clip_rewards), done uint8[N] (game over, or a lost life when
-      episode_life), info = {'lives', 'score', 'real_done'} tensors (values before the reset of a finished env).
+      reward int32[N] (sign of the summed reward when clip_rewards), done uint8[N] (game over, a lost life when
+      episode_life, or the time limit), info = {'lives', 'score', 'real_done', 'truncated', 'ep_return', 'ep_length'}
+      tensors (values before the reset of a finished env; truncated: the time limit ended the episode before its game
+      was over, all zero without a limit; ep_return / ep_length: Monitor's record where real_done or truncated).
     A finished env is reset inside the same call and `obs` then holds its reset observation (VecEnv semantics)."""
 
     def __init__(self, game, n_envs, device=None, seeds=None, config=None, frame_skip=4, noop_max=30, episode_life=True,
                  fire_reset=True, clip_rewards=True, frame_stack=4, size=(84, 84), noop_seed=0, env0=0, stack_reset="fill",
-                 grayscale=True):
+                 grayscale=True, repeat_action_probability=0.0, sticky_seed=None, max_episode_steps=None):
         """stack_reset: what a reset observation does to the other k-1 ring slots -- "fill" (FrameStack.reset,
         atari_wrappers.py:262-266: wrap_deepmind(frame_stack=True), the deepq path) or "zero" (VecFrameStack,
         vec_env/vec_frame_stack.py:17-30: make_vec_env + VecFrameStack, the ppo2 / a2c path of run.py:123-125).
         grayscale: WarpFrame's argument (atari_wrappers.py:230-244); False gives colour observations, the INTER_AREA
-        down-sample of the pixel-wise max of the last two RGB frames."""
+        down-sample of the pixel-wise max of the last two RGB frames.
+        repeat_action_probability: sticky actions (Machado et al. 2018; ALE v5 uses 0.25) on every game frame the stack
+        runs, reset-chain frames included: with this probability a frame repeats the ALE id of the env's previous frame
+        instead of applying the requested one.  The draws are counter-based, keyed by (sticky_seed, env0 + i, frame);
+        sticky_seed defaults to noop_seed.
+        max_episode_steps: gym's TimeLimit inside make_atari (baselines' make_atari(env_id, max_episode_steps); ALE v5's
+        108,000 frames are 27,000 at frame_skip 4), counting Monitor's episode length.  An env at the limit reports done
+        and takes the full reset chain; info['truncated'] flags it where its game is not over."""
         if stack_reset not in ("fill", "zero"):
             raise ValueError("stack_reset is 'fill' (FrameStack) or 'zero' (VecFrameStack)")
         self.pool = BatchedToybox(game, n_envs, device=device, obs=("gray_area", size[0], size[1]), config=config, seeds=seeds)
@@ -56,8 +65,15 @@ class DeepmindToybox:
         _lib.check(self.L.tbx_wrap_set_stack_mode(self._w, 1 if stack_reset == "zero" else 0))
         if not self.grayscale:
             _lib.check(self.L.tbx_wrap_set_obs_mode(self._w, OBS_MODES["rgb_area"]))
+        self.repeat_action_probability = float(repeat_action_probability)
+        self.max_episode_steps = None if max_episode_steps is None else int(max_episode_steps)
+        if self.repeat_action_probability != 0.0:
+            seed = noop_seed if sticky_seed is None else sticky_seed
+            _lib.check(self.L.tbx_wrap_set_sticky_actions(self._w, self.repeat_action_probability, int(seed)))
         n, dev = self.n_envs, self.device
-        # Monitor's episode record (bench/monitor.py:58-76) of the episode that ended in the last agent step, where real_done
+        self.truncated = torch.zeros(n, dtype=torch.uint8, device=dev)
+        _lib.check(self.L.tbx_wrap_set_time_limit(self._w, self.max_episode_steps or 0, _ptr(self.truncated)))
+        # Monitor's episode record (bench/monitor.py:58-76) of the episode that ended in the last agent step, where real_done or truncated
         self.ep_return = torch.zeros(n_envs, dtype=torch.int32, device=self.device)
         self.ep_length = torch.zeros(n_envs, dtype=torch.int32, device=self.device)
         _lib.check(self.L.tbx_wrap_set_episode_outputs(self._w, _ptr(self.ep_return), _ptr(self.ep_length)))
@@ -102,7 +118,7 @@ class DeepmindToybox:
                 raise ValueError("expected %d actions" % self.n_envs)
         self._call(actions, render)
         return self.obs, self.reward, self.done, {"lives": self.lives, "score": self.score, "real_done": self.real_done,
-                                                    "ep_return": self.ep_return, "ep_length": self.ep_length}
+                                                    "truncated": self.truncated, "ep_return": self.ep_return, "ep_length": self.ep_length}
 
     def check(self):
         self.pool.check()
@@ -110,7 +126,8 @@ class DeepmindToybox:
     # ------------------------------------------------------------------ state snapshots
     def save_state(self, env_ids=None):
         """A StateSnapshot of the listed wrapped envs: records, wrapper state (EpisodicLife, no-op reset counter, Monitor
-        accumulators) and observation rings.  Ids as BatchedToybox.save_state."""
+        accumulators, and with sticky actions the remembered ALE id and frame counter) and observation rings.  Ids as
+        BatchedToybox.save_state."""
         ids = _snap.id_tensor(env_ids, self.n_envs, self.device, "env id")
         k = self.n_envs if ids is None else ids.numel()
         data = torch.empty((self.L.tbx_wrap_state_rows(self._w), k), dtype=torch.int32, device=self.device)
@@ -199,7 +216,8 @@ class ToyboxVecEnv:
     """The VecEnv surface of baselines (vec_env/__init__.py:26-131) over a DeepmindToybox: numpy in, numpy out, one
     process, one GPU.  It stands for `VecFrameStack(make_vec_env(env_id, 'atari', n, seed), 4)` (run.py:123-125): the stack
     of a finished env is zeroed and holds its reset observation only (vec_frame_stack.py:17-30), and
-    `infos[i]['episode'] = {'r', 'l', 't'}` appears when env i's game ends, exactly as the Monitor between make_atari and
+    `infos[i]['episode'] = {'r', 'l', 't'}` appears when env i's game ends (or its time limit, max_episode_steps, ends the
+    episode; `infos[i]['TimeLimit.truncated'] = True` then, as gym's TimeLimit reports it), exactly as the Monitor between make_atari and
     wrap_deepmind reports it (bench/monitor.py:58-76: r = sum of raw rewards, l = MaxAndSkipEnv steps incl. those of
     FireResetEnv / EpisodicLifeEnv resets, t = seconds since start) -- both counters are kept by the step kernel.
     monitor_file: path of a Monitor-compatible CSV (bench/monitor.py:22-28,70-71,96-126: a '#{json header}' line, then the
@@ -239,13 +257,17 @@ class ToyboxVecEnv:
         rew = e.reward.cpu().numpy().astype(np.float32)
         done = e.done.cpu().numpy().astype(bool)
         real = e.real_done.cpu().numpy().astype(bool)
+        trunc = e.truncated.cpu().numpy().astype(bool)
         score = e.score.cpu().numpy().astype(np.int64)
         lives = e.lives.cpu().numpy()
         infos = [{"lives": int(lives[i]), "score": int(score[i])} for i in range(self.num_envs)]
-        if real.any():
+        for i in np.flatnonzero(trunc):
+            infos[i]["TimeLimit.truncated"] = True
+        ended = real | trunc
+        if ended.any():
             ep_r, ep_l = e.ep_return.cpu().numpy(), e.ep_length.cpu().numpy()
             t = round(time.time() - self._t0, 6)
-            for i in np.flatnonzero(real):
+            for i in np.flatnonzero(ended):
                 ep = {"r": round(float(ep_r[i]), 6), "l": int(ep_l[i]), "t": t}
                 infos[i]["episode"] = ep
                 self.episode_rewards.append(ep["r"])
