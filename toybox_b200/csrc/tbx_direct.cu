@@ -86,8 +86,9 @@ cudaError_t tbx_launch_direct(const tbx::Config &c, const RenderArgs &a, const T
       const int brk_rows = c.brk.n_rows < 1 || c.brk.n_rows > TBX_BRK_MAX_ROWS ? TBX_BRK_MAX_ROWS : c.brk.n_rows;
       /* the kernel's small tables follow the staged frame: digit patches, base-frame row classes, division table, the wall's H look-up */
       d.smem_base += TBX_BRK_TAB_BYTES + align16(brk_rows * 4 * d.hstride * (int)sizeof(float));
-      /* per warp: its env's record, the wall's H rows, the movers' records; two record stages */
-      d.warp_bytes = align16(RW * 4) + align16(brk_rows * d.hstride * (int)sizeof(float)) + 256;
+      /* per warp: the wall's H rows, the movers' records (the env's record is read in place from its team's stage); two record
+       * stages */
+      d.warp_bytes = align16(brk_rows * d.hstride * (int)sizeof(float)) + 256;
       d.smem_total = d.smem_base + 2 * RW * TBX_EPC * 4 + (TBX_DIRECT_THREADS / 32) * d.warp_bytes;
       return with_taps<5>(plan.tx, plan.ty, [&](auto X, auto Y) {
         constexpr int TX = decltype(X)::value, TY = decltype(Y)::value;

@@ -67,10 +67,57 @@ TBX_HD TbxMover brk_mover(const uint32_t *R, const BrkCfg &c, uint32_t paddle_gr
   return v;
 }
 
+/* tbx_d2i's contract (truncate, saturate to +-2^29, NaN -> 0) as one saturating conversion and two integer clamps: on the
+ * device cvt.rzi.s32.f64 already saturates to the int32 range and maps NaN to 0; the host restates that conversion */
+TBX_HD int tbx_d2i_sat(double v) {
+#if defined(__CUDA_ARCH__)
+  const int i = __double2int_rz(v);
+  return min(max(i, -536870912), 536870912);
+#else
+  const int i = !(v == v) ? 0 : v >= 2147483647.0 ? 2147483647 : v <= -2147483648.0 ? (-2147483647 - 1) : (int)v;
+  return i < -536870912 ? -536870912 : i > 536870912 ? 536870912 : i;
+#endif
+}
+
+/* brk_mover read straight from the record (any word stride), without the draw-list primitive: the same rectangle for every
+ * input.  tbx_prim_rect clips to +-30000 and keeps the extent in 16 bits, so an extent above 32767 after that clip wraps
+ * negative and the mover draws nothing; the rest of its clipping is the canvas clip below. */
+TBX_HD TbxMover brk_mover_rec(const TbxAcc &S, uint32_t paddle_gray, uint32_t ball_gray, int m) {
+  TbxMover v; v.x0 = v.y0 = v.x1 = v.y1 = 0; v.gray = m == 0 ? paddle_gray : ball_gray;
+  if (m < 0 || m >= BRK_N_MOVERS || (m > 0 && m > S.ldi(BRK_W(n_balls)))) return v;
+  int x, y, w, h;
+  if (m == 0) {
+    const double pw = S.ldd(BRK_W(paddle_width));
+    x = tbx_d2i_sat(tbx_dsub(S.ldd(BRK_W(paddle_px)), tbx_dmul(pw, 0.5)));
+    y = tbx_d2i_sat(tbx_dsub(S.ldd(BRK_W(paddle_py)), BRK_PADDLE_HALF_H));
+    w = tbx_d2i_sat(pw); h = 3;
+  } else {
+    const double r = S.ldd(BRK_W(ball_radius));
+    const int b = BRK_W(ball) + 8 * (m - 1);
+    x = tbx_d2i_sat(tbx_dsub(S.ldd(b), r));
+    y = tbx_d2i_sat(tbx_dsub(S.ldd(b + 2), r));
+    w = h = tbx_d2i_sat(tbx_dmul(r, 2.0));
+  }
+  /* |x|, |w| <= 2^29: x + w does not overflow; w <= 0 leaves x1 <= x0 */
+  const int x0 = x < 0 ? 0 : x, y0 = y < 0 ? 0 : y;
+  const int x1 = x + w > TBX_BRK_W ? TBX_BRK_W : x + w, y1 = y + h > TBX_BRK_H ? TBX_BRK_H : y + h;
+  const int ex = (x + w > 30000 ? 30000 : x + w) - (x < -30000 ? -30000 : x), ey = (y + h > 30000 ? 30000 : y + h) - (y < -30000 ? -30000 : y);
+  if (x0 >= x1 || y0 >= y1 || ex > 32767 || ey > 32767) return v;
+  v.x0 = x0; v.y0 = y0; v.x1 = x1; v.y1 = y1;
+  return v;
+}
+
 /* alive bits of brick column c (bit r = row r) */
 TBX_HD uint32_t brk_col_bits(const uint32_t *alive, int nrows, int c) {
   const int i0 = c * nrows, w = i0 >> 5, s = i0 & 31;
   const uint32_t lo = alive[w], hi = w < 4 ? alive[w + 1] : 0u;
+  const uint32_t v = s ? (lo >> s) | (hi << (32 - s)) : lo;
+  return v & ((1u << nrows) - 1u);
+}
+/* ... the same from a record of any word stride, the alive words starting at word w0 */
+TBX_HD uint32_t brk_col_bits(const TbxAcc &S, int w0, int nrows, int c) {
+  const int i0 = c * nrows, w = i0 >> 5, s = i0 & 31;
+  const uint32_t lo = S.ld(w0 + w), hi = w < 4 ? S.ld(w0 + w + 1) : 0u;
   const uint32_t v = s ? (lo >> s) | (hi << (32 - s)) : lo;
   return v & ((1u << nrows) - 1u);
 }

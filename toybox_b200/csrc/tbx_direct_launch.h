@@ -13,12 +13,13 @@ struct DirectArgs {
   const void *aux;    /* the game's closed-form tables on the device (TbxBrkDirect, TbxSiDirect) */
   const void *aux2;   /* Space Invaders: the sprite patch tables (TbxSpritePatch[]) */
   int32_t *fb_list;   /* envs handed to the tile kernel */
-  int *fb_count;
+  int *fb_count;      /* this render's hand-over count */
   int *sched;         /* [2]: next chunk id - grid size, finished CTAs (dynamic chunk scheduling of the persistent kernels) */
   int hstride;        /* floats per H row in shared memory */
   int warp_bytes;     /* shared memory per warp */
   int smem_base;      /* bytes of the staged base-frame down-sample at the start of shared memory */
   int smem_total;
+  int *fb_other;      /* the previous render's hand-over count: the last CTA zeroes it for the next render */
 };
 
 /* An owning buffer of T elements in device memory (cudaMalloc) or pinned host memory (cudaMallocHost): move-only, freed

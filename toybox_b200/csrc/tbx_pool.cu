@@ -83,7 +83,8 @@ struct tbx_pool {
   std::unique_ptr<BaseFrames> base;
   std::map<std::pair<int, int>, AreaRes> area;
   Buf<int32_t> d_dense; /* [0] = count, [8..] = env ids the patch kernel left to the canvas kernel */
-  Buf<int32_t> d_fb;    /* [0] = count, [1] = finished CTAs, [8..] = env ids the direct INTER_AREA kernel left to the tile kernel */
+  Buf<int32_t> d_fb;    /* [0], [1] = hand-over counts, [2..3] = chunk scheduling, [8..] = env ids the direct INTER_AREA kernel left to the tile kernel */
+  int fb_pair = 0;      /* the hand-over count of the next render: d_fb[fb_pair]; renders alternate between the two */
   /* JSON import / export staging (grown on demand, kept): env ids and AoS records on the device, records in pinned host memory */
   Buf<int32_t> j_ids;
   Buf<uint32_t> j_recs;
@@ -549,12 +550,17 @@ static int render_area(tbx_pool *p, RenderArgs &a, int out_w, int out_h, bool rg
       CK(cudaMemsetAsync(fb, 0, 8 * sizeof(int32_t), s));
       p->d_fb = std::move(fb);
     }
+    /* two hand-over counts, one per render in turn: the direct kernel's last CTA zeroes the other one, which the previous
+     * render's tile kernel has finished reading (stream order), so the tile kernel only reads its count */
+    const int pair = p->fb_pair;
     DirectArgs da = {};
-    da.aux = ar->d_direct; da.aux2 = ar->d_direct2; da.fb_list = p->d_fb + 8; da.fb_count = p->d_fb; da.sched = p->d_fb + 2;
+    da.aux = ar->d_direct; da.aux2 = ar->d_direct2; da.fb_list = p->d_fb + 8; da.fb_count = p->d_fb + pair; da.fb_other = p->d_fb + (pair ^ 1);
+    da.sched = p->d_fb + 2;
     CK(tbx_launch_direct(p->cfg, a, plan, da, s));
     if (p->game == TBX_SPACE_INVADERS) return TBX_OK; /* covers every env: nothing is handed over */
+    p->fb_pair = pair ^ 1;
     a.env_list = p->d_fb + 8;
-    a.env_count = p->d_fb;
+    a.env_count = p->d_fb + pair;
   }
   return with_game(p->game, [&](auto g) {
     constexpr int G = decltype(g)::value;

@@ -609,12 +609,8 @@ __global__ void __launch_bounds__(TBX_TILE_THREADS, DUAL && RGB ? TBX_TILE_DUAL_
     }
   }
   } /* chunk */
-  /* env-list mode: the last CTA to finish empties the list for the next render (every CTA has read the count by then) */
-  if (a.env_list && a.env_count && tid == 0) {
-    int *cnt = const_cast<int *>(a.env_count);
-    __threadfence();
-    if (atomicAdd(cnt + 1, 1) == (int)gridDim.x - 1) { cnt[0] = 0; cnt[1] = 0; __threadfence(); }
-  }
+  /* env-list mode leaves the count as it is: the next render counts on the other one, and the direct kernel after it zeroes
+   * this one (render_area) */
 }
 
 } /* namespace tbxk */

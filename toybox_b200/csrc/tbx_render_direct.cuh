@@ -49,12 +49,12 @@ __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wai
  * frame starts as ONE bulk shared -> global copy of it, cp.async.bulk, no per-env load/store instructions); the small tables the
  * per-pixel code indexes (digit patches of the slots in use, base frame 0 by row classes, the wall's H look-up, the plan's weights
  * and first-source indices, a division table: L1 is too small next to this much shared memory to keep them); per team two stages
- * of word-major records (cp.async prefetch of the next chunk); per warp its env's record, the wall's H rows, the movers' records. */
+ * of word-major records (cp.async prefetch of the next chunk; a warp reads its env's record there, in place); per warp the wall's H
+ * rows and the movers' records. */
 template <int TX, int TY>
 __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_direct_kernel(const __grid_constant__ RenderArgs a, const __grid_constant__ BrkCfg cfg_c,
                                                                             const __grid_constant__ TbxAreaPlan plan_c, const __grid_constant__ DirectArgs d) {
   constexpr int RW = TBX_WORDS(BrkRec);
-  constexpr int RECW_BYTES = (RW * 4 + 15) & ~15;
   extern __shared__ uint4 smem_raw[];
   uint8_t *smem = reinterpret_cast<uint8_t *>(smem_raw);
   uint8_t *sbase = smem;                                                        /* base frame 1, down-sampled */
@@ -79,8 +79,7 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
   const TbxAreaPlan &cp = plan_c;                /* warp-uniform reads: constant bank */
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   uint8_t *wmem = smem + d.smem_base + 2 * RW * TBX_EPC * 4 + wid * d.warp_bytes;
-  uint32_t *recw = reinterpret_cast<uint32_t *>(wmem);                          /* this warp's env, as a record */
-  float *hw = reinterpret_cast<float *>(wmem + RECW_BYTES);
+  float *hw = reinterpret_cast<float *>(wmem);
   int4 *mrec = reinterpret_cast<int4 *>(wmem + d.warp_bytes - 256);             /* 3 x int4 per mover */
   /* two TEAMS of 4 warps per CTA, each with its own chunks of 4 envs (one 16-byte copy per state word), record stages and
    * barrier: a team waits for the slowest of 4 envs instead of 8 */
@@ -140,7 +139,6 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
   const TbxDigitPatch *__restrict__ patches = a.patches[1];
   __syncthreads(); /* the tables are complete */
   const bool dig_smem = s_bigdig == 0;
-  const uint32_t *R = recw;
 
   int st = 0, it = 0, nxt = 0;
   for (int chunk = (int)blockIdx.x * 2 + team; chunk < n_chunks; chunk = nxt, st ^= 1, it++) {
@@ -152,14 +150,13 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
     if (ttid == 0) s_next[team][(it + 1) & 1] = n_teams + atomicAdd(d.sched, 1);
     const int env = chunk * TEAM + wt;
     if (env >= a.n) continue;
-    {
-      const uint32_t *src = tstage + st * RW * TEAM + wt;
-      for (int w = lane; w < RW; w += 32) recw[w] = src[w * TEAM];
-    }
-    __syncwarp();
+    /* the env's record, read in place from the team's stage (word w at Rs[w * TEAM]): the stage is not written again before
+     * the team's next barrier */
+    const uint32_t *Rs = tstage + st * RW * TEAM + wt;
+    const TbxAcc S{const_cast<uint32_t *>(Rs), TEAM};
     uint8_t *out = a.dst + (size_t)env * a.env_stride + (size_t)a.stack_slot * a.frame_bytes;
     /* movers: lane 0 the paddle, lanes 1..4 the balls; footprint = the output pixels the rectangle feeds */
-    const TbxMover mine = brk_mover(R, cfg_c, paddle_gray, ball_gray, lane < BRK_N_MOVERS ? lane : -1);
+    const TbxMover mine = brk_mover_rec(S, paddle_gray, ball_gray, lane < BRK_N_MOVERS ? lane : -1);
     const bool valid = mine.x0 < mine.x1;
     int fx0 = 0, fx1 = 0, fy0 = 0, fy1 = 0;
     if (valid) { fx0 = __ldg(&plan->xdlo[mine.x0]); fx1 = __ldg(&plan->xdhi[mine.x1 - 1]); fy0 = __ldg(&plan->ydlo[mine.y0]); fy1 = __ldg(&plan->ydhi[mine.y1 - 1]); }
@@ -169,14 +166,14 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
     const TbxDigitPatch *P = patches;
     if (lane < 2 * TBX_MAX_DIGITS && patches) {
       const int field = lane >= TBX_MAX_DIGITS;
-      dig = tbx_digit_at((int32_t)R[field ? TBX_HW(lives) : TBX_HW(score)], lane - field * TBX_MAX_DIGITS);
+      dig = tbx_digit_at(S.ldi(field ? TBX_HW(lives) : TBX_HW(score)), lane - field * TBX_MAX_DIGITS);
       if (dig >= 0) {
         const int cid = brk_dig_cid(lane);
         P = patches + lane * 10 + dig;
         bad |= (dig_smem && cid >= 0 ? (sdig[(cid * 10 + dig) * TBX_BRK_DIG_WORDS] >> 16) & 255u : (uint32_t)__ldg(&P->w)) == 0;
       }
     }
-    const bool covered = ok && patches && (int32_t)R[TBX_HW(tbl)] == cfg_c.default_tbl;
+    const bool covered = ok && patches && S.ldi(TBX_HW(tbl)) == cfg_c.default_tbl;
     if (!covered || __any_sync(0xffffffffu, bad)) { /* the general kernel's */
       if (lane == 0) d.fb_list[atomicAdd(d.fb_count, 1)] = env;
       continue;
@@ -208,7 +205,7 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
 #pragma unroll
     for (int m = 0; m < BRK_N_MOVERS; m++) total += mrec[3 * m + 2].x;
     const uint32_t *__restrict__ base0w = reinterpret_cast<const uint32_t *>(a.base[0]);
-    const uint32_t *alive = R + BRK_W(alive);
+    const uint32_t *alive = Rs + BRK_W(alive) * TEAM; /* alive word k at alive[k * TEAM] */
     /* pixel p0 + lane of the movers' list: its offset in the frame (-1: past the end) and its value */
     auto mover_pixel = [&](int p0, int &o) -> uint32_t {
       const int l = p0 + lane;
@@ -250,7 +247,7 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
           for (int t = 0; t < TX; t++) {
             if (cb[t] == 255u) continue;
             const uint32_t i = cb[t] * (uint32_t)nrows + r;
-            if (!((alive[i >> 5] >> (i & 31)) & 1u)) continue;
+            if (!((alive[(i >> 5) * TEAM] >> (i & 31)) & 1u)) continue;
             const uint32_t g = __ldg(&A.brickgray[i]);
             if (t < 4) lo[k] = (lo[k] & ~(255u << (8 * t))) | (g << (8 * t));
             else hi[k] = g;
@@ -295,7 +292,7 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
     if (total > 0) v_first = mover_pixel(0, o_first);
     /* 2. the wall */
     const uint32_t fullm = (1u << nrows) - 1u;
-    const uint32_t colbits = lane < ncols ? brk_col_bits(R + BRK_W(alive), nrows, lane) : fullm;
+    const uint32_t colbits = lane < ncols ? brk_col_bits(S, BRK_W(alive), nrows, lane) : fullm;
     const uint32_t deadcols = __ballot_sync(0xffffffffu, colbits != fullm);
     bool landed = false; /* the base copy must have landed before the first patch is written over it */
 #define TBX_DIRECT_LAND()                                                                       \
@@ -350,29 +347,52 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
         }
       }
     }
-    /* 3. HUD digits: one patch at a time, lanes over (row, column) */
+    /* 3. HUD digits.  The slots cached in sdig (score digits 0..3, lives digits 0..1) in ONE pass over the concatenation of their
+     * patches' pixels, lane l taking pixels l, l + 32, ...: the patches of two cached slots never share an output pixel at any
+     * size this kernel accepts (tests/test_direct_digits_cpu.py), so their order does not matter.  The other shown digits come
+     * after, one patch at a time from the table itself, in slot order: where one of them meets a cached slot it is the later
+     * slot, as in the draw list. */
     TBX_DIRECT_LAND();
     {
-      uint32_t dm = __ballot_sync(0xffffffffu, dig >= 0);
+      const int cid = brk_dig_cid(lane);
+      const bool cached = dig >= 0 && dig_smem && cid >= 0;
+      const uint32_t hdr = cached ? sdig[(cid * 10 + dig) * TBX_BRK_DIG_WORDS] : 0u; /* header word (x0, y0, w, h) */
+      /* pixel offsets of the six slots in the concatenation (warp-uniform): slot c starts at off[c] */
+      int off[TBX_BRK_DIG_SLOTS + 1];
+      off[0] = 0;
+#pragma unroll
+      for (int c = 0; c < TBX_BRK_DIG_SLOTS; c++) {
+        const uint32_t h = __shfl_sync(0xffffffffu, hdr, c < 4 ? c : TBX_MAX_DIGITS + c - 4);
+        off[c + 1] = off[c] + (int)(((h >> 16) & 255u) * (h >> 24));
+      }
+      const int ntot = off[TBX_BRK_DIG_SLOTS];
+      const uint8_t *sdigb = reinterpret_cast<const uint8_t *>(sdig);
+      for (int i0 = 0; i0 < ntot; i0 += 32) {
+        const int i = i0 + lane;
+        int c = 0, o = 0;
+#pragma unroll
+        for (int k = 1; k < TBX_BRK_DIG_SLOTS; k++)
+          if (i >= off[k]) { c = k; o = off[k]; } /* the last slot that starts at or before i: empty slots are skipped over */
+        const int src = c < 4 ? c : TBX_MAX_DIGITS + c - 4;
+        const uint32_t h = __shfl_sync(0xffffffffu, hdr, src);
+        const int dg = __shfl_sync(0xffffffffu, dig, src);
+        if (i < ntot) {
+          const int q = i - o, pw = (h >> 16) & 255u;
+          const int r = pw > 1 ? (int)__umulhi((unsigned)q, sinv[pw]) : q;
+          out[(((h >> 8) & 255u) + r) * dw + (h & 255u) + q - r * pw] = sdigb[(c * 10 + dg) * TBX_BRK_DIG_WORDS * 4 + 4 + q];
+        }
+      }
+      uint32_t dm = __ballot_sync(0xffffffffu, dig >= 0 && !cached);
       while (dm) {
         const int l = __ffs(dm) - 1;
         dm &= dm - 1;
         const int dgt = __shfl_sync(0xffffffffu, dig, l);
         const int cc = lane & 7;
-        /* the patch: header word (x0, y0, w, h), then w x h pixels -- the compact copy in shared memory, or the table itself */
-        const int cid = brk_dig_cid(l);
-        if (dig_smem && cid >= 0) {
-          const uint8_t *Q = reinterpret_cast<const uint8_t *>(sdig + (cid * 10 + dgt) * TBX_BRK_DIG_WORDS);
-          const uint32_t hdr = *reinterpret_cast<const uint32_t *>(Q);
-          const int px0 = hdr & 255u, py0 = (hdr >> 8) & 255u, pw = (hdr >> 16) & 255u, ph = hdr >> 24;
-          if (cc < pw)
-            for (int r = lane >> 3; r < ph; r += 4) out[(py0 + r) * dw + px0 + cc] = Q[4 + r * pw + cc];
-        } else {
-          const TbxDigitPatch *Q = patches + l * 10 + dgt;
-          const int px0 = __ldg(&Q->x0), py0 = __ldg(&Q->y0), pw = __ldg(&Q->w), ph = __ldg(&Q->h);
-          if (cc < pw)
-            for (int r = lane >> 3; r < ph; r += 4) out[(py0 + r) * dw + px0 + cc] = __ldg(&Q->px[r * pw + cc]);
-        }
+        /* the patch: position, size, then w x h pixels */
+        const TbxDigitPatch *Q = patches + l * 10 + dgt;
+        const int px0 = __ldg(&Q->x0), py0 = __ldg(&Q->y0), pw = __ldg(&Q->w), ph = __ldg(&Q->h);
+        if (cc < pw)
+          for (int r = lane >> 3; r < ph; r += 4) out[(py0 + r) * dw + px0 + cc] = __ldg(&Q->px[r * pw + cc]);
       }
     }
     __syncwarp(); /* the movers' pixels go over the wall's */
@@ -386,10 +406,11 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
   }
 #undef TBX_DIRECT_LAND
   __syncthreads(); /* both teams have run dry */
-  /* the last CTA to finish re-arms the chunk counter for the next launch */
+  /* the last CTA to finish re-arms the chunk counter for the next launch, and zeroes the previous render's hand-over count (its
+   * tile kernel ran before this launch): the next render appends to it */
   if (tid == 0) {
     __threadfence();
-    if (atomicAdd(d.sched + 1, 1) == (int)gridDim.x - 1) { d.sched[0] = 0; d.sched[1] = 0; __threadfence(); }
+    if (atomicAdd(d.sched + 1, 1) == (int)gridDim.x - 1) { d.sched[0] = 0; d.sched[1] = 0; *d.fb_other = 0; __threadfence(); }
   }
 }
 
@@ -1082,10 +1103,11 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) ami_d
     }
   }
   __syncthreads(); /* both teams have run dry */
-  /* the last CTA to finish re-arms the chunk counter for the next launch */
+  /* the last CTA to finish re-arms the chunk counter for the next launch, and zeroes the previous render's hand-over count (its
+   * tile kernel ran before this launch): the next render appends to it */
   if (tid == 0) {
     __threadfence();
-    if (atomicAdd(d.sched + 1, 1) == (int)gridDim.x - 1) { d.sched[0] = 0; d.sched[1] = 0; __threadfence(); }
+    if (atomicAdd(d.sched + 1, 1) == (int)gridDim.x - 1) { d.sched[0] = 0; d.sched[1] = 0; *d.fb_other = 0; __threadfence(); }
   }
 }
 
