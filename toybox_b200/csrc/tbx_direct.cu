@@ -15,12 +15,17 @@ template <class D> static cudaError_t upload_direct(const std::vector<D> &A, Buf
 }
 
 cudaError_t tbx_direct_build(const tbx::Config &c, const BrkTable *brk_default, const tbx::ResizeTab &rs, const TbxAreaPlan &plan, const uint8_t *base0_gray,
-                             Buf<uint8_t> &aux, Buf<uint8_t> &aux2) {
+                             const uint8_t *base1_out, const TbxDigitPatch *patches1, Buf<uint8_t> &aux, Buf<uint8_t> &aux2) {
   if (c.game == TBX_BREAKOUT) {
     if (!brk_default) return cudaSuccess;
     std::vector<TbxBrkDirect> A(1);
     tbx::build_brk_direct(c, *brk_default, rs, plan, base0_gray, A[0]);
-    return upload_direct(A, aux);
+    if (!A[0].ok) return cudaSuccess;
+    const Taps t = inst_taps(plan.tx, plan.ty); /* the kernel instantiation the image is laid out for */
+    std::vector<uint8_t> img;
+    tbx::build_brk_img(A[0], plan, t.x, t.y, base1_out, patches1, img);
+    const cudaError_t e = upload_direct(A, aux);
+    return e != cudaSuccess ? e : aux2.upload(img.data(), img.size());
   }
   if (c.game == TBX_AMIDAR) {
     std::vector<TbxAmiDirect> A(1);
@@ -76,7 +81,7 @@ template <class... P, class... A> static cudaError_t launch_persistent(void (*ke
   return cudaGetLastError();
 }
 
-cudaError_t tbx_launch_direct(const tbx::Config &c, const RenderArgs &a, const TbxAreaPlan &plan, DirectArgs d, cudaStream_t s) {
+cudaError_t tbx_launch_direct(const tbx::Config &c, const RenderArgs &a, const TbxAreaPlan &plan, DirectArgs d, size_t aux2_bytes, cudaStream_t s) {
   const int out_w = plan.dw, out_h = plan.dh;
   d.hstride = (out_w + 3) & ~3;
   d.smem_base = align16(out_w * out_h);
@@ -84,16 +89,14 @@ cudaError_t tbx_launch_direct(const tbx::Config &c, const RenderArgs &a, const T
     constexpr int G = decltype(g)::value, RW = Traits<G>::RW;
     if constexpr (G == TBX_BREAKOUT) {
       const int brk_rows = c.brk.n_rows < 1 || c.brk.n_rows > TBX_BRK_MAX_ROWS ? TBX_BRK_MAX_ROWS : c.brk.n_rows;
-      /* the kernel's small tables follow the staged frame: digit patches, base-frame row classes, division table, the wall's H look-up */
-      d.smem_base += TBX_BRK_TAB_BYTES + align16(brk_rows * 4 * d.hstride * (int)sizeof(float));
-      /* per warp: the wall's H rows, the movers' records (the env's record is read in place from its team's stage); two record
-       * stages */
+      /* the table image (tbx_direct.h) first; then two record stages per team; per warp the wall's H rows and the movers' records
+       * (the env's record is read in place from its team's stage).  The image's size sets the residency, and with it the grid */
+      if (aux2_bytes == 0 || aux2_bytes % 16 != 0 || aux2_bytes > 256 * 1024) return cudaErrorInvalidValue;
+      d.smem_base = (int)aux2_bytes;
       d.warp_bytes = align16(brk_rows * d.hstride * (int)sizeof(float)) + 256;
       d.smem_total = d.smem_base + 2 * RW * TBX_EPC * 4 + (TBX_DIRECT_THREADS / 32) * d.warp_bytes;
       return with_taps<5>(plan.tx, plan.ty, [&](auto X, auto Y) {
-        constexpr int TX = decltype(X)::value, TY = decltype(Y)::value;
-        /* the plan's per-pixel tables go behind the rest */
-        return launch_persistent(brk_direct_kernel<TX, TY>, d.smem_total + brk_plan_smem_bytes(TX, TY, out_w, out_h), a.n, s, a, c.brk, plan, d);
+        return launch_persistent(brk_direct_kernel<decltype(X)::value, decltype(Y)::value>, d.smem_total, a.n, s, a, c.brk, plan, d);
       });
     } else if constexpr (G == TBX_AMIDAR) {
       /* per warp: its env's record, the tile rows as looks, the movers' records; two record stages */

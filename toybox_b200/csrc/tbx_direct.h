@@ -54,6 +54,52 @@ typedef struct TbxBrkDirect {
   alignas(16) uint8_t clsrows[TBX_BD_MAX_CLS * TBX_BRK_W + 16];
 } TbxBrkDirect;
 
+/* THE SHARED-MEMORY IMAGE of the Breakout direct kernel: every table its per-env code reads, laid out on the host exactly as the
+ * kernel wants it (tbx::build_brk_img, one per (config, output size)) and copied whole, by one bulk copy, at the start of its shared
+ * memory.  The fixed-size tables come first, at offsets that depend on TY only (constants in the kernel), then the tables sized by
+ * the output size and the config (brk_img_layout).  Every offset is a multiple of 16. */
+#define TBX_A16(v) (((v) + 15) & ~15)
+#define TBX_BRK_DIG_SLOTS 6  /* digit slots whose patches are kept in the image: score digits 0..3, lives digits 0..1 */
+#define TBX_BRK_DIG_WORDS 13 /* header word + up to 48 pixels: the first 52 bytes of the TbxDigitPatch */
+#define TBX_BRK_DIG_BYTES (TBX_BRK_DIG_SLOTS * 10 * TBX_BRK_DIG_WORDS * 4)
+#define TBX_BI_FLAGS 0                                                          /* int32: 1 = every cached slot's patches fit 48 pixels */
+#define TBX_BI_DIG 16                                                           /* uint32 [6 slots x 10 digits][13] */
+#define TBX_BI_ROWCLS (TBX_BI_DIG + TBX_A16(TBX_BRK_DIG_BYTES))                 /* TbxBrkDirect.rowcls */
+#define TBX_BI_INV (TBX_BI_ROWCLS + TBX_A16(TBX_BRK_H))                         /* .inv32 */
+#define TBX_BI_XDLO (TBX_BI_INV + TBX_A16(4 * (TBX_AREA_MAX_DST + 1)))          /* plan xdlo / xdhi / ydlo / ydhi over the frame's W or H */
+#define TBX_BI_XDHI (TBX_BI_XDLO + TBX_A16(TBX_BRK_W))
+#define TBX_BI_YDLO (TBX_BI_XDHI + TBX_A16(TBX_BRK_W))
+#define TBX_BI_YDHI (TBX_BI_YDLO + TBX_A16(TBX_BRK_H))
+#define TBX_BI_XCOL (TBX_BI_YDHI + TBX_A16(TBX_BRK_H))                          /* .xcol over W */
+#define TBX_BI_YROW (TBX_BI_XCOL + TBX_A16(TBX_BRK_W))                          /* .yrow over H */
+#define TBX_BI_BGRAY (TBX_BI_YROW + TBX_A16(TBX_BRK_H))                         /* .brickgray */
+#define TBX_BI_WORDCOLS (TBX_BI_BGRAY + TBX_A16(TBX_BRK_MAX_BRICKS))            /* .wordcols */
+#define TBX_BI_COL0 (TBX_BI_WORDCOLS + 4 * 32)                                  /* .col0 */
+#define TBX_BI_DYROWS (TBX_BI_COL0 + TBX_A16(TBX_AREA_MAX_DST))                 /* .dyrows */
+#define TBX_BI_HSEL (TBX_BI_DYROWS + TBX_A16(TBX_AREA_MAX_DST))                 /* .hsel as [MAX_DST][TY] */
+#define TBX_BI_FIXED(ty) (TBX_BI_HSEL + TBX_A16(TBX_AREA_MAX_DST * (ty)))
+/* pitch of the plan's per-pixel tables in the image */
+TBX_HD int brk_plan_pitch(int dw, int dh) { return ((dw > dh ? dw : dh) + 3) & ~3; }
+struct TbxBrkImgLayout {
+  int base1;   /* uint8 [dh][dw]: the down-sample of base frame 1 (every brick alive) */
+  int plan;    /* float xalpha [TX][ps], yalpha [TY][ps]; uint16 xs0 [ps], ys0 [ps] (ps = brk_plan_pitch, clamped to dw - 1 / dh - 1) */
+  int hlut;    /* float [nrows x 4][hs]: .hlut */
+  int hstatic; /* float [n_static][hs]: the rows of .hstatic in use */
+  int cls;     /* uint8 [n_cls][W] + 16 bytes of slack: the classes of .clsrows in use */
+  int bytes;
+};
+TBX_HD TbxBrkImgLayout brk_img_layout(int tx, int ty, int dw, int dh, int nrows, int n_static, int n_cls) {
+  const int ps = brk_plan_pitch(dw, dh), hs = (dw + 3) & ~3;
+  TbxBrkImgLayout L;
+  L.base1 = TBX_BI_FIXED(ty);
+  L.plan = L.base1 + TBX_A16(dw * dh);
+  L.hlut = L.plan + TBX_A16((tx + ty) * ps * 4 + 2 * ps * 2);
+  L.hstatic = L.hlut + TBX_A16(nrows * 4 * hs * 4);
+  L.cls = L.hstatic + TBX_A16(n_static * hs * 4);
+  L.bytes = L.cls + TBX_A16(n_cls * TBX_BRK_W + 16);
+  return L;
+}
+
 /* paddle (m == 0) or ball m - 1 as a clipped rectangle */
 TBX_HD TbxMover brk_mover(const uint32_t *R, const BrkCfg &c, uint32_t paddle_gray, uint32_t ball_gray, int m) {
   TbxMover v; v.x0 = v.y0 = v.x1 = v.y1 = 0; v.gray = m == 0 ? paddle_gray : ball_gray;

@@ -11,13 +11,14 @@
 namespace tbxk {
 struct DirectArgs {
   const void *aux;    /* the game's closed-form tables on the device (TbxBrkDirect, TbxSiDirect) */
-  const void *aux2;   /* Space Invaders: the sprite patch tables (TbxSpritePatch[]) */
+  const void *aux2;   /* Space Invaders: the sprite patch tables (TbxSpritePatch[]); Breakout: the shared-memory image */
   int32_t *fb_list;   /* envs handed to the tile kernel */
   int *fb_count;      /* this render's hand-over count */
   int *sched;         /* [2]: next chunk id - grid size, finished CTAs (dynamic chunk scheduling of the persistent kernels) */
   int hstride;        /* floats per H row in shared memory */
   int warp_bytes;     /* shared memory per warp */
-  int smem_base;      /* bytes of the staged base-frame down-sample at the start of shared memory */
+  int smem_base;      /* bytes at the start of shared memory before the record stages: the staged base-frame down-sample (Breakout: the
+                       * table image at aux2, tbx_direct.h) */
   int smem_total;
   int *fb_other;      /* the previous render's hand-over count: the last CTA zeroes it for the next render */
 };
@@ -94,10 +95,12 @@ template <int MAX_TX, class F> inline auto with_taps(int tx, int ty, F &&f) {
 }
 }
 
-/* closed-form tables of one (config, output size) pair on the device; aux stays empty when the pair is not covered */
+/* closed-form tables of one (config, output size) pair on the device; aux stays empty when the pair is not covered.  Breakout also
+ * needs the down-sample of base frame 1 and its digit patches (TBX_DP_SLOTS x 10), for its shared-memory image in aux2: rebuild
+ * the tables whenever those change */
 cudaError_t tbx_direct_build(const tbx::Config &c, const BrkTable *brk_default, const tbx::ResizeTab &rs, const TbxAreaPlan &plan, const uint8_t *base0_gray,
-                             tbxk::Buf<uint8_t> &aux, tbxk::Buf<uint8_t> &aux2);
+                             const uint8_t *base1_out, const TbxDigitPatch *patches1, tbxk::Buf<uint8_t> &aux, tbxk::Buf<uint8_t> &aux2);
 /* the direct INTER_AREA kernel of the config's game for the plan's taps; d carries the tables and hand-over list, its
- * shared-memory layout is filled in here */
-cudaError_t tbx_launch_direct(const tbx::Config &c, const tbxk::RenderArgs &a, const TbxAreaPlan &plan, tbxk::DirectArgs d, cudaStream_t s);
+ * shared-memory layout is filled in here; aux2_bytes: the size of d.aux2 (Breakout: its image) */
+cudaError_t tbx_launch_direct(const tbx::Config &c, const tbxk::RenderArgs &a, const TbxAreaPlan &plan, tbxk::DirectArgs d, size_t aux2_bytes, cudaStream_t s);
 #endif

@@ -1060,6 +1060,46 @@ void build_brk_direct(const Config &c, const BrkTable &t, const ResizeTab &rs, c
   A.ok = 1;
 }
 
+void build_brk_img(const TbxBrkDirect &A, const TbxAreaPlan &pl, int tx, int ty, const uint8_t *base1_out, const TbxDigitPatch *patches1, std::vector<uint8_t> &img) {
+  const int W = TBX_BRK_W, H = TBX_BRK_H, dw = pl.dw, dh = pl.dh, hs = (dw + 3) & ~3, ps = brk_plan_pitch(dw, dh);
+  const TbxBrkImgLayout L = brk_img_layout(tx, ty, dw, dh, A.nrows, A.n_static, A.n_cls);
+  img.assign((size_t)L.bytes, 0);
+  uint8_t *b = img.data();
+  /* the cached digit slots: the first TBX_BRK_DIG_WORDS words of each patch (header, then pixels); the kernel uses them only when
+   * every one of them fits */
+  int32_t dig_cached = 1;
+  for (int e = 0; e < TBX_BRK_DIG_SLOTS * 10; e++) {
+    const int cid = e / 10, slot = cid < 4 ? cid : cid + TBX_MAX_DIGITS - 4;
+    const TbxDigitPatch &P = patches1[slot * 10 + e % 10];
+    if (P.w * P.h > 4 * (TBX_BRK_DIG_WORDS - 1)) dig_cached = 0;
+    memcpy(b + TBX_BI_DIG + e * TBX_BRK_DIG_WORDS * 4, &P, TBX_BRK_DIG_WORDS * 4);
+  }
+  memcpy(b + TBX_BI_FLAGS, &dig_cached, 4);
+  memcpy(b + TBX_BI_ROWCLS, A.rowcls, H);
+  memcpy(b + TBX_BI_INV, A.inv32, sizeof A.inv32);
+  memcpy(b + TBX_BI_XDLO, pl.xdlo, W); memcpy(b + TBX_BI_XDHI, pl.xdhi, W);
+  memcpy(b + TBX_BI_YDLO, pl.ydlo, H); memcpy(b + TBX_BI_YDHI, pl.ydhi, H);
+  memcpy(b + TBX_BI_XCOL, A.xcol, W); memcpy(b + TBX_BI_YROW, A.yrow, H);
+  memcpy(b + TBX_BI_BGRAY, A.brickgray, sizeof A.brickgray);
+  memcpy(b + TBX_BI_WORDCOLS, A.wordcols, sizeof A.wordcols);
+  memcpy(b + TBX_BI_COL0, A.col0, sizeof A.col0);
+  memcpy(b + TBX_BI_DYROWS, A.dyrows, sizeof A.dyrows);
+  for (int dy = 0; dy < TBX_AREA_MAX_DST; dy++) memcpy(b + TBX_BI_HSEL + dy * ty, A.hsel[dy], ty);
+  memcpy(b + L.base1, base1_out, (size_t)dw * dh);
+  /* the plan's weights and first-source indices at pitch ps, entries past the output size repeat its last one */
+  float *xa = reinterpret_cast<float *>(b + L.plan), *ya = xa + tx * ps;
+  uint16_t *xs = reinterpret_cast<uint16_t *>(ya + ty * ps), *ys = xs + ps;
+  for (int i = 0; i < ps; i++) {
+    const int jx = i < dw - 1 ? i : dw - 1, jy = i < dh - 1 ? i : dh - 1;
+    for (int t = 0; t < tx; t++) xa[t * ps + i] = pl.xalpha[t][jx];
+    for (int t = 0; t < ty; t++) ya[t * ps + i] = pl.yalpha[t][jy];
+    xs[i] = pl.xs0[jx]; ys[i] = pl.ys0[jy];
+  }
+  for (int rp = 0; rp < A.nrows * 4; rp++) memcpy(b + L.hlut + (size_t)rp * hs * 4, A.hlut[rp >> 2][rp & 3], sizeof(float) * dw);
+  for (int s = 0; s < A.n_static; s++) memcpy(b + L.hstatic + (size_t)s * hs * 4, A.hstatic[s], sizeof(float) * dw);
+  memcpy(b + L.cls, A.clsrows, (size_t)A.n_cls * W + 16);
+}
+
 /* Space Invaders: the score strip (TbxSiDirect.sc_*): every output pixel the ten digit slots feed, for every pair of digits in the (at
  * most two, neighbouring) slots that feed its column */
 static void build_si_score_strip(const ResizeTab &rs, const TbxAreaPlan &pl, const uint8_t *base0, TbxSiDirect &A) {

@@ -89,6 +89,9 @@ void build_digit_patches(const Config &c, const BrkTable *brk_default, const Res
 /* closed-form tables of the direct INTER_AREA kernel (tbx_direct.h) for the config's default brick table and one output
  * size; out.ok == 0 when the pair is outside its limits (irregular brick grid, output width not a multiple of 4 ...) */
 void build_brk_direct(const Config &c, const BrkTable &t, const ResizeTab &rs, const TbxAreaPlan &plan, const uint8_t *base0_gray, TbxBrkDirect &out);
+/* the Breakout direct kernel's shared-memory image (tbx_direct.h) for tables A (A.ok) and the kernel instantiated for tx x ty taps:
+ * base1_out is the down-sample of base frame 1, patches1 its TBX_DP_SLOTS x 10 digit patches */
+void build_brk_img(const TbxBrkDirect &A, const TbxAreaPlan &plan, int tx, int ty, const uint8_t *base1_out, const TbxDigitPatch *patches1, std::vector<uint8_t> &img);
 /* Space Invaders: plain-background map and pre-resolved sprite patch tables of the direct kernel (tbx_direct.h) */
 void build_si_direct(const Config &c, const ResizeTab &rs, const TbxAreaPlan &plan, const uint8_t *base0_gray, TbxSiDirect &out, std::vector<TbxSpritePatch> &patches);
 void build_ami_direct(const Config &c, const ResizeTab &rs, const TbxAreaPlan &plan, TbxAmiDirect &out); /* Amidar: tile-look tables of the direct kernel */

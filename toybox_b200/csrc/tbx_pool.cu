@@ -411,16 +411,19 @@ static int ensure_area(tbx_pool *p, int out_w, int out_h, bool rgb, const AreaRe
   if (!rgb && !ar.d_base_out[0]) {
     Buf<uint8_t> base_out[2], direct, direct2;
     Buf<TbxDigitPatch> patches[2];
+    std::vector<uint8_t> h[2];
+    std::vector<TbxDigitPatch> hp[2];
     for (int b = 0; b < 2; b++) {
       const uint8_t *gray = p->base->h_gray[b].data();
-      std::vector<uint8_t> h(((size_t)out_w * out_h + 15) & ~(size_t)15, 0);
-      tbx::area_resize(gray, rs, h.data());
-      CK(base_out[b].upload(h.data(), h.size()));
-      std::vector<TbxDigitPatch> hp((size_t)TBX_DP_SLOTS * 10);
-      tbx::build_digit_patches(p->cfg, brk_default(p), rs, ar.plan, gray, hp.data());
-      CK(patches[b].upload(hp.data(), hp.size()));
+      h[b].assign(((size_t)out_w * out_h + 15) & ~(size_t)15, 0);
+      tbx::area_resize(gray, rs, h[b].data());
+      CK(base_out[b].upload(h[b].data(), h[b].size()));
+      hp[b].resize((size_t)TBX_DP_SLOTS * 10);
+      tbx::build_digit_patches(p->cfg, brk_default(p), rs, ar.plan, gray, hp[b].data());
+      CK(patches[b].upload(hp[b].data(), hp[b].size()));
     }
-    CK(tbx_direct_build(p->cfg, brk_default(p), rs, ar.plan, p->base->h_gray[0].data(), direct, direct2));
+    /* built from the same down-sample and digit patches as the render's own (Breakout's image copies them) */
+    CK(tbx_direct_build(p->cfg, brk_default(p), rs, ar.plan, p->base->h_gray[0].data(), h[1].data(), hp[1].data(), direct, direct2));
     for (int b = 0; b < 2; b++) { ar.d_base_out[b] = std::move(base_out[b]); ar.d_patches[b] = std::move(patches[b]); }
     ar.d_direct = std::move(direct); ar.d_direct2 = std::move(direct2);
   }
@@ -556,7 +559,7 @@ static int render_area(tbx_pool *p, RenderArgs &a, int out_w, int out_h, bool rg
     DirectArgs da = {};
     da.aux = ar->d_direct; da.aux2 = ar->d_direct2; da.fb_list = p->d_fb + 8; da.fb_count = p->d_fb + pair; da.fb_other = p->d_fb + (pair ^ 1);
     da.sched = p->d_fb + 2;
-    CK(tbx_launch_direct(p->cfg, a, plan, da, s));
+    CK(tbx_launch_direct(p->cfg, a, plan, da, ar->d_direct2.size(), s));
     if (p->game == TBX_SPACE_INVADERS) return TBX_OK; /* covers every env: nothing is handed over */
     p->fb_pair = pair ^ 1;
     a.env_list = p->d_fb + 8;

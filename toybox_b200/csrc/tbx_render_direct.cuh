@@ -23,16 +23,9 @@
 namespace tbxk {
 
 #define TBX_DIRECT_THREADS 256
-#define TBX_BRK_DIG_SLOTS 6  /* digit slots whose patches are kept in shared memory: score digits 0..3, lives digits 0..1 */
-#define TBX_BRK_DIG_WORDS 13 /* header word + up to 48 pixels */
-#define TBX_BRK_DIG_BYTES (TBX_BRK_DIG_SLOTS * 10 * TBX_BRK_DIG_WORDS * 4)
-/* pitch / bytes of the plan tables the Breakout kernel keeps behind its other shared memory */
-__host__ __device__ __forceinline__ int brk_plan_pitch(int dw, int dh) { return ((dw > dh ? dw : dh) + 3) & ~3; }
-__host__ __device__ __forceinline__ int brk_plan_smem_bytes(int tx, int ty, int dw, int dh) { return ((tx + ty) * brk_plan_pitch(dw, dh) * 4 + 2 * brk_plan_pitch(dw, dh) * 2 + 15) & ~15; }
 __host__ __device__ __forceinline__ int si_tab_smem_bytes(int dw, int dh) { return ((dh * ((dw + 31) >> 5) + 3) & ~3) * 4 + ((TBX_AREA_MAX_DST + 1 + 3) & ~3) * 4; }
 __host__ __device__ __forceinline__ int ami_tab_smem_bytes(int dh) { return TBX_AMI_W + 256 + ((dh * 4 + 15) & ~15); }
 __device__ __forceinline__ int brk_dig_cid(int slot) { return slot < 4 ? slot : slot >= TBX_MAX_DIGITS && slot < TBX_MAX_DIGITS + 2 ? slot - TBX_MAX_DIGITS + 4 : -1; }
-#define TBX_BRK_TAB_BYTES (TBX_BRK_DIG_BYTES + TBX_BD_MAX_CLS * TBX_BRK_W + 16 + TBX_BRK_H + (TBX_AREA_MAX_DST + 1 + 3) / 4 * 16)
 #ifndef TBX_DIRECT_MIN_CTAS
 #define TBX_DIRECT_MIN_CTAS 4
 #endif
@@ -45,38 +38,39 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 
 /* PERSISTENT CTAs of two 4-warp TEAMS: a team renders chunks of 4 consecutive envs (one per warp), its first chunk fixed, the
- * next ones drawn from a device-wide counter.  Shared memory: the down-sample of base frame 1 (loaded once per CTA; every env's
- * frame starts as ONE bulk shared -> global copy of it, cp.async.bulk, no per-env load/store instructions); the small tables the
- * per-pixel code indexes (digit patches of the slots in use, base frame 0 by row classes, the wall's H look-up, the plan's weights
- * and first-source indices, a division table: L1 is too small next to this much shared memory to keep them); per team two stages
- * of word-major records (cp.async prefetch of the next chunk; a warp reads its env's record there, in place); per warp the wall's H
- * rows and the movers' records. */
+ * next ones drawn from a device-wide counter.  Shared memory: the host-built IMAGE of every table the per-env code reads
+ * (tbx_direct.h: the down-sample of base frame 1 -- every env's frame starts as ONE bulk shared -> global copy of it, cp.async.bulk,
+ * no per-env load/store instructions --, the digit patches of the slots in use, base frame 0 by row classes, the plan's footprints,
+ * weights and first-source indices, the brick grid, the wall's tables, a division table: L1 is too small next to this much shared
+ * memory to keep sparse global tables), d.smem_base bytes loaded by one bulk copy per CTA; per team two stages of word-major
+ * records (cp.async prefetch of the next chunk; a warp reads its env's record there, in place); per warp the wall's H rows and the
+ * movers' records. */
 template <int TX, int TY>
 __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_direct_kernel(const __grid_constant__ RenderArgs a, const __grid_constant__ BrkCfg cfg_c,
                                                                             const __grid_constant__ TbxAreaPlan plan_c, const __grid_constant__ DirectArgs d) {
   constexpr int RW = TBX_WORDS(BrkRec);
   extern __shared__ uint4 smem_raw[];
   uint8_t *smem = reinterpret_cast<uint8_t *>(smem_raw);
-  uint8_t *sbase = smem;                                                        /* base frame 1, down-sampled */
-  /* small hot tables, copied once per CTA (TBX_BRK_TAB_BYTES after the frame): the reads they replace were the kernel's main
-   * long-scoreboard stalls (L1 misses on sparse global tables) */
-  uint8_t *tab = smem + ((plan_c.dw * plan_c.dh + 15) & ~15);
-  uint32_t *sdig = reinterpret_cast<uint32_t *>(tab);                           /* [6 slots x 10 digits][13 words]: header + up to 48 pixels */
-  uint8_t *scls = tab + TBX_BRK_DIG_BYTES;                                      /* base frame 0 by row classes */
-  uint8_t *srowcls = scls + TBX_BD_MAX_CLS * TBX_BRK_W + 16;
-  uint32_t *sinv = reinterpret_cast<uint32_t *>(srowcls + TBX_BRK_H);           /* inv32[] */
-  float *shlut = reinterpret_cast<float *>(tab + TBX_BRK_TAB_BYTES);            /* [brick row][2 alive bits][hstride]: the wall's H look-up */
-  /* the resize plan's per-pixel tables, behind everything else (brk_plan_smem_bytes: the launch adds them to d.smem_total) */
-  const int ps = brk_plan_pitch(plan_c.dw, plan_c.dh);
-  float *sxa = reinterpret_cast<float *>(smem + d.smem_total);                  /* [TX][ps] */
-  float *sya = sxa + TX * ps;                                                   /* [TY][ps] */
-  uint16_t *sxs = reinterpret_cast<uint16_t *>(sya + TY * ps), *sys = sxs + ps; /* xs0, ys0 */
-  __shared__ int s_bigdig;
-  uint32_t *stage = reinterpret_cast<uint32_t *>(smem + d.smem_base);           /* [2 teams][2 stages][RW][4 envs] */
   const TbxBrkDirect *__restrict__ Ap = reinterpret_cast<const TbxBrkDirect *>(d.aux);
-  const TbxBrkDirect &A = *Ap;
-  const TbxAreaPlan *__restrict__ plan = a.plan; /* per-lane indexed reads */
-  const TbxAreaPlan &cp = plan_c;                /* warp-uniform reads: constant bank */
+  const TbxBrkDirect &A = *Ap; /* warp-uniform scalars */
+  const TbxAreaPlan &cp = plan_c;
+  const int dw = cp.dw, dh = cp.dh, nrows = A.nrows;
+  /* the image's regions (tbx_direct.h) */
+  const TbxBrkImgLayout L = brk_img_layout(TX, TY, dw, dh, nrows, A.n_static, 0);
+  const uint32_t *sdig = reinterpret_cast<const uint32_t *>(smem + TBX_BI_DIG);  /* [6 slots x 10 digits][13 words]: header + up to 48 pixels */
+  const uint8_t *scls = smem + L.cls, *srowcls = smem + TBX_BI_ROWCLS;          /* base frame 0 by row classes */
+  const uint32_t *sinv = reinterpret_cast<const uint32_t *>(smem + TBX_BI_INV);  /* inv32[] */
+  const uint8_t *sxdlo = smem + TBX_BI_XDLO, *sxdhi = smem + TBX_BI_XDHI, *sydlo = smem + TBX_BI_YDLO, *sydhi = smem + TBX_BI_YDHI;
+  const uint8_t *sxcol = smem + TBX_BI_XCOL, *syrow = smem + TBX_BI_YROW, *sbgray = smem + TBX_BI_BGRAY;
+  const uint32_t *swordcols = reinterpret_cast<const uint32_t *>(smem + TBX_BI_WORDCOLS);
+  const uint8_t *scol0 = smem + TBX_BI_COL0, *sdyrows = smem + TBX_BI_DYROWS, *shsel = smem + TBX_BI_HSEL; /* hsel: [dy][TY] */
+  uint8_t *sbase = smem + TBX_BI_FIXED(TY);                                      /* base frame 1, down-sampled */
+  const int ps = brk_plan_pitch(dw, dh);
+  const float *sxa = reinterpret_cast<const float *>(smem + L.plan);             /* [TX][ps] */
+  const float *sya = sxa + TX * ps;                                              /* [TY][ps] */
+  const uint16_t *sxs = reinterpret_cast<const uint16_t *>(sya + TY * ps), *sys = sxs + ps; /* xs0, ys0 */
+  const float *shlut = reinterpret_cast<const float *>(smem + L.hlut);           /* [brick row][2 alive bits][hstride]: the wall's H look-up */
+  uint32_t *stage = reinterpret_cast<uint32_t *>(smem + d.smem_base);           /* [2 teams][2 stages][RW][4 envs] */
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   uint8_t *wmem = smem + d.smem_base + 2 * RW * TBX_EPC * 4 + wid * d.warp_bytes;
   float *hw = reinterpret_cast<float *>(wmem);
@@ -86,7 +80,9 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
   constexpr int TEAM = 4, TEAM_THREADS = TEAM * 32;
   const int team = wid / TEAM, wt = wid % TEAM, ttid = tid % TEAM_THREADS;
   const int n_chunks = (a.n + TEAM - 1) / TEAM;
-  const int dw = cp.dw, dh = cp.dh, nwords = dw >> 2, hs = d.hstride, nb = dw * dh;
+  const int nwords = dw >> 2, hs = d.hstride, nb = dw * dh;
+  /* static rows of the wall's H sums, indexed by hsel's selector like the H rows: row sel - nrows of the image's hstatic */
+  const float *shst = reinterpret_cast<const float *>(smem + L.hstatic) - nrows * hs;
   const bool bulk = (nb & 15) == 0 && (a.env_stride & 15) == 0 && (a.frame_bytes & 15) == 0;
 
   uint32_t *tstage = stage + team * 2 * RW * TEAM; /* [2][RW][4 envs] */
@@ -100,45 +96,27 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
    * first thread draws the id one iteration ahead; the barrier at the top of the loop publishes it), so the teams finish together
    * whatever their envs cost */
   __shared__ int s_next[2][2];
+  __shared__ alignas(8) uint64_t s_img_bar; /* completes when the image has landed */
+  const uint32_t img_bar = (uint32_t)__cvta_generic_to_shared(&s_img_bar);
+  if (tid == 0) { /* the image: d.smem_base bytes at d.aux2, one bulk copy (well below the mbarrier's 2^20 - 1 transaction bytes) */
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(img_bar) : "memory");
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(img_bar), "r"(d.smem_base) : "memory");
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"((uint32_t)__cvta_generic_to_shared(smem)),
+                 "l"(d.aux2), "r"(d.smem_base), "r"(img_bar) : "memory");
+  }
   const int n_teams = (int)gridDim.x * (TBX_DIRECT_THREADS / TEAM_THREADS);
   if (ttid == 0) s_next[team][0] = n_teams + atomicAdd(d.sched, 1);
   if ((int)blockIdx.x * 2 + team < n_chunks) prefetch((int)blockIdx.x * 2 + team, 0);
-  for (int i = tid; i < ((nb + 15) >> 4); i += TBX_DIRECT_THREADS) reinterpret_cast<uint4 *>(sbase)[i] = __ldg(reinterpret_cast<const uint4 *>(a.base_out[1]) + i);
-  const TbxDigitPatch *__restrict__ gpatches = a.patches[1];
-  if (tid == 0) s_bigdig = gpatches ? 0 : 1;
-  __syncthreads();
-  if (gpatches) /* the slots that are in use in practice: the score's low 4 digits, the lives' low 2 (the others read the table itself) */
-    for (int i = tid; i < TBX_BRK_DIG_SLOTS * 10 * TBX_BRK_DIG_WORDS; i += TBX_DIRECT_THREADS) {
-      const int e = i / TBX_BRK_DIG_WORDS, w = i - e * TBX_BRK_DIG_WORDS, cid = e / 10, slot = cid < 4 ? cid : cid + TBX_MAX_DIGITS - 4;
-      const uint32_t *src = reinterpret_cast<const uint32_t *>(gpatches + slot * 10 + (e - cid * 10));
-      const uint32_t v = __ldg(src + w);
-      if (w == 0 && ((v >> 16) & 255u) * (v >> 24) > 4u * (TBX_BRK_DIG_WORDS - 1)) atomicOr(&s_bigdig, 1);
-      sdig[i] = v;
-    }
-  const int n_cls = A.n_cls;
-  for (int i = tid; i < (n_cls * TBX_BRK_W + 16) / 4; i += TBX_DIRECT_THREADS) reinterpret_cast<uint32_t *>(scls)[i] = __ldg(reinterpret_cast<const uint32_t *>(A.clsrows) + i);
-  for (int i = tid; i < TBX_BRK_H / 4; i += TBX_DIRECT_THREADS) reinterpret_cast<uint32_t *>(srowcls)[i] = __ldg(reinterpret_cast<const uint32_t *>(A.rowcls) + i);
-  for (int i = tid; i <= TBX_AREA_MAX_DST; i += TBX_DIRECT_THREADS) sinv[i] = __ldg(&A.inv32[i]);
-  for (int i = tid; i < ps; i += TBX_DIRECT_THREADS) {
-    const int jx = min(i, plan_c.dw - 1), jy = min(i, plan_c.dh - 1);
-#pragma unroll
-    for (int t = 0; t < TX; t++) sxa[t * ps + i] = __ldg(&a.plan->xalpha[t][jx]);
-#pragma unroll
-    for (int t = 0; t < TY; t++) sya[t * ps + i] = __ldg(&a.plan->yalpha[t][jy]);
-    sxs[i] = __ldg(&a.plan->xs0[jx]); sys[i] = __ldg(&a.plan->ys0[jy]);
-  }
-  for (int i = tid; i < A.nrows * 4 * (plan_c.dw >> 2); i += TBX_DIRECT_THREADS) { /* float4 pieces of the rows in use */
-    const int rp = i / (plan_c.dw >> 2), c4 = i - rp * (plan_c.dw >> 2);
-    *reinterpret_cast<float4 *>(shlut + rp * d.hstride + 4 * c4) = __ldg(reinterpret_cast<const float4 *>(&A.hlut[rp >> 2][rp & 3][4 * c4]));
-  }
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); /* the bulk copies below read sbase through the async proxy */
-
-  const int ok = A.ok, ncols = A.ncols, nrows = A.nrows, wdy0 = A.wdy0, wdy1 = A.wdy1, hud_dyhi = A.hud_dyhi;
-  const int wy0 = A.wy0, wy1 = A.wy0 + A.nrows * A.bh;
+  const int ok = A.ok, ncols = A.ncols, wdy0 = A.wdy0, wdy1 = A.wdy1, hud_dyhi = A.hud_dyhi, n_cls = A.n_cls;
+  const int wy0 = A.wy0, wy1 = A.wy0 + nrows * A.bh;
   const uint32_t paddle_gray = A.paddle_gray, ball_gray = A.ball_gray;
   const TbxDigitPatch *__restrict__ patches = a.patches[1];
-  __syncthreads(); /* the tables are complete */
-  const bool dig_smem = s_bigdig == 0;
+  __syncthreads(); /* the barrier is initialised */
+  for (uint32_t img_in = 0; !img_in;)
+    asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0; selp.u32 %0, 1, 0, p; }" : "=r"(img_in) : "r"(img_bar) : "memory");
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); /* the bulk copies below read sbase through the async proxy */
+  const bool dig_smem = *reinterpret_cast<const int32_t *>(smem + TBX_BI_FLAGS) != 0;
 
   int st = 0, it = 0, nxt = 0;
   for (int chunk = (int)blockIdx.x * 2 + team; chunk < n_chunks; chunk = nxt, st ^= 1, it++) {
@@ -159,7 +137,7 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
     const TbxMover mine = brk_mover_rec(S, paddle_gray, ball_gray, lane < BRK_N_MOVERS ? lane : -1);
     const bool valid = mine.x0 < mine.x1;
     int fx0 = 0, fx1 = 0, fy0 = 0, fy1 = 0;
-    if (valid) { fx0 = __ldg(&plan->xdlo[mine.x0]); fx1 = __ldg(&plan->xdhi[mine.x1 - 1]); fy0 = __ldg(&plan->ydlo[mine.y0]); fy1 = __ldg(&plan->ydhi[mine.y1 - 1]); }
+    if (valid) { fx0 = sxdlo[mine.x0]; fx1 = sxdhi[mine.x1 - 1]; fy0 = sydlo[mine.y0]; fy1 = sydhi[mine.y1 - 1]; }
     bool bad = valid && fy0 <= hud_dyhi;
     /* HUD digits: lanes 0..9 the score, 10..19 the lives */
     int dig = -1;
@@ -238,17 +216,17 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
       if (__any_sync(0xffffffffu, act && ys < wy1 && ys + TY > wy0)) { /* the brick grid */
         uint32_t cb[TX];
 #pragma unroll
-        for (int t = 0; t < TX; t++) cb[t] = __ldg(&A.xcol[min(xs + t, TBX_BRK_W - 1)]);
+        for (int t = 0; t < TX; t++) cb[t] = sxcol[min(xs + t, TBX_BRK_W - 1)];
 #pragma unroll
         for (int k = 0; k < TY; k++) {
-          const uint32_t r = __ldg(&A.yrow[min(ys + k, TBX_BRK_H - 1)]);
+          const uint32_t r = syrow[min(ys + k, TBX_BRK_H - 1)];
           if (r == 255u) continue;
 #pragma unroll
           for (int t = 0; t < TX; t++) {
             if (cb[t] == 255u) continue;
             const uint32_t i = cb[t] * (uint32_t)nrows + r;
             if (!((alive[(i >> 5) * TEAM] >> (i & 31)) & 1u)) continue;
-            const uint32_t g = __ldg(&A.brickgray[i]);
+            const uint32_t g = sbgray[i];
             if (t < 4) lo[k] = (lo[k] & ~(255u << (8 * t))) | (g << (8 * t));
             else hi[k] = g;
           }
@@ -306,13 +284,13 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
       uint32_t rowmask[TBX_BRK_MAX_ROWS];
 #pragma unroll
       for (int r = 0; r < TBX_BRK_MAX_ROWS; r++) rowmask[r] = __ballot_sync(0xffffffffu, (colbits >> r) & 1u);
-      const uint32_t wmask = __ballot_sync(0xffffffffu, lane < nwords && (__ldg(&A.wordcols[lane]) & deadcols));
-      const uint32_t rmask = __ballot_sync(0xffffffffu, wdy0 + lane <= wdy1 && (__ldg(&A.dyrows[wdy0 + lane]) & deadrows));
+      const uint32_t wmask = __ballot_sync(0xffffffffu, lane < nwords && (swordcols[lane] & deadcols));
+      const uint32_t rmask = __ballot_sync(0xffffffffu, wdy0 + lane <= wdy1 && (sdyrows[wdy0 + lane] & deadrows));
       if (wmask && rmask) {
         const int wlo = __ffs(wmask) - 1, whi = 31 - __clz(wmask);
         __syncwarp(); /* the previous env's readers of the H rows are done */
         for (int dx = 4 * wlo + lane; dx < 4 * whi + 4; dx += 32) {
-          const int c0 = __ldg(&A.col0[dx]);
+          const int c0 = scol0[dx];
 #pragma unroll
           for (int r = 0; r < TBX_BRK_MAX_ROWS; r++)
             if (r < nrows) hw[r * hs + dx] = shlut[(r * 4 + ((rowmask[r] >> c0) & 3u)) * hs + dx];
@@ -329,9 +307,8 @@ __global__ void __launch_bounds__(TBX_DIRECT_THREADS, TBX_DIRECT_MIN_CTAS) brk_d
           float acc[4];
 #pragma unroll
           for (int k = 0; k < TY; k++) {
-            const int sel = __ldg(&A.hsel[dy][k]);
-            const float4 h = sel < nrows ? *reinterpret_cast<const float4 *>(hw + sel * hs + 4 * myword)
-                                         : __ldg(reinterpret_cast<const float4 *>(&A.hstatic[sel - nrows][4 * myword]));
+            const int sel = shsel[dy * TY + k];
+            const float4 h = *reinterpret_cast<const float4 *>((sel < nrows ? hw : shst) + sel * hs + 4 * myword);
             const float b = sya[k * ps + dy];
             const float p0 = tbx_fmul(b, h.x), p1 = tbx_fmul(b, h.y), p2 = tbx_fmul(b, h.z), p3 = tbx_fmul(b, h.w);
             if (k == 0) { acc[0] = p0; acc[1] = p1; acc[2] = p2; acc[3] = p3; }
