@@ -199,6 +199,19 @@ int tbx_wrap_set_sticky_actions(tbx_wrap *w, double repeat_action_probability, u
  * limit truncate at the next agent step.  0 (default) = no limit.  TBX_EINVAL for a negative limit, or once the wrap has
  * stepped. */
 int tbx_wrap_set_time_limit(tbx_wrap *w, int max_episode_steps, uint8_t *truncated_dev);
+/* Final observations (SB3's infos[i]['terminal_observation'], gymnasium's final_obs): final_ring_dev has the obs ring's shape
+ * and layout (caller-owned, 16-byte aligned); NULL (default) turns the feature off.  Every tbx_wrap_step that renders
+ * (obs_ring_dev != NULL) writes, for each env whose agent step ends in done (game over, a lost life when episodic_life, or
+ * the time limit), the FrameStack the reference held just before the VecEnv worker reset it: the stack_k-1 newest ring
+ * frames before the step, in their ring slots, and in slot *slot_out the frame this step produced, WarpFrame of
+ * MaxAndSkipEnv.step's max(_obs_buffer[0], _obs_buffer[1]) -- the same under both stack modes.  MaxAndSkipEnv writes
+ * _obs_buffer[0] on frame skip-2 and [1] on frame skip-1 only and breaks at game over, so a game that ends earlier shows
+ * stale slots from earlier MaxAndSkipEnv steps (reset-chain steps or the previous episode) and a slot never written is
+ * zeros; the wrap keeps both slots as state.  Rows of other envs, and every row on steps that do not render, VecEnv resets
+ * and envs with a refused action index, are left as they are.  Adds 1 + 2 * tbx_state_rows wrapper rows per env
+ * (tbx_wrap_state_rows; a snapshot of a wrap with final observations loads only into such a wrap, and the reverse).
+ * TBX_EINVAL for a misaligned buffer, or once the wrap has stepped. */
+int tbx_wrap_set_final_observations(tbx_wrap *w, uint8_t *final_ring_dev);
 int tbx_wrap_destroy(tbx_wrap *wrap);
 /* env.step(action) of the wrapped env for every env (actions_dev: int32[N] gym action indices into the legal set), or
  * env.reset() for every env when actions_dev == NULL.  obs_ring_dev: uint8[N][stack_k][out_h][out_w] (with [3] appended
@@ -215,7 +228,8 @@ int tbx_wrap_step(tbx_wrap *wrap, const int32_t *actions_dev, uint8_t *obs_ring_
  * A snapshot of k envs is a caller-owned device buffer uint32[rows][k], word-major like the pool's planes: column j is one
  * env's whole record (both rngs, prev_score, the episode counters; rows = tbx_state_rows), followed for a wrapped env by its
  * 5 wrapper words (EpisodicLife lives, was_real_done, reset counter, Monitor return, Monitor length), 7 with sticky actions
- * (+ the remembered ALE id and the frame counter); rows = tbx_wrap_state_rows.  A loaded env continues exactly as the saved env would have.  The device-wide episode statistics
+ * (+ the remembered ALE id and the frame counter), and with final observations the written _obs_buffer slots and the two
+ * records behind them; rows = tbx_wrap_state_rows.  A loaded env continues exactly as the saved env would have.  The device-wide episode statistics
  * (tbx_stats_read) are pool state and are neither saved nor restored.
  * Breakout and Amidar records index the pool's geometry tables, so a snapshot goes with the tables blob of the moment it was
  * saved (tbx_state_tables): a tbx_state_blob_header followed by table_count tables of table_bytes bytes each (none for Space

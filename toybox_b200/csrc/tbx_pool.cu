@@ -624,7 +624,12 @@ static int render_native(tbx_pool *p, RenderArgs &a, int mode, cudaStream_t s) {
   });
 }
 
-struct DualRender { const uint32_t *planes2; const uint8_t *reset_flags; int stack_k, stack_slot, stack_mode; };
+/* planes / env_list / env_count may be NULL (the pool's planes, every env); a list renders only the envs it names (final
+ * observations), never through the direct kernel's hand-over */
+struct DualRender {
+  const uint32_t *planes2; const uint8_t *reset_flags; int stack_k, stack_slot, stack_mode;
+  const uint32_t *planes; const int32_t *env_list; const int *env_count;
+};
 static int render_impl(tbx_pool *p, uint8_t *dst, int mode, int out_w, int out_h, void *stream, const DualRender *dual) {
   if (!p || !dst) return set_err(TBX_EINVAL, "pool/dst is NULL");
   if (((uintptr_t)dst & 15) != 0) return set_err(TBX_EINVAL, "dst must be 16-byte aligned");
@@ -635,8 +640,9 @@ static int render_impl(tbx_pool *p, uint8_t *dst, int mode, int out_w, int out_h
   if (r) return r;
   const int pix = obs_pix(mode);
   RenderArgs a = {};
-  a.planes = p->planes; a.n = p->n; a.n_pad = p->n_pad; a.cfg = p->d_cfg; a.tables = p->d_tables;
+  a.planes = dual && dual->planes ? dual->planes : p->planes; a.n = p->n; a.n_pad = p->n_pad; a.cfg = p->d_cfg; a.tables = p->d_tables;
   a.planes2 = dual ? dual->planes2 : 0; a.reset_flags = dual ? dual->reset_flags : 0;
+  a.env_list = dual ? dual->env_list : 0; a.env_count = dual ? dual->env_count : 0;
   a.stack_k = dual ? dual->stack_k : 1; a.stack_slot = dual ? dual->stack_slot : 0; a.stack_mode = dual ? dual->stack_mode : 0; a.env_stride = fb * (size_t)a.stack_k;
   a.dst = dst; a.frame_bytes = fb;
   for (int b = 0; b < 2; b++) a.base[b] = pix == 4 ? p->base->rgba[b] : pix == 3 ? p->base->rgb[b] : p->base->gray[b];
@@ -670,8 +676,13 @@ struct tbx_wrap {
   uint64_t sticky_seed, sticky_thr; /* sticky actions: the draw's seed and llround(p * 2^32); thr 0 = off */
   int max_steps;           /* episode time limit in agent steps, 0 = none */
   uint8_t *truncated;      /* caller-owned device output, or NULL */
+  uint8_t *final_ring;     /* final observations: caller-owned, the obs ring's shape, or NULL (off) */
+  Buf<uint32_t> term;      /* final observations: the terminal record pair, [2][rec][n_pad] */
+  Buf<int32_t> fin_list;   /* final observations: [0], [1] = list counts, [2..] = the env list (tbx_wrap.cuh, WrapArgs::fin) */
 };
 static const int TBX_WRAP_WORDS_MAX = 7; /* wstate is allocated for the sticky layout */
+/* wrapper rows of an env: the words, then with final observations the written-slots word and the two _obs_buffer records */
+static int wrap_rows(const tbx_wrap *w) { return w->words + (w->final_ring ? 1 + 2 * w->pool->info->rec_words : 0); }
 
 extern "C" {
 
@@ -737,6 +748,31 @@ int tbx_wrap_set_time_limit(tbx_wrap *w, int max_episode_steps, uint8_t *truncat
   w->truncated = truncated_dev;
   return TBX_OK;
 }
+int tbx_wrap_set_final_observations(tbx_wrap *w, uint8_t *final_ring_dev) {
+  if (!w) return set_err(TBX_EINVAL, "wrap is NULL");
+  if (w->stepped) return set_err(TBX_EINVAL, "final observations are set before the first tbx_wrap_step");
+  if (((uintptr_t)final_ring_dev & 15) != 0) return set_err(TBX_EINVAL, "the final observation ring must be 16-byte aligned");
+  if (!final_ring_dev) {
+    w->final_ring = 0;
+    return TBX_OK;
+  }
+  tbx_pool *p = w->pool;
+  CK(cudaSetDevice(p->device));
+  return guarded([&]() -> int {
+    const size_t np = (size_t)p->n_pad, rec = (size_t)p->info->rec_words, rows = TBX_WRAP_WORDS_MAX + 1 + 2 * rec;
+    if (w->wstate.size() < rows * np) { /* room for the rows after the sticky layout's words; the new rows start at zero */
+      Buf<uint32_t> ws;
+      CK(ws.alloc(rows * np));
+      CK(cudaMemcpy(ws, w->wstate, TBX_WRAP_WORDS_MAX * np * 4, cudaMemcpyDeviceToDevice));
+      CK(cudaMemset(ws + TBX_WRAP_WORDS_MAX * np, 0, (rows - TBX_WRAP_WORDS_MAX) * np * 4));
+      w->wstate = std::move(ws);
+    }
+    CK(w->term.grow(2 * rec * np));
+    CK(w->fin_list.grow(np + 2));
+    w->final_ring = final_ring_dev;
+    return TBX_OK;
+  });
+}
 int tbx_wrap_set_episode_outputs(tbx_wrap *w, int32_t *ep_return_dev, int32_t *ep_length_dev) {
   if (!w) return set_err(TBX_EINVAL, "wrap is NULL");
   w->ep_return = ep_return_dev; w->ep_length = ep_length_dev;
@@ -767,16 +803,36 @@ int tbx_wrap_step(tbx_wrap *w, const int32_t *actions, uint8_t *obs_ring, int32_
   a.ep_return = w->ep_return; a.ep_length = w->ep_length;
   a.sticky_seed = w->sticky_seed; a.sticky_thr = w->sticky_thr; a.max_steps = w->max_steps; a.truncated = w->truncated;
   a.stats = p->d_stats; a.bad_actions = p->d_bad;
+  const bool fin = w->final_ring != 0;
+  const size_t plane_words = (size_t)p->info->rec_words * p->n_pad;
+  a.fin = fin ? w->wstate + (size_t)w->words * p->n_pad : 0;
+  a.term0 = w->term; a.term1 = w->term + plane_words;
+  a.fin_list = w->fin_list + 2; a.fin_count = w->fin_list;
+  if (fin) CK(cudaMemsetAsync(w->fin_list, 0, 2 * sizeof(int32_t), s));
   with_game(p->game, [&](auto g) {
     constexpr int G = decltype(g)::value;
-    if (w->words == 7) wrap_step_kernel<G, true><<<blocks(p->n, 128), 128, 0, s>>>(a);
+    if (fin) {
+      if (w->words == 7) wrap_step_kernel<G, true, true><<<blocks(p->n, 128), 128, 0, s>>>(a);
+      else wrap_step_kernel<G, false, true><<<blocks(p->n, 128), 128, 0, s>>>(a);
+    } else if (w->words == 7) wrap_step_kernel<G, true><<<blocks(p->n, 128), 128, 0, s>>>(a);
     else wrap_step_kernel<G, false><<<blocks(p->n, 128), 128, 0, s>>>(a);
   });
   CK(cudaGetLastError());
   if (obs_ring) {
     w->head = (w->head + 1) % w->stack_k;
-    DualRender d;
-    d.planes2 = w->planes_prev; d.reset_flags = w->was_reset; d.stack_k = w->stack_k; d.stack_slot = w->head; d.stack_mode = w->stack_mode;
+    DualRender d = {};
+    d.stack_k = w->stack_k; d.stack_slot = w->head; d.stack_mode = w->stack_mode;
+    if (fin) { /* the final stacks of the listed envs, from the ring before the render below overwrites slot head */
+      const size_t fb = tbx_obs_bytes(p, w->obs_mode, w->out_w, w->out_h);
+      const int grid = blocks(p->n, 8) < 296 ? blocks(p->n, 8) : 296;
+      final_ring_kernel<<<grid, 256, 0, s>>>(obs_ring, w->final_ring, a.fin_list, a.fin_count, p->n_pad, fb, w->stack_k, w->head);
+      CK(cudaGetLastError());
+      d.planes = a.term1; d.planes2 = a.term0; d.env_list = a.fin_list; d.env_count = a.fin_count;
+      int r = guarded([&] { return render_impl(p, w->final_ring, w->obs_mode, w->out_w, w->out_h, stream, &d); });
+      if (r) return r;
+      d.planes = 0; d.env_list = 0; d.env_count = 0;
+    }
+    d.planes2 = w->planes_prev; d.reset_flags = w->was_reset;
     int r = guarded([&] { return render_impl(p, obs_ring, w->obs_mode, w->out_w, w->out_h, stream, &d); });
     if (r) return r;
   }
@@ -1150,7 +1206,7 @@ static int state_save(tbx_pool *p, uint32_t *wstate, int words, const int32_t *i
   SnapArgs a;
   a.rows = p->info->rec_words + (wstate ? words : 0);
   a.src = pool_side(p, wstate, ids); a.dst = snap_side(snap, k, a.rows, 0);
-  a.k = k; a.tbl_row = -1; a.tbl_lim = -1; a.remap = 0; a.owner = 0; a.bad = p->d_bad + 1;
+  a.k = k; a.tbl_row[0] = a.tbl_row[1] = a.tbl_row[2] = -1; a.tbl_lim = -1; a.remap = 0; a.owner = 0; a.bad = p->d_bad + 1;
   return launch_snap_copy(a, s);
 }
 
@@ -1186,7 +1242,7 @@ static int snapshot_remap(tbx_pool *p, const uint8_t *tabs, int count, const int
   *remap = p->d_remap;
   return TBX_OK;
 }
-static int state_load(tbx_pool *p, uint32_t *wstate, int words, const uint32_t *snap, int k_snap, const int32_t *cols, const int32_t *ids, int n, const void *blob,
+static int state_load(tbx_pool *p, uint32_t *wstate, int words, bool fin, const uint32_t *snap, int k_snap, const int32_t *cols, const int32_t *ids, int n, const void *blob,
                       size_t blob_bytes, cudaStream_t s) {
   const int rows = p->info->rec_words + (wstate ? words : 0);
   if (k_snap < 0 || n < 0 || (n > 0 && !snap)) return set_err(TBX_EINVAL, "snap is NULL, or k_snap / n < 0");
@@ -1197,8 +1253,13 @@ static int state_load(tbx_pool *p, uint32_t *wstate, int words, const uint32_t *
   if (h.format != TBX_STATE_FORMAT)
     return set_err(TBX_EINVAL, "state snapshot: format " + std::to_string(h.format) + ", this library reads format " + std::to_string(TBX_STATE_FORMAT));
   if (h.game != (uint32_t)p->game) return set_err(TBX_EINVAL, std::string("state snapshot: saved from another game, this pool runs ") + p->info->name);
-  if (h.rows != (uint32_t)rows)
-    return set_err(TBX_EINVAL, "state snapshot: " + std::to_string(h.rows) + " rows per env, this " + (wstate ? "wrapped env" : "pool") + " needs " + std::to_string(rows));
+  if (h.rows != (uint32_t)rows) {
+    const int fin_rows = 1 + 2 * p->info->rec_words, d = (int)h.rows - rows;
+    const char *why = !wstate ? "" : (fin && d <= -fin_rows + 2) ? " (saved without final observations, which this wrapped env keeps)"
+                                  : (!fin && d >= fin_rows - 2) ? " (saved with final observations, which this wrapped env does not keep)" : "";
+    return set_err(TBX_EINVAL, "state snapshot: " + std::to_string(h.rows) + " rows per env, this " + (wstate ? "wrapped env" : "pool") + " needs " +
+                                   std::to_string(rows) + why);
+  }
   if (h.table_bytes != table_view(p).bytes || h.table_count > (1u << 20) || blob_bytes != sizeof h + (size_t)h.table_bytes * h.table_count)
     return set_err(TBX_EINVAL, "state snapshot: the tables blob's size does not match its header");
   if (n == 0) return TBX_OK;
@@ -1210,7 +1271,13 @@ static int state_load(tbx_pool *p, uint32_t *wstate, int words, const uint32_t *
   SnapArgs a;
   a.rows = rows;
   a.src = snap_side(const_cast<uint32_t *>(snap), k_snap, rows, cols); a.dst = pool_side(p, wstate, ids);
-  a.k = n; a.tbl_row = p->game == TBX_SPACE_INVADERS ? -1 : TBX_HW(tbl); a.tbl_lim = (int)h.table_count; a.remap = remap;
+  a.k = n;
+  /* hdr.tbl of the record and, with final observations, of the two _obs_buffer records after the written-slots word */
+  const int rec = p->info->rec_words, tbl = p->game == TBX_SPACE_INVADERS ? -1 : TBX_HW(tbl), fin0 = rec + words - 2 * rec;
+  a.tbl_row[0] = tbl;
+  a.tbl_row[1] = tbl >= 0 && fin ? fin0 + tbl : -1;
+  a.tbl_row[2] = tbl >= 0 && fin ? fin0 + rec + tbl : -1;
+  a.tbl_lim = (int)h.table_count; a.remap = remap;
   a.owner = ids ? p->d_owner.get() : 0; a.bad = p->d_bad + 1;
   if (a.owner) CK(cudaMemsetAsync(p->d_owner, 0xff, (size_t)p->n_pad * sizeof(int32_t), s)); /* -1: no entry yet */
   return launch_snap_copy(a, s);
@@ -1219,14 +1286,14 @@ static int state_load(tbx_pool *p, uint32_t *wstate, int words, const uint32_t *
 extern "C" {
 
 int tbx_state_rows(const tbx_pool *p) { return p ? p->info->rec_words : 0; }
-int tbx_wrap_state_rows(const tbx_wrap *w) { return w ? w->pool->info->rec_words + w->words : 0; }
+int tbx_wrap_state_rows(const tbx_wrap *w) { return w ? w->pool->info->rec_words + wrap_rows(w) : 0; }
 int tbx_state_tables(const tbx_pool *p, void *out_host, size_t cap, size_t *size) {
   if (!p || !size) return set_err(TBX_EINVAL, "pool/size is NULL");
   return state_tables(p, p->info->rec_words, out_host, cap, size);
 }
 int tbx_wrap_state_tables(const tbx_wrap *w, void *out_host, size_t cap, size_t *size) {
   if (!w || !size) return set_err(TBX_EINVAL, "wrap/size is NULL");
-  return state_tables(w->pool, w->pool->info->rec_words + w->words, out_host, cap, size);
+  return state_tables(w->pool, w->pool->info->rec_words + wrap_rows(w), out_host, cap, size);
 }
 int tbx_state_save(tbx_pool *p, const int32_t *ids_dev, int k, uint32_t *snap_dev, void *stream) {
   if (!p) return set_err(TBX_EINVAL, "pool is NULL");
@@ -1234,17 +1301,17 @@ int tbx_state_save(tbx_pool *p, const int32_t *ids_dev, int k, uint32_t *snap_de
 }
 int tbx_wrap_state_save(tbx_wrap *w, const int32_t *ids_dev, int k, uint32_t *snap_dev, void *stream) {
   if (!w) return set_err(TBX_EINVAL, "wrap is NULL");
-  return state_save(w->pool, w->wstate, w->words, ids_dev, k, snap_dev, (cudaStream_t)stream);
+  return state_save(w->pool, w->wstate, wrap_rows(w), ids_dev, k, snap_dev, (cudaStream_t)stream);
 }
 int tbx_state_load(tbx_pool *p, const uint32_t *snap_dev, int k_snap, const int32_t *cols_dev, const int32_t *ids_dev, int n, const void *tables_blob,
                    size_t blob_bytes, void *stream) {
   if (!p) return set_err(TBX_EINVAL, "pool is NULL");
-  return guarded([&] { return state_load(p, 0, 0, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream); });
+  return guarded([&] { return state_load(p, 0, 0, false, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream); });
 }
 int tbx_wrap_state_load(tbx_wrap *w, const uint32_t *snap_dev, int k_snap, const int32_t *cols_dev, const int32_t *ids_dev, int n, const void *tables_blob,
                         size_t blob_bytes, void *stream) {
   if (!w) return set_err(TBX_EINVAL, "wrap is NULL");
-  return guarded([&] { return state_load(w->pool, w->wstate, w->words, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream); });
+  return guarded([&] { return state_load(w->pool, w->wstate, wrap_rows(w), w->final_ring != 0, snap_dev, k_snap, cols_dev, ids_dev, n, tables_blob, blob_bytes, (cudaStream_t)stream); });
 }
 
 } /* extern "C" */

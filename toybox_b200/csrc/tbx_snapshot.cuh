@@ -1,6 +1,7 @@
 /* tbx_snapshot.cuh -- the column copy behind device-resident state snapshots (tbx_state_save / tbx_state_load and
  * their wrapped-env forms).  A snapshot of k envs is uint32[rows][k], word-major like the pool's planes: column j is one
- * env's record, followed for a wrapped env by its 5 wrapper words.  One kernel serves every direction: entry j of a list
+ * env's record, followed for a wrapped env by its wrapper rows (5 words, 7 with sticky actions, + 1 + 2 records with final
+ * observations).  One kernel serves every direction: entry j of a list
  * copies column src_idx[j] of the source to column dst_idx[j] of the destination, `rows` words.
  *
  * Mapping: lanes run over list entries, each thread copies a chunk of TBX_SNAP_ROWS rows (blockIdx.y picks the chunk), so
@@ -35,8 +36,9 @@ struct SnapSide {
 struct SnapArgs {
   SnapSide src, dst;
   int k, rows;
-  int tbl_row;          /* row of hdr.tbl, or -1 (Space Invaders) */
-  int tbl_lim;          /* >= 0: the source's tbl word must lie in 0..tbl_lim-1 (loads: the tables exported with it) */
+  int tbl_row[3];       /* rows holding a hdr.tbl word, -1 = none: the record's (-1 for Space Invaders) and, for a wrapped env
+                           with final observations, those of its two _obs_buffer records */
+  int tbl_lim;          /* >= 0: the source's tbl words must lie in 0..tbl_lim-1 (loads: the tables exported with it) */
   const int32_t *remap; /* may be NULL: tbl word -> remap[tbl] */
   int32_t *owner;       /* may be NULL: no destination can repeat */
   int *bad;
@@ -51,7 +53,9 @@ __device__ __forceinline__ bool snap_entry(const SnapArgs &a, int j, int &sc, in
   sc = a.src.idx ? a.src.idx[j] : j;
   dc = a.dst.idx ? a.dst.idx[j] : j;
   if ((unsigned)sc >= (unsigned)a.src.lim || (unsigned)dc >= (unsigned)a.dst.lim) return false;
-  if (a.tbl_row >= 0 && a.tbl_lim >= 0 && (unsigned)*snap_at(a.src, a.tbl_row, sc) >= (unsigned)a.tbl_lim) return false;
+  if (a.tbl_lim >= 0)
+    for (int t = 0; t < 3; t++)
+      if (a.tbl_row[t] >= 0 && (unsigned)*snap_at(a.src, a.tbl_row[t], sc) >= (unsigned)a.tbl_lim) return false;
   return true;
 }
 
@@ -81,7 +85,8 @@ __global__ void __launch_bounds__(TBX_SNAP_THREADS) snap_copy_kernel(SnapArgs a)
     const int r = r0 + i;
     if (r >= a.rows) break;
     /* a remapped word was bounds-checked against tbl_lim in snap_entry (remap holds tbl_lim entries) */
-    *snap_at(a.dst, r, dc) = (r == a.tbl_row && a.remap) ? (uint32_t)a.remap[v[i]] : v[i];
+    const bool tbl = r == a.tbl_row[0] || r == a.tbl_row[1] || r == a.tbl_row[2];
+    *snap_at(a.dst, r, dc) = (tbl && a.remap) ? (uint32_t)a.remap[v[i]] : v[i];
   }
 }
 

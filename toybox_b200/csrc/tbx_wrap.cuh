@@ -30,6 +30,14 @@
  * (tbx_action_index) instead of gym's np_random (a MT19937 seeded through gym's hash_seed: not part of ctoybox); the
  * sticky draws come from the same kind of generator instead of ALE's MT19937; reset-chain steps that cross the time limit
  * truncate at the next agent step.
+ *
+ * Final observations (the FINAL instantiation, tbx_wrap_set_final_observations): the FrameStack the reference held just
+ * before the VecEnv worker reset a finished env -- the k-1 newest ring frames before the step and the frame of the step that
+ * ended the episode, max(_obs_buffer[0], _obs_buffer[1]).  MaxAndSkipEnv writes _obs_buffer[0] on frame skip-2 and [1] on
+ * frame skip-1 only and breaks at game over, so a game that ends early leaves stale slots from earlier units (reset-chain
+ * steps or the previous episode) or, never written, zeros.  The kernel keeps the two records behind the slots and the set of
+ * written slots as wrapper rows, written where the reference writes the buffer (every MaxAndSkip unit; NoopResetEnv's
+ * no-ops sit below it and write nothing), and copies the pair out when the agent's own step ends in done.
  */
 #ifndef TBX_WRAP_CUH
 #define TBX_WRAP_CUH
@@ -56,6 +64,14 @@ struct WrapArgs {
   uint8_t *truncated;             /* may be NULL: the agent step hit the time limit before the game was over */
   unsigned long long *stats;
   int *bad_actions;
+  /* FINAL (final observations; the fields stay unread otherwise): fin = [1 + 2 RW][n_pad] wrapper rows -- the slots of
+   * MaxAndSkipEnv._obs_buffer written so far (bit 0: [0], bit 1: [1]), then the records behind _obs_buffer[0] and [1].
+   * A MAIN unit that ends in done copies its pair into term0 / term1 ([RW][n_pad]) and lists the env: fin_list[fin_count[0]++]
+   * when a slot was written, fin_list[n_pad - 1 - fin_count[1]++] when neither was (a zero frame).  The counts are zero
+   * before the launch. */
+  uint32_t *fin, *term0, *term1;
+  int32_t *fin_list;
+  int *fin_count;
 };
 
 /* The wrapper chain is a small state machine over UNITS of frames, so that the (large) transition and new_game code
@@ -65,7 +81,7 @@ struct WrapArgs {
 enum { TBX_U_SKIP = 0, TBX_U_NOOP = 1 };
 enum { TBX_ST_MAIN = 0, TBX_ST_ELR_A, TBX_ST_FIRE1, TBX_ST_ELR_B, TBX_ST_FIRE2, TBX_ST_ELR_C, TBX_ST_END };
 
-template <int GAME, bool STICKY>
+template <int GAME, bool STICKY, bool FINAL = false>
 __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
   typedef Traits<GAME> T;
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
@@ -86,6 +102,7 @@ __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
     sticky_ale = (int)a.wstate[5 * (size_t)a.n_pad + env];
     frame = a.wstate[6 * (size_t)a.n_pad + env];
   }
+  uint32_t fin_seen = FINAL ? a.fin[env] : 0u; /* FINAL: the _obs_buffer slots written so far */
   int unit_rew = 0, ep_ret_out = 0, ep_len_out = 0;
 
   int total = 0, sink = 0;
@@ -126,7 +143,7 @@ __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
       if (STICKY) sticky_ale = 0; /* ALE's reset_game: the remembered action is NOOP */
     }
     if (frames_left > 0) {
-      if (unit == TBX_U_SKIP && frames_left == 1 && a.skip > 1) { TBX_SNAPSHOT(); snapped = true; } /* the state before the last repeat */
+      if (!FINAL && unit == TBX_U_SKIP && frames_left == 1 && a.skip > 1) { TBX_SNAPSHOT(); snapped = true; } /* the state before the last repeat */
       /* ToyboxBaseEnv.step (base.py:115-149): one transition, reward = max(score - prev, 0), done = lives <= 0 */
       const int lives_before = S.ldi(TBX_HW(lives));
       int applied = ale;
@@ -146,6 +163,19 @@ __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
         atomicMax((long long *)(a.stats + 3), (long long)o.ep_return);
       }
       frames_left--;
+      if (FINAL && unit == TBX_U_SKIP && frames_left <= 1) {
+        /* MaxAndSkipEnv: _obs_buffer[0] = obs on frame skip-2, [1] on frame skip-1, before its "if done: break"; the
+         * frame-(skip-2) state is also the snapshot before the last repeat, taken here from the same read */
+        const bool b0 = frames_left == 1;
+        uint32_t *buf = a.fin + (size_t)(b0 ? 1 : 1 + T::RW) * a.n_pad + env;
+        for (int w_ = 0; w_ < T::RW; w_++) {
+          const uint32_t v = a.planes[(size_t)w_ * a.n_pad + env];
+          buf[(size_t)w_ * a.n_pad] = v;
+          if (b0) a.planes_prev[(size_t)w_ * a.n_pad + env] = v;
+        }
+        snapped = snapped || b0;
+        fin_seen |= b0 ? 1u : 2u;
+      }
       if (o.done) {
         if (unit == TBX_U_NOOP) need_new_game = true; /* NoopResetEnv: "if done: obs = self.env.reset()" */
         else { unit_done = true; frames_left = 0; }    /* MaxAndSkipEnv: "if done: break" */
@@ -176,6 +206,19 @@ __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
       case TBX_ST_MAIN:
         out_done = done;
         score_out = S.ldi(TBX_HW(score)); lives_out = S.ldi(TBX_HW(lives));
+        if (FINAL && done) { /* the final observation's frame, max(_obs_buffer), saved before the reset chain rewrites the buffer */
+          if (fin_seen == 0u) { /* nothing written since the wrap was created: a zero frame */
+            a.fin_list[a.n_pad - 1 - atomicAdd(a.fin_count + 1, 1)] = env;
+          } else { /* an unwritten slot is zeros, and max(0, X) = X: the written record stands in for it */
+            const uint32_t *b0 = a.fin + (size_t)((fin_seen & 1u) ? 1 : 1 + T::RW) * a.n_pad + env;
+            const uint32_t *b1 = a.fin + (size_t)((fin_seen & 2u) ? 1 + T::RW : 1) * a.n_pad + env;
+            for (int w_ = 0; w_ < T::RW; w_++) {
+              a.term0[(size_t)w_ * a.n_pad + env] = b0[(size_t)w_ * a.n_pad];
+              a.term1[(size_t)w_ * a.n_pad + env] = b1[(size_t)w_ * a.n_pad];
+            }
+            a.fin_list[atomicAdd(a.fin_count, 1)] = env;
+          }
+        }
         if (done) { reset = true; stage = TBX_ST_ELR_A; TBX_START_EL_RESET(); } /* the VecEnv worker resets a finished env at once */
         else stage = TBX_ST_END;
         break;
@@ -212,6 +255,7 @@ __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
     a.wstate[5 * (size_t)a.n_pad + env] = (uint32_t)sticky_ale;
     a.wstate[6 * (size_t)a.n_pad + env] = frame;
   }
+  if (FINAL) a.fin[env] = fin_seen;
   if (a.ep_return) a.ep_return[env] = ep_ret_out;
   if (a.ep_length) a.ep_length[env] = ep_len_out;
   if (a.reward) a.reward[env] = a.clip_rewards ? (total > 0 ? 1 : total < 0 ? -1 : 0) : total;
@@ -221,6 +265,33 @@ __global__ void __launch_bounds__(128) wrap_step_kernel(WrapArgs a) {
   if (a.truncated) a.truncated[env] = (uint8_t)out_trunc;
   if (a.score) a.score[env] = score_out;
   if (a.lives) a.lives[env] = lives_out;
+}
+
+/* Final observations, after wrap_step_kernel<..., FINAL> and before the ring's render overwrites slot `head`: the k-1 frames
+ * of each listed env's ring that survive into its final stack (slot s of the ring -> slot s of fin, s != head), and for the
+ * envs of the zero list also the zero frame in slot `head`.  The other final frames are rendered into slot `head` by the
+ * tile kernel in env-list mode (tbx_pool.cu).  One warp per listed env, a grid-stride loop over both lists. */
+__global__ void __launch_bounds__(256) final_ring_kernel(const uint8_t *ring, uint8_t *fin, const int32_t *list, const int *count, int n_pad,
+                                                         size_t frame_bytes, int stack_k, int head) {
+  const int n_drawn = count[0], n_total = n_drawn + count[1];
+  const int lane = threadIdx.x & 31, nw = (gridDim.x * blockDim.x) >> 5;
+  const size_t env_stride = frame_bytes * (size_t)stack_k;
+  for (int j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n_total; j += nw) {
+    const bool zero = j >= n_drawn;
+    const int env = zero ? list[n_pad - 1 - (j - n_drawn)] : list[j];
+    for (int s = 0; s < stack_k; s++) {
+      if (s == head && !zero) continue;
+      const bool z = s == head;
+      const uint8_t *src = ring + (size_t)env * env_stride + (size_t)s * frame_bytes;
+      uint8_t *dst = fin + (size_t)env * env_stride + (size_t)s * frame_bytes;
+      if ((frame_bytes & 15) == 0) {
+        for (size_t i = lane; i < (frame_bytes >> 4); i += 32)
+          reinterpret_cast<uint4 *>(dst)[i] = z ? make_uint4(0, 0, 0, 0) : __ldg(reinterpret_cast<const uint4 *>(src) + i);
+      } else {
+        for (size_t i = lane; i < frame_bytes; i += 32) dst[i] = z ? (uint8_t)0 : __ldg(src + i);
+      }
+    }
+  }
 }
 
 } /* namespace tbxk */

@@ -32,12 +32,13 @@ class DeepmindToybox:
       reward int32[N] (sign of the summed reward when clip_rewards), done uint8[N] (game over, a lost life when
       episode_life, or the time limit), info = {'lives', 'score', 'real_done', 'truncated', 'ep_return', 'ep_length'}
       tensors (values before the reset of a finished env; truncated: the time limit ended the episode before its game
-      was over, all zero without a limit; ep_return / ep_length: Monitor's record where real_done or truncated).
+      was over, all zero without a limit; ep_return / ep_length: Monitor's record where real_done or truncated), and
+      with final_observation=True 'final_obs', the ring `self.final_obs` (valid where done).
     A finished env is reset inside the same call and `obs` then holds its reset observation (VecEnv semantics)."""
 
     def __init__(self, game, n_envs, device=None, seeds=None, config=None, frame_skip=4, noop_max=30, episode_life=True,
                  fire_reset=True, clip_rewards=True, frame_stack=4, size=(84, 84), noop_seed=0, env0=0, stack_reset="fill",
-                 grayscale=True, repeat_action_probability=0.0, sticky_seed=None, max_episode_steps=None):
+                 grayscale=True, repeat_action_probability=0.0, sticky_seed=None, max_episode_steps=None, final_observation=False):
         """stack_reset: what a reset observation does to the other k-1 ring slots -- "fill" (FrameStack.reset,
         atari_wrappers.py:262-266: wrap_deepmind(frame_stack=True), the deepq path) or "zero" (VecFrameStack,
         vec_env/vec_frame_stack.py:17-30: make_vec_env + VecFrameStack, the ppo2 / a2c path of run.py:123-125).
@@ -49,7 +50,13 @@ class DeepmindToybox:
         sticky_seed defaults to noop_seed.
         max_episode_steps: gym's TimeLimit inside make_atari (baselines' make_atari(env_id, max_episode_steps); ALE v5's
         108,000 frames are 27,000 at frame_skip 4), counting Monitor's episode length.  An env at the limit reports done
-        and takes the full reset chain; info['truncated'] flags it where its game is not over."""
+        and takes the full reset chain; info['truncated'] flags it where its game is not over.
+        final_observation: keep the observation each finished episode ended on, the one a bootstrapping learner needs for
+        V(s_T) after a truncation or a life-loss done.  `self.final_obs` (the ring's shape and slot order; `final_stacked()`
+        gives stacked()'s layout) then holds, where done, the FrameStack the reference held just before the VecEnv worker
+        reset the env: the k-1 newest frames before the step and the frame of the step.  That frame is the max of
+        MaxAndSkipEnv's two buffer slots as the reference leaves them, stale slots of a game that ended before frame skip-2
+        or skip-1 included (DESIGN.md 4.5).  Written by steps that render; other rows keep their values."""
         if stack_reset not in ("fill", "zero"):
             raise ValueError("stack_reset is 'fill' (FrameStack) or 'zero' (VecFrameStack)")
         self.pool = BatchedToybox(game, n_envs, device=device, obs=("gray_area", size[0], size[1]), config=config, seeds=seeds)
@@ -83,6 +90,11 @@ class DeepmindToybox:
         self.real_done = torch.zeros(n, dtype=torch.uint8, device=dev)
         self.score = torch.zeros(n, dtype=torch.int32, device=dev)
         self.lives = torch.zeros(n, dtype=torch.int32, device=dev)
+        self.final_observation = bool(final_observation)
+        self.final_obs = None
+        if self.final_observation:
+            self.final_obs = torch.zeros_like(self.obs)
+            _lib.check(self.L.tbx_wrap_set_final_observations(self._w, _ptr(self.final_obs)))
         self.slot = 0
         self.n_actions = len(self.pool.get_legal_action_set())
 
@@ -117,8 +129,11 @@ class DeepmindToybox:
             if actions.numel() != self.n_envs:
                 raise ValueError("expected %d actions" % self.n_envs)
         self._call(actions, render)
-        return self.obs, self.reward, self.done, {"lives": self.lives, "score": self.score, "real_done": self.real_done,
-                                                    "truncated": self.truncated, "ep_return": self.ep_return, "ep_length": self.ep_length}
+        info = {"lives": self.lives, "score": self.score, "real_done": self.real_done, "truncated": self.truncated,
+                "ep_return": self.ep_return, "ep_length": self.ep_length}
+        if self.final_observation:
+            info["final_obs"] = self.final_obs
+        return self.obs, self.reward, self.done, info
 
     def check(self):
         self.pool.check()
@@ -126,7 +141,8 @@ class DeepmindToybox:
     # ------------------------------------------------------------------ state snapshots
     def save_state(self, env_ids=None):
         """A StateSnapshot of the listed wrapped envs: records, wrapper state (EpisodicLife, no-op reset counter, Monitor
-        accumulators, and with sticky actions the remembered ALE id and frame counter) and observation rings.  Ids as
+        accumulators, with sticky actions the remembered ALE id and frame counter, with final observations MaxAndSkipEnv's
+        two buffer records and which of them were written) and observation rings.  Ids as
         BatchedToybox.save_state."""
         ids = _snap.id_tensor(env_ids, self.n_envs, self.device, "env id")
         k = self.n_envs if ids is None else ids.numel()
@@ -159,8 +175,13 @@ class DeepmindToybox:
         cols = torch.arange(n, device=dev) if cols is None else cols.long()
         valid = (ids >= 0) & (ids < self.n_envs) & (cols >= 0) & (cols < k)
         if snap.game != "space_invaders":
-            tbl = data[_snap.TBL_WORD].long().index_select(0, cols.clamp(0, k - 1))
-            valid &= (tbl >= 0) & (tbl < snap.table_count)
+            rec = self.L.tbx_state_rows(self.pool._h)
+            rows = [_snap.TBL_WORD]
+            if self.final_observation:      # the tbl words of the two buffer records, the last 2 * rec rows
+                rows += [snap.rows - 2 * rec + _snap.TBL_WORD, snap.rows - rec + _snap.TBL_WORD]
+            for r in rows:
+                tbl = data[r].long().index_select(0, cols.clamp(0, k - 1))
+                valid &= (tbl >= 0) & (tbl < snap.table_count)
         order = torch.arange(n, device=dev)
         tgt = torch.where(valid, ids, self.n_envs)
         last = torch.full((self.n_envs + 1,), -1, dtype=torch.long, device=dev).scatter_reduce_(0, tgt, order, reduce="amax")
@@ -186,11 +207,24 @@ class DeepmindToybox:
         """FrameStack's observation (atari_wrappers.py:246-275) for every env, oldest first: uint8[N, out_h, out_w, k], or in
         colour uint8[N, out_h, out_w, 3k] with frame-major channels (the oldest frame's R, G, B first), the concatenation
         along the last axis that LazyFrames and VecFrameStack produce."""
+        return self._stack(self.obs)
+
+    def final_stacked(self, env_ids=None):
+        """stacked()'s layout of the final observations (final_observation=True), of every env or of the listed ones (a
+        device tensor or a sequence of ids); valid for the envs that were done in the last step that rendered."""
+        if self.final_obs is None:
+            raise RuntimeError("final observations are off: DeepmindToybox(final_observation=True)")
+        ring = self.final_obs
+        if env_ids is not None:
+            ring = ring.index_select(0, torch.as_tensor(env_ids, device=self.device).long().reshape(-1))
+        return self._stack(ring)
+
+    def _stack(self, ring):
         idx = torch.as_tensor(self.order(), device=self.device)
-        ring = self.obs.index_select(1, idx)
+        ring = ring.index_select(1, idx)
         if self.grayscale:
             return ring.permute(0, 2, 3, 1).contiguous()
-        return ring.permute(0, 2, 3, 1, 4).reshape(self.n_envs, self.out_h, self.out_w, 3 * self.k)
+        return ring.permute(0, 2, 3, 1, 4).reshape(ring.shape[0], self.out_h, self.out_w, 3 * self.k)
 
 
 def _got_rings(snap):
@@ -220,6 +254,8 @@ class ToyboxVecEnv:
     episode; `infos[i]['TimeLimit.truncated'] = True` then, as gym's TimeLimit reports it), exactly as the Monitor between make_atari and
     wrap_deepmind reports it (bench/monitor.py:58-76: r = sum of raw rewards, l = MaxAndSkipEnv steps incl. those of
     FireResetEnv / EpisodicLifeEnv resets, t = seconds since start) -- both counters are kept by the step kernel.
+    With final_observation=True, `infos[i]['terminal_observation']` (SB3's key) is env i's final observation where done:
+    the (h, w, c*k) stack, in the same order as obs, the reference held just before it reset the env.
     monitor_file: path of a Monitor-compatible CSV (bench/monitor.py:22-28,70-71,96-126: a '#{json header}' line, then the
     columns r,l,t), one row per finished episode."""
 
@@ -261,6 +297,11 @@ class ToyboxVecEnv:
         score = e.score.cpu().numpy().astype(np.int64)
         lives = e.lives.cpu().numpy()
         infos = [{"lives": int(lives[i]), "score": int(score[i])} for i in range(self.num_envs)]
+        if e.final_observation and done.any():
+            ids = np.flatnonzero(done)
+            fin = e.final_stacked(ids).cpu().numpy()
+            for j, i in enumerate(ids):
+                infos[i]["terminal_observation"] = fin[j]
         for i in np.flatnonzero(trunc):
             infos[i]["TimeLimit.truncated"] = True
         ended = real | trunc
